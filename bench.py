@@ -1,8 +1,13 @@
 #!/usr/bin/env python
 """bench.py -- headline benchmark of the post filter set on B200 (contract in the task statement).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N ... bench.py --gpus N --steps K --warmup W
+
+--dump-outputs DIR writes, after the timed steps, the filtered frames the last timed step produced for a fixed seeded
+sample of each rank's frames, as float32 DIR/filtered_frames.npy ([frames, 1080, 1920]; DIR/filtered_frames_rank<r>.npy
+with several ranks), at most 64 MB (64e6 bytes) in all.  The inputs depend only on the arguments, so two builds can be compared
+output for output.
 
 Workload (BASELINE.json configs[2]): a 1920x1080 8-bit x264-decoded disparity video of 1000 frames per GPU, full chain
 PostFilterSet::operator()(median_r=2, gaussian_r=1, minmax_r=3, brange_r=5, brange_th=10).  The frames are built from the
@@ -214,6 +219,23 @@ def config_dict(n_gpus, frames_per_gpu):
             "parallelism": "frame-parallel x%d, no collective" % n_gpus}
 
 
+DUMP_BYTES = 64 * 10**6
+
+
+def dump_outputs(out_dir, d_out, rank, world):
+    """Writes the frames of d_out (the device-resident output of the last timed step) at a seeded sample of frame
+    indices, as float32; the ranks share the DUMP_BYTES budget (with more ranks than frames fit, the last ranks write none)."""
+    n = d_out.shape[0]
+    total = min(world * n, DUMP_BYTES // (H * W * 4))
+    k = total // world + (1 if rank < total % world else 0)
+    if k == 0:
+        return
+    idx = np.sort(np.random.RandomState(0).choice(n, k, replace=False))
+    frames = d_out[idx.tolist()].cpu().numpy().astype(np.float32)
+    os.makedirs(out_dir, exist_ok=True)
+    np.save(os.path.join(out_dir, "filtered_frames.npy" if world == 1 else "filtered_frames_rank%d.npy" % rank), frames)
+
+
 # ------------------------------------------------------------------------------------------------ main
 def main():
     ap = argparse.ArgumentParser()
@@ -224,7 +246,12 @@ def main():
     ap.add_argument("--frames", type=int, default=1000, help="frames per GPU per step")
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--lanes", type=int, default=1, help="frame groups in flight on separate streams (device-resident path)")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write a seeded sample of the last timed step's output frames to DIR (float32 .npy)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs applies to --impl ours")
     rank = int(os.environ.get("RANK", "0")); world = int(os.environ.get("WORLD_SIZE", "1")); local = int(os.environ.get("LOCAL_RANK", "0"))
     if args.warmup < 3:
         args.warmup = 3
@@ -347,6 +374,8 @@ def main():
         ms = float(tm[0]); launches = int(ts[1])
     ms_per_step = ms / args.steps
     value = world * N * H * W / (ms_per_step * 1e-3) / 1e6
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, d_out, rank, world)
 
     # stage breakdown (untimed extra pass with every stage bracketed)
     ctx.profile_enable(15)

@@ -2,8 +2,9 @@
 
   Port       -> oracle/libdmc_oracle.so   (plain-C restatement, oracle/dmc_oracle.c)
   Reference  -> oracle/_ref/libdmc_ref.so (unmodified reference sources through oracle/refshim)
+  Shim       -> oracle/libdmc_shim.so     (oracle/refshim's cv:: stand-ins alone, no reference source)
 
-Both expose the same numpy-level methods so a test can be parametrised over them.  Only tests/,
+Port and Reference expose the same numpy-level methods so a test can be parametrised over them.  Only tests/,
 __graft_entry__.smoke() and bench.py's cpu_baseline / --impl reference legs may import this module;
 nothing in depthmapcompression_b200/ does.
 """
@@ -15,6 +16,7 @@ import numpy as np
 HERE = os.path.dirname(os.path.abspath(__file__))
 PORT_SO = os.path.join(HERE, "libdmc_oracle.so")
 REF_SO = os.path.join(HERE, "_ref", "libdmc_ref.so")
+SHIM_SO = os.path.join(HERE, "libdmc_shim.so")
 
 CV_8U, CV_16U, CV_16S, CV_32F, CV_64F = 0, 2, 3, 5, 6
 FULL_KERNEL, FULL_KERNEL_PAIR, SEPARABLE_KERNEL = 0, 1, 2
@@ -31,7 +33,7 @@ def cvtype_of(a):
 
 def build(force=False):
     """make -C oracle (the port always; the reference build only where /root/reference exists)."""
-    if force or not os.path.exists(PORT_SO) or (os.path.isdir("/root/reference") and not os.path.exists(REF_SO)):
+    if force or not os.path.exists(PORT_SO) or not os.path.exists(SHIM_SO) or (os.path.isdir("/root/reference") and not os.path.exists(REF_SO)):
         subprocess.check_call(["make", "-C", HERE, "all"], stdout=subprocess.DEVNULL)
 
 
@@ -207,7 +209,41 @@ class Port(_Base):
         return dst
 
 
-class Reference(_Base):
+class _ShimCalls:
+    """The cv:: stand-ins of oracle/refshim/minicv.hpp (shim_* entry points)."""
+
+    def median_blur(self, src, ksize):
+        src = _c(src); H, W = src.shape; dst = np.zeros_like(src)
+        assert self.lib.shim_median_blur(_p(src), _p(dst), H, W, cvtype_of(src), ksize) == 0
+        return dst
+
+    def gaussian_kernel32f(self, n, sigma):
+        k = np.zeros(n, np.float32); self.lib.shim_gaussian_kernel32f(n, C.c_double(sigma), _p(k)); return k
+
+    def gaussian_blur32f(self, src, d, sigma):
+        src = _c(src, np.float32); H, W = src.shape; dst = np.zeros_like(src)
+        assert self.lib.shim_gaussian_blur32f(_p(src), _p(dst), H, W, d, C.c_double(sigma)) == 0
+        return dst
+
+    def morph(self, src, k, is_max):
+        src = _c(src); H, W = src.shape; dst = np.zeros_like(src)
+        assert self.lib.shim_morph(_p(src), _p(dst), H, W, cvtype_of(src), k, int(is_max)) == 0
+        return dst
+
+    def copy_make_border(self, src, top, bottom, left, right, border):
+        src = _c(src); H, W = src.shape[:2]
+        dst = np.zeros((H + top + bottom, W + left + right) + src.shape[2:], src.dtype)
+        assert self.lib.shim_copy_make_border(_p(src), _p(dst), H, W, cvtype_of(src), top, bottom, left, right, border) == 0
+        return dst
+
+    def convert_to(self, src, ddtype):
+        src = _c(src); dst = np.zeros(src.shape, ddtype)
+        dt = _DEPTH_OF[np.dtype(ddtype)] + (cvtype_of(src) & ~7)
+        assert self.lib.shim_convert_to(_p(src), _p(dst), src.shape[0], src.shape[1], cvtype_of(src), dt) == 0
+        return dst
+
+
+class Reference(_Base, _ShimCalls):
     prefix = "ref_"
     kind = "reference"
 
@@ -244,39 +280,9 @@ class Reference(_Base):
         assert self.lib.ref_fill_small_hole(_p(src), _p(out), H, W, int(dst is None)) == 0
         return out
 
-    def median_blur(self, src, ksize):
-        src = _c(src); H, W = src.shape; dst = np.zeros_like(src)
-        assert self.lib.shim_median_blur(_p(src), _p(dst), H, W, cvtype_of(src), ksize) == 0
-        return dst
-
-    def gaussian_kernel32f(self, n, sigma):
-        k = np.zeros(n, np.float32); self.lib.shim_gaussian_kernel32f(n, C.c_double(sigma), _p(k)); return k
-
-    def gaussian_blur32f(self, src, d, sigma):
-        src = _c(src, np.float32); H, W = src.shape; dst = np.zeros_like(src)
-        assert self.lib.shim_gaussian_blur32f(_p(src), _p(dst), H, W, d, C.c_double(sigma)) == 0
-        return dst
-
     def small_gaussian(self, src, d, sigma):
         src = _c(src); H, W = src.shape; dst = np.zeros_like(src)
         assert self.lib.ref_small_gaussian(_p(src), _p(dst), H, W, cvtype_of(src), d, C.c_double(sigma)) == 0
-        return dst
-
-    def morph(self, src, k, is_max):
-        src = _c(src); H, W = src.shape; dst = np.zeros_like(src)
-        assert self.lib.shim_morph(_p(src), _p(dst), H, W, cvtype_of(src), k, int(is_max)) == 0
-        return dst
-
-    def copy_make_border(self, src, top, bottom, left, right, border):
-        src = _c(src); H, W = src.shape[:2]
-        dst = np.zeros((H + top + bottom, W + left + right) + src.shape[2:], src.dtype)
-        assert self.lib.shim_copy_make_border(_p(src), _p(dst), H, W, cvtype_of(src), top, bottom, left, right, border) == 0
-        return dst
-
-    def convert_to(self, src, ddtype):
-        src = _c(src); dst = np.zeros(src.shape, ddtype)
-        dt = _DEPTH_OF[np.dtype(ddtype)] + (cvtype_of(src) & ~7)
-        assert self.lib.shim_convert_to(_p(src), _p(dst), src.shape[0], src.shape[1], cvtype_of(src), dt) == 0
         return dst
 
     def bwrf(self, src, kw, kh, th, method=FULL_KERNEL, dst_init=None, inplace=False):
@@ -312,6 +318,14 @@ class Reference(_Base):
                               C.c_float(frec), C.c_float(color), C.c_float(space), int(inplace))
         assert rc >= 0, rc
         return dst
+
+
+class Shim(_ShimCalls):
+    """The stand-ins alone (oracle/libdmc_shim.so): built from oracle/refshim without the reference sources."""
+
+    def __init__(self):
+        build()
+        self.lib = C.CDLL(SHIM_SO)
 
 
 def synth_disp(H, W, seed, shift=(0, 0)):

@@ -5,10 +5,17 @@
 // buffer into a 64-byte aligned, continuous Mat (the reference uses aligned SSE
 // loads/stores on Mat data), calls the reference function, and copies the result out.
 // Used only by tests/, __graft_entry__.smoke() and bench.py's CPU-baseline legs.
+// Built with -DDMC_SHIM_ONLY (oracle/libdmc_shim.so) it holds only the shim_* entry points, which need no
+// reference source, so that the stand-ins can be pinned against cv2 without the reference tree.
+#ifdef DMC_SHIM_ONLY
+#include "minicv.hpp"
+using namespace cv;
+#else
 #include "filter.h"
 #include "util.h"
 
 void binalyWeightedRangeFilter(const Mat& src, Mat& dst, int kernelSize, float threshold, int method, int borderType);
+#endif
 
 namespace {
 Mat wrapCopy(const void* p, int rows, int cols, int type) {
@@ -24,6 +31,7 @@ void copyOut(const Mat& m, void* p) { for (int y = 0; y < m.rows; y++) memcpy((u
 
 extern "C" {
 
+#ifndef DMC_SHIM_ONLY
 int ref_version() { return 1; }
 void ref_set_num_threads(int n) {
 #ifdef _OPENMP
@@ -178,6 +186,7 @@ int ref_fill_small_hole(const uchar* src, uchar* dst, int rows, int cols, int in
     copyOut(d, dst);
     DMC_CATCH
 }
+#endif  // DMC_SHIM_ONLY
 
 // ---- the shim's own stand-ins, exported so tests can pin them against cv2 4.13 ----
 int shim_median_blur(const void* src, void* dst, int rows, int cols, int cvtype, int ksize) {

@@ -67,8 +67,8 @@ def test_port_matches_golden_depth16(port):
 
 
 @pytest.mark.parametrize("name", CHAIN_INPUTS[:2])
-def test_reference_build_matches_golden(ref, name):
+def test_reference_build_matches_golden(ref_build, name):
     """Guards against shim / compiler-flag drift of oracle/_ref."""
     img = load_png(name)
     for key, want in GOLD["inputs"][name]["golden"].items():
-        assert crc(run_chain_op(ref, key, img)) == want, (name, key)
+        assert crc(run_chain_op(ref_build, key, img)) == want, (name, key)

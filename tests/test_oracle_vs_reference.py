@@ -136,7 +136,8 @@ def test_post_filter_set_entry_points(port, ref, shape):
             assert_bits_equal(port.filter_disp8u_disp32f(a, mr, gr, mmr, br, th + 0.5), ref.filter_disp8u_disp32f(a, mr, gr, mmr, br, th + 0.5), "Disp32F")
 
 
-def test_reference_is_thread_count_invariant(ref):
+def test_reference_is_thread_count_invariant(ref_build):
+    ref = ref_build
     rs = np.random.RandomState(7); a = make_image(rs, 96, 128)
     outs = []
     for n in (1, 3, 8):
