@@ -13,10 +13,12 @@ constexpr int kTW = 128;     // output tile width  (2 warps x 32 lanes x 2 px, o
 // gathered through the border rule.  REFLECT selects BORDER_REFLECT_101 (Gaussian) instead of BORDER_REPLICATE.
 //   MODE 0: raw bytes, SW/4 words per row            MODE 1: 0x6400 | byte (fp16 1024 + byte), SW/2 words per row
 //   MODE 2: plain fp16 0..255, SW/2 words per row
+// SWW_ > 0 pads the row stride to SWW_ words (a multiple of 4).
 constexpr int kHalo16 = 16, kSW16 = kTW + 2 * kHalo16, kNV16 = kSW16 / 16;
-template <int SH, int MODE, bool REFLECT>
+template <int SH, int MODE, bool REFLECT, int SWW_ = 0>
 __device__ __forceinline__ void stage_tile16(uint32_t* __restrict__ sm, const uint8_t* __restrict__ fsrc, int X0, int ytop, int H, int W, bool al, int tid) {
-    constexpr int SWW = MODE == 0 ? kSW16 / 4 : kSW16 / 2;
+    constexpr int SWW = SWW_ > 0 ? SWW_ : (MODE == 0 ? kSW16 / 4 : kSW16 / 2);
+    static_assert(SWW % 4 == 0 && SWW >= (MODE == 0 ? kSW16 / 4 : kSW16 / 2), "16-byte aligned rows");
     for (int idx = tid; idx < SH * kNV16; idx += 256) {
         const int ty = idx / kNV16, tq = idx - ty * kNV16, gx = X0 - kHalo16 + 16 * tq;
         const int gy = REFLECT ? reflect101(ytop + ty, H) : clampi(ytop + ty, 0, H - 1);
