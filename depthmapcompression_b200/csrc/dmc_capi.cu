@@ -3,6 +3,7 @@
 // PostFilterSet chains, and the frame-batch streaming executor.  No CPU fallback exists anywhere in this file.
 #include "../../include/dmc_c.h"
 #include "dmc_common.cuh"
+#include "dmc_jpeg_enc_core.h"
 #include "dmc_kernels.cuh"
 
 #include <math.h>
@@ -44,6 +45,7 @@ struct dmc_ctx {
     struct Gateway { int device = -1; cudaStream_t stream[kSlots] = {}; Buf in[kSlots], out[kSlots]; cudaEvent_t ev_in[kSlots] = {}, ev_out[kSlots] = {}, ev_done[kSlots] = {}; } gw;
     Buf render[2]; int* render_flag = nullptr;      // point-cloud render: attempt lists etc., device flag; pinned host flag
     Buf jpeg[7];                 // JPEG decode: blob, frame descriptors, Huffman tables, quant tables, coefficients (restart streams only), output, de-stuffed scans
+    Buf jpeg_enc[9];             // JPEG encode: tables, staged frames, coefficients, block records, scan words, slots, lengths + offsets, staged output, decoder tables + descriptors
     // optional per-stage CUDA-event timing of the chain (bench.py's live roofline measurement)
     int lanes = 1;               // concurrent frame groups in the device-resident batch path
     int profile_mask = 0;
@@ -466,6 +468,7 @@ void dmc_destroy(dmc_ctx* ctx) {
     drop_gateway(ctx);
     drop_graph(ctx);
     for (auto& b : ctx->jpeg) if (b.p) cudaFree(b.p);
+    for (auto& b : ctx->jpeg_enc) if (b.p) cudaFree(b.p);
     for (auto& b : ctx->render) if (b.p) cudaFree(b.p);
     if (ctx->render_flag) cudaFreeHost(ctx->render_flag);
     for (auto& r : ctx->prof_pending) { cudaEventDestroy(r.a); cudaEventDestroy(r.b); }
@@ -936,6 +939,146 @@ int dmc_jpeg_decode_gray_batch(dmc_ctx* ctx, const void* blob, const uint64_t* o
         LAUNCH(ctx, launch_jpeg_decode((const uint8_t*)ctx->jpeg[0].p, ctx->jpeg[1].p, ctx->jpeg[2].p, ctx->jpeg[3].p, (uint8_t*)ctx->jpeg[6].p, (int16_t*)ctx->jpeg[4].p, out, nf, g.n_restart, rows, cols, s));
         if (dst_mem == DMC_MEM_HOST) CUDA_TRY(ctx, cudaMemcpyAsync((uint8_t*)dst + fpx * f0, out, fpx * nf, cudaMemcpyDeviceToHost, s));
         CUDA_TRY(ctx, cudaStreamSynchronize(s));     // the pageable host vectors (desc, tables) are reused by the next group
+    }
+    return DMC_OK;
+}
+
+// ---- JPEG encode (SURVEY.md 8f-5) ------------------------------------------------------------------------------------
+int dmc_jpeg_encode_bound(int rows, int cols, uint64_t* bytes) {
+    if (!bytes) return fail(nullptr, DMC_ERR_ARG, "dmc_jpeg_encode_bound: null bytes");
+    if (rows <= 0 || cols <= 0 || rows > 65535 || cols > 65535) return fail(nullptr, DMC_ERR_SIZE, "JPEG encode: frame size must be 1..65535 x 1..65535");
+    *bytes = dmcjpeg::jpeg_encode_bound(rows, cols);
+    if (*bytes > dmcjpeg::kEncMaxStreamBytes) return fail(nullptr, DMC_ERR_SIZE, "JPEG encode: the worst-case stream of a " + std::to_string(rows) + " x " + std::to_string(cols) + " frame exceeds 256 MB");
+    return DMC_OK;
+}
+
+namespace {
+
+// Scratch of all frames of one group; the group is as large as this allows (at least one frame, at most 2048).  A 1080p
+// frame needs about 26 MB (slot 13.4 MB, scan words 6.7 MB, coefficients 4.1 MB, staged frame).
+constexpr size_t kEncGroupBytes = (size_t)4 << 30;
+
+enum { JE_TABS, JE_SRC, JE_COEF, JE_INFO, JE_WORDS, JE_SLOTS, JE_LENS, JE_OUT, JE_DEC };
+
+// Checks the arguments shared by the encode entry points, uploads the encoder tables and returns the group size.
+int jpeg_enc_prepare(dmc_ctx* ctx, const char* what, int rows, int cols, int quality, int mem_a, int mem_b, int* group) {
+    if (quality < 0 || quality > 100) return fail(ctx, DMC_ERR_ARG, std::string(what) + ": quality must be in 0..100");
+    if ((mem_a != DMC_MEM_HOST && mem_a != DMC_MEM_DEVICE) || (mem_b != DMC_MEM_HOST && mem_b != DMC_MEM_DEVICE)) return fail(ctx, DMC_ERR_ARG, std::string(what) + ": bad mem");
+    uint64_t bound;
+    if (dmc_jpeg_encode_bound(rows, cols, &bound) != DMC_OK) return fail(ctx, DMC_ERR_SIZE, std::string(what) + ": " + g_err);
+    CUDA_TRY(ctx, cudaSetDevice(ctx->device));
+    const JpegEncLayout l = jpeg_enc_layout(rows, cols);
+    const size_t per = l.coef_bytes + l.info_bytes + l.word_bytes + l.slot_bytes + 2 * (size_t)rows * cols;
+    size_t g = kEncGroupBytes / per;
+    *group = (int)(g < 1 ? 1 : (g > 2048 ? 2048 : g));
+    dmcjpeg::EncTables t;
+    dmcjpeg::make_enc_tables(quality, rows, cols, &t);
+    TRY(reserve(ctx, ctx->jpeg_enc[JE_TABS], sizeof t));
+    CUDA_TRY(ctx, cudaMemcpyAsync(ctx->jpeg_enc[JE_TABS].p, &t, sizeof t, cudaMemcpyHostToDevice, ctx->stream));
+    CUDA_TRY(ctx, cudaStreamSynchronize(ctx->stream));          // (t lives on this stack frame)
+    return DMC_OK;
+}
+
+// Encodes frames [f0, f0 + nf) of src into the slots (lengths in JE_LENS); desc: also write the decoder's FrameDescs there.
+int jpeg_enc_group(dmc_ctx* ctx, const uint8_t* src, int src_mem, int f0, int nf, int rows, int cols, void* desc) {
+    cudaStream_t s = ctx->stream;
+    const size_t fpx = (size_t)rows * cols;
+    const JpegEncLayout l = jpeg_enc_layout(rows, cols);
+    const uint8_t* dsrc = src + fpx * f0;
+    if (src_mem == DMC_MEM_HOST) {
+        TRY(reserve(ctx, ctx->jpeg_enc[JE_SRC], fpx * nf));
+        CUDA_TRY(ctx, cudaMemcpyAsync(ctx->jpeg_enc[JE_SRC].p, dsrc, fpx * nf, cudaMemcpyHostToDevice, s));
+        dsrc = (const uint8_t*)ctx->jpeg_enc[JE_SRC].p;
+    }
+    TRY(reserve(ctx, ctx->jpeg_enc[JE_COEF], l.coef_bytes * nf));
+    TRY(reserve(ctx, ctx->jpeg_enc[JE_INFO], l.info_bytes * nf));
+    TRY(reserve(ctx, ctx->jpeg_enc[JE_WORDS], l.word_bytes * nf));
+    TRY(reserve(ctx, ctx->jpeg_enc[JE_SLOTS], l.slot_bytes * nf));
+    TRY(reserve(ctx, ctx->jpeg_enc[JE_LENS], (size_t)nf * (sizeof(uint32_t) + sizeof(uint64_t)) + 16));
+    LAUNCH(ctx, launch_jpeg_encode(dsrc, ctx->jpeg_enc[JE_TABS].p, ctx->jpeg_enc[JE_COEF].p, ctx->jpeg_enc[JE_INFO].p, ctx->jpeg_enc[JE_WORDS].p,
+                                   (uint8_t*)ctx->jpeg_enc[JE_SLOTS].p, (uint32_t*)ctx->jpeg_enc[JE_LENS].p, desc, nf, rows, cols, s));
+    return DMC_OK;
+}
+
+uint64_t* enc_offs(dmc_ctx* ctx, int nf) { return (uint64_t*)((char*)ctx->jpeg_enc[JE_LENS].p + (((size_t)nf * sizeof(uint32_t) + 15) & ~(size_t)15)); }
+
+}  // namespace
+
+// Streams are encoded group by group into per-frame slots on the device; the host reads the group's lengths back, places
+// the streams back to back after the previous group's and a gather kernel copies them there (through a device staging
+// buffer and one copy for a host blob).
+int dmc_jpeg_encode_gray_batch(dmc_ctx* ctx, const void* src, int src_mem, int n_frames, int rows, int cols, int quality, void* blob, int blob_mem,
+                               uint64_t capacity, uint64_t* offsets) {
+    if (!ctx) return fail(nullptr, DMC_ERR_ARG, "null context");
+    if (!offsets || n_frames < 0 || (n_frames > 0 && (!src || !blob))) return fail(ctx, DMC_ERR_SIZE, "dmc_jpeg_encode_gray_batch: bad arguments");
+    int group;
+    TRY(jpeg_enc_prepare(ctx, "dmc_jpeg_encode_gray_batch", rows, cols, quality, src_mem, blob_mem, &group));
+    offsets[0] = 0;
+    cudaStream_t s = ctx->stream;
+    const JpegEncLayout l = jpeg_enc_layout(rows, cols);
+    std::vector<uint32_t> lens; std::vector<uint64_t> offs;
+    for (int f0 = 0; f0 < n_frames; f0 += group) {
+        const int nf = n_frames - f0 < group ? n_frames - f0 : group;
+        TRY(jpeg_enc_group(ctx, (const uint8_t*)src, src_mem, f0, nf, rows, cols, nullptr));
+        lens.resize(nf); offs.resize(nf);
+        CUDA_TRY(ctx, cudaMemcpyAsync(lens.data(), ctx->jpeg_enc[JE_LENS].p, nf * sizeof(uint32_t), cudaMemcpyDeviceToHost, s));
+        CUDA_TRY(ctx, cudaStreamSynchronize(s));
+        const uint64_t base = offsets[f0];
+        uint64_t end = base, longest = 0;
+        for (int i = 0; i < nf; i++) { offs[i] = end - base; end += lens[i]; if (lens[i] > longest) longest = lens[i]; }
+        if (end > capacity)
+            return fail(ctx, DMC_ERR_SIZE, "dmc_jpeg_encode_gray_batch: the streams of frames 0.." + std::to_string(f0 + nf - 1) + " need " + std::to_string(end) +
+                                               " bytes, capacity is " + std::to_string(capacity));
+        for (int i = 0; i < nf; i++) offsets[f0 + i + 1] = base + offs[i] + lens[i];
+        uint64_t* d_offs = enc_offs(ctx, nf);
+        CUDA_TRY(ctx, cudaMemcpyAsync(d_offs, offs.data(), nf * sizeof(uint64_t), cudaMemcpyHostToDevice, s));
+        uint8_t* dst = (uint8_t*)blob + base;
+        if (blob_mem == DMC_MEM_HOST) { TRY(reserve(ctx, ctx->jpeg_enc[JE_OUT], end - base)); dst = (uint8_t*)ctx->jpeg_enc[JE_OUT].p; }
+        LAUNCH(ctx, launch_jpeg_enc_gather((const uint8_t*)ctx->jpeg_enc[JE_SLOTS].p, l.slot_bytes, (const uint32_t*)ctx->jpeg_enc[JE_LENS].p, d_offs, dst, nf, longest, s));
+        if (blob_mem == DMC_MEM_HOST) CUDA_TRY(ctx, cudaMemcpyAsync((uint8_t*)blob + base, dst, end - base, cudaMemcpyDeviceToHost, s));
+        CUDA_TRY(ctx, cudaStreamSynchronize(s));     // offs is reused by the next group
+    }
+    return DMC_OK;
+}
+
+// The reference's degradeJPEG on the device: encode into the slots, then decode every slot in place with the decoder of
+// dmc_jpeg_decode_gray_batch.  The decoder's tables come from parsing the encoder's header once; the encoder writes each
+// frame's FrameDesc itself, so the streams never leave the device.
+int dmc_jpeg_degrade_gray_batch(dmc_ctx* ctx, const void* src, void* dst, int n_frames, int rows, int cols, int quality, int mem, uint64_t* bytes) {
+    if (!ctx) return fail(nullptr, DMC_ERR_ARG, "null context");
+    if (n_frames < 0 || (n_frames > 0 && (!src || !dst))) return fail(ctx, DMC_ERR_SIZE, "dmc_jpeg_degrade_gray_batch: bad arguments");
+    int group;
+    TRY(jpeg_enc_prepare(ctx, "dmc_jpeg_degrade_gray_batch", rows, cols, quality, mem, mem, &group));
+    if (n_frames == 0) return DMC_OK;
+    cudaStream_t s = ctx->stream;
+    const size_t fpx = (size_t)rows * cols;
+    // decoder tables: [DC, AC Huffman tables][quantisation table][FrameDesc per frame]
+    dmcjpeg::EncTables t;
+    dmcjpeg::make_enc_tables(quality, rows, cols, &t);
+    std::vector<dmcjpeg::QuantTable> qpool; std::vector<dmcjpeg::HuffTable> hpool; dmcjpeg::FrameDesc hd;
+    const std::string why = jpeg_parse_frame(t.header, dmcjpeg::kEncHeaderBytes, 0, rows, cols, qpool, hpool, &hd);
+    if (!why.empty() || hpool.size() != 2 || qpool.size() != 1 || hd.dc != 0 || hd.ac != 1 || hd.qt != 0)
+        return fail(ctx, DMC_ERR_TYPE, "dmc_jpeg_degrade_gray_batch: encoder header does not parse: " + why);
+    const size_t o_q = 2 * sizeof(dmcjpeg::HuffTable), o_desc = (o_q + sizeof(dmcjpeg::QuantTable) + 15) & ~(size_t)15;
+    TRY(reserve(ctx, ctx->jpeg_enc[JE_DEC], o_desc + (size_t)group * sizeof(dmcjpeg::FrameDesc)));
+    char* dm = (char*)ctx->jpeg_enc[JE_DEC].p;
+    CUDA_TRY(ctx, cudaMemcpyAsync(dm, hpool.data(), 2 * sizeof(dmcjpeg::HuffTable), cudaMemcpyHostToDevice, s));
+    CUDA_TRY(ctx, cudaMemcpyAsync(dm + o_q, qpool.data(), sizeof(dmcjpeg::QuantTable), cudaMemcpyHostToDevice, s));
+    std::vector<uint32_t> lens;
+    for (int f0 = 0; f0 < n_frames; f0 += group) {
+        const int nf = n_frames - f0 < group ? n_frames - f0 : group;
+        TRY(jpeg_enc_group(ctx, (const uint8_t*)src, mem, f0, nf, rows, cols, dm + o_desc));
+        uint8_t* out = (uint8_t*)dst + fpx * f0;
+        if (mem == DMC_MEM_HOST) { TRY(reserve(ctx, ctx->jpeg_enc[JE_OUT], fpx * nf)); out = (uint8_t*)ctx->jpeg_enc[JE_OUT].p; }
+        LAUNCH(ctx, launch_jpeg_decode((const uint8_t*)ctx->jpeg_enc[JE_SLOTS].p, dm + o_desc, dm, dm + o_q, (uint8_t*)ctx->jpeg_enc[JE_WORDS].p, nullptr, out,
+                                       nf, 0, rows, cols, s));
+        if (mem == DMC_MEM_HOST) CUDA_TRY(ctx, cudaMemcpyAsync((uint8_t*)dst + fpx * f0, out, fpx * nf, cudaMemcpyDeviceToHost, s));
+        if (bytes) {
+            lens.resize(nf);
+            CUDA_TRY(ctx, cudaMemcpyAsync(lens.data(), ctx->jpeg_enc[JE_LENS].p, nf * sizeof(uint32_t), cudaMemcpyDeviceToHost, s));
+        }
+        CUDA_TRY(ctx, cudaStreamSynchronize(s));
+        if (bytes) for (int i = 0; i < nf; i++) bytes[f0 + i] = lens[i];
     }
     return DMC_OK;
 }

@@ -48,4 +48,21 @@ __host__ __device__ __forceinline__ int circle_halfwidth(int i, int rmax, int rH
     return j < rH ? j : rH;
 }
 
+// Exclusive prefix sum over a CTA of NT threads (all of them call it); *total = sum of all.
+template <int NT>
+__device__ __forceinline__ uint32_t cta_scan_excl(uint32_t v, uint32_t* warp_tot, uint32_t* total) {
+    const int lane = threadIdx.x & 31, w = threadIdx.x >> 5;
+    uint32_t x = v;
+#pragma unroll
+    for (int o = 1; o < 32; o <<= 1) { uint32_t y = __shfl_up_sync(0xffffffffu, x, o); if (lane >= o) x += y; }
+    __syncthreads();                        // warp_tot may still be read by the previous scan
+    if (lane == 31) warp_tot[w] = x;
+    __syncthreads();
+    uint32_t base = 0, tot = 0;
+#pragma unroll
+    for (int i = 0; i < NT / 32; i++) { const uint32_t t = warp_tot[i]; if (i < w) base += t; tot += t; }
+    *total = tot;
+    return base + x - v;
+}
+
 }  // namespace dmc

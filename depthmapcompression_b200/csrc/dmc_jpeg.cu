@@ -100,22 +100,6 @@ struct JpegShared {
     uint32_t marker, total, tile_total;
 };
 
-// Exclusive prefix sum over the CTA (kJT lanes); *total = sum of all.
-__device__ __forceinline__ uint32_t cta_scan_excl(uint32_t v, uint32_t* warp_tot, uint32_t* total) {
-    const int lane = threadIdx.x & 31, w = threadIdx.x >> 5;
-    uint32_t x = v;
-#pragma unroll
-    for (int o = 1; o < 32; o <<= 1) { uint32_t y = __shfl_up_sync(0xffffffffu, x, o); if (lane >= o) x += y; }
-    __syncthreads();                        // warp_tot may still be read by the previous scan
-    if (lane == 31) warp_tot[w] = x;
-    __syncthreads();
-    uint32_t base = 0, tot = 0;
-#pragma unroll
-    for (int i = 0; i < kJT / 32; i++) { const uint32_t t = warp_tot[i]; if (i < w) base += t; tot += t; }
-    *total = tot;
-    return base + x - v;
-}
-
 __global__ void __launch_bounds__(kJT, 1) jpeg_frame_kernel(const uint8_t* __restrict__ blob, const FrameDesc* __restrict__ desc, const HuffTable* __restrict__ ht,
                                                            const QuantTable* __restrict__ qts, uint8_t* scratch, uint8_t* __restrict__ dst, int H, int W) {
     extern __shared__ __align__(16) unsigned char smem_raw[];
@@ -156,7 +140,7 @@ __global__ void __launch_bounds__(kJT, 1) jpeg_frame_kernel(const uint8_t* __res
         const uint32_t m = sm.marker;
         if (m < i0 + 16u) keep &= (m <= i0) ? 0u : ((1u << (m - i0)) - 1u);       // nothing at or after the marker's 0xFF
         uint32_t tile_total;
-        uint32_t o = out_base + cta_scan_excl(__popc(keep), sm.warp_tot, &tile_total);
+        uint32_t o = out_base + cta_scan_excl<kJT>(__popc(keep), sm.warp_tot, &tile_total);
 #pragma unroll
         for (int i = 0; i < 16; i++) if (keep & (1u << i)) ds[o++] = b[i];
         out_base += tile_total;
@@ -200,8 +184,8 @@ __global__ void __launch_bounds__(kJT, 1) jpeg_frame_kernel(const uint8_t* __res
     uint32_t dummy;
     const uint32_t my_nb = (uint32_t)tid < nsub ? sm.rec_kn[tid] >> 8 : 0u;
     const uint32_t my_dc = (uint32_t)tid < nsub ? (uint32_t)sm.rec_dc[tid] : 0u;
-    uint32_t blk = cta_scan_excl(my_nb, sm.warp_tot, &dummy);
-    int pred = (int)cta_scan_excl(my_dc, sm.warp_tot, &dummy);
+    uint32_t blk = cta_scan_excl<kJT>(my_nb, sm.warp_tot, &dummy);
+    int pred = (int)cta_scan_excl<kJT>(my_dc, sm.warp_tot, &dummy);
 
     // ---- phase 4: decode again, this time for real: coefficients -> shared memory -> IDCT -> pixels ---------------------
     if ((uint32_t)tid >= nsub) return;

@@ -193,6 +193,29 @@ int dmc_chain_batch_jpeg(dmc_ctx* ctx, const void* blob, const uint64_t* offsets
  * streams (bad segment lengths, Huffman tables that are not prefix codes, ...) are refused here, never crashed on. */
 int dmc_jpeg_probe(const void* stream, size_t len, int* rows, int* cols, char* err, size_t err_len);
 
+/* ---- encode (SURVEY.md 8f-5) ----------------------------------------------------------------------------------- */
+/* Baseline JPEG encoding of 8UC1 frames, byte-identical to cv::imencode(".jpg", img, {IMWRITE_JPEG_QUALITY, quality}) with
+ * libjpeg-turbo (the encoder behind the reference's degradeJPEG): standard luminance tables scaled by quality, islow FDCT,
+ * no restart intervals, no optimised Huffman tables.
+ *
+ * Host only, needs no GPU: the worst-case stream size of one rows x cols frame.  DMC_ERR_SIZE for sizes outside
+ * 1..65535 and for frames whose bound exceeds 256 MB (the decoder's scan limit; *bytes still holds the bound). */
+int dmc_jpeg_encode_bound(int rows, int cols, uint64_t* bytes);
+/* src: n_frames dense rows x cols frames (src_mem: host or device).  The streams are written back to back into blob
+ * (blob_mem: host or device); offsets (host, n_frames + 1 entries) receives their layout -- stream i occupies
+ * [offsets[i], offsets[i+1]) -- which dmc_jpeg_decode_gray_batch and dmc_chain_batch_jpeg take as it is.  quality in
+ * 0..100 (0 acts as 1, as in cv::imencode), anything else is DMC_ERR_ARG.  If the streams do not fit into `capacity`
+ * bytes the call returns DMC_ERR_SIZE and writes nothing at or past blob + capacity; n_frames x dmc_jpeg_encode_bound
+ * always suffices.  Returns when offsets and blob are valid. */
+int dmc_jpeg_encode_gray_batch(dmc_ctx* ctx, const void* src, int src_mem, int n_frames, int rows, int cols, int quality,
+                               void* blob, int blob_mem, uint64_t capacity, uint64_t* offsets);
+/* The reference's degradeJPEG for a batch, entirely on the device: dst = cv::imdecode(cv::imencode(src, quality), 0) for
+ * every frame (src, dst: n_frames dense 8UC1 frames in `mem`; they may alias).  bytes (host, n_frames entries, may be NULL)
+ * receives the stream sizes, i.e. the bitrate.  The streams themselves never leave the device.  Returns when dst and
+ * bytes are valid. */
+int dmc_jpeg_degrade_gray_batch(dmc_ctx* ctx, const void* src, void* dst, int n_frames, int rows, int cols, int quality, int mem,
+                                uint64_t* bytes);
+
 /* ---- stand-alone operators of filter.h ------------------------------------------------------------------- */
 /* binalyWeightedRangeFilter filter.h:29 (binalyWeightedRangeFilter.cpp:1106): 8U/16S/16U/32F x C1/C3 */
 int dmc_bwrf(dmc_ctx* ctx, const dmc_image* src, dmc_image* dst, int kernel_w, int kernel_h, float threshold,

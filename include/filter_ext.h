@@ -25,3 +25,42 @@ inline void minmaxBoundaryReconstructionFilter(const Mat& src, Mat& dest, const 
 	dmc_image a = dmc_dropin::wrap(src), b = dmc_dropin::wrap(dest);
 	dmc_dropin::check(dmc_minmax_boundary_reconstruction(dmc_dropin::context(), &a, &b, r, ksize.width, ksize.height, frec, color, space), "minmaxBoundaryReconstructionFilter");
 }
+
+namespace dmc_dropin {
+inline void require_gray8(const Mat& m, const char* what) {
+	if (m.type() == CV_8UC1 && !m.empty()) return;
+#ifdef DMC_MINICV_HPP
+	throw cv::Exception((std::string(what) + ": src must be a non-empty CV_8UC1 image").c_str(), __FILE__, __LINE__);
+#else
+	CV_Error(cv::Error::StsAssert, std::string(what) + ": src must be a non-empty CV_8UC1 image");
+#endif
+}
+}  // namespace dmc_dropin
+
+// Baseline JPEG encoding of a CV_8UC1 image on the GPU: `buf` receives the same bytes as
+// cv::imencode(".jpg", src, buf, {IMWRITE_JPEG_QUALITY, quality}) with libjpeg-turbo.  quality in 0..100.
+inline void jpegEncodeGray(const Mat& src, vector<uchar>& buf, int quality)
+{
+	dmc_dropin::require_gray8(src, "jpegEncodeGray");
+	const Mat s = src.isContinuous() ? src : src.clone();
+	uint64_t cap = 0, off[2] = {0, 0};
+	dmc_dropin::check(dmc_jpeg_encode_bound(s.rows, s.cols, &cap), "jpegEncodeGray");
+	buf.resize((size_t)cap);
+	dmc_dropin::check(dmc_jpeg_encode_gray_batch(dmc_dropin::context(), s.data, DMC_MEM_HOST, 1, s.rows, s.cols, quality, buf.data(), DMC_MEM_HOST, cap, off), "jpegEncodeGray");
+	buf.resize((size_t)off[1]);
+}
+
+// JPEG round trip of a CV_8UC1 image on the GPU, the stream never leaving the device:
+// dest = cv::imdecode(cv::imencode(".jpg", src, {IMWRITE_JPEG_QUALITY, quality}), 0).  Returns the stream's size in bytes.
+inline int degradeJPEGGray(const Mat& src, Mat& dest, int quality)
+{
+	dmc_dropin::require_gray8(src, "degradeJPEGGray");
+	const Mat s = src.isContinuous() ? src : src.clone();
+	Mat d;
+	if (dest.data != src.data && dest.size() == src.size() && dest.type() == CV_8UC1 && dest.isContinuous()) d = dest;
+	else d.create(src.size(), CV_8UC1);
+	uint64_t bytes = 0;
+	dmc_dropin::check(dmc_jpeg_degrade_gray_batch(dmc_dropin::context(), s.data, d.data, 1, s.rows, s.cols, quality, DMC_MEM_HOST, &bytes), "degradeJPEGGray");
+	if (d.data != dest.data) dest = d;
+	return (int)bytes;
+}
