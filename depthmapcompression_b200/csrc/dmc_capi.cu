@@ -6,6 +6,7 @@
 #include "dmc_jpeg_enc_core.h"
 #include "dmc_kernels.cuh"
 
+#include <limits.h>
 #include <math.h>
 #include <stdio.h>
 #include <stdlib.h>
@@ -19,12 +20,17 @@ using namespace dmc;
 namespace {
 
 constexpr int kSlots = 4;        // streaming pipeline depth (H2D / kernels / D2H of different chunks overlap)
-constexpr int kBufsPerSlot = 9;  // in, out, ping, pong, float scratch; JPEG: bitstreams, descriptor block, de-stuffed scans, coefficients (restart streams)
+
+// Device buffers of a slot: the chain's staged input and output, ping-pong frames and float scratch (single-image operators
+// stage extra images there too); JPEG bitstreams, metadata block (JpegGroup), de-stuffed scans, restart-stream coefficients.
+enum { SB_IN, SB_OUT, SB_PING, SB_PONG, SB_FLOAT, SB_BITS, SB_META, SB_SCANS, SB_COEF, SB_COUNT };
+// Device buffers of dmc_jpeg_decode_gray_batch.
+enum { JD_BITS, JD_META, JD_SCANS, JD_COEF, JD_OUT, JD_COUNT };
 
 struct Buf { void* p = nullptr; size_t cap = 0; };
 
 struct Slot {
-    Buf buf[kBufsPerSlot];
+    Buf buf[SB_COUNT];
     cudaStream_t stream = nullptr;
     // pinned host staging for per-chunk metadata that is built on the host (JPEG descriptors and tables), and the event
     // after which the chunk that used it last is completely done
@@ -44,7 +50,7 @@ struct dmc_ctx {
     // device holds the staging buffers, this context's kernels reach them through NVLink peer access
     struct Gateway { int device = -1; cudaStream_t stream[kSlots] = {}; Buf in[kSlots], out[kSlots]; cudaEvent_t ev_in[kSlots] = {}, ev_out[kSlots] = {}, ev_done[kSlots] = {}; } gw;
     Buf render[2]; int* render_flag = nullptr;      // point-cloud render: attempt lists etc., device flag; pinned host flag
-    Buf jpeg[7];                 // JPEG decode: blob, frame descriptors, Huffman tables, quant tables, coefficients (restart streams only), output, de-stuffed scans
+    Buf jpeg[JD_COUNT];
     Buf jpeg_enc[9];             // JPEG encode: tables, staged frames, coefficients, block records, scan words, slots, lengths + offsets, staged output, decoder tables + descriptors
     // optional per-stage CUDA-event timing of the chain (bench.py's live roofline measurement)
     int lanes = 1;               // concurrent frame groups in the device-resident batch path
@@ -162,6 +168,21 @@ int stage_out_end(dmc_ctx* ctx, const dmc_image* dst, void* dev, cudaStream_t s)
     return DMC_OK;
 }
 
+// Prologue of a single-image operator: it runs on slot 0, which follows the context's stream; `in` is src on the device,
+// `out` where the kernels write dst (stage_out_end delivers it).
+int stage_op(dmc_ctx* ctx, const dmc_image* src, const dmc_image* dst, const void** in, void** out) {
+    CUDA_TRY(ctx, cudaSetDevice(ctx->device));
+    Slot& sl = ctx->slot[0]; sl.stream = ctx->stream;
+    TRY(stage_in(ctx, src, sl.buf[SB_IN], sl.stream, in));
+    return stage_out_begin(ctx, dst, *in, image_bytes(src), sl.buf[SB_OUT], out);
+}
+
+// The identity cases of the operators: dst becomes a copy of src.
+int copy_unless_same(dmc_ctx* ctx, void* dst, const void* src, size_t bytes, cudaStream_t s) {
+    if (dst != src) CUDA_TRY(ctx, cudaMemcpyAsync(dst, src, bytes, cudaMemcpyDeviceToDevice, s));
+    return DMC_OK;
+}
+
 int check_radius(dmc_ctx* ctx, int r, const char* what) {
     if (r < 0 || r > DMC_MAX_RADIUS) return fail(ctx, DMC_ERR_ARG, std::string(what) + " out of range [0, 10]");
     return DMC_OK;
@@ -190,7 +211,7 @@ int range_filter_8u(dmc_ctx* ctx, const uint8_t* src, uint8_t* dst, Buf& tmp, in
     size_t bytes = (size_t)n * H * W * cn;
     const int th = (int)(uint8_t)(int)threshold;                                   // (uchar)threshold :1113
     if (method == DMC_FULL_KERNEL) {
-        if (kw == 0 || kh == 0) { if (dst != src) CUDA_TRY(ctx, cudaMemcpyAsync(dst, src, bytes, cudaMemcpyDeviceToDevice, s)); return DMC_OK; }   // :1033
+        if (kw == 0 || kh == 0) return copy_unless_same(ctx, dst, src, bytes, s);   // :1033
         RowSpan rs = make_rowspan(kw, kh);
         if (cn == 1 && kw == kh && (kw & 1)) {                                     // square odd window: packed-half fast path when exact
             int nk = launch_bwrf8u_h2(src, dst, n, H, W, kw >> 1, th, rs.ntaps, s);
@@ -204,7 +225,7 @@ int range_filter_8u(dmc_ctx* ctx, const uint8_t* src, uint8_t* dst, Buf& tmp, in
         return DMC_OK;
     }
     if (method == DMC_SEPARABLE_KERNEL) {                                          // :1084-1091 (both guards test .width)
-        if (kw <= 1) { if (dst != src) CUDA_TRY(ctx, cudaMemcpyAsync(dst, src, bytes, cudaMemcpyDeviceToDevice, s)); return DMC_OK; }
+        if (kw <= 1) return copy_unless_same(ctx, dst, src, bytes, s);
         TRY(reserve(ctx, tmp, bytes));
         RowSpan rh = make_rowspan(kw, 1), rv = make_rowspan(1, kh);
         LAUNCH(ctx, launch_bwrf8u(src, (uint8_t*)tmp.p, n, H, W, cn, rh, th, s));
@@ -221,8 +242,7 @@ int range_filter_32f(dmc_ctx* ctx, const void* src, void* dst, Buf& tmp, int n, 
     if (method == DMC_FULL_KERNEL || method == DMC_FULL_KERNEL_PAIR) {
         // FULL_KERNEL_PAIR has no deterministic reference output (racy scatter, unwritten tail columns); it computes
         // the FULL_KERNEL result that it approximates.  No bit-parity claim for that method (DESIGN.md).
-        if (kw == 0 || kh == 0) { kw = 1; kh = 1; if (load_op == LOAD_F32 && store_op == STORE_F32) {
-            if (dst != src) CUDA_TRY(ctx, cudaMemcpyAsync(dst, src, count * sizeof(float), cudaMemcpyDeviceToDevice, s)); return DMC_OK; } }
+        if (kw == 0 || kh == 0) { kw = 1; kh = 1; if (load_op == LOAD_F32 && store_op == STORE_F32) return copy_unless_same(ctx, dst, src, count * sizeof(float), s); }
         RowSpan rs = make_rowspan(kw, kh);
         LAUNCH(ctx, launch_bwrf32f(src, dst, n, H, W, cn, rs, threshold, load_op, maf, store_op, s));
         return DMC_OK;
@@ -242,7 +262,7 @@ int range_filter_32f(dmc_ctx* ctx, const void* src, void* dst, Buf& tmp, int n, 
 int run_chain(dmc_ctx* ctx, Slot& sl, const uint8_t* src, void* dst, int n, int H, int W, const dmc_chain_params& p) {
     cudaStream_t s = sl.stream;
     const size_t px = (size_t)n * H * W;
-    Buf& ping = sl.buf[2]; Buf& pong = sl.buf[3]; Buf& ftmp = sl.buf[4];
+    Buf& ping = sl.buf[SB_PING]; Buf& pong = sl.buf[SB_PONG]; Buf& ftmp = sl.buf[SB_FLOAT];
     TRY(reserve(ctx, ping, px)); TRY(reserve(ctx, pong, px));
     const uint8_t* cur = src;
     uint8_t* nxt = (uint8_t*)ping.p;
@@ -333,13 +353,11 @@ int chain_single(dmc_ctx* ctx, const dmc_image* src, dmc_image* dst, const dmc_c
     if (src->cvtype != DMC_8U) return fail(ctx, DMC_ERR_TYPE, "PostFilterSet: src must be CV_8UC1");
     if (dst->cvtype != chain_out_type(p.chain)) return fail(ctx, DMC_ERR_TYPE, "PostFilterSet: dst has the wrong type for this entry point");
     if (dst->rows != src->rows || dst->cols != src->cols) return fail(ctx, DMC_ERR_SIZE, "PostFilterSet: dst size != src size");
-    CUDA_TRY(ctx, cudaSetDevice(ctx->device));
-    Slot& sl = ctx->slot[0]; sl.stream = ctx->stream;
     const void* in; void* out;
-    TRY(stage_in(ctx, src, sl.buf[0], sl.stream, &in));
-    TRY(stage_out_begin(ctx, dst, in, image_bytes(src), sl.buf[1], &out));
+    TRY(stage_op(ctx, src, dst, &in, &out));
+    Slot& sl = ctx->slot[0];
     int rc = DMC_OK;
-    const bool direct = in != sl.buf[0].p && out != sl.buf[1].p;  // device-resident (or mapped host memory), dense, not aliased: nothing but kernels
+    const bool direct = in != sl.buf[SB_IN].p && out != sl.buf[SB_OUT].p;  // device-resident (or mapped host memory), dense, not aliased: nothing but kernels
     if (direct && graph_eligible(ctx, sl.stream)) {
         dmc_ctx::GraphKey key; memset(&key, 0, sizeof key);
         key.in = in; key.out = out; key.rows = src->rows; key.cols = src->cols; key.stream = sl.stream;
@@ -378,23 +396,85 @@ void drop_gateway(dmc_ctx* ctx) {
     ctx->gw.device = -1;
 }
 
-// Staging buffers of a pipeline slot: on this context's device, or on the gateway's (allocated there).
-int reserve_io(dmc_ctx* ctx, int slot, size_t in_bytes, size_t out_bytes, void** in, void** out) {
-    if (ctx->gw.device < 0) {
-        TRY(reserve(ctx, ctx->slot[slot].buf[0], in_bytes)); TRY(reserve(ctx, ctx->slot[slot].buf[1], out_bytes));
-        *in = ctx->slot[slot].buf[0].p; *out = ctx->slot[slot].buf[1].p;
-        return DMC_OK;
-    }
-    Buf& bi = ctx->gw.in[slot]; Buf& bo = ctx->gw.out[slot];
-    if (bi.cap < in_bytes || bo.cap < out_bytes) {
+// A tuning knob of the batch entry points: `name` in MiB when it is set to a positive number, else `dflt` bytes.
+size_t env_mib(const char* name, size_t dflt) {
+    if (const char* e = getenv(name)) { long v = atol(e); if (v > 0) return (size_t)v << 20; }
+    return dflt;
+}
+
+// Frames per group or chunk of a batch: `target` bytes of `frame_bytes` each, at least one frame, at most `cap` (a grid
+// dimension limit) and n_frames.  spread: at least kSlots chunks when there are that many frames, so every slot has work.
+int chunk_frames(size_t target, size_t frame_bytes, int n_frames, int cap, bool spread) {
+    size_t c = target / frame_bytes;
+    if (c > (size_t)cap) c = cap;
+    if (c > (size_t)n_frames) c = n_frames;
+    const int chunk = c < 1 ? 1 : (int)c;
+    return spread && n_frames / chunk < kSlots && n_frames >= kSlots ? (n_frames + kSlots - 1) / kSlots : chunk;
+}
+
+// Frames [f0, f0 + nf) of a streamed batch on slot `si`.  routed: its host traffic runs over the gateway's link; `copy` is
+// the stream that carries it (the gateway's copy stream of the slot, or the slot's own).
+struct Chunk { int f0, nf, si; Slot* sl; bool routed; cudaStream_t copy; };
+
+// Staging buffers of a chunk's host traffic: `local_in` / `local_out` of its slot, or when routed the slot's buffers on
+// the gateway's device (allocated there).  out_bytes == 0: no output staging.
+int reserve_io(dmc_ctx* ctx, const Chunk& c, size_t in_bytes, size_t out_bytes, Buf& local_in, Buf& local_out, void** in, void** out) {
+    Buf& bi = c.routed ? ctx->gw.in[c.si] : local_in;
+    Buf& bo = c.routed ? ctx->gw.out[c.si] : local_out;
+    if (!c.routed) {
+        TRY(reserve(ctx, bi, in_bytes));
+        if (out_bytes) TRY(reserve(ctx, bo, out_bytes));
+    } else if (bi.cap < in_bytes || bo.cap < out_bytes) {
         CUDA_TRY(ctx, cudaDeviceSynchronize());                  // this device's kernels may still be reading the old buffers
         CUDA_TRY(ctx, cudaSetDevice(ctx->gw.device));
-        int rc = reserve(ctx, bi, in_bytes); if (rc == DMC_OK) rc = reserve(ctx, bo, out_bytes);
+        int rc = reserve(ctx, bi, in_bytes); if (rc == DMC_OK && out_bytes) rc = reserve(ctx, bo, out_bytes);
         cudaSetDevice(ctx->device);
         if (rc != DMC_OK) return rc;
     }
     *in = bi.p; *out = bo.p;
     return DMC_OK;
+}
+
+// Streams n_frames through the kSlots slots in chunks of `chunk` frames, so that the copies in, the kernels and the copies
+// out of different chunks overlap.  Chunk i runs on slot i % kSlots (slot 0 follows ctx->stream); a slot's first chunk
+// waits for the work queued on ctx->stream before the call.  Per chunk the caller's prepare (host work, reservations),
+// copy_in (on c.copy), kernels (on the slot's stream) and copy_out (on c.copy) run in turn.  routed: the copies run on the
+// gateway's device (dmc_set_gateway), fenced against the kernels with events.  staged: prepare refills the slot's pinned
+// hstage, so it first waits until the slot's previous chunk is done.  Stops at the first error; drains every stream it used.
+template <class Prepare, class CopyIn, class Kernels, class CopyOut>
+int stream_chunks(dmc_ctx* ctx, int n_frames, int chunk, bool routed, bool staged, Prepare prepare, CopyIn copy_in, Kernels kernels, CopyOut copy_out) {
+    dmc_ctx::Gateway& gw = ctx->gw;
+    cudaEvent_t ready;
+    CUDA_TRY(ctx, cudaEventCreateWithFlags(&ready, cudaEventDisableTiming));
+    CUDA_TRY(ctx, cudaEventRecord(ready, ctx->stream));
+    int rc = DMC_OK;
+    for (int f0 = 0, ci = 0; f0 < n_frames && rc == DMC_OK; f0 += chunk, ci++) {
+        const int si = ci % kSlots;
+        Slot& sl = ctx->slot[si]; if (si == 0) sl.stream = ctx->stream;
+        const Chunk c = {f0, n_frames - f0 < chunk ? n_frames - f0 : chunk, si, &sl, routed, routed ? gw.stream[si] : sl.stream};
+        if (ci < kSlots && sl.stream != ctx->stream) cudaStreamWaitEvent(sl.stream, ready, 0);
+        if (sl.done_pending) { cudaError_t e = cudaEventSynchronize(routed ? gw.ev_done[si] : sl.done); sl.done_pending = false; if (e != cudaSuccess) { rc = fail(ctx, DMC_ERR_CUDA, cudaGetErrorString(e)); break; } }
+        if (staged && !sl.done && cudaEventCreateWithFlags(&sl.done, cudaEventDisableTiming) != cudaSuccess) { rc = fail(ctx, DMC_ERR_CUDA, "cudaEventCreate"); break; }
+        if ((rc = prepare(c)) != DMC_OK) break;
+        if (routed) { cudaSetDevice(gw.device); if (ci < kSlots) cudaStreamWaitEvent(c.copy, ready, 0); }
+        cudaError_t e = copy_in(c);
+        if (e == cudaSuccess && routed) { e = cudaEventRecord(gw.ev_in[si], c.copy); cudaSetDevice(ctx->device); if (e == cudaSuccess) e = cudaStreamWaitEvent(sl.stream, gw.ev_in[si], 0); }
+        if (e != cudaSuccess) { cudaSetDevice(ctx->device); rc = fail(ctx, DMC_ERR_CUDA, cudaGetErrorString(e)); break; }
+        if ((rc = kernels(c)) != DMC_OK) break;
+        if (routed) { e = cudaEventRecord(gw.ev_out[si], sl.stream); cudaSetDevice(gw.device); if (e == cudaSuccess) e = cudaStreamWaitEvent(c.copy, gw.ev_out[si], 0); }
+        if (e == cudaSuccess) e = copy_out(c);
+        if (e == cudaSuccess && staged) { e = cudaEventRecord(routed ? gw.ev_done[si] : sl.done, c.copy); sl.done_pending = e == cudaSuccess; }   // (an event lives on its stream's device)
+        if (routed) cudaSetDevice(ctx->device);
+        if (e != cudaSuccess) { rc = fail(ctx, DMC_ERR_CUDA, cudaGetErrorString(e)); break; }
+    }
+    for (int i = 0; i < kSlots; i++) {
+        cudaError_t e = cudaStreamSynchronize(ctx->slot[i].stream);
+        if (e == cudaSuccess && routed) e = cudaStreamSynchronize(gw.stream[i]);
+        ctx->slot[i].done_pending = false;
+        if (e != cudaSuccess && rc == DMC_OK) rc = fail(ctx, DMC_ERR_CUDA, cudaGetErrorString(e));
+    }
+    cudaEventDestroy(ready);
+    return rc;
 }
 
 }  // namespace
@@ -459,7 +539,7 @@ void dmc_destroy(dmc_ctx* ctx) {
     cudaSetDevice(ctx->device);
     cudaDeviceSynchronize();
     for (int i = 0; i < kSlots; i++) {
-        for (int b = 0; b < kBufsPerSlot; b++) if (ctx->slot[i].buf[b].p) cudaFree(ctx->slot[i].buf[b].p);
+        for (int b = 0; b < SB_COUNT; b++) if (ctx->slot[i].buf[b].p) cudaFree(ctx->slot[i].buf[b].p);
         if (ctx->slot[i].hstage) cudaFreeHost(ctx->slot[i].hstage);
         if (ctx->slot[i].done) cudaEventDestroy(ctx->slot[i].done);
         if (i > 0 && ctx->slot[i].stream) cudaStreamDestroy(ctx->slot[i].stream);
@@ -586,11 +666,9 @@ int dmc_chain_batch(dmc_ctx* ctx, const void* src, void* dst, int n_frames, int 
         // instruction-bound), small enough that scratch stays modest (two group-sized buffers).
         uint8_t* out = (uint8_t*)dst;
         ctx->slot[0].stream = ctx->stream;
-        if (overlaps(dst, obytes * n_frames, src, fpx * n_frames)) { TRY(reserve(ctx, ctx->slot[0].buf[1], obytes * n_frames)); out = (uint8_t*)ctx->slot[0].buf[1].p; }
+        if (overlaps(dst, obytes * n_frames, src, fpx * n_frames)) { TRY(reserve(ctx, ctx->slot[0].buf[SB_OUT], obytes * n_frames)); out = (uint8_t*)ctx->slot[0].buf[SB_OUT].p; }
         const int lanes = ctx->lanes < 1 ? 1 : (ctx->lanes > kSlots ? kSlots : ctx->lanes);
-        size_t group_bytes = (size_t)256 << 20;
-        if (const char* e = getenv("DMC_GROUP_MB")) { long v = atol(e); if (v > 0) group_bytes = (size_t)v << 20; }   // tuning knob
-        int group = (int)((group_bytes / lanes) / fpx); if (group < 1) group = 1; if (group > 65535) group = 65535;   // gridDim.z limit
+        const int group = chunk_frames(env_mib("DMC_GROUP_MB", (size_t)256 << 20) / lanes, fpx, n_frames, 65535, false);
         // lanes > 1: consecutive groups run on different streams so that the tail of one kernel (partially filled last
         // wave) overlaps the head of another group's kernel.  The extra streams are fenced against ctx->stream.
         cudaEvent_t fence = nullptr;
@@ -613,48 +691,19 @@ int dmc_chain_batch(dmc_ctx* ctx, const void* src, void* dst, int n_frames, int 
         return DMC_OK;
     }
     // host: chunked streaming
-    size_t target = (size_t)48 << 20;                       // input bytes per chunk; per 1000 1080p frames host-to-host: 16 MB 42.0, 32 MB 42.5, 48 MB 45.5, 64 MB 45.0, 128 MB 43.5 Gpx/s
-    if (const char* e = getenv("DMC_CHUNK_MB")) { long v = atol(e); if (v > 0) target = (size_t)v << 20; }   // tuning knob
-    int chunk = (int)(target / fpx); if (chunk < 1) chunk = 1; if (chunk > 65535) chunk = 65535; if (chunk > n_frames) chunk = n_frames;
-    if (n_frames / chunk < kSlots && n_frames >= kSlots) chunk = (n_frames + kSlots - 1) / kSlots;
-    cudaEvent_t ready;                                       // slots wait for work queued earlier on ctx->stream
-    CUDA_TRY(ctx, cudaEventCreateWithFlags(&ready, cudaEventDisableTiming));
-    CUDA_TRY(ctx, cudaEventRecord(ready, ctx->stream));
-    const bool gw = ctx->gw.device >= 0;
-    int rc = DMC_OK, ci = 0;
-    for (int f0 = 0; f0 < n_frames && rc == DMC_OK; f0 += chunk, ci++) {
-        int nf = n_frames - f0 < chunk ? n_frames - f0 : chunk;
-        const int si = ci % kSlots;
-        Slot& sl = ctx->slot[si]; if (si == 0) sl.stream = ctx->stream;
-        if (ci < kSlots && sl.stream != ctx->stream) cudaStreamWaitEvent(sl.stream, ready, 0);
-        void *din = nullptr, *dout = nullptr;
-        if ((rc = reserve_io(ctx, si, fpx * nf, obytes * nf, &din, &dout)) != DMC_OK) break;
-        // copies run on the stream of the device whose link carries them; with a gateway the kernels (on this device's
-        // stream) are fenced against them with events and read / write the gateway's buffers over NVLink
-        cudaStream_t cps = gw ? ctx->gw.stream[si] : sl.stream;
-        if (gw) { cudaSetDevice(ctx->gw.device); if (ci < kSlots) cudaStreamWaitEvent(cps, ready, 0); }
-        cudaError_t e = cudaMemcpyAsync(din, (const uint8_t*)src + fpx * f0, fpx * nf, cudaMemcpyHostToDevice, cps);
-        if (e == cudaSuccess && gw) { e = cudaEventRecord(ctx->gw.ev_in[si], cps); cudaSetDevice(ctx->device); if (e == cudaSuccess) e = cudaStreamWaitEvent(sl.stream, ctx->gw.ev_in[si], 0); }
-        if (e != cudaSuccess) { cudaSetDevice(ctx->device); rc = fail(ctx, DMC_ERR_CUDA, cudaGetErrorString(e)); break; }
-        rc = run_chain(ctx, sl, (const uint8_t*)din, dout, nf, rows, cols, p);
-        if (rc != DMC_OK) break;
-        if (gw) { e = cudaEventRecord(ctx->gw.ev_out[si], sl.stream); cudaSetDevice(ctx->gw.device); if (e == cudaSuccess) e = cudaStreamWaitEvent(cps, ctx->gw.ev_out[si], 0); }
-        if (e == cudaSuccess) e = cudaMemcpyAsync((uint8_t*)dst + obytes * f0, dout, obytes * nf, cudaMemcpyDeviceToHost, cps);
-        if (gw) cudaSetDevice(ctx->device);
-        if (e != cudaSuccess) { rc = fail(ctx, DMC_ERR_CUDA, cudaGetErrorString(e)); break; }
-    }
-    for (int i = 0; i < kSlots; i++) {
-        cudaError_t e = cudaStreamSynchronize(ctx->slot[i].stream);
-        if (e == cudaSuccess && gw) e = cudaStreamSynchronize(ctx->gw.stream[i]);
-        if (e != cudaSuccess && rc == DMC_OK) rc = fail(ctx, DMC_ERR_CUDA, cudaGetErrorString(e));
-    }
-    cudaEventDestroy(ready);
-    return rc;
+    const int chunk = chunk_frames(env_mib("DMC_CHUNK_MB", (size_t)48 << 20), fpx, n_frames, 65535, true);   // input bytes per chunk; per 1000 1080p frames host-to-host: 16 MB 42.0, 32 MB 42.5, 48 MB 45.5, 64 MB 45.0, 128 MB 43.5 Gpx/s
+    void *din = nullptr, *dout = nullptr;
+    return stream_chunks(ctx, n_frames, chunk, ctx->gw.device >= 0, false,
+        [&](const Chunk& c) { return reserve_io(ctx, c, fpx * c.nf, obytes * c.nf, c.sl->buf[SB_IN], c.sl->buf[SB_OUT], &din, &dout); },
+        [&](const Chunk& c) { return cudaMemcpyAsync(din, (const uint8_t*)src + fpx * c.f0, fpx * c.nf, cudaMemcpyHostToDevice, c.copy); },
+        [&](const Chunk& c) { return run_chain(ctx, *c.sl, (const uint8_t*)din, dout, c.nf, rows, cols, p); },
+        [&](const Chunk& c) { return cudaMemcpyAsync((uint8_t*)dst + obytes * c.f0, dout, obytes * c.nf, cudaMemcpyDeviceToHost, c.copy); });
 }
 
 // The same chain on a batch given as ARRAYS OF IMAGE DESCRIPTORS (frames anywhere in host or device memory, any row step):
 // every frame is packed into the slot's dense buffer (H2D or D2D), chunks of frames run through run_chain and are
-// unpacked into their own dst -- the 3-slot pipeline of the dense host path.  Returns when every dst is valid.
+// unpacked into their own dst -- the slot pipeline of the dense host path, always on this context's own device (frames
+// may be device-resident).  Returns when every dst is valid.
 int dmc_chain_batch_images(dmc_ctx* ctx, const dmc_image* srcs, dmc_image* dsts, int n_frames, const dmc_chain_params* pp) {
     if (!ctx) return fail(nullptr, DMC_ERR_ARG, "null context");
     if (!srcs || !dsts || !pp || n_frames < 0) return fail(ctx, DMC_ERR_ARG, "dmc_chain_batch_images: bad arguments");
@@ -670,44 +719,35 @@ int dmc_chain_batch_images(dmc_ctx* ctx, const dmc_image* srcs, dmc_image* dsts,
     }
     CUDA_TRY(ctx, cudaSetDevice(ctx->device));
     const size_t fpx = (size_t)rows * cols, obytes = fpx * depth_size(otype), orow = (size_t)cols * depth_size(otype);
-    size_t target = (size_t)48 << 20;
-    int chunk = (int)(target / fpx); if (chunk < 1) chunk = 1; if (chunk > 65535) chunk = 65535; if (chunk > n_frames) chunk = n_frames;
-    if (n_frames / chunk < kSlots && n_frames >= kSlots) chunk = (n_frames + kSlots - 1) / kSlots;
-    cudaEvent_t ready;
-    CUDA_TRY(ctx, cudaEventCreateWithFlags(&ready, cudaEventDisableTiming));
-    CUDA_TRY(ctx, cudaEventRecord(ready, ctx->stream));
-    int rc = DMC_OK, ci = 0;
-    for (int f0 = 0; f0 < n_frames && rc == DMC_OK; f0 += chunk, ci++) {
-        const int nf = n_frames - f0 < chunk ? n_frames - f0 : chunk;
-        Slot& sl = ctx->slot[ci % kSlots]; if (ci % kSlots == 0) sl.stream = ctx->stream;
-        if (ci < kSlots && sl.stream != ctx->stream) cudaStreamWaitEvent(sl.stream, ready, 0);
-        if ((rc = reserve(ctx, sl.buf[0], fpx * nf)) != DMC_OK) break;
-        if ((rc = reserve(ctx, sl.buf[1], obytes * nf)) != DMC_OK) break;
-        cudaError_t e = cudaSuccess;
-        for (int i = 0; i < nf && e == cudaSuccess; i++) {
-            const dmc_image& im = srcs[f0 + i];
-            e = cudaMemcpy2DAsync((uint8_t*)sl.buf[0].p + fpx * i, cols, im.data, step_of(&im), cols, rows,
-                                  im.mem == DMC_MEM_HOST ? cudaMemcpyHostToDevice : cudaMemcpyDeviceToDevice, sl.stream);
-        }
-        if (e != cudaSuccess) { rc = fail(ctx, DMC_ERR_CUDA, cudaGetErrorString(e)); break; }
-        rc = run_chain(ctx, sl, (const uint8_t*)sl.buf[0].p, sl.buf[1].p, nf, rows, cols, p);
-        if (rc != DMC_OK) break;
-        for (int i = 0; i < nf && e == cudaSuccess; i++) {
-            const dmc_image& im = dsts[f0 + i];
-            e = cudaMemcpy2DAsync(im.data, step_of(&im), (uint8_t*)sl.buf[1].p + obytes * i, orow, orow, rows,
-                                  im.mem == DMC_MEM_HOST ? cudaMemcpyDeviceToHost : cudaMemcpyDeviceToDevice, sl.stream);
-        }
-        if (e != cudaSuccess) { rc = fail(ctx, DMC_ERR_CUDA, cudaGetErrorString(e)); break; }
-    }
-    for (int i = 0; i < kSlots; i++) { cudaError_t e = cudaStreamSynchronize(ctx->slot[i].stream); if (e != cudaSuccess && rc == DMC_OK) rc = fail(ctx, DMC_ERR_CUDA, cudaGetErrorString(e)); }
-    cudaEventDestroy(ready);
-    return rc;
+    const int chunk = chunk_frames((size_t)48 << 20, fpx, n_frames, 65535, true);
+    void *din = nullptr, *dout = nullptr;
+    return stream_chunks(ctx, n_frames, chunk, false, false,
+        [&](const Chunk& c) { return reserve_io(ctx, c, fpx * c.nf, obytes * c.nf, c.sl->buf[SB_IN], c.sl->buf[SB_OUT], &din, &dout); },
+        [&](const Chunk& c) {
+            cudaError_t e = cudaSuccess;
+            for (int i = 0; i < c.nf && e == cudaSuccess; i++) {
+                const dmc_image& im = srcs[c.f0 + i];
+                e = cudaMemcpy2DAsync((uint8_t*)din + fpx * i, cols, im.data, step_of(&im), cols, rows,
+                                      im.mem == DMC_MEM_HOST ? cudaMemcpyHostToDevice : cudaMemcpyDeviceToDevice, c.copy);
+            }
+            return e;
+        },
+        [&](const Chunk& c) { return run_chain(ctx, *c.sl, (const uint8_t*)din, dout, c.nf, rows, cols, p); },
+        [&](const Chunk& c) {
+            cudaError_t e = cudaSuccess;
+            for (int i = 0; i < c.nf && e == cudaSuccess; i++) {
+                const dmc_image& im = dsts[c.f0 + i];
+                e = cudaMemcpy2DAsync(im.data, step_of(&im), (uint8_t*)dout + obytes * i, orow, orow, rows,
+                                      im.mem == DMC_MEM_HOST ? cudaMemcpyDeviceToHost : cudaMemcpyDeviceToDevice, c.copy);
+            }
+            return e;
+        });
 }
 
 // ---- frame-batch scheduler across the GPUs of one box ---------------------------------------------------------------
 // One context per listed device, kept alive between runs (device buffers, streams); every run cuts the batch into
 // contiguous shards (dmc_shard_frames) and streams each shard through its device on its own host thread with
-// dmc_chain_batch (3-slot H2D / kernels / D2H pipeline).  Frames are independent: no exchange between devices.
+// dmc_chain_batch (its slot pipeline of H2D / kernels / D2H).  Frames are independent: no exchange between devices.
 struct dmc_sched {
     std::vector<dmc_ctx*> ctxs;
     std::string err;
@@ -787,12 +827,20 @@ int dmc_multi_chain_batch(const int* devices, int n_devices, const void* src, vo
 // ---- JPEG decode feeding the chain (SURVEY.md 8f-1) -----------------------------------------------------------------
 namespace {
 
-// Host side of one group of streams: parsed descriptors + de-duplicated tables, packed into ONE staging block so that a
-// single H2D copy brings everything the kernels need besides the bitstreams themselves.
+// Host side of one group of streams: parsed descriptors + de-duplicated tables, packed into ONE metadata block so that a
+// single H2D copy brings everything the kernels need besides the bitstreams themselves.  The block is
+// [FrameDesc...][HuffTable...][QuantTable...] with 16-byte aligned parts; o_huff and o_quant are the tables' offsets.
 struct JpegGroup {
     std::vector<dmcjpeg::FrameDesc> desc; std::vector<dmcjpeg::QuantTable> qpool; std::vector<dmcjpeg::HuffTable> hpool;
     size_t scratch_bytes = 0; int n_restart = 0;
+    size_t o_huff = 0, o_quant = 0, meta_bytes = 0;
 };
+
+void jpeg_write_meta(const JpegGroup& g, void* block) {
+    memcpy(block, g.desc.data(), g.desc.size() * sizeof(dmcjpeg::FrameDesc));
+    memcpy((char*)block + g.o_huff, g.hpool.data(), g.hpool.size() * sizeof(dmcjpeg::HuffTable));
+    memcpy((char*)block + g.o_quant, g.qpool.data(), g.qpool.size() * sizeof(dmcjpeg::QuantTable));
+}
 
 // Parses streams [f0, f0 + nf) of the blob; scan offsets are relative to `blob_base` (the first byte that will be copied).
 int jpeg_parse_group(dmc_ctx* ctx, const uint8_t* blob, const uint64_t* offsets, int f0, int nf, uint64_t blob_base, int rows, int cols, JpegGroup* g) {
@@ -807,6 +855,9 @@ int jpeg_parse_group(dmc_ctx* ctx, const uint8_t* blob, const uint64_t* offsets,
         g->scratch_bytes += jpeg_scratch_bytes(g->desc[i].scan_end - g->desc[i].scan_offset);
         if (g->desc[i].restart_interval) g->n_restart++;
     }
+    g->o_huff = (g->desc.size() * sizeof(dmcjpeg::FrameDesc) + 15) & ~(size_t)15;
+    g->o_quant = (g->o_huff + g->hpool.size() * sizeof(dmcjpeg::HuffTable) + 15) & ~(size_t)15;
+    g->meta_bytes = g->o_quant + g->qpool.size() * sizeof(dmcjpeg::QuantTable);
     return DMC_OK;
 }
 
@@ -827,77 +878,45 @@ int dmc_chain_batch_jpeg(dmc_ctx* ctx, const void* blob, const uint64_t* offsets
     if (n_frames == 0) return DMC_OK;
     CUDA_TRY(ctx, cudaSetDevice(ctx->device));
     const size_t fpx = (size_t)rows * cols, obytes = fpx * depth_size(chain_out_type(p.chain)), blocks = (size_t)((rows + 7) / 8) * ((cols + 7) / 8);
-    size_t target = (size_t)128 << 20;                      // decoded bytes per chunk: enough frames (one CTA each) to fill the SMs together with the neighbouring slots
-    if (const char* e = getenv("DMC_CHUNK_MB")) { long v = atol(e); if (v > 0) target = (size_t)v << 20; }
-    int chunk = (int)(target / fpx); if (chunk < 1) chunk = 1; if (chunk > 4096) chunk = 4096; if (chunk > n_frames) chunk = n_frames;
-    if (n_frames / chunk < kSlots && n_frames >= kSlots) chunk = (n_frames + kSlots - 1) / kSlots;
-    cudaEvent_t ready;
-    CUDA_TRY(ctx, cudaEventCreateWithFlags(&ready, cudaEventDisableTiming));
-    CUDA_TRY(ctx, cudaEventRecord(ready, ctx->stream));
-    const bool gw = ctx->gw.device >= 0, host_out = dst_mem == DMC_MEM_HOST;
+    const int chunk = chunk_frames(env_mib("DMC_CHUNK_MB", (size_t)128 << 20), fpx, n_frames, 4096, true);   // decoded bytes per chunk: enough frames (one CTA each) to fill the SMs together with the neighbouring slots
+    const bool host_out = dst_mem == DMC_MEM_HOST;
     JpegGroup g;
-    int rc = DMC_OK, ci = 0;
-    for (int f0 = 0; f0 < n_frames && rc == DMC_OK; f0 += chunk, ci++) {
-        const int nf = n_frames - f0 < chunk ? n_frames - f0 : chunk;
-        const int si = ci % kSlots;
-        Slot& sl = ctx->slot[si]; if (si == 0) sl.stream = ctx->stream;
-        if (ci < kSlots && sl.stream != ctx->stream) cudaStreamWaitEvent(sl.stream, ready, 0);
-        if (sl.done_pending) { cudaError_t e = cudaEventSynchronize(gw ? ctx->gw.ev_done[si] : sl.done); sl.done_pending = false; if (e != cudaSuccess) { rc = fail(ctx, DMC_ERR_CUDA, cudaGetErrorString(e)); break; } }
-        const uint64_t b0 = offsets[f0], b1 = offsets[f0 + nf];
-        if (b1 < b0) { rc = fail(ctx, DMC_ERR_ARG, "dmc_chain_batch_jpeg: offsets must be non-decreasing"); break; }
-        if ((rc = jpeg_parse_group(ctx, (const uint8_t*)blob, offsets, f0, nf, b0, rows, cols, &g)) != DMC_OK) break;
-        // metadata block: [descriptors][Huffman tables][quantisation tables], 16-byte aligned parts
-        const size_t o_desc = 0, o_h = (g.desc.size() * sizeof(dmcjpeg::FrameDesc) + 15) & ~(size_t)15,
-                     o_q = (o_h + g.hpool.size() * sizeof(dmcjpeg::HuffTable) + 15) & ~(size_t)15, meta = o_q + g.qpool.size() * sizeof(dmcjpeg::QuantTable);
-        if (sl.hcap < meta) {
-            if (sl.hstage) cudaFreeHost(sl.hstage);
-            sl.hstage = nullptr; sl.hcap = 0;
-            const size_t cap = (meta * 2 + 65535) & ~(size_t)65535;
-            if (cudaHostAlloc(&sl.hstage, cap, cudaHostAllocDefault) != cudaSuccess) { rc = fail(ctx, DMC_ERR_CUDA, "cudaHostAlloc (JPEG metadata staging)"); break; }
-            sl.hcap = cap;
-        }
-        if (!sl.done && cudaEventCreateWithFlags(&sl.done, cudaEventDisableTiming) != cudaSuccess) { rc = fail(ctx, DMC_ERR_CUDA, "cudaEventCreate"); break; }
-        memcpy((char*)sl.hstage + o_desc, g.desc.data(), g.desc.size() * sizeof(dmcjpeg::FrameDesc));
-        memcpy((char*)sl.hstage + o_h, g.hpool.data(), g.hpool.size() * sizeof(dmcjpeg::HuffTable));
-        memcpy((char*)sl.hstage + o_q, g.qpool.data(), g.qpool.size() * sizeof(dmcjpeg::QuantTable));
-        // device buffers: bitstreams and results on the device whose link carries them, everything else local
-        void *dblob = nullptr, *dout = nullptr;
-        if (gw) { if ((rc = reserve_io(ctx, si, (size_t)(b1 - b0) + 16, host_out ? obytes * nf : 16, &dblob, &dout)) != DMC_OK) break; }
-        else {
-            if ((rc = reserve(ctx, sl.buf[5], (size_t)(b1 - b0) + 16)) != DMC_OK) break;
-            if (host_out && (rc = reserve(ctx, sl.buf[1], obytes * nf)) != DMC_OK) break;
-            dblob = sl.buf[5].p; dout = sl.buf[1].p;
-        }
-        if (!host_out) dout = (uint8_t*)dst + obytes * f0;
-        if ((rc = reserve(ctx, sl.buf[0], fpx * nf)) != DMC_OK) break;
-        if ((rc = reserve(ctx, sl.buf[6], meta)) != DMC_OK) break;
-        if ((rc = reserve(ctx, sl.buf[7], g.scratch_bytes + 16)) != DMC_OK) break;
-        if (g.n_restart && (rc = reserve(ctx, sl.buf[8], (size_t)nf * blocks * 64 * sizeof(int16_t))) != DMC_OK) break;
-        cudaStream_t cps = gw ? ctx->gw.stream[si] : sl.stream;
-        if (gw) { cudaSetDevice(ctx->gw.device); if (ci < kSlots) cudaStreamWaitEvent(cps, ready, 0); }
-        cudaError_t e = cudaMemcpyAsync(dblob, (const uint8_t*)blob + b0, (size_t)(b1 - b0), cudaMemcpyHostToDevice, cps);
-        if (e == cudaSuccess && gw) { e = cudaEventRecord(ctx->gw.ev_in[si], cps); cudaSetDevice(ctx->device); if (e == cudaSuccess) e = cudaStreamWaitEvent(sl.stream, ctx->gw.ev_in[si], 0); }
-        if (e == cudaSuccess) e = cudaMemcpyAsync(sl.buf[6].p, sl.hstage, meta, cudaMemcpyHostToDevice, sl.stream);
-        if (e != cudaSuccess) { cudaSetDevice(ctx->device); rc = fail(ctx, DMC_ERR_CUDA, cudaGetErrorString(e)); break; }
-        const char* dm = (const char*)sl.buf[6].p;
-        int nk = launch_jpeg_decode((const uint8_t*)dblob, dm + o_desc, dm + o_h, dm + o_q, (uint8_t*)sl.buf[7].p, (int16_t*)sl.buf[8].p, (uint8_t*)sl.buf[0].p, nf, g.n_restart, rows, cols, sl.stream);
-        if ((rc = after_launch(ctx, nk)) != DMC_OK) break;
-        rc = run_chain(ctx, sl, (const uint8_t*)sl.buf[0].p, dout, nf, rows, cols, p);
-        if (rc != DMC_OK) break;
-        if (gw) { e = cudaEventRecord(ctx->gw.ev_out[si], sl.stream); cudaSetDevice(ctx->gw.device); if (e == cudaSuccess) e = cudaStreamWaitEvent(cps, ctx->gw.ev_out[si], 0); }
-        if (e == cudaSuccess && host_out) e = cudaMemcpyAsync((uint8_t*)dst + obytes * f0, dout, obytes * nf, cudaMemcpyDeviceToHost, cps);
-        if (e == cudaSuccess) { e = cudaEventRecord(gw ? ctx->gw.ev_done[si] : sl.done, cps); sl.done_pending = e == cudaSuccess; }      // (an event lives on its stream's device)
-        if (gw) cudaSetDevice(ctx->device);
-        if (e != cudaSuccess) { rc = fail(ctx, DMC_ERR_CUDA, cudaGetErrorString(e)); break; }
-    }
-    for (int i = 0; i < kSlots; i++) {
-        cudaError_t e = cudaStreamSynchronize(ctx->slot[i].stream);
-        if (e == cudaSuccess && gw) e = cudaStreamSynchronize(ctx->gw.stream[i]);
-        ctx->slot[i].done_pending = false;
-        if (e != cudaSuccess && rc == DMC_OK) rc = fail(ctx, DMC_ERR_CUDA, cudaGetErrorString(e));
-    }
-    cudaEventDestroy(ready);
-    return rc;
+    uint64_t b0 = 0, b1 = 0;
+    void *dblob = nullptr, *dout = nullptr;
+    return stream_chunks(ctx, n_frames, chunk, ctx->gw.device >= 0, true,
+        [&](const Chunk& c) -> int {
+            Slot& sl = *c.sl;
+            b0 = offsets[c.f0]; b1 = offsets[c.f0 + c.nf];
+            if (b1 < b0) return fail(ctx, DMC_ERR_ARG, "dmc_chain_batch_jpeg: offsets must be non-decreasing");
+            TRY(jpeg_parse_group(ctx, (const uint8_t*)blob, offsets, c.f0, c.nf, b0, rows, cols, &g));
+            if (sl.hcap < g.meta_bytes) {
+                if (sl.hstage) cudaFreeHost(sl.hstage);
+                sl.hstage = nullptr; sl.hcap = 0;
+                const size_t cap = (g.meta_bytes * 2 + 65535) & ~(size_t)65535;
+                if (cudaHostAlloc(&sl.hstage, cap, cudaHostAllocDefault) != cudaSuccess) return fail(ctx, DMC_ERR_CUDA, "cudaHostAlloc (JPEG metadata staging)");
+                sl.hcap = cap;
+            }
+            jpeg_write_meta(g, sl.hstage);
+            // bitstreams and results on the device whose link carries them, everything else local
+            TRY(reserve_io(ctx, c, (size_t)(b1 - b0) + 16, host_out ? obytes * c.nf : 0, sl.buf[SB_BITS], sl.buf[SB_OUT], &dblob, &dout));
+            if (!host_out) dout = (uint8_t*)dst + obytes * c.f0;
+            TRY(reserve(ctx, sl.buf[SB_IN], fpx * c.nf));
+            TRY(reserve(ctx, sl.buf[SB_META], g.meta_bytes));
+            TRY(reserve(ctx, sl.buf[SB_SCANS], g.scratch_bytes + 16));
+            if (g.n_restart) TRY(reserve(ctx, sl.buf[SB_COEF], (size_t)c.nf * blocks * 64 * sizeof(int16_t)));
+            return DMC_OK;
+        },
+        [&](const Chunk& c) { return cudaMemcpyAsync(dblob, (const uint8_t*)blob + b0, (size_t)(b1 - b0), cudaMemcpyHostToDevice, c.copy); },
+        [&](const Chunk& c) -> int {
+            Slot& sl = *c.sl;
+            cudaError_t e = cudaMemcpyAsync(sl.buf[SB_META].p, sl.hstage, g.meta_bytes, cudaMemcpyHostToDevice, sl.stream);
+            if (e != cudaSuccess) return fail(ctx, DMC_ERR_CUDA, cudaGetErrorString(e));
+            const char* dm = (const char*)sl.buf[SB_META].p;
+            LAUNCH(ctx, launch_jpeg_decode((const uint8_t*)dblob, dm, dm + g.o_huff, dm + g.o_quant, (uint8_t*)sl.buf[SB_SCANS].p, (int16_t*)sl.buf[SB_COEF].p,
+                                           (uint8_t*)sl.buf[SB_IN].p, c.nf, g.n_restart, rows, cols, sl.stream));
+            return run_chain(ctx, sl, (const uint8_t*)sl.buf[SB_IN].p, dout, c.nf, rows, cols, p);
+        },
+        [&](const Chunk& c) { return host_out ? cudaMemcpyAsync((uint8_t*)dst + obytes * c.f0, dout, obytes * c.nf, cudaMemcpyDeviceToHost, c.copy) : cudaSuccess; });
 }
 
 int dmc_jpeg_probe(const void* stream, size_t len, int* rows, int* cols, char* err, size_t err_len) {
@@ -919,26 +938,27 @@ int dmc_jpeg_decode_gray_batch(dmc_ctx* ctx, const void* blob, const uint64_t* o
     const size_t fpx = (size_t)rows * cols, blocks = (size_t)((rows + 7) / 8) * ((cols + 7) / 8);
     const int group_max = 2048;
     JpegGroup g;
+    std::vector<char> meta;
     for (int f0 = 0; f0 < n_frames; f0 += group_max) {
         const int nf = n_frames - f0 < group_max ? n_frames - f0 : group_max;
         const uint64_t b0 = offsets[f0], b1 = offsets[f0 + nf];
         if (b1 < b0) return fail(ctx, DMC_ERR_ARG, "dmc_jpeg_decode_gray_batch: offsets must be non-decreasing");
         TRY(jpeg_parse_group(ctx, (const uint8_t*)blob, offsets, f0, nf, b0, rows, cols, &g));
-        TRY(reserve(ctx, ctx->jpeg[0], (size_t)(b1 - b0) + 16));
-        TRY(reserve(ctx, ctx->jpeg[1], g.desc.size() * sizeof(dmcjpeg::FrameDesc)));
-        TRY(reserve(ctx, ctx->jpeg[2], g.hpool.size() * sizeof(dmcjpeg::HuffTable)));
-        TRY(reserve(ctx, ctx->jpeg[3], g.qpool.size() * sizeof(dmcjpeg::QuantTable)));
-        if (g.n_restart) TRY(reserve(ctx, ctx->jpeg[4], (size_t)nf * blocks * 64 * sizeof(int16_t)));
-        TRY(reserve(ctx, ctx->jpeg[6], g.scratch_bytes + 16));
+        TRY(reserve(ctx, ctx->jpeg[JD_BITS], (size_t)(b1 - b0) + 16));
+        TRY(reserve(ctx, ctx->jpeg[JD_META], g.meta_bytes));
+        if (g.n_restart) TRY(reserve(ctx, ctx->jpeg[JD_COEF], (size_t)nf * blocks * 64 * sizeof(int16_t)));
+        TRY(reserve(ctx, ctx->jpeg[JD_SCANS], g.scratch_bytes + 16));
         uint8_t* out = (uint8_t*)dst + fpx * f0;
-        if (dst_mem == DMC_MEM_HOST) { TRY(reserve(ctx, ctx->jpeg[5], fpx * nf)); out = (uint8_t*)ctx->jpeg[5].p; }
-        CUDA_TRY(ctx, cudaMemcpyAsync(ctx->jpeg[0].p, (const uint8_t*)blob + b0, (size_t)(b1 - b0), cudaMemcpyHostToDevice, s));
-        CUDA_TRY(ctx, cudaMemcpyAsync(ctx->jpeg[1].p, g.desc.data(), g.desc.size() * sizeof(dmcjpeg::FrameDesc), cudaMemcpyHostToDevice, s));
-        CUDA_TRY(ctx, cudaMemcpyAsync(ctx->jpeg[2].p, g.hpool.data(), g.hpool.size() * sizeof(dmcjpeg::HuffTable), cudaMemcpyHostToDevice, s));
-        CUDA_TRY(ctx, cudaMemcpyAsync(ctx->jpeg[3].p, g.qpool.data(), g.qpool.size() * sizeof(dmcjpeg::QuantTable), cudaMemcpyHostToDevice, s));
-        LAUNCH(ctx, launch_jpeg_decode((const uint8_t*)ctx->jpeg[0].p, ctx->jpeg[1].p, ctx->jpeg[2].p, ctx->jpeg[3].p, (uint8_t*)ctx->jpeg[6].p, (int16_t*)ctx->jpeg[4].p, out, nf, g.n_restart, rows, cols, s));
+        if (dst_mem == DMC_MEM_HOST) { TRY(reserve(ctx, ctx->jpeg[JD_OUT], fpx * nf)); out = (uint8_t*)ctx->jpeg[JD_OUT].p; }
+        meta.resize(g.meta_bytes);
+        jpeg_write_meta(g, meta.data());
+        CUDA_TRY(ctx, cudaMemcpyAsync(ctx->jpeg[JD_BITS].p, (const uint8_t*)blob + b0, (size_t)(b1 - b0), cudaMemcpyHostToDevice, s));
+        CUDA_TRY(ctx, cudaMemcpyAsync(ctx->jpeg[JD_META].p, meta.data(), g.meta_bytes, cudaMemcpyHostToDevice, s));
+        const char* dm = (const char*)ctx->jpeg[JD_META].p;
+        LAUNCH(ctx, launch_jpeg_decode((const uint8_t*)ctx->jpeg[JD_BITS].p, dm, dm + g.o_huff, dm + g.o_quant, (uint8_t*)ctx->jpeg[JD_SCANS].p, (int16_t*)ctx->jpeg[JD_COEF].p,
+                                       out, nf, g.n_restart, rows, cols, s));
         if (dst_mem == DMC_MEM_HOST) CUDA_TRY(ctx, cudaMemcpyAsync((uint8_t*)dst + fpx * f0, out, fpx * nf, cudaMemcpyDeviceToHost, s));
-        CUDA_TRY(ctx, cudaStreamSynchronize(s));     // the pageable host vectors (desc, tables) are reused by the next group
+        CUDA_TRY(ctx, cudaStreamSynchronize(s));     // the pageable metadata block is reused by the next group
     }
     return DMC_OK;
 }
@@ -969,8 +989,7 @@ int jpeg_enc_prepare(dmc_ctx* ctx, const char* what, int rows, int cols, int qua
     CUDA_TRY(ctx, cudaSetDevice(ctx->device));
     const JpegEncLayout l = jpeg_enc_layout(rows, cols);
     const size_t per = l.coef_bytes + l.info_bytes + l.word_bytes + l.slot_bytes + 2 * (size_t)rows * cols;
-    size_t g = kEncGroupBytes / per;
-    *group = (int)(g < 1 ? 1 : (g > 2048 ? 2048 : g));
+    *group = chunk_frames(kEncGroupBytes, per, INT_MAX, 2048, false);
     dmcjpeg::EncTables t;
     dmcjpeg::make_enc_tables(quality, rows, cols, &t);
     TRY(reserve(ctx, ctx->jpeg_enc[JE_TABS], sizeof t));
@@ -1098,24 +1117,23 @@ int dmc_bwrf(dmc_ctx* ctx, const dmc_image* src, dmc_image* dst, int kw, int kh,
     if (!runs) return DMC_UNSUPPORTED;
     if (cn != 1 && cn != 3) return fail(ctx, DMC_ERR_TYPE, "binalyWeightedRangeFilter: CV_Assert(type is C1 or C3)");   // :1038 / :985
     if (dst->cvtype != src->cvtype || dst->rows != src->rows || dst->cols != src->cols) return fail(ctx, DMC_ERR_TYPE, "binalyWeightedRangeFilter: CV_Assert(src.type()==dst.type() && src.size()==dst.size())");
-    CUDA_TRY(ctx, cudaSetDevice(ctx->device));
-    Slot& sl = ctx->slot[0]; sl.stream = ctx->stream; cudaStream_t s = sl.stream;
     const void* in; void* out;
-    TRY(stage_in(ctx, src, sl.buf[0], s, &in));
-    TRY(stage_out_begin(ctx, dst, in, image_bytes(src), sl.buf[1], &out));
+    TRY(stage_op(ctx, src, dst, &in, &out));
+    const cudaStream_t s = ctx->stream;
+    Buf& ftmp = ctx->slot[0].buf[SB_FLOAT];
     const int H = src->rows, W = src->cols;
     int rc;
-    if (depth == DMC_8U) rc = range_filter_8u(ctx, (const uint8_t*)in, (uint8_t*)out, sl.buf[4], 1, H, W, cn, kw, kh, threshold, method, s);
+    if (depth == DMC_8U) rc = range_filter_8u(ctx, (const uint8_t*)in, (uint8_t*)out, ftmp, 1, H, W, cn, kw, kh, threshold, method, s);
     else {
         int lop = depth == DMC_32F ? LOAD_F32 : depth == DMC_16U ? LOAD_U16 : LOAD_S16;
         int sop = depth == DMC_32F ? STORE_F32 : depth == DMC_16U ? STORE_U16 : STORE_S16;
         if (method == DMC_SEPARABLE_KERNEL && kw <= 1) {          // SP_32f: src.copyTo(dst) and nothing else
-            if (out != in) CUDA_TRY(ctx, cudaMemcpyAsync(out, in, image_bytes(src), cudaMemcpyDeviceToDevice, s));
+            TRY(copy_unless_same(ctx, out, in, image_bytes(src), s));
             rc = DMC_OK;
         } else if (method == DMC_SEPARABLE_KERNEL && kh == 0) {  // vertical pass with height 0 copies
             RowSpan rh = make_rowspan(kw, 1);
             rc = DMC_OK; LAUNCH(ctx, launch_bwrf32f(in, out, 1, H, W, cn, rh, threshold, lop, 0.f, sop, s));
-        } else rc = range_filter_32f(ctx, in, out, sl.buf[4], 1, H, W, cn, kw, kh, threshold, method, lop, 0.f, sop, s);
+        } else rc = range_filter_32f(ctx, in, out, ftmp, 1, H, W, cn, kw, kh, threshold, method, lop, 0.f, sop, s);
     }
     if (rc != DMC_OK) { cudaStreamSynchronize(s); return rc; }
     return stage_out_end(ctx, dst, out, s);
@@ -1131,16 +1149,15 @@ int dmc_joint_bwrf(dmc_ctx* ctx, const dmc_image* src, const dmc_image* guide, d
     if (cv_depth(guide->cvtype) != DMC_8U || (gcn != 1 && gcn != 3)) return fail(ctx, DMC_ERR_TYPE, "jointBinalyWeightedRangeFilter: guide must be CV_8UC1 or CV_8UC3");
     if (guide->rows != src->rows || guide->cols != src->cols) return fail(ctx, DMC_ERR_SIZE, "jointBinalyWeightedRangeFilter: guide size != src size");
     if (dst->cvtype != src->cvtype || dst->rows != src->rows || dst->cols != src->cols) return fail(ctx, DMC_ERR_TYPE, "jointBinalyWeightedRangeFilter: dst must match src");
-    CUDA_TRY(ctx, cudaSetDevice(ctx->device));
-    Slot& sl = ctx->slot[0]; sl.stream = ctx->stream; cudaStream_t s = sl.stream;
     const void* in; const void* gd; void* out;
-    TRY(stage_in(ctx, src, sl.buf[0], s, &in));
-    TRY(stage_in(ctx, guide, sl.buf[2], s, &gd));
-    TRY(stage_out_begin(ctx, dst, in, image_bytes(src), sl.buf[1], &out));
-    if (out != sl.buf[1].p && overlaps(out, image_bytes(dst), gd, image_bytes(guide))) { TRY(reserve(ctx, sl.buf[1], image_bytes(dst))); out = sl.buf[1].p; }      // dst aliases the guide
+    TRY(stage_op(ctx, src, dst, &in, &out));
+    const cudaStream_t s = ctx->stream;
+    Buf& bout = ctx->slot[0].buf[SB_OUT];
+    TRY(stage_in(ctx, guide, ctx->slot[0].buf[SB_PING], s, &gd));
+    if (out != bout.p && overlaps(out, image_bytes(dst), gd, image_bytes(guide))) { TRY(reserve(ctx, bout, image_bytes(dst))); out = bout.p; }      // dst aliases the guide
     const int H = src->rows, W = src->cols;
     int rc = DMC_OK;
-    if (kw == 0 || kh == 0) { if (out != in) CUDA_TRY(ctx, cudaMemcpyAsync(out, in, image_bytes(src), cudaMemcpyDeviceToDevice, s)); }
+    if (kw == 0 || kh == 0) TRY(copy_unless_same(ctx, out, in, image_bytes(src), s));
     else {
         RowSpan rs = make_rowspan(kw, kh);
         int nk = launch_joint_bwrf8u((const uint8_t*)in, (const uint8_t*)gd, (uint8_t*)out, 1, H, W, gcn, rs, (int)(uint8_t)(int)threshold, s);
@@ -1155,15 +1172,12 @@ int dmc_blur_remove_minmax(dmc_ctx* ctx, const dmc_image* src, dmc_image* dst, i
     TRY(check_image(ctx, src, "src")); TRY(check_image(ctx, dst, "dst")); TRY(check_radius(ctx, r, "r"));
     const int depth = cv_depth(src->cvtype), cn = cv_cn(src->cvtype);
     if (dst->cvtype != src->cvtype || dst->rows != src->rows || dst->cols != src->cols) return fail(ctx, DMC_ERR_SIZE, "blurRemoveMinMax: dst must match src");
-    CUDA_TRY(ctx, cudaSetDevice(ctx->device));
-    Slot& sl = ctx->slot[0]; sl.stream = ctx->stream; cudaStream_t s = sl.stream;
     const void* in; void* out;
-    TRY(stage_in(ctx, src, sl.buf[0], s, &in));
-    TRY(stage_out_begin(ctx, dst, in, image_bytes(src), sl.buf[1], &out));
+    TRY(stage_op(ctx, src, dst, &in, &out));
+    const cudaStream_t s = ctx->stream;
     const bool known = depth == DMC_8U || depth == DMC_16S || depth == DMC_16U || depth == DMC_32F || depth == DMC_64F;
-    if (!known || r == 0) {        // other depths: only src.copyTo(dest) happens (:52); r == 0 is the identity
-        if (out != in) CUDA_TRY(ctx, cudaMemcpyAsync(out, in, image_bytes(src), cudaMemcpyDeviceToDevice, s));
-    } else LAUNCH(ctx, launch_minmax(in, out, 1, src->rows, src->cols, depth, cn, r, s));
+    if (!known || r == 0) TRY(copy_unless_same(ctx, out, in, image_bytes(src), s));     // other depths: only src.copyTo(dest) happens (:52); r == 0 is the identity
+    else LAUNCH(ctx, launch_minmax(in, out, 1, src->rows, src->cols, depth, cn, r, s));
     return stage_out_end(ctx, dst, out, s);
 }
 
@@ -1175,14 +1189,13 @@ static int minmax_filter(dmc_ctx* ctx, const dmc_image* src, dmc_image* dst, int
     const int t = src->cvtype;
     if (t != DMC_8U && t != DMC_16S && t != DMC_16U && t != DMC_32F) return DMC_UNSUPPORTED;    // `src.type()==CV_8U` ... :316-333
     if (dst->cvtype != t || dst->rows != src->rows || dst->cols != src->cols) return fail(ctx, DMC_ERR_SIZE, "maxFilter/minFilter: dst must match src");
-    CUDA_TRY(ctx, cudaSetDevice(ctx->device));
-    Slot& sl = ctx->slot[0]; sl.stream = ctx->stream; cudaStream_t s = sl.stream;
     const void* in; void* out;
-    TRY(stage_in(ctx, src, sl.buf[0], s, &in));
-    TRY(stage_out_begin(ctx, dst, in, image_bytes(src), sl.buf[1], &out));
+    TRY(stage_op(ctx, src, dst, &in, &out));
+    const cudaStream_t s = ctx->stream;
     if (t == DMC_32F) {
-        TRY(reserve(ctx, sl.buf[4], image_bytes(src)));
-        LAUNCH(ctx, launch_minmax_filter_f32_seeded((const float*)in, (float*)out, (float*)sl.buf[4].p, src->rows, src->cols, kw, kh, is_max, s));
+        Buf& ftmp = ctx->slot[0].buf[SB_FLOAT];
+        TRY(reserve(ctx, ftmp, image_bytes(src)));
+        LAUNCH(ctx, launch_minmax_filter_f32_seeded((const float*)in, (float*)out, (float*)ftmp.p, src->rows, src->cols, kw, kh, is_max, s));
     } else LAUNCH(ctx, launch_morph(in, out, 1, src->rows, src->cols, t, kw, kh, is_max, s));
     return stage_out_end(ctx, dst, out, s);
 }
@@ -1196,11 +1209,9 @@ int dmc_boundary_reconstruction(dmc_ctx* ctx, const dmc_image* src, dmc_image* d
     const int t = src->cvtype;
     if (t != DMC_8U && t != DMC_16S && t != DMC_16U && t != DMC_32F && t != DMC_64F) return DMC_UNSUPPORTED;   // :133-155 single channel only
     if (dst->cvtype != t || dst->rows != src->rows || dst->cols != src->cols) return fail(ctx, DMC_ERR_SIZE, "boundaryReconstructionFilter: dst must match src");
-    CUDA_TRY(ctx, cudaSetDevice(ctx->device));
-    Slot& sl = ctx->slot[0]; sl.stream = ctx->stream; cudaStream_t s = sl.stream;
     const void* in; void* out;
-    TRY(stage_in(ctx, src, sl.buf[0], s, &in));
-    TRY(stage_out_begin(ctx, dst, in, image_bytes(src), sl.buf[1], &out));
+    TRY(stage_op(ctx, src, dst, &in, &out));
+    const cudaStream_t s = ctx->stream;
     int nk = launch_brf(in, out, src->rows, src->cols, t, kw, kh, frec, color, space, s);
     if (nk == 0) return fail(ctx, DMC_ERR_ARG, "boundaryReconstructionFilter: window too large");
     TRY(after_launch(ctx, nk));
@@ -1215,11 +1226,9 @@ int dmc_minmax_boundary_reconstruction(dmc_ctx* ctx, const dmc_image* src, dmc_i
     const int t = src->cvtype;
     if (t != DMC_8U && t != DMC_16S && t != DMC_16U) return fail(ctx, DMC_ERR_TYPE, "minmaxBoundaryReconstructionFilter: single channel 8U / 16U / 16S only");
     if (dst->cvtype != t || dst->rows != src->rows || dst->cols != src->cols) return fail(ctx, DMC_ERR_SIZE, "minmaxBoundaryReconstructionFilter: dst must match src");
-    CUDA_TRY(ctx, cudaSetDevice(ctx->device));
-    Slot& sl = ctx->slot[0]; sl.stream = ctx->stream; cudaStream_t s = sl.stream;
     const void* in; void* out;
-    TRY(stage_in(ctx, src, sl.buf[0], s, &in));
-    TRY(stage_out_begin(ctx, dst, in, image_bytes(src), sl.buf[1], &out));
+    TRY(stage_op(ctx, src, dst, &in, &out));
+    const cudaStream_t s = ctx->stream;
     int nk = launch_minmax_brf(in, out, src->rows, src->cols, t, minmax_r, kw, kh, frec, color, space, s);
     if (nk == 0) return fail(ctx, DMC_ERR_ARG, "minmaxBoundaryReconstructionFilter: window too large");
     TRY(after_launch(ctx, nk));
@@ -1232,14 +1241,12 @@ int dmc_small_gaussian(dmc_ctx* ctx, const dmc_image* src, dmc_image* dst, int d
     if (src->cvtype != DMC_8U || dst->cvtype != DMC_8U) return fail(ctx, DMC_ERR_TYPE, "smallGaussianBlur: CV_8UC1 only");
     if (dst->rows != src->rows || dst->cols != src->cols) return fail(ctx, DMC_ERR_SIZE, "smallGaussianBlur: dst must match src");
     if (d < 0 || (d > 0 && (d & 1) == 0) || d / 2 > DMC_MAX_RADIUS) return fail(ctx, DMC_ERR_ARG, "smallGaussianBlur: d must be 0 or odd, <= 21");
-    CUDA_TRY(ctx, cudaSetDevice(ctx->device));
-    Slot& sl = ctx->slot[0]; sl.stream = ctx->stream; cudaStream_t s = sl.stream;
     const void* in; void* out;
-    TRY(stage_in(ctx, src, sl.buf[0], s, &in));
-    TRY(stage_out_begin(ctx, dst, in, image_bytes(src), sl.buf[1], &out));
+    TRY(stage_op(ctx, src, dst, &in, &out));
+    const cudaStream_t s = ctx->stream;
     GaussTaps t; t.rx = t.ry = 0;
     if (d > 1 && !make_gauss_taps(d, sigma, src->rows, src->cols, &t)) return fail(ctx, DMC_ERR_ARG, "smallGaussianBlur: bad kernel");
-    if (d <= 1 || (t.rx == 0 && t.ry == 0)) { if (out != in) CUDA_TRY(ctx, cudaMemcpyAsync(out, in, image_bytes(src), cudaMemcpyDeviceToDevice, s)); }
+    if (d <= 1 || (t.rx == 0 && t.ry == 0)) TRY(copy_unless_same(ctx, out, in, image_bytes(src), s));
     else LAUNCH(ctx, launch_gauss8u((const uint8_t*)in, (uint8_t*)out, 1, src->rows, src->cols, t, s));
     return stage_out_end(ctx, dst, out, s);
 }
@@ -1250,12 +1257,10 @@ int dmc_median_blur(dmc_ctx* ctx, const dmc_image* src, dmc_image* dst, int ksiz
     if (src->cvtype != DMC_8U || dst->cvtype != DMC_8U) return fail(ctx, DMC_ERR_TYPE, "medianBlur: CV_8UC1 only");
     if (dst->rows != src->rows || dst->cols != src->cols) return fail(ctx, DMC_ERR_SIZE, "medianBlur: dst must match src");
     if (ksize < 1 || (ksize & 1) == 0 || ksize / 2 > DMC_MAX_RADIUS) return fail(ctx, DMC_ERR_ARG, "medianBlur: ksize must be odd, <= 21");
-    CUDA_TRY(ctx, cudaSetDevice(ctx->device));
-    Slot& sl = ctx->slot[0]; sl.stream = ctx->stream; cudaStream_t s = sl.stream;
     const void* in; void* out;
-    TRY(stage_in(ctx, src, sl.buf[0], s, &in));
-    TRY(stage_out_begin(ctx, dst, in, image_bytes(src), sl.buf[1], &out));
-    if (ksize == 1) { if (out != in) CUDA_TRY(ctx, cudaMemcpyAsync(out, in, image_bytes(src), cudaMemcpyDeviceToDevice, s)); }
+    TRY(stage_op(ctx, src, dst, &in, &out));
+    const cudaStream_t s = ctx->stream;
+    if (ksize == 1) TRY(copy_unless_same(ctx, out, in, image_bytes(src), s));
     else LAUNCH(ctx, launch_median8u((const uint8_t*)in, (uint8_t*)out, 1, src->rows, src->cols, ksize / 2, s));
     return stage_out_end(ctx, dst, out, s);
 }
@@ -1266,13 +1271,11 @@ static int convert_op(dmc_ctx* ctx, int kind, int stype, int dtype, const dmc_im
     TRY(check_image(ctx, src, "src")); TRY(check_image(ctx, dst, "dst"));
     if (src->cvtype != stype || dst->cvtype != dtype) return fail(ctx, DMC_ERR_TYPE, "converter: wrong src/dst type");
     if (dst->rows != src->rows || dst->cols != src->cols) return fail(ctx, DMC_ERR_SIZE, "converter: dst must match src");
-    CUDA_TRY(ctx, cudaSetDevice(ctx->device));
-    Slot& sl = ctx->slot[0]; sl.stream = ctx->stream; cudaStream_t s = sl.stream;
     const void* in; void* out;
-    TRY(stage_in(ctx, src, sl.buf[0], s, &in));
+    TRY(stage_op(ctx, src, dst, &in, &out));
+    const cudaStream_t s = ctx->stream;
     // disp8U2depth32F with b != 0 leaves most of dst untouched, so dst's previous contents are staged too
-    if (kind == 0 && b != 0.f) { const void* prev; TRY(stage_in(ctx, dst, sl.buf[1], s, &prev)); out = (void*)prev; }
-    else TRY(stage_out_begin(ctx, dst, in, image_bytes(src), sl.buf[1], &out));
+    if (kind == 0 && b != 0.f) { const void* prev; TRY(stage_in(ctx, dst, ctx->slot[0].buf[SB_OUT], s, &prev)); out = (void*)prev; }
     LAUNCH(ctx, launch_convert(kind, in, out, (long)src->rows * src->cols, fb, a, b, s));
     return stage_out_end(ctx, dst, out, s);
 }
@@ -1290,12 +1293,12 @@ int dmc_fill_occlusion(dmc_ctx* ctx, dmc_image* img, int invalid_value, int disp
     CUDA_TRY(ctx, cudaSetDevice(ctx->device));
     Slot& sl = ctx->slot[0]; sl.stream = ctx->stream; cudaStream_t s = sl.stream;
     size_t row = dense_step(img), bytes = image_bytes(img);
-    TRY(reserve(ctx, sl.buf[0], bytes)); TRY(reserve(ctx, sl.buf[1], bytes));
+    TRY(reserve(ctx, sl.buf[SB_IN], bytes)); TRY(reserve(ctx, sl.buf[SB_OUT], bytes));
     cudaMemcpyKind in_kind = img->mem == DMC_MEM_HOST ? cudaMemcpyHostToDevice : cudaMemcpyDeviceToDevice;
-    CUDA_TRY(ctx, cudaMemcpy2DAsync(sl.buf[0].p, row, img->data, step_of(img), row, img->rows, in_kind, s));
-    CUDA_TRY(ctx, cudaMemcpyAsync(sl.buf[1].p, sl.buf[0].p, bytes, cudaMemcpyDeviceToDevice, s));
-    LAUNCH(ctx, launch_fill_occlusion(sl.buf[1].p, sl.buf[0].p, img->rows, img->cols, t, (double)invalid_value, disp_or_depth == DMC_FILL_DEPTH, s));
-    return stage_out_end(ctx, img, sl.buf[1].p, s);
+    CUDA_TRY(ctx, cudaMemcpy2DAsync(sl.buf[SB_IN].p, row, img->data, step_of(img), row, img->rows, in_kind, s));
+    CUDA_TRY(ctx, cudaMemcpyAsync(sl.buf[SB_OUT].p, sl.buf[SB_IN].p, bytes, cudaMemcpyDeviceToDevice, s));
+    LAUNCH(ctx, launch_fill_occlusion(sl.buf[SB_OUT].p, sl.buf[SB_IN].p, img->rows, img->cols, t, (double)invalid_value, disp_or_depth == DMC_FILL_DEPTH, s));
+    return stage_out_end(ctx, img, sl.buf[SB_OUT].p, s);
 }
 
 int dmc_transpose(dmc_ctx* ctx, const dmc_image* src, dmc_image* dst) {
@@ -1303,11 +1306,9 @@ int dmc_transpose(dmc_ctx* ctx, const dmc_image* src, dmc_image* dst) {
     TRY(check_image(ctx, src, "src")); TRY(check_image(ctx, dst, "dst"));
     if (cv_cn(src->cvtype) != 1) return fail(ctx, DMC_ERR_TYPE, "transpose: single-channel images only");
     if (dst->cvtype != src->cvtype || dst->rows != src->cols || dst->cols != src->rows) return fail(ctx, DMC_ERR_SIZE, "transpose: dst must be cols x rows of the same type");
-    CUDA_TRY(ctx, cudaSetDevice(ctx->device));
-    Slot& sl = ctx->slot[0]; sl.stream = ctx->stream; cudaStream_t s = sl.stream;
     const void* in; void* out;
-    TRY(stage_in(ctx, src, sl.buf[0], s, &in));
-    TRY(stage_out_begin(ctx, dst, in, image_bytes(src), sl.buf[1], &out));
+    TRY(stage_op(ctx, src, dst, &in, &out));
+    const cudaStream_t s = ctx->stream;
     LAUNCH(ctx, launch_transpose(in, out, src->rows, src->cols, (int)elem_size(src->cvtype), s));
     return stage_out_end(ctx, dst, out, s);
 }
@@ -1320,8 +1321,9 @@ int dmc_reproject_xyz(dmc_ctx* ctx, const dmc_image* depth, dmc_image* xyz, doub
     const int H = depth->rows, W = depth->cols;
     if (xyz->cvtype != DMC_MAKETYPE(DMC_32F, 3) || (size_t)xyz->rows * xyz->cols != (size_t)H * W) return fail(ctx, DMC_ERR_TYPE, "reprojectXYZ: xyz must be 32FC3 with rows*cols == depth.total()");
     if (xyz->step && xyz->step != dense_step(xyz)) return fail(ctx, DMC_ERR_SIZE, "reprojectXYZ: xyz must be dense");
-    CUDA_TRY(ctx, cudaSetDevice(ctx->device));
-    Slot& sl = ctx->slot[0]; sl.stream = ctx->stream; cudaStream_t s = sl.stream;
+    const void* in; void* out;
+    TRY(stage_op(ctx, depth, xyz, &in, &out));
+    const cudaStream_t s = ctx->stream;
     const float fxinv = (float)(1.0 / f), fyinv = (float)(1.0 / f);
     const float cw = (W - 1) * 0.5f, ch = (H - 1) * 0.5f;
     if (!ctx->xtab || ctx->xtab_w != W || ctx->xtab_f != f) {       // x = (-cw)*fxinv; x += fxinv per column (:469, :478)
@@ -1333,9 +1335,6 @@ int dmc_reproject_xyz(dmc_ctx* ctx, const dmc_image* depth, dmc_image* xyz, doub
         CUDA_TRY(ctx, cudaMemcpy(ctx->xtab, tab.data(), W * sizeof(float), cudaMemcpyHostToDevice));
         ctx->xtab_w = W; ctx->xtab_f = f;
     }
-    const void* in; void* out;
-    TRY(stage_in(ctx, depth, sl.buf[0], s, &in));
-    TRY(stage_out_begin(ctx, xyz, in, image_bytes(depth), sl.buf[1], &out));
     LAUNCH(ctx, launch_reproject(in, (float*)out, ctx->xtab, H, W, t, fyinv, ch, s));
     return stage_out_end(ctx, xyz, out, s);
 }
@@ -1355,11 +1354,9 @@ int dmc_project_points(dmc_ctx* ctx, const dmc_image* xyz, const double* R, cons
     if (xyz->cvtype != DMC_MAKETYPE(DMC_32F, 3) || pt->cvtype != DMC_MAKETYPE(DMC_32F, 2)) return fail(ctx, DMC_ERR_TYPE, "projectPointsSimple: xyz must be 32FC3, pt 32FC2");
     const long n = (long)xyz->rows * xyz->cols;
     if ((long)pt->rows * pt->cols != n || (xyz->step && xyz->step != dense_step(xyz)) || (pt->step && pt->step != dense_step(pt))) return fail(ctx, DMC_ERR_SIZE, "projectPointsSimple: pt must hold one point per xyz entry, both dense");
-    CUDA_TRY(ctx, cudaSetDevice(ctx->device));
-    Slot& sl = ctx->slot[0]; sl.stream = ctx->stream; cudaStream_t s = sl.stream;
     const void* in; void* out;
-    TRY(stage_in(ctx, xyz, sl.buf[0], s, &in));
-    TRY(stage_out_begin(ctx, pt, in, image_bytes(xyz), sl.buf[1], &out));
+    TRY(stage_op(ctx, xyz, pt, &in, &out));
+    const cudaStream_t s = ctx->stream;
     float kr[9], tt[3]; camera_floats(R, t, K, kr, tt);
     LAUNCH(ctx, launch_project_points((const float*)in, (float*)out, n, kr, tt, flags & DMC_RENDER_EXACT_DIVIDE, s));
     return stage_out_end(ctx, pt, out, s);
@@ -1380,11 +1377,11 @@ int dmc_project_image_from_xyz(dmc_ctx* ctx, const dmc_image* image, dmc_image* 
     CUDA_TRY(ctx, cudaSetDevice(ctx->device));
     Slot& sl = ctx->slot[0]; sl.stream = ctx->stream; cudaStream_t s = sl.stream;
     const void *d_img, *d_xyz; void *d_dest, *d_depth = nullptr, *d_pt = nullptr;
-    TRY(stage_in(ctx, image, sl.buf[0], s, &d_img));
-    TRY(stage_in(ctx, xyz, sl.buf[2], s, &d_xyz));
-    TRY(stage_out_begin(ctx, dest, d_img, image_bytes(image), sl.buf[1], &d_dest));
-    if (depth) { if (depth->mem == DMC_MEM_DEVICE && step_of(depth) == dense_step(depth)) d_depth = depth->data; else { TRY(reserve(ctx, sl.buf[3], (size_t)n * 4)); d_depth = sl.buf[3].p; } }
-    if (pt && pt->mem == DMC_MEM_DEVICE) d_pt = pt->data; else { TRY(reserve(ctx, sl.buf[4], (size_t)n * 8)); d_pt = sl.buf[4].p; }
+    TRY(stage_in(ctx, image, sl.buf[SB_IN], s, &d_img));
+    TRY(stage_in(ctx, xyz, sl.buf[SB_PING], s, &d_xyz));
+    TRY(stage_out_begin(ctx, dest, d_img, image_bytes(image), sl.buf[SB_OUT], &d_dest));
+    if (depth) { if (depth->mem == DMC_MEM_DEVICE && step_of(depth) == dense_step(depth)) d_depth = depth->data; else { TRY(reserve(ctx, sl.buf[SB_PONG], (size_t)n * 4)); d_depth = sl.buf[SB_PONG].p; } }
+    if (pt && pt->mem == DMC_MEM_DEVICE) d_pt = pt->data; else { TRY(reserve(ctx, sl.buf[SB_FLOAT], (size_t)n * 8)); d_pt = sl.buf[SB_FLOAT].p; }
     TRY(reserve(ctx, ctx->render[0], render_scratch_bytes(H, W)));
     TRY(reserve(ctx, ctx->render[1], 64));
     if (!ctx->render_flag) CUDA_TRY(ctx, cudaHostAlloc((void**)&ctx->render_flag, 64, cudaHostAllocDefault));
@@ -1407,12 +1404,12 @@ int dmc_fill_small_hole(dmc_ctx* ctx, const dmc_image* src, dmc_image* dst) {
     CUDA_TRY(ctx, cudaSetDevice(ctx->device));
     Slot& sl = ctx->slot[0]; sl.stream = ctx->stream; cudaStream_t s = sl.stream;
     const void* in; void* out;
-    TRY(stage_in(ctx, src, sl.buf[0], s, &in));
+    TRY(stage_in(ctx, src, sl.buf[SB_IN], s, &in));
     const bool same = dst->data == src->data;
     if (!same && dst->mem == DMC_MEM_DEVICE && step_of(dst) == dense_step(dst) && !overlaps(dst->data, image_bytes(dst), in, image_bytes(src))) out = dst->data;   // only holes are written: dest keeps the rest
     else {          // staged: dest's own previous content (or, in place, a copy of src -- `src.copyTo(src_)` :189-193) is the canvas
-        TRY(reserve(ctx, sl.buf[1], image_bytes(dst)));
-        out = sl.buf[1].p;
+        TRY(reserve(ctx, sl.buf[SB_OUT], image_bytes(dst)));
+        out = sl.buf[SB_OUT].p;
         const size_t row = dense_step(dst);
         if (same) CUDA_TRY(ctx, cudaMemcpyAsync(out, in, image_bytes(src), cudaMemcpyDeviceToDevice, s));
         else CUDA_TRY(ctx, cudaMemcpy2DAsync(out, row, dst->data, step_of(dst), row, dst->rows, dst->mem == DMC_MEM_HOST ? cudaMemcpyHostToDevice : cudaMemcpyDeviceToDevice, s));
@@ -1429,11 +1426,9 @@ int dmc_split_bgr_line_interleave(dmc_ctx* ctx, const dmc_image* src, dmc_image*
     const int depth = cv_depth(src->cvtype);
     if (cv_cn(src->cvtype) != 3 || (depth != DMC_8U && depth != DMC_32F)) return DMC_UNSUPPORTED;      // other types: nothing happens (:169-176)
     if (dst->cvtype != depth || dst->rows != 3 * src->rows || dst->cols != src->cols) return fail(ctx, DMC_ERR_SIZE, "splitBGRLineInterleave: dest must be single channel, 3*rows x cols");
-    CUDA_TRY(ctx, cudaSetDevice(ctx->device));
-    Slot& sl = ctx->slot[0]; sl.stream = ctx->stream; cudaStream_t s = sl.stream;
     const void* in; void* out;
-    TRY(stage_in(ctx, src, sl.buf[0], s, &in));
-    TRY(stage_out_begin(ctx, dst, in, image_bytes(src), sl.buf[1], &out));
+    TRY(stage_op(ctx, src, dst, &in, &out));
+    const cudaStream_t s = ctx->stream;
     LAUNCH(ctx, launch_split_line_interleave(in, out, src->rows, src->cols, (int)depth_size(depth), s));
     return stage_out_end(ctx, dst, out, s);
 }

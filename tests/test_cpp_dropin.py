@@ -9,16 +9,18 @@ ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 CPP = os.path.join(ROOT, "tests", "cpp")
 
 
-def _build():
+def _build(out_dir):
+    """Builds the drop-in program into out_dir: the source tree may be read-only."""
     import __graft_entry__ as g
     g.build()
-    subprocess.check_call(["make", "-C", CPP, "test_dropin"], stdout=subprocess.DEVNULL)
-    return os.path.join(CPP, "test_dropin")
+    exe = str(out_dir / "test_dropin")
+    subprocess.check_call(["make", "-C", CPP, "OUT=" + exe], stdout=subprocess.DEVNULL)
+    return exe
 
 
-def test_dropin_headers_compile_and_link():
+def test_dropin_headers_compile_and_link(tmp_path):
     """CPU-side: the reference's declarations compile against our headers and link against libdmc_b200.so."""
-    exe = _build()
+    exe = _build(tmp_path)
     assert os.path.exists(exe)
     hdr = open(os.path.join(ROOT, "include", "filter.h")).read()
     ref_decls = [   # PostFilterSetForDepthCoding/filter.h:12-45, verbatim
@@ -55,8 +57,8 @@ def test_dropin_headers_compile_and_link():
 
 
 @pytest.mark.gpu
-def test_dropin_call_sites_bit_exact():
-    exe = _build()
+def test_dropin_call_sites_bit_exact(tmp_path):
+    exe = _build(tmp_path)
     res = subprocess.run([exe, os.path.join(ROOT, "oracle", "libdmc_oracle.so")], capture_output=True, text=True, cwd=ROOT, timeout=600)
     print(res.stdout[-3000:], res.stderr[-2000:])
     assert res.returncode == 0 and "ALL OK" in res.stdout

@@ -104,6 +104,64 @@ def test_streamed_bitstream_to_chain_1080p(dmc, port):
     assert_bits_equal(out2, out, "second streamed call")
 
 
+def _streams_1080p(n):
+    """n 1080p q80 streams cycling over three degraded synthetic frames -> (streams, index of each frame's base)"""
+    from oracle.oracle_py import synth_disp, degrade_blocks
+    base = [enc(degrade_blocks(synth_disp(1080, 1920, 2000 + k, shift=(3 * k, k)), k), 80) for k in range(3)]
+    return [base[f % 3] for f in range(n)], base
+
+
+def test_streamed_error_in_a_later_chunk(dmc, port, monkeypatch):
+    """dmc_chain_batch_jpeg stops at a malformed stream found while earlier chunks are still in flight, drains its slots
+    and leaves the context usable.  DMC_CHUNK_MB=1 makes every 1080p frame a chunk of its own, so the slots come round
+    three times in a 12-frame batch."""
+    from depthmapcompression_b200.filters import chain_params
+    from depthmapcompression_b200 import capi
+    monkeypatch.setenv("DMC_CHUNK_MB", "1")
+    H, W, N = 1080, 1920, 12
+    streams, base = _streams_1080p(N)
+    p8 = chain_params(capi.CHAIN_DISP8U, 2, 1, 3, 5, 10)
+    ctx = dmc.Context(0)
+    bad = list(streams); bad[9] = b"not a jpeg at all"
+    with pytest.raises(dmc.DmcError, match="JPEG frame 9"):
+        ctx.chain_batch_jpeg(bad, H, W, np.zeros((N, H, W), np.uint8), p8)
+    out = np.zeros((N, H, W), np.uint8)
+    ctx.chain_batch_jpeg(streams, H, W, out, p8)
+    want = [port.post_filter_set(cv2.imdecode(s, 0), 2, 1, 3, 5, 10) for s in base]
+    for i in range(N):
+        assert_bits_equal(out[i], want[i % 3], "call after the failed one, frame %d" % i)
+    ctx.close()
+
+
+def test_streamed_jpeg_through_gateway(dmc, monkeypatch):
+    """dmc_chain_batch_jpeg with dmc_set_gateway: the bitstreams and results travel over another device's link, the kernels
+    reach its buffers over NVLink.  Results equal the own-link ones, on repeated calls (buffers and events reused) and for a
+    device destination.  Needs two GPUs with peer access (skipped on a one-GPU box)."""
+    import torch
+    from depthmapcompression_b200.filters import chain_params
+    from depthmapcompression_b200 import capi
+    if capi.lib.dmc_device_count() < 2:
+        pytest.skip("needs two GPUs")
+    monkeypatch.setenv("DMC_CHUNK_MB", "1")
+    H, W, N = 1080, 1920, 12
+    streams, _ = _streams_1080p(N)
+    p8 = chain_params(capi.CHAIN_DISP8U, 2, 1, 3, 5, 10)
+    ctx = dmc.Context(0)
+    own = np.zeros((N, H, W), np.uint8); ctx.chain_batch_jpeg(streams, H, W, own, p8)
+    d_own = torch.zeros((N, H, W), dtype=torch.uint8, device="cuda:0")
+    ctx.chain_batch_jpeg(streams, H, W, d_own.data_ptr(), p8, device=True); ctx.synchronize()
+    ctx.set_gateway(1)
+    assert ctx.gateway == 1
+    for rep in range(2):
+        routed = np.zeros_like(own); ctx.chain_batch_jpeg(streams, H, W, routed, p8)
+        assert_bits_equal(routed, own, "through the gateway, repetition %d" % rep)
+    d_routed = torch.zeros_like(d_own)
+    ctx.chain_batch_jpeg(streams, H, W, d_routed.data_ptr(), p8, device=True); ctx.synchronize()
+    assert_bits_equal(d_routed.cpu().numpy(), d_own.cpu().numpy(), "through the gateway, device destination")
+    ctx.set_gateway(-1)
+    ctx.close()
+
+
 def test_probe_and_hostile_streams(dmc):
     img = make_image(np.random.RandomState(3), 24, 40)
     good = bytes(enc(img, 75))
