@@ -51,7 +51,8 @@ struct dmc_ctx {
     struct Gateway { int device = -1; cudaStream_t stream[kSlots] = {}; Buf in[kSlots], out[kSlots]; cudaEvent_t ev_in[kSlots] = {}, ev_out[kSlots] = {}, ev_done[kSlots] = {}; } gw;
     Buf render[2]; int* render_flag = nullptr;      // point-cloud render: attempt lists etc., device flag; pinned host flag
     Buf jpeg[JD_COUNT];
-    Buf jpeg_enc[9];             // JPEG encode: tables, staged frames, coefficients, block records, scan words, slots, lengths + offsets, staged output, decoder tables + descriptors
+    Buf jpeg_enc[11];            // JPEG encode: tables, staged frames, coefficients, block records, scan words, slots, lengths + offsets, staged output, decoder tables + descriptors,
+                                 // optimised-table scratch, per-frame decoder Huffman tables
     // optional per-stage CUDA-event timing of the chain (bench.py's live roofline measurement)
     int lanes = 1;               // concurrent frame groups in the device-resident batch path
     int profile_mask = 0;
@@ -831,24 +832,24 @@ namespace {
 // single H2D copy brings everything the kernels need besides the bitstreams themselves.  The block is
 // [FrameDesc...][HuffTable...][QuantTable...] with 16-byte aligned parts; o_huff and o_quant are the tables' offsets.
 struct JpegGroup {
-    std::vector<dmcjpeg::FrameDesc> desc; std::vector<dmcjpeg::QuantTable> qpool; std::vector<dmcjpeg::HuffTable> hpool;
+    std::vector<dmcjpeg::FrameDesc> desc; JpegTablePools pools;
     size_t scratch_bytes = 0; int n_restart = 0;
     size_t o_huff = 0, o_quant = 0, meta_bytes = 0;
 };
 
 void jpeg_write_meta(const JpegGroup& g, void* block) {
     memcpy(block, g.desc.data(), g.desc.size() * sizeof(dmcjpeg::FrameDesc));
-    memcpy((char*)block + g.o_huff, g.hpool.data(), g.hpool.size() * sizeof(dmcjpeg::HuffTable));
-    memcpy((char*)block + g.o_quant, g.qpool.data(), g.qpool.size() * sizeof(dmcjpeg::QuantTable));
+    memcpy((char*)block + g.o_huff, g.pools.h.items.data(), g.pools.h.items.size() * sizeof(dmcjpeg::HuffTable));
+    memcpy((char*)block + g.o_quant, g.pools.q.items.data(), g.pools.q.items.size() * sizeof(dmcjpeg::QuantTable));
 }
 
 // Parses streams [f0, f0 + nf) of the blob; scan offsets are relative to `blob_base` (the first byte that will be copied).
 int jpeg_parse_group(dmc_ctx* ctx, const uint8_t* blob, const uint64_t* offsets, int f0, int nf, uint64_t blob_base, int rows, int cols, JpegGroup* g) {
-    g->desc.resize(nf); g->qpool.clear(); g->hpool.clear(); g->scratch_bytes = 0; g->n_restart = 0;
+    g->desc.resize(nf); g->pools.q.clear(); g->pools.h.clear(); g->scratch_bytes = 0; g->n_restart = 0;
     for (int i = 0; i < nf; i++) {
         const uint64_t o = offsets[f0 + i], e = offsets[f0 + i + 1];
         if (e < o || o < blob_base) return fail(ctx, DMC_ERR_ARG, "JPEG batch: offsets must be non-decreasing");
-        std::string why = jpeg_parse_frame(blob + o, e - o, o - blob_base, rows, cols, g->qpool, g->hpool, &g->desc[i]);
+        std::string why = jpeg_parse_frame(blob + o, e - o, o - blob_base, rows, cols, g->pools, &g->desc[i]);
         if (!why.empty()) return fail(ctx, DMC_ERR_TYPE, "JPEG frame " + std::to_string(f0 + i) + ": " + why);
         if (g->desc[i].scan_end - g->desc[i].scan_offset >= (1ull << 28)) return fail(ctx, DMC_ERR_SIZE, "JPEG frame " + std::to_string(f0 + i) + ": scan larger than 256 MB");
         g->desc[i].ds_offset = g->scratch_bytes;
@@ -856,8 +857,8 @@ int jpeg_parse_group(dmc_ctx* ctx, const uint8_t* blob, const uint64_t* offsets,
         if (g->desc[i].restart_interval) g->n_restart++;
     }
     g->o_huff = (g->desc.size() * sizeof(dmcjpeg::FrameDesc) + 15) & ~(size_t)15;
-    g->o_quant = (g->o_huff + g->hpool.size() * sizeof(dmcjpeg::HuffTable) + 15) & ~(size_t)15;
-    g->meta_bytes = g->o_quant + g->qpool.size() * sizeof(dmcjpeg::QuantTable);
+    g->o_quant = (g->o_huff + g->pools.h.items.size() * sizeof(dmcjpeg::HuffTable) + 15) & ~(size_t)15;
+    g->meta_bytes = g->o_quant + g->pools.q.items.size() * sizeof(dmcjpeg::QuantTable);
     return DMC_OK;
 }
 
@@ -964,13 +965,16 @@ int dmc_jpeg_decode_gray_batch(dmc_ctx* ctx, const void* blob, const uint64_t* o
 }
 
 // ---- JPEG encode (SURVEY.md 8f-5) ------------------------------------------------------------------------------------
-int dmc_jpeg_encode_bound(int rows, int cols, uint64_t* bytes) {
+int dmc_jpeg_encode_bound_ex(int rows, int cols, int flags, uint64_t* bytes) {
     if (!bytes) return fail(nullptr, DMC_ERR_ARG, "dmc_jpeg_encode_bound: null bytes");
+    if (flags & ~DMC_JPEG_OPTIMIZE_HUFFMAN) return fail(nullptr, DMC_ERR_ARG, "JPEG encode: unknown flags " + std::to_string(flags));
     if (rows <= 0 || cols <= 0 || rows > 65535 || cols > 65535) return fail(nullptr, DMC_ERR_SIZE, "JPEG encode: frame size must be 1..65535 x 1..65535");
-    *bytes = dmcjpeg::jpeg_encode_bound(rows, cols);
+    *bytes = dmcjpeg::jpeg_encode_bound(rows, cols, (flags & DMC_JPEG_OPTIMIZE_HUFFMAN) != 0);
     if (*bytes > dmcjpeg::kEncMaxStreamBytes) return fail(nullptr, DMC_ERR_SIZE, "JPEG encode: the worst-case stream of a " + std::to_string(rows) + " x " + std::to_string(cols) + " frame exceeds 256 MB");
     return DMC_OK;
 }
+
+int dmc_jpeg_encode_bound(int rows, int cols, uint64_t* bytes) { return dmc_jpeg_encode_bound_ex(rows, cols, 0, bytes); }
 
 namespace {
 
@@ -978,17 +982,18 @@ namespace {
 // frame needs about 26 MB (slot 13.4 MB, scan words 6.7 MB, coefficients 4.1 MB, staged frame).
 constexpr size_t kEncGroupBytes = (size_t)4 << 30;
 
-enum { JE_TABS, JE_SRC, JE_COEF, JE_INFO, JE_WORDS, JE_SLOTS, JE_LENS, JE_OUT, JE_DEC };
+enum { JE_TABS, JE_SRC, JE_COEF, JE_INFO, JE_WORDS, JE_SLOTS, JE_LENS, JE_OUT, JE_DEC, JE_OPT, JE_HUFF };
 
 // Checks the arguments shared by the encode entry points, uploads the encoder tables and returns the group size.
-int jpeg_enc_prepare(dmc_ctx* ctx, const char* what, int rows, int cols, int quality, int mem_a, int mem_b, int* group) {
+int jpeg_enc_prepare(dmc_ctx* ctx, const char* what, int rows, int cols, int quality, int flags, int mem_a, int mem_b, int* group) {
     if (quality < 0 || quality > 100) return fail(ctx, DMC_ERR_ARG, std::string(what) + ": quality must be in 0..100");
     if ((mem_a != DMC_MEM_HOST && mem_a != DMC_MEM_DEVICE) || (mem_b != DMC_MEM_HOST && mem_b != DMC_MEM_DEVICE)) return fail(ctx, DMC_ERR_ARG, std::string(what) + ": bad mem");
+    if (flags & ~DMC_JPEG_OPTIMIZE_HUFFMAN) return fail(ctx, DMC_ERR_ARG, std::string(what) + ": unknown flags " + std::to_string(flags));
     uint64_t bound;
-    if (dmc_jpeg_encode_bound(rows, cols, &bound) != DMC_OK) return fail(ctx, DMC_ERR_SIZE, std::string(what) + ": " + g_err);
+    if (dmc_jpeg_encode_bound_ex(rows, cols, flags, &bound) != DMC_OK) return fail(ctx, DMC_ERR_SIZE, std::string(what) + ": " + g_err);
     CUDA_TRY(ctx, cudaSetDevice(ctx->device));
-    const JpegEncLayout l = jpeg_enc_layout(rows, cols);
-    const size_t per = l.coef_bytes + l.info_bytes + l.word_bytes + l.slot_bytes + 2 * (size_t)rows * cols;
+    const JpegEncLayout l = jpeg_enc_layout(rows, cols, flags != 0);
+    const size_t per = l.coef_bytes + l.info_bytes + l.word_bytes + l.slot_bytes + 2 * (size_t)rows * cols + (flags ? l.opt_bytes + 2 * sizeof(dmcjpeg::HuffTable) : 0);
     *group = chunk_frames(kEncGroupBytes, per, INT_MAX, 2048, false);
     dmcjpeg::EncTables t;
     dmcjpeg::make_enc_tables(quality, rows, cols, &t);
@@ -998,11 +1003,12 @@ int jpeg_enc_prepare(dmc_ctx* ctx, const char* what, int rows, int cols, int qua
     return DMC_OK;
 }
 
-// Encodes frames [f0, f0 + nf) of src into the slots (lengths in JE_LENS); desc: also write the decoder's FrameDescs there.
-int jpeg_enc_group(dmc_ctx* ctx, const uint8_t* src, int src_mem, int f0, int nf, int rows, int cols, void* desc) {
+// Encodes frames [f0, f0 + nf) of src into the slots (lengths in JE_LENS); desc: also write the decoder's FrameDescs there
+// (with optimised tables their Huffman tables go to JE_HUFF, a pair per frame).
+int jpeg_enc_group(dmc_ctx* ctx, const uint8_t* src, int src_mem, int f0, int nf, int rows, int cols, bool optimize, void* desc) {
     cudaStream_t s = ctx->stream;
     const size_t fpx = (size_t)rows * cols;
-    const JpegEncLayout l = jpeg_enc_layout(rows, cols);
+    const JpegEncLayout l = jpeg_enc_layout(rows, cols, optimize);
     const uint8_t* dsrc = src + fpx * f0;
     if (src_mem == DMC_MEM_HOST) {
         TRY(reserve(ctx, ctx->jpeg_enc[JE_SRC], fpx * nf));
@@ -1014,8 +1020,14 @@ int jpeg_enc_group(dmc_ctx* ctx, const uint8_t* src, int src_mem, int f0, int nf
     TRY(reserve(ctx, ctx->jpeg_enc[JE_WORDS], l.word_bytes * nf));
     TRY(reserve(ctx, ctx->jpeg_enc[JE_SLOTS], l.slot_bytes * nf));
     TRY(reserve(ctx, ctx->jpeg_enc[JE_LENS], (size_t)nf * (sizeof(uint32_t) + sizeof(uint64_t)) + 16));
+    void *opt = nullptr, *huff = nullptr;
+    if (optimize) {
+        TRY(reserve(ctx, ctx->jpeg_enc[JE_OPT], l.opt_bytes * nf));
+        opt = ctx->jpeg_enc[JE_OPT].p;
+        if (desc) { TRY(reserve(ctx, ctx->jpeg_enc[JE_HUFF], 2 * sizeof(dmcjpeg::HuffTable) * nf)); huff = ctx->jpeg_enc[JE_HUFF].p; }
+    }
     LAUNCH(ctx, launch_jpeg_encode(dsrc, ctx->jpeg_enc[JE_TABS].p, ctx->jpeg_enc[JE_COEF].p, ctx->jpeg_enc[JE_INFO].p, ctx->jpeg_enc[JE_WORDS].p,
-                                   (uint8_t*)ctx->jpeg_enc[JE_SLOTS].p, (uint32_t*)ctx->jpeg_enc[JE_LENS].p, desc, nf, rows, cols, s));
+                                   (uint8_t*)ctx->jpeg_enc[JE_SLOTS].p, (uint32_t*)ctx->jpeg_enc[JE_LENS].p, desc, nf, rows, cols, s, opt, huff));
     return DMC_OK;
 }
 
@@ -1026,19 +1038,20 @@ uint64_t* enc_offs(dmc_ctx* ctx, int nf) { return (uint64_t*)((char*)ctx->jpeg_e
 // Streams are encoded group by group into per-frame slots on the device; the host reads the group's lengths back, places
 // the streams back to back after the previous group's and a gather kernel copies them there (through a device staging
 // buffer and one copy for a host blob).
-int dmc_jpeg_encode_gray_batch(dmc_ctx* ctx, const void* src, int src_mem, int n_frames, int rows, int cols, int quality, void* blob, int blob_mem,
-                               uint64_t capacity, uint64_t* offsets) {
+int dmc_jpeg_encode_gray_batch_ex(dmc_ctx* ctx, const void* src, int src_mem, int n_frames, int rows, int cols, int quality, int flags, void* blob, int blob_mem,
+                                  uint64_t capacity, uint64_t* offsets) {
     if (!ctx) return fail(nullptr, DMC_ERR_ARG, "null context");
     if (!offsets || n_frames < 0 || (n_frames > 0 && (!src || !blob))) return fail(ctx, DMC_ERR_SIZE, "dmc_jpeg_encode_gray_batch: bad arguments");
     int group;
-    TRY(jpeg_enc_prepare(ctx, "dmc_jpeg_encode_gray_batch", rows, cols, quality, src_mem, blob_mem, &group));
+    TRY(jpeg_enc_prepare(ctx, "dmc_jpeg_encode_gray_batch", rows, cols, quality, flags, src_mem, blob_mem, &group));
     offsets[0] = 0;
     cudaStream_t s = ctx->stream;
-    const JpegEncLayout l = jpeg_enc_layout(rows, cols);
+    const bool optimize = (flags & DMC_JPEG_OPTIMIZE_HUFFMAN) != 0;
+    const JpegEncLayout l = jpeg_enc_layout(rows, cols, optimize);
     std::vector<uint32_t> lens; std::vector<uint64_t> offs;
     for (int f0 = 0; f0 < n_frames; f0 += group) {
         const int nf = n_frames - f0 < group ? n_frames - f0 : group;
-        TRY(jpeg_enc_group(ctx, (const uint8_t*)src, src_mem, f0, nf, rows, cols, nullptr));
+        TRY(jpeg_enc_group(ctx, (const uint8_t*)src, src_mem, f0, nf, rows, cols, optimize, nullptr));
         lens.resize(nf); offs.resize(nf);
         CUDA_TRY(ctx, cudaMemcpyAsync(lens.data(), ctx->jpeg_enc[JE_LENS].p, nf * sizeof(uint32_t), cudaMemcpyDeviceToHost, s));
         CUDA_TRY(ctx, cudaStreamSynchronize(s));
@@ -1060,14 +1073,21 @@ int dmc_jpeg_encode_gray_batch(dmc_ctx* ctx, const void* src, int src_mem, int n
     return DMC_OK;
 }
 
+int dmc_jpeg_encode_gray_batch(dmc_ctx* ctx, const void* src, int src_mem, int n_frames, int rows, int cols, int quality, void* blob, int blob_mem,
+                               uint64_t capacity, uint64_t* offsets) {
+    return dmc_jpeg_encode_gray_batch_ex(ctx, src, src_mem, n_frames, rows, cols, quality, 0, blob, blob_mem, capacity, offsets);
+}
+
 // The reference's degradeJPEG on the device: encode into the slots, then decode every slot in place with the decoder of
-// dmc_jpeg_decode_gray_batch.  The decoder's tables come from parsing the encoder's header once; the encoder writes each
-// frame's FrameDesc itself, so the streams never leave the device.
-int dmc_jpeg_degrade_gray_batch(dmc_ctx* ctx, const void* src, void* dst, int n_frames, int rows, int cols, int quality, int mem, uint64_t* bytes) {
+// dmc_jpeg_decode_gray_batch.  The decoder's tables come from parsing the encoder's header once (with optimised tables,
+// the Huffman tables are every frame's own, derived by the encoder's table kernel); the encoder writes each frame's
+// FrameDesc itself, so the streams never leave the device.
+int dmc_jpeg_degrade_gray_batch_ex(dmc_ctx* ctx, const void* src, void* dst, int n_frames, int rows, int cols, int quality, int flags, int mem, uint64_t* bytes) {
     if (!ctx) return fail(nullptr, DMC_ERR_ARG, "null context");
     if (n_frames < 0 || (n_frames > 0 && (!src || !dst))) return fail(ctx, DMC_ERR_SIZE, "dmc_jpeg_degrade_gray_batch: bad arguments");
     int group;
-    TRY(jpeg_enc_prepare(ctx, "dmc_jpeg_degrade_gray_batch", rows, cols, quality, mem, mem, &group));
+    TRY(jpeg_enc_prepare(ctx, "dmc_jpeg_degrade_gray_batch", rows, cols, quality, flags, mem, mem, &group));
+    const bool optimize = (flags & DMC_JPEG_OPTIMIZE_HUFFMAN) != 0;
     if (n_frames == 0) return DMC_OK;
     cudaStream_t s = ctx->stream;
     const size_t fpx = (size_t)rows * cols;
@@ -1086,11 +1106,11 @@ int dmc_jpeg_degrade_gray_batch(dmc_ctx* ctx, const void* src, void* dst, int n_
     std::vector<uint32_t> lens;
     for (int f0 = 0; f0 < n_frames; f0 += group) {
         const int nf = n_frames - f0 < group ? n_frames - f0 : group;
-        TRY(jpeg_enc_group(ctx, (const uint8_t*)src, mem, f0, nf, rows, cols, dm + o_desc));
+        TRY(jpeg_enc_group(ctx, (const uint8_t*)src, mem, f0, nf, rows, cols, optimize, dm + o_desc));
         uint8_t* out = (uint8_t*)dst + fpx * f0;
         if (mem == DMC_MEM_HOST) { TRY(reserve(ctx, ctx->jpeg_enc[JE_OUT], fpx * nf)); out = (uint8_t*)ctx->jpeg_enc[JE_OUT].p; }
-        LAUNCH(ctx, launch_jpeg_decode((const uint8_t*)ctx->jpeg_enc[JE_SLOTS].p, dm + o_desc, dm, dm + o_q, (uint8_t*)ctx->jpeg_enc[JE_WORDS].p, nullptr, out,
-                                       nf, 0, rows, cols, s));
+        LAUNCH(ctx, launch_jpeg_decode((const uint8_t*)ctx->jpeg_enc[JE_SLOTS].p, dm + o_desc, optimize ? ctx->jpeg_enc[JE_HUFF].p : dm, dm + o_q,
+                                       (uint8_t*)ctx->jpeg_enc[JE_WORDS].p, nullptr, out, nf, 0, rows, cols, s));
         if (mem == DMC_MEM_HOST) CUDA_TRY(ctx, cudaMemcpyAsync((uint8_t*)dst + fpx * f0, out, fpx * nf, cudaMemcpyDeviceToHost, s));
         if (bytes) {
             lens.resize(nf);
@@ -1100,6 +1120,10 @@ int dmc_jpeg_degrade_gray_batch(dmc_ctx* ctx, const void* src, void* dst, int n_
         if (bytes) for (int i = 0; i < nf; i++) bytes[f0 + i] = lens[i];
     }
     return DMC_OK;
+}
+
+int dmc_jpeg_degrade_gray_batch(dmc_ctx* ctx, const void* src, void* dst, int n_frames, int rows, int cols, int quality, int mem, uint64_t* bytes) {
+    return dmc_jpeg_degrade_gray_batch_ex(ctx, src, dst, n_frames, rows, cols, quality, 0, mem, bytes);
 }
 
 // ---- stand-alone operators ---------------------------------------------------------------------------------------

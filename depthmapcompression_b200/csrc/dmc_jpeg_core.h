@@ -10,6 +10,7 @@
 // by one from libjpeg-turbo, tools/nvjpeg_probe.py).
 #pragma once
 #include <stdint.h>
+#include <string.h>
 
 #if defined(__CUDACC__)
 #define DMC_HD __host__ __device__ __forceinline__
@@ -86,6 +87,42 @@ DMC_HD void br_fill(BitReader& br) {
 }
 DMC_HD uint32_t br_peek(BitReader& br, int n) { return (uint32_t)(br.acc >> (64 - n)); }     // n in 1..32, after br_fill
 DMC_HD void br_skip(BitReader& br, int n) { br.acc <<= n; br.nbits -= n; }
+
+// Derives the decoding tables of one DHT entry (bits[1..16], vals[nvals]); used by the host parser and by the encoder's
+// table kernel, which derives the decoder tables of the optimised tables it builds.  Returns false for tables libjpeg's
+// jpeg_make_d_derived_tbl rejects with JERR_BAD_HUFF_TABLE: more than 256 symbols, or code lengths that do not form a
+// prefix code (a code of length l must be < 2^l; an over-subscribed BITS array would otherwise index past look[]).
+DMC_HD bool derive_table(const uint8_t bits[17], const uint8_t* vals, int nvals, HuffTable* t) {
+    memset(t, 0, sizeof *t);
+    int huffsize[257], huffcode[257], p = 0;
+    for (int l = 1; l <= 16; l++) {
+        if (p + bits[l] > 256) return false;
+        for (int i = 0; i < bits[l]; i++) huffsize[p++] = l;
+    }
+    if (p != nvals) return false;
+    huffsize[p] = 0;
+    int code = 0, si = huffsize[0]; p = 0;
+    while (huffsize[p]) {
+        while (huffsize[p] == si) huffcode[p++] = code++;
+        if (code > (1 << si)) return false;                   // jdhuff.c: "code is now 1 more than the last code used for codelength si"
+        code <<= 1; si++;
+    }
+    p = 0;
+    for (int l = 1; l <= 16; l++) {
+        if (bits[l]) { t->valoffset[l] = p - huffcode[p]; p += bits[l]; t->maxcode[l] = huffcode[p - 1]; }
+        else t->maxcode[l] = -1;
+    }
+    t->maxcode[17] = 0xFFFFF;
+    for (int i = 0; i < nvals; i++) t->huffval[i] = vals[i];
+    p = 0;
+    for (int l = 1; l <= 9; l++)
+        for (int i = 0; i < bits[l]; i++, p++) {
+            const int lookbits = huffcode[p] << (9 - l), span = 1 << (9 - l);
+            if (lookbits + span > 512) return false;          // (cannot happen once the prefix-code check passed; belt and braces)
+            for (int c = 0; c < span; c++) t->look[lookbits + c] = (uint16_t)((l << 8) | vals[p]);
+        }
+    return true;
+}
 
 DMC_HD int huff_decode(BitReader& br, const HuffTable& t) {
     br_fill(br);

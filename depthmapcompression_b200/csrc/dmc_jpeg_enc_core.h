@@ -5,7 +5,7 @@
 //
 // The target is byte equality with cv2.imencode(img, [IMWRITE_JPEG_QUALITY, q]) of an 8UC1 image (libjpeg-turbo with
 // OpenCV's settings: JFIF 1.1 APP0, one DQT, the standard luminance Huffman tables of ITU T.81 K.3 / K.5, no restart
-// intervals, no optimised tables).  That encoder is fully determined by these rules:
+// intervals).  That encoder is fully determined by these rules:
 //   * quality: q clamped to [1, 100]; scale = q < 50 ? 5000 / q : 200 - 2q; entry = clamp((std * scale + 50) / 100, 1, 255)
 //     (jcparam.c jpeg_quality_scaling / jpeg_add_quant_table with force_baseline);
 //   * the last column and row are replicated to a multiple of 8 (jccoefct.c / jcsample.c edge expansion);
@@ -14,6 +14,9 @@
 //   * Huffman coding in raster block order, one DC predictor starting at 0, 0xF0 (ZRL) before a non-zero coefficient
 //     preceded by 16 or more zeros, 0x00 (EOB) after the last non-zero one; MSB-first bits, 0x00 stuffed after every 0xFF,
 //     the last byte padded with 1-bits (jchuff.c).
+// With optimised Huffman tables (cv2.IMWRITE_JPEG_OPTIMIZE = 1, libjpeg's optimize_coding) the stream is the same except
+// for the two DHT segments: each frame gets the tables jchuff.c's jpeg_gen_optimal_table builds from its own DC category
+// and AC symbol counts (see the optimised-table section below).
 #pragma once
 #include "dmc_jpeg_core.h"
 #include <string.h>
@@ -26,6 +29,11 @@ constexpr int kEncHeaderBytes = 328;                       // SOI + APP0 + DQT +
 // non-zero coefficients they replace, so a block never needs more.
 constexpr uint32_t kEncMaxBlockBits = (9 + 11) + 63 * (16 + 10);
 constexpr uint64_t kEncMaxStreamBytes = 1ull << 28;       // the decoder's scan limit
+// With optimised tables: a Huffman code over at most 12 DC categories + the reserved symbol 256 (13 leaves) is at most
+// 12 bits long, and AC codes (ZRL, EOB included) are limited to 16 bits as before, so a block takes at most
+// (12 + 11) + 63 * (16 + 10) bits; ZRL and EOB, at most 16 bits each, still cost less than the non-zero coefficients they
+// replace.  The header is at most as long as the standard one (12 DC + 162 AC symbols).
+constexpr uint32_t kEncMaxBlockBitsOpt = (12 + 11) + 63 * (16 + 10);
 
 struct EncTables {
     uint32_t dc[16];          // (code length << 16) | code of DC category s; s <= 11
@@ -35,13 +43,24 @@ struct EncTables {
     uint8_t header[kEncHeaderBytes];
 };
 
+// A frame's own Huffman coding in optimised mode (written by the table kernel): code tables as in EncTables, and the
+// frame's header of header_bytes = 154 + (DC symbols) + (AC symbols) bytes.
+struct EncFrameCode {
+    uint32_t dc[16];
+    uint32_t ac[256];
+    uint32_t header_bytes;
+    uint8_t header[kEncHeaderBytes];
+};
+constexpr int kEncHeaderDhtAt = 20 + 69 + 13;             // the DHT segments follow SOI + APP0, DQT and SOF0
+constexpr int kEncSosBytes = 10;
+
 // One block after the transform.  nz: bit k set iff zigzag coefficient k (1..63) is non-zero.
 struct EncBlock { uint64_t nz; uint32_t ac_bits; int32_t dc; };
 
 // Worst-case stream size of a rows x cols frame: header, EOI, and every scan byte followed by a stuffed zero.
-inline uint64_t jpeg_encode_bound(int rows, int cols) {
+inline uint64_t jpeg_encode_bound(int rows, int cols, bool optimize = false) {
     const uint64_t blocks = (uint64_t)((rows + 7) / 8) * (uint64_t)((cols + 7) / 8);
-    return (uint64_t)kEncHeaderBytes + 2 + 2 * ((blocks * kEncMaxBlockBits + 7) / 8);
+    return (uint64_t)kEncHeaderBytes + 2 + 2 * ((blocks * (optimize ? kEncMaxBlockBitsOpt : kEncMaxBlockBits) + 7) / 8);
 }
 
 // ---- tables and header (host) -----------------------------------------------------------------------------------------
@@ -214,10 +233,135 @@ DMC_HD uint32_t block_ac_bits(const int16_t* zz, const uint32_t* ac) {
     return bits;
 }
 
+// The Huffman symbols of the AC part of one block as emit_block emits them: add(symbol, count) for every run/size
+// symbol, ZRL (0xF0) and EOB (0x00).  zz is indexed with constants only, so a register array stays in registers.
+template <class Add>
+DMC_HD void block_ac_symbols(const int16_t* zz, Add add) {
+    int last = 0;
+#pragma unroll
+    for (int k = 1; k < 64; k++) {
+        const int v = zz[k];
+        if (v != 0) {
+            const int r = k - last - 1, s = bit_length((uint32_t)(v < 0 ? -v : v));
+            if (r >= 16) add(0xF0, r >> 4);
+            add(((r & 15) << 4) | s, 1);
+            last = k;
+        }
+    }
+    if (last < 63) add(0x00, 1);
+}
+
+// block_ac_bits from the non-zero mask, reading only the non-zero coefficients zz(k).
+template <class Coef>
+DMC_HD uint32_t block_ac_bits_sparse(uint64_t nz, Coef zz, const uint32_t* ac) {
+    uint32_t bits = 0; int last = 0;
+    while (nz) {
+#if defined(__CUDA_ARCH__)
+        const int k = __ffsll((long long)nz) - 1;
+#else
+        const int k = __builtin_ctzll(nz);
+#endif
+        nz &= nz - 1;
+        const int r = k - last - 1, v = zz(k), s = bit_length((uint32_t)(v < 0 ? -v : v));
+        bits += (uint32_t)(r >> 4) * code_len(ac[0xF0]) + code_len(ac[((r & 15) << 4) | s]) + (uint32_t)s;
+        last = k;
+    }
+    if (last < 63) bits += code_len(ac[0x00]);
+    return bits;
+}
+
 // Bits of the DC part: code of the category of `diff` + the category's value bits.
 DMC_HD uint32_t block_dc_bits(int diff, const uint32_t* dc) {
     const int s = bit_length((uint32_t)(diff < 0 ? -diff : diff));
     return code_len(dc[s]) + (uint32_t)s;
+}
+
+// ---- optimised Huffman tables ----------------------------------------------------------------------------------------
+// jchuff.c's jpeg_gen_optimal_table, restated for one warp.  The serial original, with freq[256] = 1 reserving the
+// all-ones code:
+//   repeat: c1 = the symbol of the smallest non-zero freq, c2 = that of the next smallest (c2 != c1), both searches
+//           taking the LARGER symbol on ties; stop when there is no c2; freq[c1] += freq[c2], freq[c2] = 0; codesize++
+//           for every symbol of c1's tree and of c2's tree (walked through the `others` chains), c2's tree joins c1's.
+//   bits[l] = number of symbols with codesize l; lengths over 16 are folded back (opt_fold); the reserved symbol is
+//   taken from the longest length; HUFFVAL lists the symbols 0..255 by codesize, then by value.
+// Here lane i owns the symbols i + 32 k (k < 9; symbol 256 is lane 0's k = 8).  The non-zero frequencies are exactly
+// the roots of the trees, so a symbol's tree is named by its root: set[] starts as the symbol itself, and a merge
+// increments codesize for the symbols of sets c1 and c2 and renames set c2 to c1 -- the increments of the chain walks.
+// The searches combine the lanes' opt_lane_min with a warp min of the frequency, then a warp max of the symbol among
+// the lanes holding that minimum.  Total counts stay below 2^26 (at most 64 symbols per block and 2^28 / 1661 * 8
+// blocks), far from jchuff.c's 10^9 search sentinel, and a code length needs a total of at least Fibonacci(length + 2),
+// so lengths stay below 40 < kOptMaxLen.
+constexpr int kOptPer = 9, kOptMaxLen = 64;
+struct OptLane { uint32_t fr[kOptPer]; uint16_t set[kOptPer], cs[kOptPer]; };
+
+// hist: counts of symbols 0 .. nsym-1 (nsym <= 256)
+DMC_HD void opt_lane_init(OptLane& L, const uint32_t* hist, int nsym, int lane) {
+#pragma unroll
+    for (int k = 0; k < kOptPer; k++) {
+        const int s = lane + 32 * k;
+        L.fr[k] = s < nsym ? hist[s] : (s == 256 ? 1u : 0u);
+        L.set[k] = (uint16_t)s; L.cs[k] = 0;
+    }
+}
+
+// The lane's smallest non-zero frequency among its symbols other than excl, the larger symbol on ties (ascending k):
+// *f = 0xFFFFFFFF and *s = -1 when there is none.
+DMC_HD void opt_lane_min(const OptLane& L, int lane, int excl, uint32_t* f, int* s) {
+    uint32_t bf = 0xFFFFFFFFu; int bs = -1;
+#pragma unroll
+    for (int k = 0; k < kOptPer; k++) {
+        const int sym = lane + 32 * k;
+        if (L.fr[k] != 0u && sym != excl && L.fr[k] <= bf) { bf = L.fr[k]; bs = sym; }
+    }
+    *f = bf; *s = bs;
+}
+
+// Merges tree c2 (frequency f2) into tree c1.
+DMC_HD void opt_lane_merge(OptLane& L, int lane, int c1, int c2, uint32_t f2) {
+#pragma unroll
+    for (int k = 0; k < kOptPer; k++) {
+        const int sym = lane + 32 * k;
+        if (sym == c1) L.fr[k] += f2;
+        if (sym == c2) L.fr[k] = 0u;
+        if (L.set[k] == c1 || L.set[k] == c2) { L.cs[k]++; L.set[k] = (uint16_t)c1; }
+    }
+}
+
+// cnt[l] (l <= kOptMaxLen): symbols with codesize l, the reserved one included.  Folds lengths over 16 back exactly as
+// jchuff.c, removes the reserved symbol from the longest length and returns BITS (bits[l - 1] = codes of length l) and
+// the number of symbols.  cnt is clobbered.
+DMC_HD int opt_fold(uint32_t* cnt, uint8_t bits[16]) {
+    int i;
+    for (i = kOptMaxLen; i > 16; i--)
+        while (cnt[i] > 0) {
+            int j = i - 2;
+            while (cnt[j] == 0) j--;
+            cnt[i] -= 2; cnt[i - 1]++; cnt[j + 1] += 2; cnt[j]--;
+        }
+    while (cnt[i] == 0) i--;
+    cnt[i]--;
+    int n = 0;
+    for (int l = 1; l <= 16; l++) { bits[l - 1] = (uint8_t)cnt[l]; n += (int)cnt[l]; }
+    return n;
+}
+
+// (length << 16) | code of the symbol at HUFFVAL position p: make_code_table's canonical assignment.
+DMC_HD uint32_t opt_code(const uint8_t bits[16], int p) {
+    uint32_t code = 0; int pos = 0;
+    for (int l = 1; l <= 16; l++) {
+        if (p < pos + bits[l - 1]) return ((uint32_t)l << 16) | (code + (uint32_t)(p - pos));
+        code = (code + bits[l - 1]) << 1; pos += bits[l - 1];
+    }
+    return 0;
+}
+
+// One DHT segment (table class tc: 0 DC, 1 AC; table 0) at h; returns its length, 21 + n.
+DMC_HD int opt_write_dht(uint8_t* h, int tc, const uint8_t bits[16], const uint8_t* vals, int n) {
+    const int len = 19 + n;
+    h[0] = 0xFF; h[1] = 0xC4; h[2] = (uint8_t)(len >> 8); h[3] = (uint8_t)len; h[4] = (uint8_t)(tc << 4);
+    for (int l = 0; l < 16; l++) h[5 + l] = bits[l];
+    for (int i = 0; i < n; i++) h[21 + i] = vals[i];
+    return 21 + n;
 }
 
 // ---- bit packing ------------------------------------------------------------------------------------------------------

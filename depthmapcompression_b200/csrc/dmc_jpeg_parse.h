@@ -1,11 +1,12 @@
-// dmc_jpeg_parse.h -- host-side marker parsing of baseline grayscale JPEG streams (DQT / SOF0 / DHT / DRI / SOS), Huffman
-// table derivation and validation.  Host only; shared by dmc_jpeg.cu and by the CPU emulation harness of the parallel
-// decoder (tests/cpp/jpeg_emul.cpp).  Reference counterpart: libjpeg's jdmarker.c / jdhuff.c as reached through
-// cv::imdecode(buf, 0) (main.cpp:284, :521) and jpeg_decode() (jpegTurboDemo.cpp:217-271).
+// dmc_jpeg_parse.h -- host-side marker parsing of baseline grayscale JPEG streams (DQT / SOF0 / DHT / DRI / SOS), table
+// validation and de-duplication (the derivation itself, derive_table, is in dmc_jpeg_core.h).  Host only; shared by
+// dmc_jpeg.cu and by the CPU emulation harness of the parallel decoder (tests/cpp/jpeg_emul.cpp).  Reference
+// counterpart: libjpeg's jdmarker.c / jdhuff.c as reached through cv::imdecode(buf, 0) (main.cpp:284, :521) and jpeg_decode() (jpegTurboDemo.cpp:217-271).
 #pragma once
 #include "dmc_jpeg_core.h"
 #include <string.h>
 #include <string>
+#include <unordered_map>
 #include <vector>
 
 namespace dmc {
@@ -13,50 +14,46 @@ namespace dmc {
 using namespace dmcjpeg;
 
 // ---- host: marker parsing ----------------------------------------------------------------------------------------
-// Derives the decoding tables of one DHT entry.  Returns false for tables libjpeg's jpeg_make_d_derived_tbl rejects with
-// JERR_BAD_HUFF_TABLE: more than 256 symbols, or code lengths that do not form a prefix code (a code of length l must be
-// < 2^l; an over-subscribed BITS array would otherwise index past look[]).
-static inline bool derive_table(const uint8_t bits[17], const uint8_t* vals, int nvals, HuffTable* t) {
-    memset(t, 0, sizeof *t);
-    int huffsize[257], huffcode[257], p = 0;
-    for (int l = 1; l <= 16; l++) {
-        if (p + bits[l] > 256) return false;
-        for (int i = 0; i < bits[l]; i++) huffsize[p++] = l;
+// De-duplicated table pool: the distinct tables in first-occurrence order, found again by a hash of their bytes (equal
+// hashes are confirmed with memcmp), so that interning is linear in the number of tables -- a batch of streams with
+// optimised Huffman tables brings two distinct tables per frame.
+template <class T> struct TablePool {
+    std::vector<T> items;
+    std::unordered_multimap<uint64_t, int> index;
+    static uint64_t hash(const T& v) {
+        static_assert(sizeof(T) % 8 == 0, "tables are hashed as 64-bit words");
+        uint64_t w[sizeof(T) / 8], h = 0x9E3779B97F4A7C15ull;
+        memcpy(w, &v, sizeof w);
+        for (uint64_t x : w) { h ^= x; h *= 0xFF51AFD7ED558CCDull; h ^= h >> 32; }
+        return h;
     }
-    if (p != nvals) return false;
-    huffsize[p] = 0;
-    int code = 0, si = huffsize[0]; p = 0;
-    while (huffsize[p]) {
-        while (huffsize[p] == si) huffcode[p++] = code++;
-        if (code > (1 << si)) return false;                   // jdhuff.c: "code is now 1 more than the last code used for codelength si"
-        code <<= 1; si++;
+    int find(const T& v, uint64_t h) const {
+        auto r = index.equal_range(h);
+        for (auto it = r.first; it != r.second; ++it) if (memcmp(&items[it->second], &v, sizeof(T)) == 0) return it->second;
+        return -1;
     }
-    p = 0;
-    for (int l = 1; l <= 16; l++) {
-        if (bits[l]) { t->valoffset[l] = p - huffcode[p]; p += bits[l]; t->maxcode[l] = huffcode[p - 1]; }
-        else t->maxcode[l] = -1;
+    int intern(const T& v) {
+        const uint64_t h = hash(v);
+        const int i = find(v, h);
+        if (i >= 0) return i;
+        items.push_back(v);
+        index.emplace(h, (int)items.size() - 1);
+        return (int)items.size() - 1;
     }
-    t->maxcode[17] = 0xFFFFF;
-    for (int i = 0; i < nvals; i++) t->huffval[i] = vals[i];
-    p = 0;
-    for (int l = 1; l <= 9; l++)
-        for (int i = 0; i < bits[l]; i++, p++) {
-            const int lookbits = huffcode[p] << (9 - l), span = 1 << (9 - l);
-            if (lookbits + span > 512) return false;          // (cannot happen once the prefix-code check passed; belt and braces)
-            for (int c = 0; c < span; c++) t->look[lookbits + c] = (uint16_t)((l << 8) | vals[p]);
-        }
-    return true;
-}
-
-template <class T> static inline int intern(std::vector<T>& pool, const T& v) {
-    for (size_t i = 0; i < pool.size(); i++) if (memcmp(&pool[i], &v, sizeof(T)) == 0) return (int)i;
-    pool.push_back(v); return (int)pool.size() - 1;
-}
+    void assign(const std::vector<T>& v) {         // takes v as the pool; equal entries resolve to the first of them
+        clear();
+        items = v;
+        for (size_t i = 0; i < items.size(); i++) { const uint64_t h = hash(items[i]); if (find(items[i], h) < 0) index.emplace(h, (int)i); }
+    }
+    void clear() { items.clear(); index.clear(); }
+};
+struct JpegTablePools { TablePool<QuantTable> q; TablePool<HuffTable> h; };
 
 // Parses one stream [p, p+len).  Returns an empty string on success, else the reason it is not supported.
 // rows < 0: any frame size is accepted (reported through out_rows / out_cols).
+// The frame's tables are interned into `pools` (FrameDesc::qt / dc / ac index pools.q.items / pools.h.items).
 inline std::string jpeg_parse_frame(const uint8_t* p, uint64_t len, uint64_t blob_offset, int rows, int cols,
-                             std::vector<QuantTable>& qpool, std::vector<HuffTable>& hpool, FrameDesc* d, int* out_rows = nullptr, int* out_cols = nullptr) {
+                                    JpegTablePools& pools, FrameDesc* d, int* out_rows = nullptr, int* out_cols = nullptr) {
     QuantTable qt[4]; bool have_q[4] = {false, false, false, false};
     HuffTable dc[4], ac[4]; bool have_dc[4] = {false, false, false, false}, have_ac[4] = {false, false, false, false};
     int comp_tq = -1, restart = 0; bool have_sof = false;
@@ -119,13 +116,23 @@ inline std::string jpeg_parse_frame(const uint8_t* p, uint64_t len, uint64_t blo
             int td = s[2] >> 4, ta = s[2] & 15;
             if (td > 3 || ta > 3 || comp_tq < 0 || comp_tq > 3 || !have_dc[td] || !have_ac[ta] || !have_q[comp_tq]) return "scan refers to a missing table";
             d->scan_offset = blob_offset + i + 2 + seg; d->scan_end = blob_offset + len; d->restart_interval = restart;
-            d->qt = intern(qpool, qt[comp_tq]);
-            d->dc = intern(hpool, dc[td]); d->ac = intern(hpool, ac[ta]);
+            d->qt = pools.q.intern(qt[comp_tq]);
+            d->dc = pools.h.intern(dc[td]); d->ac = pools.h.intern(ac[ta]);
             return "";
         }
         i += 2 + seg;
     }
     return "no SOS marker";
+}
+
+// The same with plain vectors as the pools (tables already in them are found again, the first of equal ones first).
+inline std::string jpeg_parse_frame(const uint8_t* p, uint64_t len, uint64_t blob_offset, int rows, int cols,
+                                    std::vector<QuantTable>& qpool, std::vector<HuffTable>& hpool, FrameDesc* d, int* out_rows = nullptr, int* out_cols = nullptr) {
+    JpegTablePools pools;
+    pools.q.assign(qpool); pools.h.assign(hpool);
+    std::string why = jpeg_parse_frame(p, len, blob_offset, rows, cols, pools, d, out_rows, out_cols);
+    qpool.swap(pools.q.items); hpool.swap(pools.h.items);
+    return why;
 }
 
 }  // namespace dmc

@@ -82,12 +82,15 @@ int launch_jpeg_decode(const uint8_t* blob, const void* desc, const void* hts, c
                        int n, int n_restart, int H, int W, cudaStream_t s);
 // Baseline grayscale JPEG encoding (dmc_jpeg_enc.cu).  Per-frame scratch of a rows x cols frame: int16 coefficients, block
 // records, packed scan words (reused by the decoder as de-stuffing scratch) and the slot the frame's stream is written to.
-struct JpegEncLayout { size_t blocks, coef_bytes, info_bytes, word_bytes, slot_bytes; };
-JpegEncLayout jpeg_enc_layout(int rows, int cols);
+// optimize: optimised Huffman tables, which take opt_bytes more per frame (symbol counts, the frame's code tables and header).
+struct JpegEncLayout { size_t blocks, coef_bytes, info_bytes, word_bytes, slot_bytes, opt_bytes; };
+JpegEncLayout jpeg_enc_layout(int rows, int cols, bool optimize = false);
 // n frames of src -> one stream per slot (slots + f * slot_bytes), its length in lens[f]; with desc != nullptr also the
 // FrameDesc that decodes slot f in place (scan_offset / scan_end relative to `slots`, ds_offset relative to `words`).
+// opt != nullptr (n x opt_bytes of a layout with optimize): optimised Huffman tables, every frame its own; the FrameDescs
+// then refer to the HuffTable pair huff[2 f], huff[2 f + 1], which the encoder writes when huff != nullptr.
 int launch_jpeg_encode(const uint8_t* src, const void* tabs, void* coefs, void* info, void* words, uint8_t* slots, uint32_t* lens, void* desc,
-                       int n, int H, int W, cudaStream_t s);
+                       int n, int H, int W, cudaStream_t s, void* opt = nullptr, void* huff = nullptr);
 // copies stream f (lens[f] bytes of slot f) to dst + offs[f]; max_len >= every lens[f]
 int launch_jpeg_enc_gather(const uint8_t* slots, size_t slot_bytes, const uint32_t* lens, const uint64_t* offs, uint8_t* dst, int n, uint64_t max_len, cudaStream_t s);
 }

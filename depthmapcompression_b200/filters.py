@@ -216,11 +216,15 @@ def jpegDecodeGrayBatch(streams, rows, cols, dst=None, ctx=None):
     return dst
 
 
-def jpegEncodeBound(rows, cols):
-    """dmc_jpeg_encode_bound (host only): worst-case bytes of one rows x cols stream; raises DmcError for sizes the encoder
-    refuses (outside 1..65535, or a bound above 256 MB)."""
+def _jpeg_flags(optimize):
+    return capi.JPEG_OPTIMIZE_HUFFMAN if optimize else 0
+
+
+def jpegEncodeBound(rows, cols, optimize=False):
+    """dmc_jpeg_encode_bound_ex (host only): worst-case bytes of one rows x cols stream (optimize: with optimised Huffman
+    tables); raises DmcError for sizes the encoder refuses (outside 1..65535, or a bound above 256 MB)."""
     b = C.c_uint64()
-    rc = lib.dmc_jpeg_encode_bound(int(rows), int(cols), C.byref(b))
+    rc = lib.dmc_jpeg_encode_bound_ex(int(rows), int(cols), _jpeg_flags(optimize), C.byref(b))
     if rc != capi.DMC_OK:
         raise DmcError(rc, (lib.dmc_last_error(None) or b"").decode())
     return int(b.value)
@@ -238,9 +242,10 @@ def _frames(frames):
     return a.ctypes.data, n, rows, cols, MEM_HOST, a
 
 
-def jpegEncodeGrayBatch(frames, quality, ctx=None, blob=None):
+def jpegEncodeGrayBatch(frames, quality, ctx=None, blob=None, optimize=False):
     """Baseline JPEG encode of 8-bit frames on the GPU, byte-identical to cv2.imencode(".jpg", f, [IMWRITE_JPEG_QUALITY,
-    quality]) of each frame.  frames: uint8 numpy [n, rows, cols] (or one [rows, cols] frame), or (device pointer, n, rows,
+    quality]) of each frame; with optimize=True every frame gets its own optimised Huffman tables, byte-identical to
+    cv2.imencode(".jpg", f, [IMWRITE_JPEG_QUALITY, quality, IMWRITE_JPEG_OPTIMIZE, 1]).  frames: uint8 numpy [n, rows, cols] (or one [rows, cols] frame), or (device pointer, n, rows,
     cols).  Returns (blob, offsets) in the layout of pack_streams: stream i is blob[offsets[i]:offsets[i+1]], ready for
     jpegDecodeGrayBatch and Context.chain_batch_jpeg.  blob=None: a new host array; blob=(device pointer, capacity): the
     streams go to device memory and (pointer, offsets) is returned."""
@@ -248,22 +253,23 @@ def jpegEncodeGrayBatch(frames, quality, ctx=None, blob=None):
     sp, n, rows, cols, smem, keep = _frames(frames)
     offsets = np.zeros(n + 1, np.uint64)
     if blob is None:
-        cap = n * jpegEncodeBound(rows, cols)
+        cap = n * jpegEncodeBound(rows, cols, optimize)
         host = np.empty(cap, np.uint8)          # pages the streams never reach are never touched
         bp, bmem = host.ctypes.data, MEM_HOST
     else:
         bp, cap = int(blob[0]), int(blob[1])
         bmem = MEM_DEVICE
-    ctx.check(lib.dmc_jpeg_encode_gray_batch(ctx.h, C.c_void_p(sp), smem, n, rows, cols, int(quality), C.c_void_p(bp), bmem, cap,
-                                             offsets.ctypes.data_as(C.POINTER(C.c_uint64))))
+    ctx.check(lib.dmc_jpeg_encode_gray_batch_ex(ctx.h, C.c_void_p(sp), smem, n, rows, cols, int(quality), _jpeg_flags(optimize), C.c_void_p(bp), bmem,
+                                                cap, offsets.ctypes.data_as(C.POINTER(C.c_uint64))))
     if blob is None:
         return host[:int(offsets[-1])].copy(), offsets
     return bp, offsets
 
 
-def degradeJPEG(frames, quality, dst=None, ctx=None):
+def degradeJPEG(frames, quality, dst=None, ctx=None, optimize=False):
     """The reference's degradeJPEG on the device: decoded = cv2.imdecode(cv2.imencode(f, q), 0) for every frame, and the
-    stream sizes in bytes.  frames: uint8 numpy [n, rows, cols] (or one [rows, cols] frame; nbytes is then an int), or
+    stream sizes in bytes (optimize=True: the sizes of the streams with optimised Huffman tables; the decoded frames are
+    the same).  frames: uint8 numpy [n, rows, cols] (or one [rows, cols] frame; nbytes is then an int), or
     (device pointer, n, rows, cols) with dst a device pointer.  Returns (decoded, nbytes)."""
     ctx = ctx or default_context()
     sp, n, rows, cols, mem, a = _frames(frames)
@@ -276,8 +282,8 @@ def degradeJPEG(frames, quality, dst=None, ctx=None):
             dst = np.empty(a.shape, np.uint8)
         dp = dst.ctypes.data
     nbytes = np.zeros(n, np.uint64)
-    ctx.check(lib.dmc_jpeg_degrade_gray_batch(ctx.h, C.c_void_p(sp), C.c_void_p(dp), n, rows, cols, int(quality), mem,
-                                              nbytes.ctypes.data_as(C.POINTER(C.c_uint64))))
+    ctx.check(lib.dmc_jpeg_degrade_gray_batch_ex(ctx.h, C.c_void_p(sp), C.c_void_p(dp), n, rows, cols, int(quality), _jpeg_flags(optimize), mem,
+                                                 nbytes.ctypes.data_as(C.POINTER(C.c_uint64))))
     if a is not None and a.ndim == 2:
         return dst, int(nbytes[0])
     return dst, nbytes

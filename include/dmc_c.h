@@ -196,11 +196,21 @@ int dmc_jpeg_probe(const void* stream, size_t len, int* rows, int* cols, char* e
 /* ---- encode (SURVEY.md 8f-5) ----------------------------------------------------------------------------------- */
 /* Baseline JPEG encoding of 8UC1 frames, byte-identical to cv::imencode(".jpg", img, {IMWRITE_JPEG_QUALITY, quality}) with
  * libjpeg-turbo (the encoder behind the reference's degradeJPEG): standard luminance tables scaled by quality, islow FDCT,
- * no restart intervals, no optimised Huffman tables.
+ * no restart intervals, the standard Huffman tables of ITU T.81 K.3 / K.5.  The _ex entry points take `flags`:
+ *   0                          the calls without _ex, same bytes;
+ *   DMC_JPEG_OPTIMIZE_HUFFMAN  every frame gets its own optimal Huffman tables, built from its own symbol counts as
+ *                              libjpeg's optimize_coding builds them: byte-identical to cv::imencode(".jpg", img,
+ *                              {IMWRITE_JPEG_QUALITY, quality, IMWRITE_JPEG_OPTIMIZE, 1}).  The same decoded pixels
+ *                              in fewer bytes (the header's two DHT segments and the scan differ).
+ * Any other flag bit is DMC_ERR_ARG.
  *
  * Host only, needs no GPU: the worst-case stream size of one rows x cols frame.  DMC_ERR_SIZE for sizes outside
  * 1..65535 and for frames whose bound exceeds 256 MB (the decoder's scan limit; *bytes still holds the bound). */
+enum { DMC_JPEG_OPTIMIZE_HUFFMAN = 1 };   /* cv::IMWRITE_JPEG_OPTIMIZE = 1 */
 int dmc_jpeg_encode_bound(int rows, int cols, uint64_t* bytes);
+/* The bound of a stream encoded with `flags` (with DMC_JPEG_OPTIMIZE_HUFFMAN a little larger: 1661 instead of 1658 bits
+ * per 8x8 block). */
+int dmc_jpeg_encode_bound_ex(int rows, int cols, int flags, uint64_t* bytes);
 /* src: n_frames dense rows x cols frames (src_mem: host or device).  The streams are written back to back into blob
  * (blob_mem: host or device); offsets (host, n_frames + 1 entries) receives their layout -- stream i occupies
  * [offsets[i], offsets[i+1]) -- which dmc_jpeg_decode_gray_batch and dmc_chain_batch_jpeg take as it is.  quality in
@@ -209,12 +219,19 @@ int dmc_jpeg_encode_bound(int rows, int cols, uint64_t* bytes);
  * always suffices.  Returns when offsets and blob are valid. */
 int dmc_jpeg_encode_gray_batch(dmc_ctx* ctx, const void* src, int src_mem, int n_frames, int rows, int cols, int quality,
                                void* blob, int blob_mem, uint64_t capacity, uint64_t* offsets);
+/* The same with flags; n_frames x dmc_jpeg_encode_bound_ex(rows, cols, flags) always suffices. */
+int dmc_jpeg_encode_gray_batch_ex(dmc_ctx* ctx, const void* src, int src_mem, int n_frames, int rows, int cols, int quality, int flags,
+                                  void* blob, int blob_mem, uint64_t capacity, uint64_t* offsets);
 /* The reference's degradeJPEG for a batch, entirely on the device: dst = cv::imdecode(cv::imencode(src, quality), 0) for
  * every frame (src, dst: n_frames dense 8UC1 frames in `mem`; they may alias).  bytes (host, n_frames entries, may be NULL)
  * receives the stream sizes, i.e. the bitrate.  The streams themselves never leave the device.  Returns when dst and
  * bytes are valid. */
 int dmc_jpeg_degrade_gray_batch(dmc_ctx* ctx, const void* src, void* dst, int n_frames, int rows, int cols, int quality, int mem,
                                 uint64_t* bytes);
+/* The same with flags: with DMC_JPEG_OPTIMIZE_HUFFMAN dst is unchanged (the coefficients are the same) and bytes receives
+ * the sizes of the optimised streams. */
+int dmc_jpeg_degrade_gray_batch_ex(dmc_ctx* ctx, const void* src, void* dst, int n_frames, int rows, int cols, int quality, int flags,
+                                   int mem, uint64_t* bytes);
 
 /* ---- stand-alone operators of filter.h ------------------------------------------------------------------- */
 /* binalyWeightedRangeFilter filter.h:29 (binalyWeightedRangeFilter.cpp:1106): 8U/16S/16U/32F x C1/C3 */

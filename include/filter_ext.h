@@ -39,20 +39,23 @@ inline void require_gray8(const Mat& m, const char* what) {
 
 // Baseline JPEG encoding of a CV_8UC1 image on the GPU: `buf` receives the same bytes as
 // cv::imencode(".jpg", src, buf, {IMWRITE_JPEG_QUALITY, quality}) with libjpeg-turbo.  quality in 0..100.
-inline void jpegEncodeGray(const Mat& src, vector<uchar>& buf, int quality)
+// optimize: optimised Huffman tables, the bytes of {IMWRITE_JPEG_QUALITY, quality, IMWRITE_JPEG_OPTIMIZE, 1}.
+inline void jpegEncodeGray(const Mat& src, vector<uchar>& buf, int quality, bool optimize = false)
 {
 	dmc_dropin::require_gray8(src, "jpegEncodeGray");
 	const Mat s = src.isContinuous() ? src : src.clone();
+	const int flags = optimize ? DMC_JPEG_OPTIMIZE_HUFFMAN : 0;
 	uint64_t cap = 0, off[2] = {0, 0};
-	dmc_dropin::check(dmc_jpeg_encode_bound(s.rows, s.cols, &cap), "jpegEncodeGray");
+	dmc_dropin::check(dmc_jpeg_encode_bound_ex(s.rows, s.cols, flags, &cap), "jpegEncodeGray");
 	buf.resize((size_t)cap);
-	dmc_dropin::check(dmc_jpeg_encode_gray_batch(dmc_dropin::context(), s.data, DMC_MEM_HOST, 1, s.rows, s.cols, quality, buf.data(), DMC_MEM_HOST, cap, off), "jpegEncodeGray");
+	dmc_dropin::check(dmc_jpeg_encode_gray_batch_ex(dmc_dropin::context(), s.data, DMC_MEM_HOST, 1, s.rows, s.cols, quality, flags, buf.data(), DMC_MEM_HOST, cap, off), "jpegEncodeGray");
 	buf.resize((size_t)off[1]);
 }
 
 // JPEG round trip of a CV_8UC1 image on the GPU, the stream never leaving the device:
-// dest = cv::imdecode(cv::imencode(".jpg", src, {IMWRITE_JPEG_QUALITY, quality}), 0).  Returns the stream's size in bytes.
-inline int degradeJPEGGray(const Mat& src, Mat& dest, int quality)
+// dest = cv::imdecode(cv::imencode(".jpg", src, {IMWRITE_JPEG_QUALITY, quality}), 0).  Returns the stream's size in bytes
+// (optimize: the size with optimised Huffman tables; dest is the same).
+inline int degradeJPEGGray(const Mat& src, Mat& dest, int quality, bool optimize = false)
 {
 	dmc_dropin::require_gray8(src, "degradeJPEGGray");
 	const Mat s = src.isContinuous() ? src : src.clone();
@@ -60,7 +63,8 @@ inline int degradeJPEGGray(const Mat& src, Mat& dest, int quality)
 	if (dest.data != src.data && dest.size() == src.size() && dest.type() == CV_8UC1 && dest.isContinuous()) d = dest;
 	else d.create(src.size(), CV_8UC1);
 	uint64_t bytes = 0;
-	dmc_dropin::check(dmc_jpeg_degrade_gray_batch(dmc_dropin::context(), s.data, d.data, 1, s.rows, s.cols, quality, DMC_MEM_HOST, &bytes), "degradeJPEGGray");
+	dmc_dropin::check(dmc_jpeg_degrade_gray_batch_ex(dmc_dropin::context(), s.data, d.data, 1, s.rows, s.cols, quality, optimize ? DMC_JPEG_OPTIMIZE_HUFFMAN : 0,
+	                                                 DMC_MEM_HOST, &bytes), "degradeJPEGGray");
 	if (d.data != dest.data) dest = d;
 	return (int)bytes;
 }
