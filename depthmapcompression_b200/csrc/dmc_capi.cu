@@ -26,6 +26,10 @@ constexpr int kSlots = 4;        // streaming pipeline depth (H2D / kernels / D2
 enum { SB_IN, SB_OUT, SB_PING, SB_PONG, SB_FLOAT, SB_BITS, SB_META, SB_SCANS, SB_COEF, SB_COUNT };
 // Device buffers of dmc_jpeg_decode_gray_batch.
 enum { JD_BITS, JD_META, JD_SCANS, JD_COEF, JD_OUT, JD_COUNT };
+// Device buffers of dmc_sse_gray_batch and dmc_jpeg_rd_sweep: every quality's encoder + decoder tables, the decoder's
+// FrameDescs of a group, its staged source, coded and filtered frames (the staged second batch of dmc_sse_gray_batch),
+// and the group's results (SSE, stream lengths) that one copy brings back.
+enum { RD_TABS, RD_DESC, RD_SRC, RD_CODED, RD_FILT, RD_RES, RD_COUNT };
 
 struct Buf { void* p = nullptr; size_t cap = 0; };
 
@@ -51,6 +55,7 @@ struct dmc_ctx {
     struct Gateway { int device = -1; cudaStream_t stream[kSlots] = {}; Buf in[kSlots], out[kSlots]; cudaEvent_t ev_in[kSlots] = {}, ev_out[kSlots] = {}, ev_done[kSlots] = {}; } gw;
     Buf render[2]; int* render_flag = nullptr;      // point-cloud render: attempt lists etc., device flag; pinned host flag
     Buf jpeg[JD_COUNT];
+    Buf rd[RD_COUNT];
     Buf jpeg_enc[11];            // JPEG encode: tables, staged frames, coefficients, block records, scan words, slots, lengths + offsets, staged output, decoder tables + descriptors,
                                  // optimised-table scratch, per-frame decoder Huffman tables
     // optional per-stage CUDA-event timing of the chain (bench.py's live roofline measurement)
@@ -550,6 +555,7 @@ void dmc_destroy(dmc_ctx* ctx) {
     drop_graph(ctx);
     for (auto& b : ctx->jpeg) if (b.p) cudaFree(b.p);
     for (auto& b : ctx->jpeg_enc) if (b.p) cudaFree(b.p);
+    for (auto& b : ctx->rd) if (b.p) cudaFree(b.p);
     for (auto& b : ctx->render) if (b.p) cudaFree(b.p);
     if (ctx->render_flag) cudaFreeHost(ctx->render_flag);
     for (auto& r : ctx->prof_pending) { cudaEventDestroy(r.a); cudaEventDestroy(r.b); }
@@ -1003,9 +1009,9 @@ int jpeg_enc_prepare(dmc_ctx* ctx, const char* what, int rows, int cols, int qua
     return DMC_OK;
 }
 
-// Encodes frames [f0, f0 + nf) of src into the slots (lengths in JE_LENS); desc: also write the decoder's FrameDescs there
-// (with optimised tables their Huffman tables go to JE_HUFF, a pair per frame).
-int jpeg_enc_group(dmc_ctx* ctx, const uint8_t* src, int src_mem, int f0, int nf, int rows, int cols, bool optimize, void* desc) {
+// Encodes frames [f0, f0 + nf) of src with the device EncTables `tabs` into the slots (lengths in JE_LENS); desc: also
+// write the decoder's FrameDescs there (with optimised tables their Huffman tables go to JE_HUFF, a pair per frame).
+int jpeg_enc_group(dmc_ctx* ctx, const void* tabs, const uint8_t* src, int src_mem, int f0, int nf, int rows, int cols, bool optimize, void* desc) {
     cudaStream_t s = ctx->stream;
     const size_t fpx = (size_t)rows * cols;
     const JpegEncLayout l = jpeg_enc_layout(rows, cols, optimize);
@@ -1026,7 +1032,7 @@ int jpeg_enc_group(dmc_ctx* ctx, const uint8_t* src, int src_mem, int f0, int nf
         opt = ctx->jpeg_enc[JE_OPT].p;
         if (desc) { TRY(reserve(ctx, ctx->jpeg_enc[JE_HUFF], 2 * sizeof(dmcjpeg::HuffTable) * nf)); huff = ctx->jpeg_enc[JE_HUFF].p; }
     }
-    LAUNCH(ctx, launch_jpeg_encode(dsrc, ctx->jpeg_enc[JE_TABS].p, ctx->jpeg_enc[JE_COEF].p, ctx->jpeg_enc[JE_INFO].p, ctx->jpeg_enc[JE_WORDS].p,
+    LAUNCH(ctx, launch_jpeg_encode(dsrc, tabs, ctx->jpeg_enc[JE_COEF].p, ctx->jpeg_enc[JE_INFO].p, ctx->jpeg_enc[JE_WORDS].p,
                                    (uint8_t*)ctx->jpeg_enc[JE_SLOTS].p, (uint32_t*)ctx->jpeg_enc[JE_LENS].p, desc, nf, rows, cols, s, opt, huff));
     return DMC_OK;
 }
@@ -1051,7 +1057,7 @@ int dmc_jpeg_encode_gray_batch_ex(dmc_ctx* ctx, const void* src, int src_mem, in
     std::vector<uint32_t> lens; std::vector<uint64_t> offs;
     for (int f0 = 0; f0 < n_frames; f0 += group) {
         const int nf = n_frames - f0 < group ? n_frames - f0 : group;
-        TRY(jpeg_enc_group(ctx, (const uint8_t*)src, src_mem, f0, nf, rows, cols, optimize, nullptr));
+        TRY(jpeg_enc_group(ctx, ctx->jpeg_enc[JE_TABS].p, (const uint8_t*)src, src_mem, f0, nf, rows, cols, optimize, nullptr));
         lens.resize(nf); offs.resize(nf);
         CUDA_TRY(ctx, cudaMemcpyAsync(lens.data(), ctx->jpeg_enc[JE_LENS].p, nf * sizeof(uint32_t), cudaMemcpyDeviceToHost, s));
         CUDA_TRY(ctx, cudaStreamSynchronize(s));
@@ -1106,7 +1112,7 @@ int dmc_jpeg_degrade_gray_batch_ex(dmc_ctx* ctx, const void* src, void* dst, int
     std::vector<uint32_t> lens;
     for (int f0 = 0; f0 < n_frames; f0 += group) {
         const int nf = n_frames - f0 < group ? n_frames - f0 : group;
-        TRY(jpeg_enc_group(ctx, (const uint8_t*)src, mem, f0, nf, rows, cols, optimize, dm + o_desc));
+        TRY(jpeg_enc_group(ctx, ctx->jpeg_enc[JE_TABS].p, (const uint8_t*)src, mem, f0, nf, rows, cols, optimize, dm + o_desc));
         uint8_t* out = (uint8_t*)dst + fpx * f0;
         if (mem == DMC_MEM_HOST) { TRY(reserve(ctx, ctx->jpeg_enc[JE_OUT], fpx * nf)); out = (uint8_t*)ctx->jpeg_enc[JE_OUT].p; }
         LAUNCH(ctx, launch_jpeg_decode((const uint8_t*)ctx->jpeg_enc[JE_SLOTS].p, dm + o_desc, optimize ? ctx->jpeg_enc[JE_HUFF].p : dm, dm + o_q,
@@ -1124,6 +1130,143 @@ int dmc_jpeg_degrade_gray_batch_ex(dmc_ctx* ctx, const void* src, void* dst, int
 
 int dmc_jpeg_degrade_gray_batch(dmc_ctx* ctx, const void* src, void* dst, int n_frames, int rows, int cols, int quality, int mem, uint64_t* bytes) {
     return dmc_jpeg_degrade_gray_batch_ex(ctx, src, dst, n_frames, rows, cols, quality, 0, mem, bytes);
+}
+
+// ---- distortion and the rate-distortion sweep ----------------------------------------------------------------------------
+// cv::PSNR (OpenCV 4.x, core/src/norm.cpp) with R = 255: 20 log10(R / (sqrt(||a - b||^2 / pixels) + DBL_EPSILON)).
+double dmc_psnr_from_sse(uint64_t sse, uint64_t pixels) {
+    return 20.0 * log10(255.0 / (sqrt((double)sse / (double)pixels) + DBL_EPSILON));
+}
+
+// Device frames: one launch over the whole batch.  Host frames: groups of ~256 MB per batch are copied in first (once
+// when a and b are the same pointer).
+int dmc_sse_gray_batch(dmc_ctx* ctx, const void* a, const void* b, int n_frames, int rows, int cols, int mem, uint64_t* sse) {
+    if (!ctx) return fail(nullptr, DMC_ERR_ARG, "null context");
+    if (mem != DMC_MEM_HOST && mem != DMC_MEM_DEVICE) return fail(ctx, DMC_ERR_ARG, "dmc_sse_gray_batch: bad mem");
+    if (n_frames < 0 || rows <= 0 || cols <= 0 || (n_frames > 0 && (!a || !b || !sse))) return fail(ctx, DMC_ERR_SIZE, "dmc_sse_gray_batch: bad arguments");
+    if (n_frames == 0) return DMC_OK;
+    CUDA_TRY(ctx, cudaSetDevice(ctx->device));
+    cudaStream_t s = ctx->stream;
+    const size_t fpx = (size_t)rows * cols;
+    const int group = mem == DMC_MEM_HOST ? chunk_frames((size_t)256 << 20, fpx, n_frames, INT_MAX, false) : n_frames;
+    TRY(reserve(ctx, ctx->rd[RD_RES], (size_t)group * sizeof(uint64_t)));
+    uint64_t* dsse = (uint64_t*)ctx->rd[RD_RES].p;
+    for (int f0 = 0; f0 < n_frames; f0 += group) {
+        const int nf = n_frames - f0 < group ? n_frames - f0 : group;
+        const uint8_t* da = (const uint8_t*)a + fpx * f0;
+        const uint8_t* db = (const uint8_t*)b + fpx * f0;
+        if (mem == DMC_MEM_HOST) {
+            TRY(reserve(ctx, ctx->rd[RD_SRC], fpx * nf));
+            CUDA_TRY(ctx, cudaMemcpyAsync(ctx->rd[RD_SRC].p, da, fpx * nf, cudaMemcpyHostToDevice, s));
+            if (b != a) {
+                TRY(reserve(ctx, ctx->rd[RD_CODED], fpx * nf));
+                CUDA_TRY(ctx, cudaMemcpyAsync(ctx->rd[RD_CODED].p, db, fpx * nf, cudaMemcpyHostToDevice, s));
+            }
+            da = (const uint8_t*)ctx->rd[RD_SRC].p;
+            db = b != a ? (const uint8_t*)ctx->rd[RD_CODED].p : da;
+        }
+        LAUNCH(ctx, launch_sse_u8(da, db, nullptr, dsse, nullptr, nf, fpx, s));
+        CUDA_TRY(ctx, cudaMemcpyAsync(sse + f0, dsse, nf * sizeof(uint64_t), cudaMemcpyDeviceToHost, s));
+        CUDA_TRY(ctx, cudaStreamSynchronize(s));
+    }
+    return DMC_OK;
+}
+
+// The sweep runs group by group (a group is sized like the encoder's, counting the coded and filtered frames and the
+// chain's ping-pong too) and, inside a group, quality by quality: a host source is copied to the device once per group.
+// Every quality's encoder tables and the decoder tables parsed from its header are built once and uploaded in one copy.
+// Per (group, quality) everything runs on ctx->stream without a host synchronisation: encode, decode into the coded
+// frames, the chain into the filtered frames, one SSE launch (source vs coded and vs filtered) and a device-side copy of
+// the stream lengths; one copy and one synchronisation per group bring the results back.
+int dmc_jpeg_rd_sweep(dmc_ctx* ctx, const void* src, int src_mem, int n_frames, int rows, int cols, const int* qualities, int n_q,
+                      int flags, const dmc_chain_params* p, uint64_t* bytes, uint64_t* sse_coded, uint64_t* sse_filtered) {
+    if (!ctx) return fail(nullptr, DMC_ERR_ARG, "null context");
+    if (!qualities || n_q < 1) return fail(ctx, DMC_ERR_ARG, "dmc_jpeg_rd_sweep: no qualities");
+    for (int k = 0; k < n_q; k++)
+        if (qualities[k] < 0 || qualities[k] > 100) return fail(ctx, DMC_ERR_ARG, "dmc_jpeg_rd_sweep: quality must be in 0..100");
+    if (flags & ~DMC_JPEG_OPTIMIZE_HUFFMAN) return fail(ctx, DMC_ERR_ARG, "dmc_jpeg_rd_sweep: unknown flags " + std::to_string(flags));
+    if (p) {
+        TRY(check_chain_params(ctx, *p));
+        if (p->chain != DMC_CHAIN_DISP8U) return fail(ctx, DMC_ERR_ARG, "dmc_jpeg_rd_sweep: the chain must be DMC_CHAIN_DISP8U (8-bit output, comparable with the 8-bit source)");
+        // (the reference's 8U range filter leaves dst unwritten for FULL_KERNEL_PAIR: there would be nothing to measure)
+        if (p->brange_method != DMC_FULL_KERNEL && p->brange_method != DMC_SEPARABLE_KERNEL) return fail(ctx, DMC_ERR_ARG, "dmc_jpeg_rd_sweep: brange_method must be FULL_KERNEL or SEPARABLE_KERNEL");
+    }
+    if (src_mem != DMC_MEM_HOST && src_mem != DMC_MEM_DEVICE) return fail(ctx, DMC_ERR_ARG, "dmc_jpeg_rd_sweep: bad mem");
+    uint64_t bound;
+    if (dmc_jpeg_encode_bound_ex(rows, cols, flags, &bound) != DMC_OK) return fail(ctx, DMC_ERR_SIZE, "dmc_jpeg_rd_sweep: " + g_err);
+    if (n_frames < 0 || (n_frames > 0 && (!src || !bytes || !sse_coded || (p && !sse_filtered)))) return fail(ctx, DMC_ERR_SIZE, "dmc_jpeg_rd_sweep: bad arguments");
+    if (n_frames == 0) return DMC_OK;
+    CUDA_TRY(ctx, cudaSetDevice(ctx->device));
+    cudaStream_t s = ctx->stream;
+    const bool optimize = (flags & DMC_JPEG_OPTIMIZE_HUFFMAN) != 0, host = src_mem == DMC_MEM_HOST;
+    const size_t fpx = (size_t)rows * cols;
+    const JpegEncLayout l = jpeg_enc_layout(rows, cols, optimize);
+    const size_t per = l.coef_bytes + l.info_bytes + l.word_bytes + l.slot_bytes + (optimize ? l.opt_bytes + 2 * sizeof(dmcjpeg::HuffTable) : 0) +
+                       sizeof(dmcjpeg::FrameDesc) + fpx * ((host ? 1 : 0) + 1 + (p ? 3 : 0));      // staged source, coded, filtered, ping, pong
+    const int group = chunk_frames(kEncGroupBytes, per, n_frames, 2048, false);
+    // per quality: [EncTables][DC, AC HuffTable][QuantTable]
+    const size_t o_h = (sizeof(dmcjpeg::EncTables) + 15) & ~(size_t)15, o_q = o_h + 2 * sizeof(dmcjpeg::HuffTable);
+    const size_t rec = (o_q + sizeof(dmcjpeg::QuantTable) + 255) & ~(size_t)255;
+    std::vector<char> tabs(rec * n_q);
+    for (int k = 0; k < n_q; k++) {
+        dmcjpeg::EncTables t;
+        dmcjpeg::make_enc_tables(qualities[k], rows, cols, &t);
+        std::vector<dmcjpeg::QuantTable> qpool; std::vector<dmcjpeg::HuffTable> hpool; dmcjpeg::FrameDesc hd;
+        const std::string why = jpeg_parse_frame(t.header, dmcjpeg::kEncHeaderBytes, 0, rows, cols, qpool, hpool, &hd);
+        if (!why.empty() || hpool.size() != 2 || qpool.size() != 1 || hd.dc != 0 || hd.ac != 1 || hd.qt != 0)
+            return fail(ctx, DMC_ERR_TYPE, "dmc_jpeg_rd_sweep: encoder header does not parse: " + why);
+        char* r = tabs.data() + rec * k;
+        memcpy(r, &t, sizeof t);
+        memcpy(r + o_h, hpool.data(), 2 * sizeof(dmcjpeg::HuffTable));
+        memcpy(r + o_q, qpool.data(), sizeof(dmcjpeg::QuantTable));
+    }
+    TRY(reserve(ctx, ctx->rd[RD_TABS], tabs.size()));
+    TRY(reserve(ctx, ctx->rd[RD_DESC], (size_t)group * sizeof(dmcjpeg::FrameDesc)));
+    TRY(reserve(ctx, ctx->rd[RD_CODED], fpx * group));
+    if (p) TRY(reserve(ctx, ctx->rd[RD_FILT], fpx * group));
+    if (host) TRY(reserve(ctx, ctx->rd[RD_SRC], fpx * group));
+    // results of a group of nf frames: [sse_coded][sse_filtered] (uint64, [quality][frame]), then the lengths (uint32)
+    const size_t res_bytes = (size_t)n_q * group * (2 * sizeof(uint64_t) + sizeof(uint32_t));
+    TRY(reserve(ctx, ctx->rd[RD_RES], res_bytes));
+    CUDA_TRY(ctx, cudaMemcpyAsync(ctx->rd[RD_TABS].p, tabs.data(), tabs.size(), cudaMemcpyHostToDevice, s));
+    Slot& sl = ctx->slot[0]; sl.stream = s;
+    uint8_t* coded = (uint8_t*)ctx->rd[RD_CODED].p;
+    uint8_t* filt = (uint8_t*)ctx->rd[RD_FILT].p;
+    std::vector<char> res;
+    for (int f0 = 0; f0 < n_frames; f0 += group) {
+        const int nf = n_frames - f0 < group ? n_frames - f0 : group;
+        const uint8_t* dsrc = (const uint8_t*)src + fpx * f0;
+        if (host) {
+            CUDA_TRY(ctx, cudaMemcpyAsync(ctx->rd[RD_SRC].p, dsrc, fpx * nf, cudaMemcpyHostToDevice, s));
+            dsrc = (const uint8_t*)ctx->rd[RD_SRC].p;
+        }
+        uint64_t* d_sc = (uint64_t*)ctx->rd[RD_RES].p;
+        uint64_t* d_sf = d_sc + (size_t)n_q * nf;
+        uint32_t* d_len = (uint32_t*)(d_sf + (size_t)n_q * nf);
+        for (int k = 0; k < n_q; k++) {
+            const char* tk = (const char*)ctx->rd[RD_TABS].p + rec * k;
+            TRY(jpeg_enc_group(ctx, tk, dsrc, DMC_MEM_DEVICE, 0, nf, rows, cols, optimize, ctx->rd[RD_DESC].p));
+            LAUNCH(ctx, launch_jpeg_decode((const uint8_t*)ctx->jpeg_enc[JE_SLOTS].p, ctx->rd[RD_DESC].p, optimize ? ctx->jpeg_enc[JE_HUFF].p : tk + o_h, tk + o_q,
+                                           (uint8_t*)ctx->jpeg_enc[JE_WORDS].p, nullptr, coded, nf, 0, rows, cols, s));
+            if (p) TRY(run_chain(ctx, sl, coded, filt, nf, rows, cols, *p));
+            LAUNCH(ctx, launch_sse_u8(dsrc, coded, p ? filt : nullptr, d_sc + (size_t)k * nf, p ? d_sf + (size_t)k * nf : nullptr, nf, fpx, s));
+            CUDA_TRY(ctx, cudaMemcpyAsync(d_len + (size_t)k * nf, ctx->jpeg_enc[JE_LENS].p, nf * sizeof(uint32_t), cudaMemcpyDeviceToDevice, s));
+        }
+        const size_t used = (size_t)n_q * nf * (2 * sizeof(uint64_t) + sizeof(uint32_t));
+        res.resize(used);
+        CUDA_TRY(ctx, cudaMemcpyAsync(res.data(), ctx->rd[RD_RES].p, used, cudaMemcpyDeviceToHost, s));
+        CUDA_TRY(ctx, cudaStreamSynchronize(s));
+        const uint64_t* sc = (const uint64_t*)res.data();
+        const uint64_t* sf = sc + (size_t)n_q * nf;
+        const uint32_t* len = (const uint32_t*)(sf + (size_t)n_q * nf);
+        for (int k = 0; k < n_q; k++)
+            for (int i = 0; i < nf; i++) {
+                const size_t o = (size_t)k * n_frames + f0 + i, j = (size_t)k * nf + i;
+                bytes[o] = len[j]; sse_coded[o] = sc[j];
+                if (p) sse_filtered[o] = sf[j];
+            }
+    }
+    return DMC_OK;
 }
 
 // ---- stand-alone operators ---------------------------------------------------------------------------------------

@@ -96,6 +96,12 @@ int launch_jpeg_enc_gather(const uint8_t* slots, size_t slot_bytes, const uint32
 }
 
 namespace dmc {
+// Exact per-frame sum of squared differences of n dense 8-bit frames of frame_bytes each (dmc_metrics.cu): sse0[f] = SSE(a, b0)
+// and, when b1 != nullptr, sse1[f] = SSE(a, b1) in the same launch (a is read once).  Zeroes the outputs first.
+int launch_sse_u8(const uint8_t* a, const uint8_t* b0, const uint8_t* b1, uint64_t* sse0, uint64_t* sse1, int n, size_t frame_bytes, cudaStream_t s);
+}
+
+namespace dmc {
 // point-cloud render (dmc_render.cu)
 int launch_project_points(const float* xyz, float* pt, long n, const float kr[9], const float t[3], int exact_divide, cudaStream_t s);
 size_t render_scratch_bytes(int rows, int cols);

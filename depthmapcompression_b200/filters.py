@@ -289,6 +289,51 @@ def degradeJPEG(frames, quality, dst=None, ctx=None, optimize=False):
     return dst, nbytes
 
 
+def frameSSE(a, b, ctx=None):
+    """Exact per-frame sum of squared differences of two batches of 8-bit frames on the GPU (dmc_sse_gray_batch).  a, b:
+    uint8 numpy [n, rows, cols] (or one [rows, cols] frame), or both (device pointer, n, rows, cols).  -> np.uint64[n]"""
+    ctx = ctx or default_context()
+    ap, n, rows, cols, mem, ka = _frames(a)
+    bp, bn, brows, bcols, bmem, kb = _frames(b)
+    if (n, rows, cols, mem) != (bn, brows, bcols, bmem):
+        raise DmcError(capi.DMC_ERR_SIZE, "frameSSE: a and b must be batches of one shape in the same memory")
+    sse = np.zeros(n, np.uint64)
+    ctx.check(lib.dmc_sse_gray_batch(ctx.h, C.c_void_p(ap), C.c_void_p(bp), n, rows, cols, mem, sse.ctypes.data_as(C.POINTER(C.c_uint64))))
+    return sse
+
+
+_psnr = np.vectorize(lambda sse, pixels: lib.dmc_psnr_from_sse(int(sse), int(pixels)), otypes=[np.float64])
+
+
+def psnrFromSSE(sse, pixels):
+    """PSNR in dB of 8-bit frames of `pixels` pixels from their exact SSE, by the formula of cv2.PSNR (dmc_psnr_from_sse);
+    vectorised over both arguments."""
+    r = _psnr(np.asarray(sse, np.uint64), np.asarray(pixels, np.uint64))
+    return float(r) if r.ndim == 0 else r
+
+
+def jpegRateDistortion(frames, qualities, params=None, optimize=False, ctx=None):
+    """The JPEG rate-distortion sweep on the GPU (dmc_jpeg_rd_sweep): every frame is coded at every quality as cv2.imencode
+    codes it (optimize: with optimised Huffman tables), decoded, and with `params` (a chain_params(CHAIN_DISP8U, ...))
+    post-filtered; no frame or stream leaves the device.  frames as for degradeJPEG.  Returns a dict of (n_q, n) arrays:
+    bytes, sse_coded, psnr_coded, and with params also sse_filtered, psnr_filtered."""
+    ctx = ctx or default_context()
+    sp, n, rows, cols, mem, keep = _frames(frames)
+    q = np.ascontiguousarray(np.asarray(qualities).ravel(), dtype=np.int32)
+    shape = (len(q), n)
+    U64 = C.POINTER(C.c_uint64)
+    nbytes, sc = np.zeros(shape, np.uint64), np.zeros(shape, np.uint64)
+    sf = np.zeros(shape, np.uint64) if params is not None else None
+    ctx.check(lib.dmc_jpeg_rd_sweep(ctx.h, C.c_void_p(sp), mem, n, rows, cols, q.ctypes.data_as(C.POINTER(C.c_int)), len(q), _jpeg_flags(optimize),
+                                    C.byref(params) if params is not None else None, nbytes.ctypes.data_as(U64), sc.ctypes.data_as(U64),
+                                    sf.ctypes.data_as(U64) if sf is not None else None))
+    out = {"bytes": nbytes, "sse_coded": sc, "psnr_coded": psnrFromSSE(sc, rows * cols)}
+    if sf is not None:
+        out["sse_filtered"] = sf
+        out["psnr_filtered"] = psnrFromSSE(sf, rows * cols)
+    return out
+
+
 _default = {}
 
 

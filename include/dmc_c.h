@@ -233,6 +233,26 @@ int dmc_jpeg_degrade_gray_batch(dmc_ctx* ctx, const void* src, void* dst, int n_
 int dmc_jpeg_degrade_gray_batch_ex(dmc_ctx* ctx, const void* src, void* dst, int n_frames, int rows, int cols, int quality, int flags,
                                    int mem, uint64_t* bytes);
 
+/* ---- distortion and the JPEG rate-distortion sweep ---------------------------------------------------------- */
+/* Per-frame sum of squared differences of two batches of n dense rows x cols 8UC1 frames (both in `mem`), exact:
+ * sse[i] = sum over the pixels of (a_i - b_i)^2 (host, n_frames entries).  a and b may be the same pointer.
+ * Returns when sse is valid. */
+int dmc_sse_gray_batch(dmc_ctx* ctx, const void* a, const void* b, int n_frames, int rows, int cols, int mem, uint64_t* sse);
+/* Host only, no GPU: PSNR in dB of an 8-bit frame of `pixels` pixels with sum of squared differences `sse`, by the formula of
+ * cv::PSNR: 20*log10(255 / (sqrt(sse / pixels) + DBL_EPSILON)) -- identical frames give 361.20199909921956, as cv2.PSNR does. */
+double dmc_psnr_from_sse(uint64_t sse, uint64_t pixels);
+/* The rate-distortion sweep: for every quality qualities[k] and every frame i of src (n dense 8UC1 frames, src_mem host or
+ * device): bytes[k*n+i]        = size of cv::imencode(frame, {QUALITY, q} [+ OPTIMIZE with DMC_JPEG_OPTIMIZE_HUFFMAN]),
+ *          sse_coded[k*n+i]    = SSE(frame, imdecode(that stream)),
+ *          sse_filtered[k*n+i] = SSE(frame, chain(imdecode(that stream))) -- only when p != NULL; p->chain must be DMC_CHAIN_DISP8U.
+ * No stream and no decoded or filtered frame leaves the device.  Outputs are host arrays of n_q * n_frames entries.
+ * DMC_ERR_ARG (nothing written): n_q < 1, a quality outside 0..100 (0 acts as 1, as in cv::imencode), unknown flag bits,
+ * a chain other than DMC_CHAIN_DISP8U, a bad radius, or a brange_method other than FULL_KERNEL / SEPARABLE_KERNEL (the
+ * 8-bit chain writes nothing for the others).  p == NULL: sse_filtered may be NULL and is not written.  Sizes follow
+ * dmc_jpeg_encode_bound_ex.  Returns when the outputs are valid. */
+int dmc_jpeg_rd_sweep(dmc_ctx* ctx, const void* src, int src_mem, int n_frames, int rows, int cols, const int* qualities, int n_q,
+                      int flags, const dmc_chain_params* p, uint64_t* bytes, uint64_t* sse_coded, uint64_t* sse_filtered);
+
 /* ---- stand-alone operators of filter.h ------------------------------------------------------------------- */
 /* binalyWeightedRangeFilter filter.h:29 (binalyWeightedRangeFilter.cpp:1106): 8U/16S/16U/32F x C1/C3 */
 int dmc_bwrf(dmc_ctx* ctx, const dmc_image* src, dmc_image* dst, int kernel_w, int kernel_h, float threshold,

@@ -68,3 +68,27 @@ inline int degradeJPEGGray(const Mat& src, Mat& dest, int quality, bool optimize
 	if (d.data != dest.data) dest = d;
 	return (int)bytes;
 }
+
+// The JPEG rate-distortion sweep of one CV_8UC1 image on the GPU (the reference's simpleTest, main.cpp:516-526, for several
+// qualities at once): for every qualities[k], bytes[k] = the size of cv::imencode(".jpg", src, {IMWRITE_JPEG_QUALITY, q}
+// [, IMWRITE_JPEG_OPTIMIZE, 1]), psnr_coded[k] = cv::PSNR(src, the decoded image) and psnr_filtered[k] = cv::PSNR(src,
+// PostFilterSet()(decoded, median_r, gaussian_r, minmax_r, brange_r, brange_th)).  Neither stream nor image leaves the device.
+inline void jpegRateDistortionGray(const Mat& src, const vector<int>& qualities, vector<int>& bytes, vector<double>& psnr_coded,
+                                   vector<double>& psnr_filtered, int median_r, int gaussian_r, int minmax_r, int brange_r, int brange_th,
+                                   bool optimize = false)
+{
+	dmc_dropin::require_gray8(src, "jpegRateDistortionGray");
+	const Mat s = src.isContinuous() ? src : src.clone();
+	const size_t nq = qualities.size();
+	vector<uint64_t> b(nq), sc(nq), sf(nq);
+	dmc_chain_params p = {DMC_CHAIN_DISP8U, median_r, gaussian_r, minmax_r, brange_r, (float)brange_th, DMC_FULL_KERNEL, 0, 0, 0};
+	dmc_dropin::check(dmc_jpeg_rd_sweep(dmc_dropin::context(), s.data, DMC_MEM_HOST, 1, s.rows, s.cols, qualities.data(), (int)nq,
+	                                    optimize ? DMC_JPEG_OPTIMIZE_HUFFMAN : 0, &p, b.data(), sc.data(), sf.data()), "jpegRateDistortionGray");
+	const uint64_t pixels = (uint64_t)s.rows * s.cols;
+	bytes.resize(nq); psnr_coded.resize(nq); psnr_filtered.resize(nq);
+	for (size_t k = 0; k < nq; k++) {
+		bytes[k] = (int)b[k];
+		psnr_coded[k] = dmc_psnr_from_sse(sc[k], pixels);
+		psnr_filtered[k] = dmc_psnr_from_sse(sf[k], pixels);
+	}
+}
