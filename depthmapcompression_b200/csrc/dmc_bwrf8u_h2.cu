@@ -17,9 +17,8 @@
 // tall block of outputs; for every input row it loads 7 aligned half2 words, funnel-shifts the odd offsets, and
 // reuses each tap vector for all the output rows whose window contains it (register tiling: ~0.5 LDS per 2x81 taps).
 // R = 4 at radius >= 4 keeps the fully unrolled body near the 32 KB instruction cache (R = 8, 56 KB, ran 5x slower;
-// R = 4 with the flat path below, 2224 instructions = 34.8 KB at radius 5: uniform noise, which never leaves the tap
-// loop, runs 2.3 % slower, flat test included).  A
-// variant with a run-time loop over the horizontal offset, R = 8 and two shifted shared-memory copies was measured
+// R = 4 with the flat-strip path below, 2328 instructions = 36.4 KB at radius 5: uniform noise, which never leaves
+// the tap loop, runs about 2 % slower than the tap loop alone, centre pre-test included).  A variant with a run-time loop over the horizontal offset, R = 8 and two shifted shared-memory copies was measured
 // too: fewer loads per tap but more staging/loop instructions, 17.9 ms vs 16.0 ms per 1000 frames -- not kept.
 #include "dmc_common.cuh"
 #include "dmc_kernels.cuh"
@@ -70,14 +69,28 @@ __host__ __device__ constexpr int stride_of(int R) {
 // input row (a row contributes at most 2*RAD+1 taps, so |S| <= (2*RAD+1)*th <= 2048 stays exact); +5 instructions
 // per output row and input row.
 //
-// Warps.  A warp owns a 32 x 2R pixel block of the 128 x 4R tile: lanes 0-15 the upper R rows, lanes 16-31 the lower.
-// On the chain's real input 32 x 8 blocks pass the flat test below about 10 points more often than 64 x 4 blocks.
+// Strips.  A thread computes one strip of 2 x R outputs; the CTA's 256 strips tile its 128 x 4R outputs, strip id
+// s = 32 * (4 * wy + wx) + lane at pixels (32 * wx + 2 * (lane % 16), 2R * wy + R * (lane / 16)), so that with the
+// identity assignment a warp owns a 32 x 2R block, lanes 0-15 the upper R rows, lanes 16-31 the lower.
 //
-// Flat warps.  Let F be a warp's square footprint in the staged tile (its block plus RAD on every side, widened to whole
-// 4-pixel chunks; the staged tile already holds the REPLICATE border values, so F holds every value a tap of the warp can
-// read), m and M the min and max over F, cmin and cmax over the warp's centres.  If M - cmin <= th and cmax - m <= th,
-// every tap of every pixel of the warp is within th of its centre: N = ntaps and the filter is the disc mean
-// RNE(sum v / ntaps).  cmax - cmin <= th is necessary for that and costs little, so F is read only when it holds.
+// Flat strips.  Let F be a strip's footprint in the staged tile: the NW words the tap loop reads (pixels x - E .. x + E + 1)
+// over its R + 2*RAD input rows.  The staged tile already holds the REPLICATE border values, so F holds every value a
+// tap of the strip can read.  Let m and M be the min and max over F, cmin and cmax over the strip's centres.  If
+// M - cmin <= th and cmax - m <= th, every tap of every pixel of the strip is within th of its centre: N = ntaps and
+// the filter is the disc mean RNE(sum v / ntaps).  cmax - cmin <= th is necessary for that and costs little, so F is
+// read only in CTAs where some strip passes it (uniform noise never does).  F is taken separably: the CTA first writes
+// the column min / max of every word column over the input rows of each strip row to shared memory (strip rows 2p and
+// 2p+1 share all but R of their rows, so one thread takes both), then each thread folds its NW columns.
+// The CTA then reassigns strips to threads: flat strips first, tap strips after, each in id order, and the one warp
+// that would hold both runs the tap loop for all of its strips, so no warp pays for both paths.  On the chain's real
+// input (bench.py, radius 5, th 10) 75 % of the 2 x 4 strips pass, against 39 % of 32 x 8 warps under the warp-wide
+// test this replaced, and 29 % of the warps run the tap loop after regrouping.  Measured on a B200 (1000 W), range
+// filter alone on 8 stacked frames of that input: 0.1022 -> 0.0801 ms; a constant frame 0.0414 -> 0.0433 ms (the
+// strip test costs more than the warp test); uniform noise 0.1237 -> 0.1233 ms.  The timings imply that 54 % of the warps take the
+// flat path, not 71 %: a CTA keeps its slot until its last tap warp ends, so flat warps beside tap warps free nothing
+// (25 % tap strips cost 0.0739 ms as two tap warps in every CTA, 0.0674 ms as a quarter of the CTAs all tap).  Tap
+// warps of scattered strips read shared memory with bank conflicts and store 2 bytes per lane at scattered rows; both
+// measured at about 1 % (coalescing the stores through shared memory was slower).
 // The flat path adds, per input row, the packed segment sums for every half-width (2 pixels per 32-bit word, 16-bit
 // fields) into the R output rows.  The fields hold sum (v - m) <= ntaps * (M - m) <= ntaps * 2 * th < 2^16
 // (static_assert below), so 32-bit adds of the biased words, wrapping, and one subtraction of ntaps * (0x6400 + m) per
@@ -87,64 +100,94 @@ __host__ __device__ constexpr int stride_of(int R) {
 // m + (sum(v - m) + ntaps / 2) / ntaps  in integers.
 template <int RAD, int R, bool FLUSH, bool EVEN>     // EVEN: W and dst allow 2-byte stores
 __global__ void __launch_bounds__(256) bwrf8u_h2_kernel(const uint8_t* __restrict__ src, uint8_t* __restrict__ dst, int H, int W, int th) {
-    constexpr int TILE_H = 4 * R;                         // 2 warp rows of 2R
+    constexpr int TILE_H = 4 * R;                         // 4 strip rows of R
     constexpr int SH = TILE_H + 2 * RAD;
     constexpr int SWW = stride_of(R);                     // row stride in 32-bit words
     constexpr int NT = ntaps_of(RAD);
+    constexpr int E = RAD <= 6 ? 6 : (RAD <= 8 ? 8 : 10), NW = E + 1;     // words (x-E, x-E+1) .. (x+E, x+E+1) cover offsets -E .. E+1
+    constexpr int NC = 64 + E;                            // word columns any strip's footprint touches, from word (kHalo - E) / 2
     static_assert(NT % 2 == 1 && (long)NT * 2 * (2048 / (2 * RAD + 1)) < 65536, "flat-path fields must not overflow");
     __shared__ __align__(16) uint32_t sm[SH * SWW];
+    __shared__ uint2 colmm[4][NC];                        // per strip row and word column: packed (min, max) over its input rows
+    __shared__ uint32_t order[256];                       // thread -> strip id | footprint min << 8
+    __shared__ uint32_t wflat[8];
 
     const size_t fo = (size_t)blockIdx.z * H * W;
     const int X0 = blockIdx.x * kTileW, Y0 = blockIdx.y * TILE_H;
-    const int tid = threadIdx.y * 32 + threadIdx.x;
+    const int tid = threadIdx.y * 32 + threadIdx.x, lane = threadIdx.x;
     stage_tile16<SH, 1, false, SWW>(sm, src + fo, X0, Y0 - RAD, H, W, aligned16(src, W), tid);      // biased half2 words (0x6400 | byte)
     __syncthreads();
 
-    const int lane = threadIdx.x, wx = threadIdx.y & 3, wy = threadIdx.y >> 2;
-    const int xl = 32 * wx + 2 * (lane & 15);             // first pixel of this thread's pair inside the tile
-    const int yl = 2 * R * wy + R * (lane >> 4);          // first output row of this thread inside the tile
-    constexpr int E = RAD <= 6 ? 6 : (RAD <= 8 ? 8 : 10), NW = E + 1;     // words (x-E, x-E+1) .. (x+E, x+E+1) cover offsets -E .. E+1
-    const uint32_t* base = sm + yl * SWW + (xl + kHalo - E) / 2;      // word holding pixels (x-E, x-E+1)
-
+    int xl, yl;                                           // first pixel and first output row of this thread's strip inside the tile
+    const uint32_t* base;                                 // word holding pixels (x-E, x-E+1) of the strip's first input row
     __half2 c[R];
+    auto take_strip = [&](int s) {
+        xl = 32 * ((s >> 5) & 3) + 2 * (s & 15);
+        yl = R * (s >> 7 << 1 | (s >> 4 & 1));
+        base = sm + yl * SWW + (xl + kHalo - E) / 2;
 #pragma unroll
-    for (int r = 0; r < R; r++) {
-        uint32_t cw = base[(r + RAD) * SWW + E / 2];      // pixels (x, x+1) of output row r
-        c[r] = *reinterpret_cast<__half2*>(&cw);
-    }
+        for (int r = 0; r < R; r++) {
+            uint32_t cw = base[(r + RAD) * SWW + E / 2];  // pixels (x, x+1) of output row r
+            c[r] = *reinterpret_cast<__half2*>(&cw);
+        }
+    };
+    take_strip(tid);
 
-    // ---- flat-warp test.  The biased halves 0x6400 | byte order like their bit patterns: min / max of 16-bit fields ----
+    // ---- flat-strip test.  The biased halves 0x6400 | byte order like their bit patterns: min / max of 16-bit fields ----
     auto h2u = [](__half2 h) { return *reinterpret_cast<const uint32_t*>(&h); };
     __half2 cmn = c[0], cmx = c[0];
 #pragma unroll
     for (int r = 1; r < R; r++) { cmn = __hmin2(cmn, c[r]); cmx = __hmax2(cmx, c[r]); }
-    const uint32_t cmin = __reduce_min_sync(0xFFFFFFFFu, min(h2u(cmn) & 0xFFFFu, h2u(cmn) >> 16));
-    const uint32_t cmax = __reduce_max_sync(0xFFFFFFFFu, max(h2u(cmx) & 0xFFFFu, h2u(cmx) >> 16));
-    bool flat = (int)(cmax - cmin) <= th;
+    const uint32_t cmin = min(h2u(cmn) & 0xFFFFu, h2u(cmn) >> 16), cmax = max(h2u(cmx) & 0xFFFFu, h2u(cmx) >> 16);
+    const bool outside = X0 + xl >= W || Y0 + yl >= H;    // never stored: counted with the flat strips
+    bool flat = false;
     uint32_t m = 0;
-    if (flat) {
-        // F: rows 2R*wy .. 2R*wy + 2R + 2*RAD - 1, 4-pixel chunks Q0 .. Q0 + NQ - 1 of the warp's columns; lane l reads
-        // chunk l % NQ of rows l / NQ, l / NQ + RPI, ... (lanes from RPI * NQ on read none)
-        constexpr int Q0 = (kHalo - RAD) >> 2, NQ = ((kHalo + 31 + RAD) >> 2) - Q0 + 1, RPI = 32 / NQ, FR = 2 * R + 2 * RAD;
-        __half2 fmn = c[0], fmx = c[0];
-        const int fr = lane / NQ;
-        const uint2* fp = reinterpret_cast<const uint2*>(sm + (2 * R * wy + fr) * SWW) + 8 * wx + Q0 + lane % NQ;
+    if (__syncthreads_or(!outside && (int)(cmax - cmin) <= th)) {
+        if (tid < 2 * NC) {
+            // strip rows 2p and 2p+1 read input rows 2pR .. 2pR + R + 2RAD - 1 and (2p+1)R .. (2p+1)R + R + 2RAD - 1
+            const int p = tid / NC, j = tid - p * NC;
+            const uint32_t* col = sm + 2 * p * R * SWW + (kHalo - E) / 2 + j;
+            uint32_t mn = col[R * SWW], mx = mn;
 #pragma unroll
-        for (int k = 0; k < (FR + RPI - 1) / RPI; k++) {
-            if (fr < RPI && fr + k * RPI < FR) {
-                const uint2 q = fp[k * RPI * (SWW / 2)];
-                const __half2 a = *reinterpret_cast<const __half2*>(&q.x), b = *reinterpret_cast<const __half2*>(&q.y);
-                fmn = __hmin2(fmn, __hmin2(a, b)); fmx = __hmax2(fmx, __hmax2(a, b));
-            }
+            for (int y = R + 1; y < R + 2 * RAD; y++) { mn = __vminu2(mn, col[y * SWW]); mx = __vmaxu2(mx, col[y * SWW]); }
+            uint32_t amn = mn, amx = mx, bmn = mn, bmx = mx;
+#pragma unroll
+            for (int y = 0; y < R; y++) { amn = __vminu2(amn, col[y * SWW]); amx = __vmaxu2(amx, col[y * SWW]); }
+#pragma unroll
+            for (int y = R + 2 * RAD; y < 2 * R + 2 * RAD; y++) { bmn = __vminu2(bmn, col[y * SWW]); bmx = __vmaxu2(bmx, col[y * SWW]); }
+            colmm[2 * p][j] = make_uint2(amn, amx);
+            colmm[2 * p + 1][j] = make_uint2(bmn, bmx);
         }
-        m = __reduce_min_sync(0xFFFFFFFFu, min(h2u(fmn) & 0xFFFFu, h2u(fmn) >> 16));
-        const uint32_t M = __reduce_max_sync(0xFFFFFFFFu, max(h2u(fmx) & 0xFFFFu, h2u(fmx) >> 16));
-        flat = (int)(M - cmin) <= th && (int)(cmax - m) <= th;
-    }
+        __syncthreads();
+        const uint2* cm = &colmm[yl / R][xl / 2];
+        uint32_t fmn = cm[0].x, fmx = cm[0].y;
+#pragma unroll
+        for (int i = 1; i < NW; i++) { const uint2 q = cm[i]; fmn = __vminu2(fmn, q.x); fmx = __vmaxu2(fmx, q.y); }
+        m = min(fmn & 0xFFFFu, fmn >> 16);
+        const uint32_t M = max(fmx & 0xFFFFu, fmx >> 16);
+        flat = outside || ((int)(M - cmin) <= th && (int)(cmax - m) <= th);
 
+        // ---- regroup: flat strips to the first threads, tap strips after them, both in id order.  The warp that would
+        // hold both runs the tap loop for all its strips (exact for any strip): no warp runs both paths ----
+        const uint32_t bal = __ballot_sync(0xFFFFFFFFu, flat);
+        if (lane == 0) wflat[threadIdx.y] = __popc(bal);
+        const int nflat = __syncthreads_count(flat);
+        if (nflat >= 32 && nflat < 256) {                 // otherwise every thread keeps its own strip
+            uint32_t before = 0;
+#pragma unroll
+            for (int w = 0; w < 8; w++) before += w < (int)threadIdx.y ? wflat[w] : 0u;
+            const uint32_t rank = __popc(bal & ((1u << lane) - 1u));
+            order[flat ? before + rank : nflat + 32 * threadIdx.y - before + lane - rank] = (uint32_t)tid | (m & 0xFFu) << 8;
+            __syncthreads();
+            const uint32_t o = order[tid];
+            m = o >> 8;
+            take_strip(o & 0xFFu);
+        }
+        flat = tid < (nflat & ~31);
+    }
     uint32_t o0[R], o1[R];                                // results, in the low byte
     if (flat) {
-        // ---- flat warp: disc mean from packed per-row segment sums ----
+        // ---- flat strip: disc mean from packed per-row segment sums ----
         uint32_t acc[R];
 #pragma unroll
         for (int r = 0; r < R; r++) acc[r] = 0u;

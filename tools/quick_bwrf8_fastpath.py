@@ -1,12 +1,14 @@
 #!/usr/bin/env python
-"""Range filter alone (8UC1, radius 5, th 10: the chain's last stage) on three inputs, to see what the flat-warp path
+"""Range filter alone (8UC1, radius 5, th 10: the chain's last stage) on three inputs, to see what the flat-strip path
 of dmc_bwrf8u_h2.cu buys and costs:
     video   the range filter's real input in bench.py: median 5 -> Gaussian 3 -> min-max 3 of frames of its video
-    noise   uniform random bytes: no warp passes the flat test, every warp runs the tap loop
-    const   a constant frame: every warp passes the flat test
-Each input is --frames 1080p frames stacked into one tall image.  Prints ms per launch (CUDA events over --reps launches)
-and the share of warps that pass the flat test, as predicted by a numpy copy of the test.  Both paths cost the same
-for any data, so  (noise - video) / (noise - const)  is the share of the flat path measured from the timings.
+    noise   uniform random bytes: no strip passes the flat test, every warp runs the tap loop
+    const   a constant frame: every strip passes the flat test
+Each input is --frames 1080p frames stacked into one tall image.  Prints ms per launch (CUDA events over --reps launches),
+and from a numpy copy of the kernel's test the share of strips that pass and the share of warps that run the tap loop
+once the CTA has regrouped its strips (flat strips first; the one warp holding both counts as a tap warp).  A warp costs
+about the same on either path for any data, so  (noise - video) / (noise - const)  is the share of warps that take the
+flat path, measured from the timings.
 
     python tools/quick_bwrf8_fastpath.py [--frames 8] [--reps 50]"""
 import argparse
@@ -24,31 +26,34 @@ RAD, TH = 5, 10
 H, W = 1080, 1920
 
 
-def flat_warp_share(img, rad, th, R):
-    """numpy copy of the kernel's flat-warp test: warps of 32 x 2R pixels in tiles of 128 x 4R; footprint = the warp's
-    rows +- rad and the 4-pixel chunks (counted from 16 pixels left of the tile) that hold its columns +- rad, all read
-    through BORDER_REPLICATE; the warp passes iff max(F) - min(centres) <= th and max(centres) - min(F) <= th."""
+def _win(x, axis, lo, hi, fn):
+    """fn over offsets lo .. hi along axis, BORDER_REPLICATE"""
+    n = x.shape[axis]
+    p = np.pad(x, [(-lo, hi) if a == axis else (0, 0) for a in range(x.ndim)], mode="edge")
+    out = np.take(p, range(0, n), axis=axis)
+    for k in range(1, hi - lo + 1):
+        out = fn(out, np.take(p, range(k, k + n), axis=axis))
+    return out
+
+
+def flat_strip_model(img, rad, th, R):
+    """numpy copy of the kernel's flat-strip test and regrouping: a strip is 2 pixels x R rows, its footprint the words
+    the tap loop reads (pixels x - E .. x + E + 1) over rows y - rad .. y + R - 1 + rad, read through BORDER_REPLICATE; it
+    passes iff max(F) - min(centres) <= th and max(centres) - min(F) <= th.  A CTA (128 x 4R pixels, 256 strips, 8 warps)
+    runs ceil(tap strips / 32) tap warps.  Returns (share of strips that pass, share of warps that run the tap loop)."""
     x = img.astype(np.int16)
     Hh, Ww = x.shape
-    q0 = (16 - rad) >> 2
-    nq = ((16 + 31 + rad) >> 2) - q0 + 1
-    ntx, nty = (Ww + 127) // 128, (Hh + 4 * R - 1) // (4 * R)
-    pl, pt = 16, rad
-    xp = np.pad(x, ((pt, nty * 4 * R + rad - Hh), (pl, ntx * 128 + 16 - Ww + 8)), mode="edge")      # xp[pt + y, pl + x] = x[clamp(y), clamp(x)]
-    passed = total = 0
-    for ty in range(nty):
-        for wy in range(2):
-            y0 = ty * 4 * R + wy * 2 * R
-            rows = xp[y0:y0 + 2 * R + 2 * rad]
-            cen = xp[pt + y0:pt + y0 + 2 * R]
-            for tx in range(ntx):
-                for wx in range(4):
-                    s0 = tx * 128 + 4 * (8 * wx + q0)          # padded column of the first chunk (staged column - 16 + pl)
-                    f = rows[:, s0:s0 + 4 * nq]
-                    c = cen[:, pl + tx * 128 + 32 * wx:pl + tx * 128 + 32 * wx + 32]
-                    passed += (f.max() - c.min() <= th) and (c.max() - f.min() <= th)
-                    total += 1
-    return passed / total
+    E = 6 if rad <= 6 else (8 if rad <= 8 else 10)
+    fmin = _win(_win(x, 0, -rad, R - 1 + rad, np.minimum), 1, -E, E + 1, np.minimum)[::R, ::2]
+    fmax = _win(_win(x, 0, -rad, R - 1 + rad, np.maximum), 1, -E, E + 1, np.maximum)[::R, ::2]
+    cmin = _win(_win(x, 0, 0, R - 1, np.minimum), 1, 0, 1, np.minimum)[::R, ::2]
+    cmax = _win(_win(x, 0, 0, R - 1, np.maximum), 1, 0, 1, np.maximum)[::R, ::2]
+    flat = (fmax - cmin <= th) & (cmax - fmin <= th)
+    ty, tx = -(-flat.shape[0] // 4), -(-flat.shape[1] // 64)
+    tiles = np.ones((4 * ty, 64 * tx), bool)           # strips outside the image go with the flat ones
+    tiles[:flat.shape[0], :flat.shape[1]] = flat
+    ntap = (~tiles).reshape(ty, 4, tx, 64).sum(axis=(1, 3))
+    return float(flat.mean()), float(np.ceil(ntap / 32).sum() / (8 * ty * tx))
 
 
 def main():
@@ -94,7 +99,9 @@ def main():
         e1.record(stream)
         torch.cuda.synchronize()
         ms = e0.elapsed_time(e1) / args.reps
-        res[name] = {"ms": round(ms, 4), "gpx_s": round(n * H * W / ms / 1e6, 1), "predicted_flat_warps": round(flat_warp_share(img, RAD, TH, 4), 4)}
+        strips, tap_warps = flat_strip_model(img, RAD, TH, 4)
+        res[name] = {"ms": round(ms, 4), "gpx_s": round(n * H * W / ms / 1e6, 1), "predicted_flat_strips": round(strips, 4),
+                     "predicted_tap_warps": round(tap_warps, 4)}
     t = {k: res[k]["ms"] for k in inputs}
     if t["noise"] > t["const"]:
         res["measured_flat_share_video"] = round((t["noise"] - t["video"]) / (t["noise"] - t["const"]), 4)
