@@ -31,7 +31,7 @@ EXPORTS = [
     "dmc_disp8u2depth32f", "dmc_depth32f2disp8u", "dmc_depth16u2disp8u", "dmc_disp16s2depth16u",
     "dmc_fill_occlusion", "dmc_reproject_xyz", "dmc_transpose",
     "dmc_chain_batch_jpeg", "dmc_jpeg_probe", "dmc_jpeg_encode_bound", "dmc_jpeg_encode_gray_batch", "dmc_jpeg_degrade_gray_batch", "dmc_jpeg_encode_bound_ex", "dmc_jpeg_encode_gray_batch_ex", "dmc_jpeg_degrade_gray_batch_ex", "dmc_split_bgr_line_interleave", "dmc_project_points", "dmc_project_image_from_xyz", "dmc_fill_small_hole", "dmc_hostlink_probe", "dmc_release_device", "dmc_set_gateway", "dmc_get_gateway", "dmc_sched_get_routing",
-    "dmc_sse_gray_batch", "dmc_psnr_from_sse", "dmc_jpeg_rd_sweep",
+    "dmc_sse_gray_batch", "dmc_psnr_from_sse", "dmc_jpeg_rd_sweep", "dmc_jpeg_view_rd_sweep",
 ]
 MAX_DEVICES = 16
 RENDER_EXACT_DIVIDE = 1
@@ -92,6 +92,8 @@ def _load():
         "dmc_sse_gray_batch": (I, [P, P, P, I, I, I, I, C.POINTER(C.c_uint64)]),
         "dmc_psnr_from_sse": (D, [C.c_uint64, C.c_uint64]),
         "dmc_jpeg_rd_sweep": (I, [P, P, I, I, I, I, C.POINTER(I), I, I, C.POINTER(DmcChainParams), C.POINTER(C.c_uint64), C.POINTER(C.c_uint64), C.POINTER(C.c_uint64)]),
+        "dmc_jpeg_view_rd_sweep": (I, [P, P, P, I, I, I, I, C.POINTER(I), I, I, C.POINTER(DmcChainParams), D, C.POINTER(D), C.POINTER(D), I, C.POINTER(D), I, I,
+                                       C.POINTER(C.c_uint64), C.POINTER(C.c_uint64), C.POINTER(C.c_uint64)]),
         "dmc_sched_create": (I, [C.POINTER(I), I, C.POINTER(P)]), "dmc_sched_destroy": (None, [P]), "dmc_sched_device_count": (I, [P]),
         "dmc_sched_last_error": (C.c_char_p, [P]), "dmc_sched_chain_batch": (I, [P, P, P, I, I, I, C.POINTER(DmcChainParams)]),
         "dmc_multi_chain_batch": (I, [C.POINTER(I), I, P, P, I, I, I, C.POINTER(DmcChainParams), C.c_char_p, C.c_size_t]),

@@ -30,6 +30,9 @@ enum { JD_BITS, JD_META, JD_SCANS, JD_COEF, JD_OUT, JD_COUNT };
 // FrameDescs of a group, its staged source, coded and filtered frames (the staged second batch of dmc_sse_gray_batch),
 // and the group's results (SSE, stream lengths) that one copy brings back.
 enum { RD_TABS, RD_DESC, RD_SRC, RD_CODED, RD_FILT, RD_RES, RD_COUNT };
+// Device buffers of dmc_jpeg_view_rd_sweep: the group's staged textures, a depth frame, the points of the coded and of the
+// filtered depth (xyz), their projections, a raw render, the coded and filtered views, and the reference views.
+enum { VS_TEX, VS_DEPTH, VS_XYZ, VS_PT, VS_RAW, VS_VIEW, VS_REF, VS_COUNT };
 
 struct Buf { void* p = nullptr; size_t cap = 0; };
 
@@ -56,6 +59,7 @@ struct dmc_ctx {
     Buf render[2]; int* render_flag = nullptr;      // point-cloud render: attempt lists etc., device flag; pinned host flag
     Buf jpeg[JD_COUNT];
     Buf rd[RD_COUNT];
+    Buf vs[VS_COUNT];
     Buf jpeg_enc[11];            // JPEG encode: tables, staged frames, coefficients, block records, scan words, slots, lengths + offsets, staged output, decoder tables + descriptors,
                                  // optimised-table scratch, per-frame decoder Huffman tables
     // optional per-stage CUDA-event timing of the chain (bench.py's live roofline measurement)
@@ -557,6 +561,7 @@ void dmc_destroy(dmc_ctx* ctx) {
     for (auto& b : ctx->jpeg_enc) if (b.p) cudaFree(b.p);
     for (auto& b : ctx->rd) if (b.p) cudaFree(b.p);
     for (auto& b : ctx->render) if (b.p) cudaFree(b.p);
+    for (auto& b : ctx->vs) if (b.p) cudaFree(b.p);
     if (ctx->render_flag) cudaFreeHost(ctx->render_flag);
     for (auto& r : ctx->prof_pending) { cudaEventDestroy(r.a); cudaEventDestroy(r.b); }
     for (auto e : ctx->prof_free) cudaEventDestroy(e);
@@ -1172,6 +1177,45 @@ int dmc_sse_gray_batch(dmc_ctx* ctx, const void* a, const void* b, int n_frames,
     return DMC_OK;
 }
 
+namespace {
+
+// The sweeps' per-quality tables in RD_TABS, kRdRec bytes a quality: [EncTables][DC, AC HuffTable][QuantTable].
+constexpr size_t kRdHuff = (sizeof(dmcjpeg::EncTables) + 15) & ~(size_t)15, kRdQuant = kRdHuff + 2 * sizeof(dmcjpeg::HuffTable);
+constexpr size_t kRdRec = (kRdQuant + sizeof(dmcjpeg::QuantTable) + 255) & ~(size_t)255;
+
+// Builds every quality's encoder tables and the decoder tables parsed from its header, and uploads them in one copy.
+// `host` holds them until the copy has been made.
+int rd_tables(dmc_ctx* ctx, const char* what, int rows, int cols, const int* qualities, int n_q, std::vector<char>& host) {
+    host.assign(kRdRec * n_q, 0);
+    for (int k = 0; k < n_q; k++) {
+        dmcjpeg::EncTables t;
+        dmcjpeg::make_enc_tables(qualities[k], rows, cols, &t);
+        std::vector<dmcjpeg::QuantTable> qpool; std::vector<dmcjpeg::HuffTable> hpool; dmcjpeg::FrameDesc hd;
+        const std::string why = jpeg_parse_frame(t.header, dmcjpeg::kEncHeaderBytes, 0, rows, cols, qpool, hpool, &hd);
+        if (!why.empty() || hpool.size() != 2 || qpool.size() != 1 || hd.dc != 0 || hd.ac != 1 || hd.qt != 0)
+            return fail(ctx, DMC_ERR_TYPE, std::string(what) + ": encoder header does not parse: " + why);
+        char* r = host.data() + kRdRec * k;
+        memcpy(r, &t, sizeof t);
+        memcpy(r + kRdHuff, hpool.data(), 2 * sizeof(dmcjpeg::HuffTable));
+        memcpy(r + kRdQuant, qpool.data(), sizeof(dmcjpeg::QuantTable));
+    }
+    TRY(reserve(ctx, ctx->rd[RD_TABS], host.size()));
+    CUDA_TRY(ctx, cudaMemcpyAsync(ctx->rd[RD_TABS].p, host.data(), host.size(), cudaMemcpyHostToDevice, ctx->stream));
+    return DMC_OK;
+}
+
+// Codes the nf device frames dsrc at the sweep's k-th quality and decodes them into `coded`; the stream lengths stay in
+// JE_LENS.  RD_DESC holds the group's FrameDescs.
+int rd_degrade(dmc_ctx* ctx, int k, const uint8_t* dsrc, int nf, int rows, int cols, bool optimize, uint8_t* coded) {
+    const char* tk = (const char*)ctx->rd[RD_TABS].p + kRdRec * k;
+    TRY(jpeg_enc_group(ctx, tk, dsrc, DMC_MEM_DEVICE, 0, nf, rows, cols, optimize, ctx->rd[RD_DESC].p));
+    LAUNCH(ctx, launch_jpeg_decode((const uint8_t*)ctx->jpeg_enc[JE_SLOTS].p, ctx->rd[RD_DESC].p, optimize ? ctx->jpeg_enc[JE_HUFF].p : tk + kRdHuff, tk + kRdQuant,
+                                   (uint8_t*)ctx->jpeg_enc[JE_WORDS].p, nullptr, coded, nf, 0, rows, cols, ctx->stream));
+    return DMC_OK;
+}
+
+}  // namespace
+
 // The sweep runs group by group (a group is sized like the encoder's, counting the coded and filtered frames and the
 // chain's ping-pong too) and, inside a group, quality by quality: a host source is copied to the device once per group.
 // Every quality's encoder tables and the decoder tables parsed from its header are built once and uploaded in one copy.
@@ -1204,23 +1248,8 @@ int dmc_jpeg_rd_sweep(dmc_ctx* ctx, const void* src, int src_mem, int n_frames, 
     const size_t per = l.coef_bytes + l.info_bytes + l.word_bytes + l.slot_bytes + (optimize ? l.opt_bytes + 2 * sizeof(dmcjpeg::HuffTable) : 0) +
                        sizeof(dmcjpeg::FrameDesc) + fpx * ((host ? 1 : 0) + 1 + (p ? 3 : 0));      // staged source, coded, filtered, ping, pong
     const int group = chunk_frames(kEncGroupBytes, per, n_frames, 2048, false);
-    // per quality: [EncTables][DC, AC HuffTable][QuantTable]
-    const size_t o_h = (sizeof(dmcjpeg::EncTables) + 15) & ~(size_t)15, o_q = o_h + 2 * sizeof(dmcjpeg::HuffTable);
-    const size_t rec = (o_q + sizeof(dmcjpeg::QuantTable) + 255) & ~(size_t)255;
-    std::vector<char> tabs(rec * n_q);
-    for (int k = 0; k < n_q; k++) {
-        dmcjpeg::EncTables t;
-        dmcjpeg::make_enc_tables(qualities[k], rows, cols, &t);
-        std::vector<dmcjpeg::QuantTable> qpool; std::vector<dmcjpeg::HuffTable> hpool; dmcjpeg::FrameDesc hd;
-        const std::string why = jpeg_parse_frame(t.header, dmcjpeg::kEncHeaderBytes, 0, rows, cols, qpool, hpool, &hd);
-        if (!why.empty() || hpool.size() != 2 || qpool.size() != 1 || hd.dc != 0 || hd.ac != 1 || hd.qt != 0)
-            return fail(ctx, DMC_ERR_TYPE, "dmc_jpeg_rd_sweep: encoder header does not parse: " + why);
-        char* r = tabs.data() + rec * k;
-        memcpy(r, &t, sizeof t);
-        memcpy(r + o_h, hpool.data(), 2 * sizeof(dmcjpeg::HuffTable));
-        memcpy(r + o_q, qpool.data(), sizeof(dmcjpeg::QuantTable));
-    }
-    TRY(reserve(ctx, ctx->rd[RD_TABS], tabs.size()));
+    std::vector<char> tabs;
+    TRY(rd_tables(ctx, "dmc_jpeg_rd_sweep", rows, cols, qualities, n_q, tabs));
     TRY(reserve(ctx, ctx->rd[RD_DESC], (size_t)group * sizeof(dmcjpeg::FrameDesc)));
     TRY(reserve(ctx, ctx->rd[RD_CODED], fpx * group));
     if (p) TRY(reserve(ctx, ctx->rd[RD_FILT], fpx * group));
@@ -1228,7 +1257,6 @@ int dmc_jpeg_rd_sweep(dmc_ctx* ctx, const void* src, int src_mem, int n_frames, 
     // results of a group of nf frames: [sse_coded][sse_filtered] (uint64, [quality][frame]), then the lengths (uint32)
     const size_t res_bytes = (size_t)n_q * group * (2 * sizeof(uint64_t) + sizeof(uint32_t));
     TRY(reserve(ctx, ctx->rd[RD_RES], res_bytes));
-    CUDA_TRY(ctx, cudaMemcpyAsync(ctx->rd[RD_TABS].p, tabs.data(), tabs.size(), cudaMemcpyHostToDevice, s));
     Slot& sl = ctx->slot[0]; sl.stream = s;
     uint8_t* coded = (uint8_t*)ctx->rd[RD_CODED].p;
     uint8_t* filt = (uint8_t*)ctx->rd[RD_FILT].p;
@@ -1244,10 +1272,7 @@ int dmc_jpeg_rd_sweep(dmc_ctx* ctx, const void* src, int src_mem, int n_frames, 
         uint64_t* d_sf = d_sc + (size_t)n_q * nf;
         uint32_t* d_len = (uint32_t*)(d_sf + (size_t)n_q * nf);
         for (int k = 0; k < n_q; k++) {
-            const char* tk = (const char*)ctx->rd[RD_TABS].p + rec * k;
-            TRY(jpeg_enc_group(ctx, tk, dsrc, DMC_MEM_DEVICE, 0, nf, rows, cols, optimize, ctx->rd[RD_DESC].p));
-            LAUNCH(ctx, launch_jpeg_decode((const uint8_t*)ctx->jpeg_enc[JE_SLOTS].p, ctx->rd[RD_DESC].p, optimize ? ctx->jpeg_enc[JE_HUFF].p : tk + o_h, tk + o_q,
-                                           (uint8_t*)ctx->jpeg_enc[JE_WORDS].p, nullptr, coded, nf, 0, rows, cols, s));
+            TRY(rd_degrade(ctx, k, dsrc, nf, rows, cols, optimize, coded));
             if (p) TRY(run_chain(ctx, sl, coded, filt, nf, rows, cols, *p));
             LAUNCH(ctx, launch_sse_u8(dsrc, coded, p ? filt : nullptr, d_sc + (size_t)k * nf, p ? d_sf + (size_t)k * nf : nullptr, nf, fpx, s));
             CUDA_TRY(ctx, cudaMemcpyAsync(d_len + (size_t)k * nf, ctx->jpeg_enc[JE_LENS].p, nf * sizeof(uint32_t), cudaMemcpyDeviceToDevice, s));
@@ -1480,6 +1505,26 @@ int dmc_transpose(dmc_ctx* ctx, const dmc_image* src, dmc_image* dst) {
     return stage_out_end(ctx, dst, out, s);
 }
 
+}  // extern "C"
+
+namespace {
+// reprojectXYZ's column table of width W and focal length f in ctx->xtab: x = (-cw)*fxinv; x += fxinv per column (:469, :478)
+int reproject_table(dmc_ctx* ctx, int W, double f) {
+    if (ctx->xtab && ctx->xtab_w == W && ctx->xtab_f == f) return DMC_OK;
+    const float fxinv = (float)(1.0 / f), cw = (W - 1) * 0.5f;
+    std::vector<float> tab(W);
+    volatile float x = (-cw) * fxinv;
+    for (int i = 0; i < W; i++) { tab[i] = x; x = x + fxinv; }
+    if (ctx->xtab) { CUDA_TRY(ctx, cudaStreamSynchronize(ctx->stream)); CUDA_TRY(ctx, cudaFree(ctx->xtab)); ctx->xtab = nullptr; }
+    CUDA_TRY(ctx, cudaMalloc(&ctx->xtab, W * sizeof(float)));
+    CUDA_TRY(ctx, cudaMemcpy(ctx->xtab, tab.data(), W * sizeof(float), cudaMemcpyHostToDevice));
+    ctx->xtab_w = W; ctx->xtab_f = f;
+    return DMC_OK;
+}
+}  // namespace
+
+extern "C" {
+
 int dmc_reproject_xyz(dmc_ctx* ctx, const dmc_image* depth, dmc_image* xyz, double f) {
     if (!ctx) return fail(nullptr, DMC_ERR_ARG, "null context");
     TRY(check_image(ctx, depth, "depth")); TRY(check_image(ctx, xyz, "xyz"));
@@ -1490,20 +1535,9 @@ int dmc_reproject_xyz(dmc_ctx* ctx, const dmc_image* depth, dmc_image* xyz, doub
     if (xyz->step && xyz->step != dense_step(xyz)) return fail(ctx, DMC_ERR_SIZE, "reprojectXYZ: xyz must be dense");
     const void* in; void* out;
     TRY(stage_op(ctx, depth, xyz, &in, &out));
-    const cudaStream_t s = ctx->stream;
-    const float fxinv = (float)(1.0 / f), fyinv = (float)(1.0 / f);
-    const float cw = (W - 1) * 0.5f, ch = (H - 1) * 0.5f;
-    if (!ctx->xtab || ctx->xtab_w != W || ctx->xtab_f != f) {       // x = (-cw)*fxinv; x += fxinv per column (:469, :478)
-        std::vector<float> tab(W);
-        volatile float x = (-cw) * fxinv;
-        for (int i = 0; i < W; i++) { tab[i] = x; x = x + fxinv; }
-        if (ctx->xtab) { CUDA_TRY(ctx, cudaStreamSynchronize(s)); CUDA_TRY(ctx, cudaFree(ctx->xtab)); ctx->xtab = nullptr; }
-        CUDA_TRY(ctx, cudaMalloc(&ctx->xtab, W * sizeof(float)));
-        CUDA_TRY(ctx, cudaMemcpy(ctx->xtab, tab.data(), W * sizeof(float), cudaMemcpyHostToDevice));
-        ctx->xtab_w = W; ctx->xtab_f = f;
-    }
-    LAUNCH(ctx, launch_reproject(in, (float*)out, ctx->xtab, H, W, t, fyinv, ch, s));
-    return stage_out_end(ctx, xyz, out, s);
+    TRY(reproject_table(ctx, W, f));
+    LAUNCH(ctx, launch_reproject(in, (float*)out, ctx->xtab, 1, H, W, t, (float)(1.0 / f), (H - 1) * 0.5f, ctx->stream));
+    return stage_out_end(ctx, xyz, out, ctx->stream);
 }
 
 // ---- point-cloud render (SURVEY.md 8f-3) ------------------------------------------------------------------------------
@@ -1511,6 +1545,16 @@ namespace {
 void camera_floats(const double* R, const double* t, const double* K, float kr[9], float tt[3]) {      // Mat kr = K*R; (float)kr(i,j)  depthmapUtil.cpp:12-29
     for (int i = 0; i < 3; i++) for (int j = 0; j < 3; j++) { double s = 0; for (int k = 0; k < 3; k++) s += K[3 * i + k] * R[3 * k + j]; kr[3 * i + j] = (float)s; }
     for (int i = 0; i < 3; i++) tt[i] = (float)t[i];
+}
+
+// projectImagefromXYZ's splat of `frames` frames (pt already projected) into dest (and depth, if not NULL).
+int render(dmc_ctx* ctx, const uint8_t* image, const float* xyz, const float* pt, int frames, int rows, int cols, int is_sub, uint8_t* dest, float* depth) {
+    TRY(reserve(ctx, ctx->render[0], render_scratch_bytes(frames, rows, cols)));
+    TRY(reserve(ctx, ctx->render[1], 64));
+    if (!ctx->render_flag) CUDA_TRY(ctx, cudaHostAlloc((void**)&ctx->render_flag, 64, cudaHostAllocDefault));
+    const int nk = launch_render(image, xyz, pt, frames, rows, cols, is_sub, dest, depth, ctx->render[0].p, (int*)ctx->render[1].p, ctx->render_flag, ctx->stream);
+    if (nk < 0) return fail(ctx, DMC_ERR_CUDA, std::string("projectImagefromXYZ: the splat did not settle: ") + cudaGetErrorString(cudaGetLastError()));
+    return after_launch(ctx, nk);
 }
 }  // namespace
 
@@ -1525,7 +1569,7 @@ int dmc_project_points(dmc_ctx* ctx, const dmc_image* xyz, const double* R, cons
     TRY(stage_op(ctx, xyz, pt, &in, &out));
     const cudaStream_t s = ctx->stream;
     float kr[9], tt[3]; camera_floats(R, t, K, kr, tt);
-    LAUNCH(ctx, launch_project_points((const float*)in, (float*)out, n, kr, tt, flags & DMC_RENDER_EXACT_DIVIDE, s));
+    LAUNCH(ctx, launch_project_points((const float*)in, (float*)out, 1, n, kr, tt, flags & DMC_RENDER_EXACT_DIVIDE, s));
     return stage_out_end(ctx, pt, out, s);
 }
 
@@ -1549,15 +1593,9 @@ int dmc_project_image_from_xyz(dmc_ctx* ctx, const dmc_image* image, dmc_image* 
     TRY(stage_out_begin(ctx, dest, d_img, image_bytes(image), sl.buf[SB_OUT], &d_dest));
     if (depth) { if (depth->mem == DMC_MEM_DEVICE && step_of(depth) == dense_step(depth)) d_depth = depth->data; else { TRY(reserve(ctx, sl.buf[SB_PONG], (size_t)n * 4)); d_depth = sl.buf[SB_PONG].p; } }
     if (pt && pt->mem == DMC_MEM_DEVICE) d_pt = pt->data; else { TRY(reserve(ctx, sl.buf[SB_FLOAT], (size_t)n * 8)); d_pt = sl.buf[SB_FLOAT].p; }
-    TRY(reserve(ctx, ctx->render[0], render_scratch_bytes(H, W)));
-    TRY(reserve(ctx, ctx->render[1], 64));
-    if (!ctx->render_flag) CUDA_TRY(ctx, cudaHostAlloc((void**)&ctx->render_flag, 64, cudaHostAllocDefault));
     float kr[9], tt[3]; camera_floats(R, t, K, kr, tt);
-    LAUNCH(ctx, launch_project_points((const float*)d_xyz, (float*)d_pt, n, kr, tt, flags & DMC_RENDER_EXACT_DIVIDE, s));
-    int nk = launch_render((const uint8_t*)d_img, (const float*)d_xyz, (const float*)d_pt, H, W, is_sub, (uint8_t*)d_dest, (float*)d_depth,
-                           ctx->render[0].p, (int*)ctx->render[1].p, ctx->render_flag, s);
-    if (nk < 0) return fail(ctx, DMC_ERR_CUDA, std::string("projectImagefromXYZ: ") + cudaGetErrorString(cudaGetLastError()));
-    TRY(after_launch(ctx, nk));
+    LAUNCH(ctx, launch_project_points((const float*)d_xyz, (float*)d_pt, 1, n, kr, tt, flags & DMC_RENDER_EXACT_DIVIDE, s));
+    TRY(render(ctx, (const uint8_t*)d_img, (const float*)d_xyz, (const float*)d_pt, 1, H, W, is_sub, (uint8_t*)d_dest, (float*)d_depth));
     if (depth && d_depth != depth->data) TRY(stage_out_end(ctx, depth, d_depth, s));
     if (pt && d_pt != pt->data) TRY(stage_out_end(ctx, pt, d_pt, s));
     return stage_out_end(ctx, dest, d_dest, s);
@@ -1581,9 +1619,157 @@ int dmc_fill_small_hole(dmc_ctx* ctx, const dmc_image* src, dmc_image* dst) {
         if (same) CUDA_TRY(ctx, cudaMemcpyAsync(out, in, image_bytes(src), cudaMemcpyDeviceToDevice, s));
         else CUDA_TRY(ctx, cudaMemcpy2DAsync(out, row, dst->data, step_of(dst), row, dst->rows, dst->mem == DMC_MEM_HOST ? cudaMemcpyHostToDevice : cudaMemcpyDeviceToDevice, s));
     }
-    int nk = launch_fill_small_hole((const uint8_t*)in, (uint8_t*)out, src->rows, src->cols, s);
+    int nk = launch_fill_small_hole((const uint8_t*)in, (uint8_t*)out, 1, src->rows, src->cols, s);
     TRY(after_launch(ctx, nk));
     return stage_out_end(ctx, dst, out, s);
+}
+
+}  // extern "C"
+
+namespace {
+// view(depth) of nf frames for one camera: projectImagefromXYZ of the textures at the points xyz into `raw`, then
+// fillSmallHole in place, which reads a copy of its source (src.copyTo(src_), depthmapUtil.cpp:189-193): `out` starts as
+// the raw render and receives the filled holes.
+int render_view(dmc_ctx* ctx, const uint8_t* tex, const float* xyz, float* pt, uint8_t* raw, uint8_t* out, int nf, int rows, int cols,
+                const float* kr, const float* tt, int is_sub, int exact) {
+    const cudaStream_t s = ctx->stream;
+    const long n = (long)rows * cols;
+    LAUNCH(ctx, launch_project_points(xyz, pt, nf, n, kr, tt, exact, s));
+    TRY(render(ctx, tex, xyz, pt, nf, rows, cols, is_sub, raw, nullptr));
+    CUDA_TRY(ctx, cudaMemcpyAsync(out, raw, (size_t)3 * n * nf, cudaMemcpyDeviceToDevice, s));
+    LAUNCH(ctx, launch_fill_small_hole(raw, out, nf, rows, cols, s));
+    return DMC_OK;
+}
+
+// D(x) of nf 8-bit frames: disp8U2depth32F(x, focus * baseline, amp, 0), one launch per frame because the converter's
+// SIMD body / scalar tail split is per call; then reprojectXYZ into xyz.
+int depth_points(dmc_ctx* ctx, const uint8_t* disp, float* depth, float* xyz, int nf, int rows, int cols, const dmc_chain_params& p, double f) {
+    const size_t fpx = (size_t)rows * cols;
+    for (int i = 0; i < nf; i++)
+        LAUNCH(ctx, launch_convert(0, disp + fpx * i, depth + fpx * i, (long)fpx, (float)(p.focus * p.baseline), (float)p.amp, 0.f, ctx->stream));
+    LAUNCH(ctx, launch_reproject(depth, xyz, ctx->xtab, nf, rows, cols, DMC_32F, (float)(1.0 / f), (rows - 1) * 0.5f, ctx->stream));
+    return DMC_OK;
+}
+}  // namespace
+
+extern "C" {
+
+// Group by group (sized like dmc_jpeg_rd_sweep's groups, plus the render's scratch, the points and the views), the reference
+// views of every camera are rendered once; then quality by quality the frames are coded, decoded, converted (D) and
+// filtered, both depths reprojected, and per camera both rendered and compared with the reference view in one SSE launch.
+// Every render of nf frames is one batched render; its fixed point costs one host read per iteration.  One copy per group
+// brings the results back.
+int dmc_jpeg_view_rd_sweep(dmc_ctx* ctx, const void* disp, const void* texture, int src_mem, int n_frames, int rows, int cols,
+                           const int* qualities, int n_q, int flags, const dmc_chain_params* p, double f,
+                           const double* R, const double* t, int n_views, const double* K, int is_sub, int render_flags,
+                           uint64_t* bytes, uint64_t* sse_view_coded, uint64_t* sse_view_filtered) {
+    if (!ctx) return fail(nullptr, DMC_ERR_ARG, "null context");
+    if (!qualities || n_q < 1) return fail(ctx, DMC_ERR_ARG, "dmc_jpeg_view_rd_sweep: no qualities");
+    for (int k = 0; k < n_q; k++)
+        if (qualities[k] < 0 || qualities[k] > 100) return fail(ctx, DMC_ERR_ARG, "dmc_jpeg_view_rd_sweep: quality must be in 0..100");
+    if (flags & ~DMC_JPEG_OPTIMIZE_HUFFMAN) return fail(ctx, DMC_ERR_ARG, "dmc_jpeg_view_rd_sweep: unknown flags " + std::to_string(flags));
+    if (render_flags & ~DMC_RENDER_EXACT_DIVIDE) return fail(ctx, DMC_ERR_ARG, "dmc_jpeg_view_rd_sweep: unknown render_flags " + std::to_string(render_flags));
+    if (!p) return fail(ctx, DMC_ERR_ARG, "dmc_jpeg_view_rd_sweep: chain parameters are required");
+    TRY(check_chain_params(ctx, *p));
+    if (p->chain != DMC_CHAIN_DEPTH32F) return fail(ctx, DMC_ERR_ARG, "dmc_jpeg_view_rd_sweep: the chain must be DMC_CHAIN_DEPTH32F (filterDisp8U2Depth32F, the depth that is rendered)");
+    // (for any other method the reference's 32F chain leaves dest unwritten: there would be nothing to render)
+    if (p->brange_method != DMC_FULL_KERNEL && p->brange_method != DMC_FULL_KERNEL_PAIR && p->brange_method != DMC_SEPARABLE_KERNEL)
+        return fail(ctx, DMC_ERR_ARG, "dmc_jpeg_view_rd_sweep: brange_method must be FULL_KERNEL, FULL_KERNEL_PAIR or SEPARABLE_KERNEL");
+    if (n_views < 1 || !R || !t || !K) return fail(ctx, DMC_ERR_ARG, "dmc_jpeg_view_rd_sweep: at least one camera (R, t, K) is required");
+    if (src_mem != DMC_MEM_HOST && src_mem != DMC_MEM_DEVICE) return fail(ctx, DMC_ERR_ARG, "dmc_jpeg_view_rd_sweep: bad mem");
+    uint64_t bound;
+    if (dmc_jpeg_encode_bound_ex(rows, cols, flags, &bound) != DMC_OK) return fail(ctx, DMC_ERR_SIZE, "dmc_jpeg_view_rd_sweep: " + g_err);
+    const size_t fpx = (size_t)rows * cols;
+    if (fpx >= ((size_t)1 << 29)) return fail(ctx, DMC_ERR_SIZE, "dmc_jpeg_view_rd_sweep: frame too large for the renderer");
+    if (n_frames < 0 || (n_frames > 0 && (!disp || !texture || !bytes || !sse_view_coded || !sse_view_filtered))) return fail(ctx, DMC_ERR_SIZE, "dmc_jpeg_view_rd_sweep: bad arguments");
+    if (n_frames == 0) return DMC_OK;
+    CUDA_TRY(ctx, cudaSetDevice(ctx->device));
+    cudaStream_t s = ctx->stream;
+    const bool optimize = (flags & DMC_JPEG_OPTIMIZE_HUFFMAN) != 0, host = src_mem == DMC_MEM_HOST;
+    const int exact = render_flags & DMC_RENDER_EXACT_DIVIDE;
+    const JpegEncLayout l = jpeg_enc_layout(rows, cols, optimize);
+    // per frame: the encoder's scratch and FrameDesc; staged source and texture; coded, ping, pong, float scratch of the chain;
+    // depth, two sets of points, their projection; raw render, coded and filtered views, reference views; the render's scratch
+    const size_t per = l.coef_bytes + l.info_bytes + l.word_bytes + l.slot_bytes + (optimize ? l.opt_bytes + 2 * sizeof(dmcjpeg::HuffTable) : 0) +
+                       sizeof(dmcjpeg::FrameDesc) + fpx * ((host ? 4 : 0) + 3 + 4 + 4 + 24 + 8 + 9 + 3 * (size_t)n_views) + render_scratch_bytes(1, rows, cols);
+    // the render's attempt offsets are uint32 (at most 7 attempts a point) and the frame is a grid dimension
+    const size_t cap = ((size_t)UINT32_MAX / (7 * fpx)) < 2048 ? (size_t)UINT32_MAX / (7 * fpx) : 2048;
+    const int group = chunk_frames(kEncGroupBytes, per, n_frames, (int)cap, false);
+    std::vector<char> tabs;
+    TRY(rd_tables(ctx, "dmc_jpeg_view_rd_sweep", rows, cols, qualities, n_q, tabs));
+    TRY(reproject_table(ctx, cols, f));
+    TRY(reserve(ctx, ctx->rd[RD_DESC], (size_t)group * sizeof(dmcjpeg::FrameDesc)));
+    TRY(reserve(ctx, ctx->rd[RD_CODED], fpx * group));
+    if (host) { TRY(reserve(ctx, ctx->rd[RD_SRC], fpx * group)); TRY(reserve(ctx, ctx->vs[VS_TEX], 3 * fpx * group)); }
+    TRY(reserve(ctx, ctx->vs[VS_DEPTH], 4 * fpx * group));
+    TRY(reserve(ctx, ctx->vs[VS_XYZ], 2 * 12 * fpx * group));
+    TRY(reserve(ctx, ctx->vs[VS_PT], 8 * fpx * group));
+    TRY(reserve(ctx, ctx->vs[VS_RAW], 3 * fpx * group));
+    TRY(reserve(ctx, ctx->vs[VS_VIEW], 2 * 3 * fpx * group));
+    TRY(reserve(ctx, ctx->vs[VS_REF], 3 * fpx * group * (size_t)n_views));
+    TRY(reserve(ctx, ctx->render[0], render_scratch_bytes(group, rows, cols)));
+    // results of a group of nf frames: [sse_view_coded][sse_view_filtered] (uint64, [quality][view][frame]), the lengths (uint32)
+    const size_t per_res = (size_t)n_q * (2 * sizeof(uint64_t) * n_views + sizeof(uint32_t));
+    TRY(reserve(ctx, ctx->rd[RD_RES], per_res * group));
+    std::vector<float> kr(9 * (size_t)n_views), tt(3 * (size_t)n_views);
+    for (int v = 0; v < n_views; v++) camera_floats(R + 9 * v, t + 3 * v, K, &kr[9 * v], &tt[3 * v]);
+    Slot& sl = ctx->slot[0]; sl.stream = s;
+    uint8_t* coded = (uint8_t*)ctx->rd[RD_CODED].p;
+    float* depth = (float*)ctx->vs[VS_DEPTH].p;
+    float* pt = (float*)ctx->vs[VS_PT].p;
+    uint8_t* raw = (uint8_t*)ctx->vs[VS_RAW].p;
+    std::vector<char> res;
+    for (int f0 = 0; f0 < n_frames; f0 += group) {
+        const int nf = n_frames - f0 < group ? n_frames - f0 : group;
+        const size_t vb = 3 * fpx * nf;           // bytes of the group's views of one camera
+        float* xyz_c = (float*)ctx->vs[VS_XYZ].p;
+        float* xyz_f = xyz_c + 3 * fpx * nf;
+        uint8_t* view_c = (uint8_t*)ctx->vs[VS_VIEW].p;
+        uint8_t* view_f = view_c + vb;
+        uint8_t* ref = (uint8_t*)ctx->vs[VS_REF].p;
+        const uint8_t* dsrc = (const uint8_t*)disp + fpx * f0;
+        const uint8_t* dtex = (const uint8_t*)texture + 3 * fpx * f0;
+        if (host) {
+            CUDA_TRY(ctx, cudaMemcpyAsync(ctx->rd[RD_SRC].p, dsrc, fpx * nf, cudaMemcpyHostToDevice, s));
+            CUDA_TRY(ctx, cudaMemcpyAsync(ctx->vs[VS_TEX].p, dtex, vb, cudaMemcpyHostToDevice, s));
+            dsrc = (const uint8_t*)ctx->rd[RD_SRC].p;
+            dtex = (const uint8_t*)ctx->vs[VS_TEX].p;
+        }
+        TRY(depth_points(ctx, dsrc, depth, xyz_c, nf, rows, cols, *p, f));
+        for (int v = 0; v < n_views; v++) TRY(render_view(ctx, dtex, xyz_c, pt, raw, ref + vb * v, nf, rows, cols, &kr[9 * v], &tt[3 * v], is_sub, exact));
+        uint64_t* d_sc = (uint64_t*)ctx->rd[RD_RES].p;
+        uint64_t* d_sf = d_sc + (size_t)n_q * n_views * nf;
+        uint32_t* d_len = (uint32_t*)(d_sf + (size_t)n_q * n_views * nf);
+        for (int k = 0; k < n_q; k++) {
+            TRY(rd_degrade(ctx, k, dsrc, nf, rows, cols, optimize, coded));
+            CUDA_TRY(ctx, cudaMemcpyAsync(d_len + (size_t)k * nf, ctx->jpeg_enc[JE_LENS].p, nf * sizeof(uint32_t), cudaMemcpyDeviceToDevice, s));
+            TRY(depth_points(ctx, coded, depth, xyz_c, nf, rows, cols, *p, f));
+            TRY(run_chain(ctx, sl, coded, depth, nf, rows, cols, *p));
+            LAUNCH(ctx, launch_reproject(depth, xyz_f, ctx->xtab, nf, rows, cols, DMC_32F, (float)(1.0 / f), (rows - 1) * 0.5f, s));
+            for (int v = 0; v < n_views; v++) {
+                TRY(render_view(ctx, dtex, xyz_c, pt, raw, view_c, nf, rows, cols, &kr[9 * v], &tt[3 * v], is_sub, exact));
+                TRY(render_view(ctx, dtex, xyz_f, pt, raw, view_f, nf, rows, cols, &kr[9 * v], &tt[3 * v], is_sub, exact));
+                const size_t o = ((size_t)k * n_views + v) * nf;
+                LAUNCH(ctx, launch_sse_u8(ref + vb * v, view_c, view_f, d_sc + o, d_sf + o, nf, 3 * fpx, s));
+            }
+        }
+        const size_t used = per_res * nf;
+        res.resize(used);
+        CUDA_TRY(ctx, cudaMemcpyAsync(res.data(), ctx->rd[RD_RES].p, used, cudaMemcpyDeviceToHost, s));
+        CUDA_TRY(ctx, cudaStreamSynchronize(s));
+        const uint64_t* sc = (const uint64_t*)res.data();
+        const uint64_t* sf = sc + (size_t)n_q * n_views * nf;
+        const uint32_t* len = (const uint32_t*)(sf + (size_t)n_q * n_views * nf);
+        for (int k = 0; k < n_q; k++)
+            for (int i = 0; i < nf; i++) {
+                bytes[(size_t)k * n_frames + f0 + i] = len[(size_t)k * nf + i];
+                for (int v = 0; v < n_views; v++) {
+                    const size_t o = ((size_t)k * n_views + v) * n_frames + f0 + i, j = ((size_t)k * n_views + v) * nf + i;
+                    sse_view_coded[o] = sc[j]; sse_view_filtered[o] = sf[j];
+                }
+            }
+    }
+    return DMC_OK;
 }
 
 // splitBGRLineInterleave filter.h:12 (split.cpp:167-177): 8UC3 / 32FC3 -> single channel, 3*rows x cols

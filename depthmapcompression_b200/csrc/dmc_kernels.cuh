@@ -46,9 +46,10 @@ int launch_convert(int kind, const void* src, void* dst, long n, float fb, float
 int launch_f32_to_u16(const float* src, uint16_t* dst, long n, cudaStream_t s);   // Mat::convertTo(CV_16U)
 // fillOcclusion_<T> / Inv_ (depthmapUtil.cpp:548-636): `pristine` is an untouched copy of `img`
 int launch_fill_occlusion(void* img, const void* pristine, int H, int W, int depth, double invalid, int inv, cudaStream_t s);
-// reprojectXYZ_<T> (depthmapUtil.cpp:450-481): xtab[i] = running FP32 sum along the row, computed by the host
 int launch_transpose(const void* src, void* dst, int H, int W, int elem_size, cudaStream_t s);   // cv::transpose, single channel
-int launch_reproject(const void* depth, float* xyz, const float* xtab, int H, int W, int dtype, float fyinv, float ch, cudaStream_t s);
+// reprojectXYZ_<T> (depthmapUtil.cpp:450-481) of `frames` frames: xtab[i] = running FP32 sum along the row, computed by the
+// host and shared by the frames
+int launch_reproject(const void* depth, float* xyz, const float* xtab, int frames, int H, int W, int dtype, float fyinv, float ch, cudaStream_t s);
 
 }  // namespace dmc
 
@@ -102,12 +103,12 @@ int launch_sse_u8(const uint8_t* a, const uint8_t* b0, const uint8_t* b1, uint64
 }
 
 namespace dmc {
-// point-cloud render (dmc_render.cu)
-int launch_project_points(const float* xyz, float* pt, long n, const float kr[9], const float t[3], int exact_divide, cudaStream_t s);
-size_t render_scratch_bytes(int rows, int cols);
-int launch_render(const uint8_t* image, const float* xyz, const float* pt, int rows, int cols, int is_sub, uint8_t* dest, float* depth,
+// point-cloud render (dmc_render.cu), `frames` dense frames of n = rows x cols points / pixels back to back, one camera
+int launch_project_points(const float* xyz, float* pt, int frames, long n, const float kr[9], const float t[3], int exact_divide, cudaStream_t s);
+size_t render_scratch_bytes(int frames, int rows, int cols);
+int launch_render(const uint8_t* image, const float* xyz, const float* pt, int frames, int rows, int cols, int is_sub, uint8_t* dest, float* depth,
                   void* scratch, int* changed_dev, int* changed_host, cudaStream_t s);
-int launch_fill_small_hole(const uint8_t* src, uint8_t* dst, int rows, int cols, cudaStream_t s);
+int launch_fill_small_hole(const uint8_t* src, uint8_t* dst, int frames, int rows, int cols, cudaStream_t s);
 int launch_split_line_interleave(const void* src, void* dst, int rows, int cols, int elem, cudaStream_t s);
 }
 

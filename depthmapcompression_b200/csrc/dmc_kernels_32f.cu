@@ -202,20 +202,22 @@ int launch_fill_occlusion(void* img, const void* pristine, int H, int W, int dep
 
 // ----------------------------------------------------------------------------------------------------------
 // reprojectXYZ_<T> (depthmapUtil.cpp:450-481): xyz = (x*z, y*z, z==0 ? 10000 : z); x is the reference's running
-// FP32 sum along the row (xtab, built by the host with the same serial adds), y = (j - ch) * fyinv.
+// FP32 sum along the row (xtab, built by the host with the same serial adds), y = (j - ch) * fyinv.  Frame = blockIdx.z.
 // ----------------------------------------------------------------------------------------------------------
 template <typename T>
 __global__ void reproject_kernel(const T* __restrict__ depth, float* __restrict__ xyz, const float* __restrict__ xtab, int H, int W, float fyinv, float ch) {
     int i = blockIdx.x * blockDim.x + threadIdx.x, j = blockIdx.y;
     if (i >= W) return;
+    const size_t g = ((size_t)blockIdx.z * H + j) * W + i;
     float y = __fmul_rn(__fsub_rn((float)j, ch), fyinv);
-    float z = (float)depth[(size_t)j * W + i];
-    float* o = xyz + ((size_t)j * W + i) * 3;
+    float z = (float)depth[g];
+    float* o = xyz + g * 3;
     o[0] = __fmul_rn(xtab[i], z); o[1] = __fmul_rn(y, z); o[2] = (z == 0) ? 10000.f : z;
 }
 
-int launch_reproject(const void* depth, float* xyz, const float* xtab, int H, int W, int dtype, float fyinv, float ch, cudaStream_t s) {
-    dim3 grid((W + 255) / 256, H), block(256);
+int launch_reproject(const void* depth, float* xyz, const float* xtab, int frames, int H, int W, int dtype, float fyinv, float ch, cudaStream_t s) {
+    if (frames <= 0) return 0;
+    dim3 grid((W + 255) / 256, H, frames), block(256);
     switch (dtype) {
     case 0: reproject_kernel<uint8_t><<<grid, block, 0, s>>>((const uint8_t*)depth, xyz, xtab, H, W, fyinv, ch); return 1;
     case 3: reproject_kernel<int16_t><<<grid, block, 0, s>>>((const int16_t*)depth, xyz, xtab, H, W, fyinv, ch); return 1;

@@ -16,6 +16,10 @@
 //     iteration that changes nothing has reached it (typically 3-5 iterations).
 //   * the colour of a pixel is that of the LATEST fired attempt that colours it (atomicMax on time), its depth the final
 //     running minimum.
+//   * a batch of F frames (one camera) is rendered at once: the kernels take the frame from the grid, a pixel's global
+//     index is frame * n + local, while times, coloured pixels and the `fired` bits stay frame-local.  Only interior points
+//     make attempts, so no attempt reaches into another frame.  One scan covers all F * n counters, and the fixed point
+//     is iterated until no frame changed (one host read per iteration for the whole batch).
 //
 // The projection uses the reference's reciprocal: _mm_rcp_ps (:78) is a 2048-entry look-up on Intel CPUs, carried here as
 // a table (dmc_rcp_intel.inc, verified against the instruction on all 2^32 operands by tools/gen_rcp_table.c); the last
@@ -46,17 +50,20 @@ __device__ __forceinline__ int sub_wrap(int a, int b) { return (int)((unsigned)a
 
 struct RenderCam { float r[3][3]; float t[3]; };
 
+// F frames of n points, frame = blockIdx.y; the rcp / exact split is per frame (the reference's tail is per call)
 __global__ void project_points_kernel(const float* __restrict__ xyz, float2* __restrict__ pt, long n, long n_rcp, RenderCam cam) {
     const long i = (long)blockIdx.x * blockDim.x + threadIdx.x;
     if (i >= n) return;
-    const float x = __fadd_rn(xyz[3 * i], cam.t[0]), y = __fadd_rn(xyz[3 * i + 1], cam.t[1]), z = __fadd_rn(xyz[3 * i + 2], cam.t[2]);
+    const long g = (long)blockIdx.y * n + i;
+    const float x = __fadd_rn(xyz[3 * g], cam.t[0]), y = __fadd_rn(xyz[3 * g + 1], cam.t[1]), z = __fadd_rn(xyz[3 * g + 2], cam.t[2]);
     auto dot = [&](int k) { return __fadd_rn(__fadd_rn(__fmul_rn(cam.r[k][0], x), __fmul_rn(cam.r[k][1], y)), __fmul_rn(cam.r[k][2], z)); };
     const float den = dot(2);
     const float div = i < n_rcp ? rcp_intel(den) : __fdiv_rn(1.f, den);
-    pt[i] = make_float2(__fmul_rn(dot(0), div), __fmul_rn(dot(1), div));
+    pt[g] = make_float2(__fmul_rn(dot(0), div), __fmul_rn(dot(1), div));
 }
 
-// The attempts of interior point p: calls f(ordinal, z-tested pixel index, coloured pixel index).
+// The attempts of interior point p of one frame (pt: that frame's points): calls f(ordinal, z-tested pixel index,
+// coloured pixel index), all frame-local.  p +- 1 and p +- cols stay inside the frame because p is interior.
 template <class F>
 __device__ __forceinline__ void for_each_attempt(const float2* __restrict__ pt, long p, int rows, int cols, int is_sub, F f) {
     const float2 me = pt[p];
@@ -76,22 +83,25 @@ __device__ __forceinline__ void for_each_attempt(const float2* __restrict__ pt, 
     else if (up) f(ord++, q0 - cols, q0 - cols);
 }
 
-struct Attempt { uint32_t time; float z; uint32_t c; };      // time = point * 8 + ordinal
+// time = frame-local point * 8 + ordinal; c = frame-local coloured pixel.  Pixel lists hold one frame's attempts only.
+struct Attempt { uint32_t time; float z; uint32_t c; };
 
+// frame = blockIdx.z; counters, cursors and offsets are indexed by the global pixel frame * n + q
 __global__ void attempts_count_kernel(const float2* __restrict__ pt, uint32_t* __restrict__ cnt, int rows, int cols, int is_sub) {
     const int i = blockIdx.x * blockDim.x + threadIdx.x + 1, j = blockIdx.y + 1;
     if (i >= cols - 1 || j >= rows - 1) return;
-    for_each_attempt(pt, (long)j * cols + i, rows, cols, is_sub, [&](int, long q, long) { atomicAdd(&cnt[q], 1u); });
+    const long base = (long)blockIdx.z * rows * cols;
+    for_each_attempt(pt + base, (long)j * cols + i, rows, cols, is_sub, [&](int, long q, long) { atomicAdd(&cnt[base + q], 1u); });
 }
 
 __global__ void attempts_fill_kernel(const float2* __restrict__ pt, const float* __restrict__ xyz, const uint32_t* __restrict__ offs, uint32_t* __restrict__ cursor,
                                      Attempt* __restrict__ att, int rows, int cols, int is_sub) {
     const int i = blockIdx.x * blockDim.x + threadIdx.x + 1, j = blockIdx.y + 1;
     if (i >= cols - 1 || j >= rows - 1) return;
-    const long p = (long)j * cols + i;
-    const float z = xyz[3 * p + 2];
-    for_each_attempt(pt, p, rows, cols, is_sub, [&](int ord, long q, long c) {
-        const uint32_t slot = offs[q] + atomicAdd(&cursor[q], 1u);
+    const long base = (long)blockIdx.z * rows * cols, p = (long)j * cols + i;
+    const float z = xyz[3 * (base + p) + 2];
+    for_each_attempt(pt + base, p, rows, cols, is_sub, [&](int ord, long q, long c) {
+        const uint32_t slot = offs[base + q] + atomicAdd(&cursor[base + q], 1u);
         Attempt a; a.time = (uint32_t)p * 8u + (uint32_t)ord; a.z = z; a.c = (uint32_t)c;
         att[slot] = a;
     });
@@ -143,12 +153,14 @@ __global__ void scan_add_kernel(uint32_t* __restrict__ out, const uint32_t* __re
     for (int k = 0; k < kScanPer; k++) if (base + k < n) out[base + k] += add;
 }
 
+// Pixel q of frame blockIdx.y (global pixel index frame * n + q) in the kernels below.
 __global__ void attempts_sort_kernel(const uint32_t* __restrict__ offs, const uint32_t* __restrict__ cnt, Attempt* __restrict__ att, long n) {
     const long q = (long)blockIdx.x * blockDim.x + threadIdx.x;
     if (q >= n) return;
-    const uint32_t m = cnt[q];
+    const long g = (long)blockIdx.y * n + q;
+    const uint32_t m = cnt[g];
     if (m < 2) return;
-    Attempt* a = att + offs[q];
+    Attempt* a = att + offs[g];
     if (m <= 48) {                                      // the usual case: a handful of entries
         for (uint32_t i = 1; i < m; i++) {
             const Attempt key = a[i]; uint32_t k = i;
@@ -171,42 +183,46 @@ __global__ void attempts_sort_kernel(const uint32_t* __restrict__ offs, const ui
     for (uint32_t end = m; end-- > 1;) { const Attempt t = a[0]; a[0] = a[end]; a[end] = t; sift(0, end); }
 }
 
-// One sweep of the fixed-point iteration; FINAL: also emits colours and depth.
+// One sweep of the fixed-point iteration over every frame; FINAL: also emits colours and depth.  `changed` is shared by
+// the frames: the batch iterates until no frame changed.
 template <bool FINAL>
 __global__ void attempts_sweep_kernel(const uint32_t* __restrict__ offs, const uint32_t* __restrict__ cnt, const Attempt* __restrict__ att, uint8_t* fired,
                                       int* __restrict__ changed, uint32_t* __restrict__ ckey, float* __restrict__ depth, long n) {
     const long q = (long)blockIdx.x * blockDim.x + threadIdx.x;
     if (q >= n) return;
-    const uint32_t m = cnt[q];
-    const Attempt* a = att + offs[q];
+    const long base = (long)blockIdx.y * n, g = base + q;
+    const uint32_t m = cnt[g];
+    const Attempt* a = att + offs[g];
+    uint8_t* fr = fired + base;
     float cur = 10000.f;                                // depth.setTo(10000.f) :306
     for (uint32_t i = 0; i < m; i++) {
         const Attempt e = a[i];
         const uint32_t p = e.time >> 3, ord = e.time & 7u;
-        const bool considered = ord == 0u || fired[p] != 0;
+        const bool considered = ord == 0u || fr[p] != 0;
         const bool fires = considered && cur > e.z;     // `*zbuff > z` :325 (false for NaN)
-        if (fires) { cur = e.z; if (FINAL) atomicMax(&ckey[e.c], e.time + 1u); }
-        if (!FINAL && ord == 0u && (fired[p] != 0) != fires) { fired[p] = fires ? 1 : 0; *changed = 1; }
+        if (fires) { cur = e.z; if (FINAL) atomicMax(&ckey[base + e.c], e.time + 1u); }
+        if (!FINAL && ord == 0u && (fr[p] != 0) != fires) { fr[p] = fires ? 1 : 0; *changed = 1; }
     }
-    if (FINAL && depth) depth[q] = cur;
+    if (FINAL && depth) depth[g] = cur;
 }
 
 __global__ void render_resolve_kernel(const uint8_t* __restrict__ image, const uint32_t* __restrict__ ckey, uint8_t* __restrict__ dest, long n) {
     const long q = (long)blockIdx.x * blockDim.x + threadIdx.x;
     if (q >= n) return;
-    const uint32_t k = ckey[q];
-    uint8_t b = 0, g = 0, r = 0;                        // destimage.setTo(0) :288
-    if (k) { const uint8_t* c = image + 3 * (long)((k - 1u) >> 3); b = c[0]; g = c[1]; r = c[2]; }
-    dest[3 * q] = b; dest[3 * q + 1] = g; dest[3 * q + 2] = r;
+    const long base = (long)blockIdx.y * n, g = base + q;
+    const uint32_t k = ckey[g];
+    uint8_t b = 0, gr = 0, r = 0;                       // destimage.setTo(0) :288
+    if (k) { const uint8_t* c = image + 3 * (base + (long)((k - 1u) >> 3)); b = c[0]; gr = c[1]; r = c[2]; }
+    dest[3 * g] = b; dest[3 * g + 1] = gr; dest[3 * g + 2] = r;
 }
 
 // fillSmallHole :187-283: a pixel whose GREEN is 0 becomes the mean of the neighbours whose BLUE is not 0 (s[lstep+1-1]);
-// cvRound of a double quotient; border pixels and non-holes keep dst's previous content.
+// cvRound of a double quotient; border pixels and non-holes keep dst's previous content.  Frame = blockIdx.z.
 __global__ void fill_small_hole_kernel(const uint8_t* __restrict__ src, uint8_t* __restrict__ dst, int rows, int cols) {
     const int i = blockIdx.x * blockDim.x + threadIdx.x + 1, j = blockIdx.y + 1;
     if (i >= cols - 1 || j >= rows - 1) return;
-    const long step = (long)cols * 3;
-    const uint8_t* s = src + j * step + 3 * i;
+    const long step = (long)cols * 3, frame = (long)blockIdx.z * rows * step;
+    const uint8_t* s = src + frame + j * step + 3 * i;
     if (s[1] != 0) return;
     int count = 0, b = 0, g = 0, r = 0;
 #pragma unroll
@@ -217,7 +233,7 @@ __global__ void fill_small_hole_kernel(const uint8_t* __restrict__ src, uint8_t*
             const uint8_t* q = s + dy * step + 3 * dx;
             if (q[0] != 0) { b += q[0]; g += q[1]; r += q[2]; count++; }
         }
-    uint8_t* d = dst + j * step + 3 * i;
+    uint8_t* d = dst + frame + j * step + 3 * i;
     d[0] = count ? (uint8_t)__double2int_rn(__ddiv_rn((double)b, (double)count)) : 0;
     d[1] = count ? (uint8_t)__double2int_rn(__ddiv_rn((double)g, (double)count)) : 0;
     d[2] = count ? (uint8_t)__double2int_rn(__ddiv_rn((double)r, (double)count)) : 0;
@@ -240,37 +256,41 @@ int launch_split_line_interleave(const void* src, void* dst, int rows, int cols,
 }
 
 // ---- launchers ----------------------------------------------------------------------------------------------------
-int launch_project_points(const float* xyz, float* pt, long n, const float kr[9], const float t[3], int exact_divide, cudaStream_t s) {
+int launch_project_points(const float* xyz, float* pt, int frames, long n, const float kr[9], const float t[3], int exact_divide, cudaStream_t s) {
+    if (frames <= 0 || n <= 0) return 0;
     RenderCam cam;
     for (int i = 0; i < 3; i++) { for (int j = 0; j < 3; j++) cam.r[i][j] = kr[3 * i + j]; cam.t[i] = t[i]; }
-    project_points_kernel<<<(unsigned)((n + 255) / 256), 256, 0, s>>>(xyz, (float2*)pt, n, exact_divide ? 0 : 4 * (n / 4), cam);
+    project_points_kernel<<<dim3((unsigned)((n + 255) / 256), frames), 256, 0, s>>>(xyz, (float2*)pt, n, exact_divide ? 0 : 4 * (n / 4), cam);
     return 1;
 }
 
-size_t render_scratch_bytes(int rows, int cols) {
-    const size_t n = (size_t)rows * cols, nb = (n + kScanT * kScanPer - 1) / (kScanT * kScanPer);
+size_t render_scratch_bytes(int frames, int rows, int cols) {
+    const size_t n = (size_t)frames * rows * cols, nb = (n + kScanT * kScanPer - 1) / (kScanT * kScanPer);
     return n * 4 * 3 + nb * 4 + 256 + n * 7 * sizeof(Attempt) + n + 64;      // cnt, offs, cursor/ckey, block sums, attempts, fired
 }
 
-// Everything after the projection, up to the fixed point.  `changed_host` is pinned memory the sweeps report through.
-// Returns the number of kernels launched, or -1 if the iteration did not settle (cannot happen: see the header).
-int launch_render(const uint8_t* image, const float* xyz, const float* pt, int rows, int cols, int is_sub, uint8_t* dest, float* depth,
+// Everything after the projection, up to the fixed point, for `frames` frames of rows x cols at once (one scan over all
+// their counters: the caller keeps frames * rows * cols * 7 below 2^32).  `changed_host` is pinned memory the sweeps report
+// through: one read per iteration for the whole batch.  Returns the number of kernels launched, or -1 if the iteration did
+// not settle (cannot happen: see the header).
+int launch_render(const uint8_t* image, const float* xyz, const float* pt, int frames, int rows, int cols, int is_sub, uint8_t* dest, float* depth,
                   void* scratch, int* changed_dev, int* changed_host, cudaStream_t s) {
-    const long n = (long)rows * cols;
-    const int nb = (int)((n + kScanT * kScanPer - 1) / (kScanT * kScanPer));
-    uint32_t* cnt = (uint32_t*)scratch; uint32_t* offs = cnt + n; uint32_t* cursor = offs + n; uint32_t* sums = cursor + n;
+    const long n = (long)rows * cols, nt = n * frames;
+    if (nt <= 0) return 0;
+    const int nb = (int)((nt + kScanT * kScanPer - 1) / (kScanT * kScanPer));
+    uint32_t* cnt = (uint32_t*)scratch; uint32_t* offs = cnt + nt; uint32_t* cursor = offs + nt; uint32_t* sums = cursor + nt;
     Attempt* att = (Attempt*)(((uintptr_t)(sums + nb) + 63) & ~(uintptr_t)63);
-    uint8_t* fired = (uint8_t*)(att + (size_t)n * 7);
+    uint8_t* fired = (uint8_t*)(att + (size_t)nt * 7);
     int nk = 0;
-    cudaMemsetAsync(cnt, 0, (size_t)n * 4, s); cudaMemsetAsync(cursor, 0, (size_t)n * 4, s); cudaMemsetAsync(fired, 1, (size_t)n, s);
-    dim3 grid((cols + 255) / 256, rows > 2 ? rows - 2 : 1);
+    cudaMemsetAsync(cnt, 0, (size_t)nt * 4, s); cudaMemsetAsync(cursor, 0, (size_t)nt * 4, s); cudaMemsetAsync(fired, 1, (size_t)nt, s);
+    dim3 grid((cols + 255) / 256, rows > 2 ? rows - 2 : 1, frames);
     if (rows > 2 && cols > 2) { attempts_count_kernel<<<grid, 256, 0, s>>>((const float2*)pt, cnt, rows, cols, is_sub); nk++; }
-    scan_blocks_kernel<<<nb, kScanT, 0, s>>>(cnt, offs, sums, n);
+    scan_blocks_kernel<<<nb, kScanT, 0, s>>>(cnt, offs, sums, nt);
     scan_sums_kernel<<<1, 1024, 0, s>>>(sums, nb);
-    scan_add_kernel<<<nb, kScanT, 0, s>>>(offs, sums, n);
+    scan_add_kernel<<<nb, kScanT, 0, s>>>(offs, sums, nt);
     nk += 3;
     if (rows > 2 && cols > 2) { attempts_fill_kernel<<<grid, 256, 0, s>>>((const float2*)pt, xyz, offs, cursor, att, rows, cols, is_sub); nk++; }
-    const unsigned gq = (unsigned)((n + 255) / 256);
+    const dim3 gq((unsigned)((n + 255) / 256), frames);
     attempts_sort_kernel<<<gq, 256, 0, s>>>(offs, cnt, att, n); nk++;
     if (is_sub) {
         for (int it = 0;; it++) {
@@ -283,15 +303,15 @@ int launch_render(const uint8_t* image, const float* xyz, const float* pt, int r
         }
     }
     uint32_t* ckey = cursor;                            // the fill cursors are no longer needed
-    cudaMemsetAsync(ckey, 0, (size_t)n * 4, s);
+    cudaMemsetAsync(ckey, 0, (size_t)nt * 4, s);
     attempts_sweep_kernel<true><<<gq, 256, 0, s>>>(offs, cnt, att, fired, nullptr, ckey, depth, n);
     render_resolve_kernel<<<gq, 256, 0, s>>>(image, ckey, dest, n);
     return nk + 2;
 }
 
-int launch_fill_small_hole(const uint8_t* src, uint8_t* dst, int rows, int cols, cudaStream_t s) {
-    if (rows <= 2 || cols <= 2) return 0;
-    dim3 grid((cols + 255) / 256, rows - 2);
+int launch_fill_small_hole(const uint8_t* src, uint8_t* dst, int frames, int rows, int cols, cudaStream_t s) {
+    if (rows <= 2 || cols <= 2 || frames <= 0) return 0;
+    dim3 grid((cols + 255) / 256, rows - 2, frames);
     fill_small_hole_kernel<<<grid, 256, 0, s>>>(src, dst, rows, cols);
     return 1;
 }

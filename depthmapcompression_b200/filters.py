@@ -334,6 +334,47 @@ def jpegRateDistortion(frames, qualities, params=None, optimize=False, ctx=None)
     return out
 
 
+def jpegViewRateDistortion(disp, texture, qualities, params, f, R, t, K, isSub=True, optimize=False, exact_divide=False, ctx=None):
+    """The view-synthesis rate-distortion sweep on the GPU (dmc_jpeg_view_rd_sweep): coded depth scored by the views it
+    renders, as pointcloudTest renders a decoded depth map.  For every frame, quality and camera (R[v], t[v], shared K) the
+    reference view fillSmallHole(projectImagefromXYZ(texture, reprojectXYZ(D(disp), f), ...)), with D the unfiltered
+    disp8U2depth32F, is compared with the view of D(decoded) and with the view of filterDisp8U2Depth32F(decoded, params).
+    disp: frames as for degradeJPEG; texture: uint8 numpy [n, rows, cols, 3] (or one [rows, cols, 3] image), or (device
+    pointer, n, rows, cols) when disp is a device tuple.  params: chain_params(CHAIN_DEPTH32F, ..., focus, baseline, amp).
+    R: [n_views, 3, 3] (or one 3x3), t: [n_views, 3].  Returns a dict: bytes (n_q, n), and sse_view_coded, psnr_view_coded,
+    sse_view_filtered, psnr_view_filtered (n_q, n_views, n); the PSNR is cv2.PSNR of the two 8UC3 views."""
+    ctx = ctx or default_context()
+    sp, n, rows, cols, mem, keep = _frames(disp)
+    if isinstance(texture, tuple):
+        tp, tn, trows, tcols = (int(x) for x in texture)
+        tmem, tkeep = MEM_DEVICE, None
+    else:
+        tkeep = np.ascontiguousarray(texture)
+        if tkeep.dtype != np.uint8 or tkeep.ndim not in (3, 4) or tkeep.shape[-1] != 3:
+            raise DmcError(capi.DMC_ERR_TYPE, "texture must be uint8 [n, rows, cols, 3] or [rows, cols, 3]")
+        tn, trows, tcols = (1,) + tkeep.shape[:2] if tkeep.ndim == 3 else tkeep.shape[:3]
+        tp, tmem = tkeep.ctypes.data, MEM_HOST
+    if (tn, trows, tcols, tmem) != (n, rows, cols, mem):
+        raise DmcError(capi.DMC_ERR_SIZE, "jpegViewRateDistortion: disp and texture must be batches of one size in the same memory")
+    q = np.ascontiguousarray(np.asarray(qualities).ravel(), dtype=np.int32)
+    Rs = np.ascontiguousarray(R, np.float64).reshape(-1, 9)
+    ts = np.ascontiguousarray(t, np.float64).reshape(-1, 3)
+    Ks = np.ascontiguousarray(K, np.float64).reshape(9)
+    if Rs.shape[0] != ts.shape[0]:
+        raise DmcError(capi.DMC_ERR_ARG, "jpegViewRateDistortion: R and t must hold one camera each")
+    nv = Rs.shape[0]
+    U64, DP = C.POINTER(C.c_uint64), C.POINTER(C.c_double)
+    nbytes = np.zeros((len(q), n), np.uint64)
+    sc, sf = np.zeros((len(q), nv, n), np.uint64), np.zeros((len(q), nv, n), np.uint64)
+    ctx.check(lib.dmc_jpeg_view_rd_sweep(ctx.h, C.c_void_p(sp), C.c_void_p(tp), mem, n, rows, cols, q.ctypes.data_as(C.POINTER(C.c_int)), len(q),
+                                         _jpeg_flags(optimize), C.byref(params), float(f), Rs.ctypes.data_as(DP), ts.ctypes.data_as(DP), nv,
+                                         Ks.ctypes.data_as(DP), int(bool(isSub)), capi.RENDER_EXACT_DIVIDE if exact_divide else 0,
+                                         nbytes.ctypes.data_as(U64), sc.ctypes.data_as(U64), sf.ctypes.data_as(U64)))
+    px = 3 * rows * cols
+    return {"bytes": nbytes, "sse_view_coded": sc, "psnr_view_coded": psnrFromSSE(sc, px),
+            "sse_view_filtered": sf, "psnr_view_filtered": psnrFromSSE(sf, px)}
+
+
 _default = {}
 
 

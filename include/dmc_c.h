@@ -316,6 +316,30 @@ int dmc_project_image_from_xyz(dmc_ctx* ctx, const dmc_image* image, dmc_image* 
  * dest keeps everything else (call it in place, like main.cpp:355, or with dest pre-filled). */
 int dmc_fill_small_hole(dmc_ctx* ctx, const dmc_image* src, dmc_image* dest);
 
+/* ---- the view-synthesis rate-distortion sweep ------------------------------------------------------------------- */
+/* Scores coded depth by the views it renders, as pointcloudTest (main.cpp:276-373) consumes a decoded depth map.  For every
+ * frame i of disp (n dense 8UC1 disparity frames) with its texture i (n dense 8UC3 images, the pixels that are splatted, in
+ * the same memory src_mem as disp), every camera v (R + 9v, t + 3v: row-major doubles; K shared) and every qualities[k]:
+ *   D(x)     = disp8U2depth32F(x, (float)(p->focus * p->baseline), (float)p->amp, 0), the unfiltered depth.  It equals the
+ *              32F chain with all four radii 0 except where x is 0: there D is +inf and the chain NaN, and neither point is
+ *              drawn, so the views are the same;
+ *   view(z)  = fillSmallHole(projectImagefromXYZ(texture_i, reprojectXYZ(z, f), R_v, t_v, K, is_sub)), the fill in place
+ *              as at main.cpp:355;
+ *   dec      = imdecode(imencode(disp_i, {QUALITY, q} [+ OPTIMIZE with DMC_JPEG_OPTIMIZE_HUFFMAN]));
+ *   bytes[k*n + i]                          = the size of that stream (as dmc_jpeg_rd_sweep reports it);
+ *   sse_view_coded[(k*n_views + v)*n + i]    = SSE(view(D(disp_i)), view(D(dec))), over all 3*rows*cols bytes;
+ *   sse_view_filtered[(k*n_views + v)*n + i] = SSE(view(D(disp_i)), view(filterDisp8U2Depth32F(dec, p))).
+ * PSNR of a view is dmc_psnr_from_sse(sse, 3*rows*cols), which is cv::PSNR of the two 8UC3 images.  p->chain must be
+ * DMC_CHAIN_DEPTH32F (focus, baseline, amp and the radii of pointcloudTest's filter); render_flags: DMC_RENDER_EXACT_DIVIDE
+ * or 0, as the flags of dmc_project_image_from_xyz.  No frame, stream or view leaves the device.
+ * DMC_ERR_ARG (nothing written): n_q < 1, a quality outside 0..100, unknown flags or render_flags bits, p == NULL, a chain
+ * other than DMC_CHAIN_DEPTH32F, a bad radius, a brange_method for which the 32F chain writes nothing, n_views < 1 or a NULL
+ * camera.  Sizes follow dmc_jpeg_encode_bound_ex and rows * cols < 2^29 (DMC_ERR_SIZE).  Returns when the outputs are valid. */
+int dmc_jpeg_view_rd_sweep(dmc_ctx* ctx, const void* disp, const void* texture, int src_mem, int n_frames, int rows, int cols,
+                           const int* qualities, int n_q, int flags, const dmc_chain_params* p, double f,
+                           const double* R, const double* t, int n_views, const double* K, int is_sub, int render_flags,
+                           uint64_t* bytes, uint64_t* sse_view_coded, uint64_t* sse_view_filtered);
+
 #ifdef __cplusplus
 }
 #endif

@@ -2,6 +2,7 @@
 // own header so that include/filter.h stays a truthful drop-in of the reference API (SURVEY.md section 8f-4).
 #pragma once
 #include "filter.h"
+#include "util.h"
 
 // Joint ("colour-guided") binary-weighted range filter: `src` (CV_8UC1 depth / disparity) is averaged over the window
 // of binalyWeightedRangeFilter with the binary weights computed on `guide` (CV_8UC3: the saturated L1 colour distance of
@@ -90,5 +91,46 @@ inline void jpegRateDistortionGray(const Mat& src, const vector<int>& qualities,
 		bytes[k] = (int)b[k];
 		psnr_coded[k] = dmc_psnr_from_sse(sc[k], pixels);
 		psnr_filtered[k] = dmc_psnr_from_sse(sf[k], pixels);
+	}
+}
+
+// The view-synthesis rate-distortion sweep of one frame on the GPU (pointcloudTest's view, main.cpp:276-373, for several
+// qualities and cameras at once): `disp` (CV_8UC1 disparity) is coded at every qualities[k] (optimize: with optimised Huffman
+// tables); bytes[k] is the stream's size.  For every camera v (R[v], t[v]: CV_64F 3x3 and 3x1; K shared), the reference view
+// is fillSmallHole(projectImagefromXYZ(texture, reprojectXYZ(disp8U2depth32F(disp, focus*baseline, amp), f), R, t, K, isSub))
+// in place, and psnr_coded[k][v] / psnr_filtered[k][v] = cv::PSNR of that view against the same view rendered from the
+// decoded disparity (converted the same way) / from filterDisp8U2Depth32F(decoded, focus, baseline, amp, median_r,
+// gaussian_r, minmax_r, brange_r, brange_th).  texture: CV_8UC3, the image that is splatted.  Nothing leaves the device.
+inline void jpegViewRateDistortionGray(const Mat& disp, const Mat& texture, const vector<int>& qualities, double focus, double baseline, double amp,
+                                       int median_r, int gaussian_r, int minmax_r, int brange_r, float brange_th, double f,
+                                       const vector<Mat>& R, const vector<Mat>& t, const Mat& K, bool isSub, vector<int>& bytes,
+                                       vector<vector<double> >& psnr_coded, vector<vector<double> >& psnr_filtered, bool optimize = false)
+{
+	dmc_dropin::require_gray8(disp, "jpegViewRateDistortionGray");
+	if (texture.type() != CV_8UC3 || texture.rows != disp.rows || texture.cols != disp.cols) {
+#ifdef DMC_MINICV_HPP
+		throw cv::Exception("jpegViewRateDistortionGray: texture must be CV_8UC3 of the size of disp", __FILE__, __LINE__);
+#else
+		CV_Error(cv::Error::StsAssert, "jpegViewRateDistortionGray: texture must be CV_8UC3 of the size of disp");
+#endif
+	}
+	const Mat s = disp.isContinuous() ? disp : disp.clone();
+	const Mat tex = texture.isContinuous() ? texture : texture.clone();
+	const size_t nq = qualities.size(), nv = R.size() < t.size() ? R.size() : t.size();
+	vector<double> r(9 * nv), tt(3 * nv), k(9);
+	for (size_t v = 0; v < nv; v++) dmc_dropin::camera(R[v], t[v], K, &r[9 * v], &tt[3 * v], &k[0], "jpegViewRateDistortionGray");
+	vector<uint64_t> b(nq), sc(nq * nv), sf(nq * nv);
+	dmc_chain_params p = {DMC_CHAIN_DEPTH32F, median_r, gaussian_r, minmax_r, brange_r, brange_th, DMC_FULL_KERNEL, focus, baseline, amp};
+	dmc_dropin::check(dmc_jpeg_view_rd_sweep(dmc_dropin::context(), s.data, tex.data, DMC_MEM_HOST, 1, s.rows, s.cols, qualities.data(), (int)nq,
+	                                         optimize ? DMC_JPEG_OPTIMIZE_HUFFMAN : 0, &p, f, nv ? &r[0] : 0, nv ? &tt[0] : 0, (int)nv, &k[0], isSub ? 1 : 0, 0,
+	                                         b.data(), sc.data(), sf.data()), "jpegViewRateDistortionGray");
+	const uint64_t pixels = 3 * (uint64_t)s.rows * s.cols;
+	bytes.resize(nq); psnr_coded.assign(nq, vector<double>(nv)); psnr_filtered.assign(nq, vector<double>(nv));
+	for (size_t q = 0; q < nq; q++) {
+		bytes[q] = (int)b[q];
+		for (size_t v = 0; v < nv; v++) {
+			psnr_coded[q][v] = dmc_psnr_from_sse(sc[q * nv + v], pixels);
+			psnr_filtered[q][v] = dmc_psnr_from_sse(sf[q * nv + v], pixels);
+		}
 	}
 }
