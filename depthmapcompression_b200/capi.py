@@ -32,6 +32,7 @@ EXPORTS = [
     "dmc_fill_occlusion", "dmc_reproject_xyz", "dmc_transpose",
     "dmc_chain_batch_jpeg", "dmc_jpeg_probe", "dmc_jpeg_encode_bound", "dmc_jpeg_encode_gray_batch", "dmc_jpeg_degrade_gray_batch", "dmc_jpeg_encode_bound_ex", "dmc_jpeg_encode_gray_batch_ex", "dmc_jpeg_degrade_gray_batch_ex", "dmc_split_bgr_line_interleave", "dmc_project_points", "dmc_project_image_from_xyz", "dmc_fill_small_hole", "dmc_hostlink_probe", "dmc_release_device", "dmc_set_gateway", "dmc_get_gateway", "dmc_sched_get_routing",
     "dmc_sse_gray_batch", "dmc_psnr_from_sse", "dmc_jpeg_rd_sweep", "dmc_jpeg_view_rd_sweep",
+    "dmc_brf_batch", "dmc_jpeg_rd_sweep_ex", "dmc_jpeg_view_rd_sweep_ex",
 ]
 MAX_DEVICES = 16
 RENDER_EXACT_DIVIDE = 1
@@ -46,6 +47,10 @@ class DmcChainParams(C.Structure):
     _fields_ = [("chain", C.c_int), ("median_r", C.c_int), ("gaussian_r", C.c_int), ("minmax_r", C.c_int),
                 ("brange_r", C.c_int), ("brange_th", C.c_float), ("brange_method", C.c_int),
                 ("focus", C.c_double), ("baseline", C.c_double), ("amp", C.c_double)]
+
+
+class DmcBrfParams(C.Structure):
+    _fields_ = [("kernel_w", C.c_int), ("kernel_h", C.c_int), ("frec", C.c_float), ("color", C.c_float), ("space", C.c_float)]
 
 
 class DmcHostlinkInfo(C.Structure):
@@ -94,6 +99,12 @@ def _load():
         "dmc_jpeg_rd_sweep": (I, [P, P, I, I, I, I, C.POINTER(I), I, I, C.POINTER(DmcChainParams), C.POINTER(C.c_uint64), C.POINTER(C.c_uint64), C.POINTER(C.c_uint64)]),
         "dmc_jpeg_view_rd_sweep": (I, [P, P, P, I, I, I, I, C.POINTER(I), I, I, C.POINTER(DmcChainParams), D, C.POINTER(D), C.POINTER(D), I, C.POINTER(D), I, I,
                                        C.POINTER(C.c_uint64), C.POINTER(C.c_uint64), C.POINTER(C.c_uint64)]),
+        "dmc_brf_batch": (I, [P, P, P, I, I, I, I, C.POINTER(DmcBrfParams), I]),
+        "dmc_jpeg_rd_sweep_ex": (I, [P, P, I, I, I, I, C.POINTER(I), I, I, C.POINTER(DmcChainParams), C.POINTER(DmcBrfParams),
+                                     C.POINTER(C.c_uint64), C.POINTER(C.c_uint64), C.POINTER(C.c_uint64), C.POINTER(C.c_uint64)]),
+        "dmc_jpeg_view_rd_sweep_ex": (I, [P, P, P, I, I, I, I, C.POINTER(I), I, I, C.POINTER(DmcChainParams), C.POINTER(DmcBrfParams), D, C.POINTER(D),
+                                          C.POINTER(D), I, C.POINTER(D), I, I, C.POINTER(C.c_uint64), C.POINTER(C.c_uint64), C.POINTER(C.c_uint64),
+                                          C.POINTER(C.c_uint64)]),
         "dmc_sched_create": (I, [C.POINTER(I), I, C.POINTER(P)]), "dmc_sched_destroy": (None, [P]), "dmc_sched_device_count": (I, [P]),
         "dmc_sched_last_error": (C.c_char_p, [P]), "dmc_sched_chain_batch": (I, [P, P, P, I, I, I, C.POINTER(DmcChainParams)]),
         "dmc_multi_chain_batch": (I, [C.POINTER(I), I, P, P, I, I, I, C.POINTER(DmcChainParams), C.c_char_p, C.c_size_t]),

@@ -129,6 +129,8 @@ template <typename T> __device__ __forceinline__ T minmax_pick(T v, T mn, T mx) 
 // Shared memory (dynamic): [pool: kPool x 8 B][order: kPool B][ids: tile bytes][vals: 256 x sizeof(key)]
 //   while ranking, the pool area holds the hash keys (kSlots x sizeof(key)) followed by slot -> id (kSlots x 2 B), and the
 //   order area holds the tile as slot numbers (2 B each).
+// A launch covers a batch of dense H x W frames: blockIdx.z is the frame.  Everything else is per CTA (staged tile, rank
+// table, flat-tile exit, list fallback), so frames of one launch may take different paths.
 template <typename T, int TY, bool FUSED>
 __global__ void __launch_bounds__(kTX * TY) brf_rank_kernel(const T* __restrict__ src, T* __restrict__ dst, int H, int W, int rw, int rh, int mr,
                                                         const __grid_constant__ BrfTaps taps, float frec, float color, float space) {
@@ -146,6 +148,9 @@ __global__ void __launch_bounds__(kTX * TY) brf_rank_kernel(const T* __restrict_
     uint16_t* slot_id = (uint16_t*)(keys + NS + 2);                 // keys[NS] is the reserved slot of a value whose bits equal EMPTY (an all-ones NaN)
     uint16_t* slot_tile = (uint16_t*)order;
     __shared__ int s_warp[kNT / 32], s_m, s_odd;
+    // Frame 0 keeps the parameters as they are, and the fused kernel rebases dst only once its min-max tile is staged: both
+    // keep register pressure at the single-image kernel's (rebasing unconditionally costs 1-8 registers, profiles/r09_brf_ptxas.md)
+    if (blockIdx.z) { const size_t fo = (size_t)blockIdx.z * H * W; src += fo; if constexpr (!FUSED) dst += fo; }
     const int tid = threadIdx.x;
     const int x0 = blockIdx.x * kTX, y0 = blockIdx.y * TY;
 
@@ -258,6 +263,7 @@ __global__ void __launch_bounds__(kTX * TY) brf_rank_kernel(const T* __restrict_
         }
     }
     __syncthreads();
+    if constexpr (FUSED) if (blockIdx.z) dst += (size_t)blockIdx.z * H * W;
     const int M = s_m;
     const bool ranked = M <= kMaxRanks && M * 32 <= kPool && s_odd == 0;     // at least one warp of pixels per pass
     if (M == 1) {                                                   // a flat tile: every window holds that one value
@@ -392,7 +398,7 @@ __global__ void __launch_bounds__(kTX * TY) brf_rank_kernel(const T* __restrict_
 }
 
 template <typename T, int TY, bool FUSED>
-static int launch_brf_rank(const void* src, void* dst, int H, int W, int rw, int rh, int mr, const BrfTaps& taps, float frec, float color, float space, cudaStream_t s) {
+static int launch_brf_rank(const void* src, void* dst, int nf, int H, int W, int rw, int rh, int mr, const BrfTaps& taps, float frec, float color, float space, cudaStream_t s) {
     typedef typename BrfT<T>::key_t key_t;
     const int ntile = (kTX + 2 * rw) * (TY + 2 * rh);
     constexpr int kNT = kTX * TY, kPool = kNT * kPoolPerPixel;
@@ -401,7 +407,7 @@ static int launch_brf_rank(const void* src, void* dst, int H, int W, int rw, int
     auto kern = brf_rank_kernel<T, TY, FUSED>;
     // (the attribute is per function AND per device: set on every call, ~1 us, so that every GPU of a scheduler gets it)
     if (cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)(kPool * 9 + kMaxTile + 16 + kMaxRanks * sizeof(key_t))) != cudaSuccess) return 0;
-    dim3 grid((W + kTX - 1) / kTX, (H + TY - 1) / TY);
+    dim3 grid((W + kTX - 1) / kTX, (H + TY - 1) / TY, nf);
     kern<<<grid, kNT, smem, s>>>((const T*)src, (T*)dst, H, W, rw, rh, mr, taps, frec, color, space);
     return 1;
 }
@@ -421,26 +427,27 @@ static bool make_brf_taps(int kw, int kh, BrfTaps* taps) {
 constexpr int kBrfTY8 = 4;          // 8-bit tile height (a direct 256-slot table: small CTAs are cheap); hashed types keep 8 rows
 
 template <bool FUSED>
-static int launch_brf_any(const void* src, void* dst, int H, int W, int depth, int kw, int kh, int mr, float frec, float color, float space, cudaStream_t s) {
+static int launch_brf_any(const void* src, void* dst, int nf, int H, int W, int depth, int kw, int kh, int mr, float frec, float color, float space, cudaStream_t s) {
     BrfTaps taps;
     if (!make_brf_taps(kw, kh, &taps)) return 0;
     const int rw = kw / 2, rh = kh / 2;
+    if (nf < 1 || nf > 65535) return 0;                                                   // grid z
     switch (depth) {
-    case 0: return launch_brf_rank<uint8_t, FUSED ? 8 : kBrfTY8, FUSED>(src, dst, H, W, rw, rh, mr, taps, frec, color, space, s);      // fused: taller tiles, less halo to min-max
-    case 2: return launch_brf_rank<uint16_t, 8, FUSED>(src, dst, H, W, rw, rh, mr, taps, frec, color, space, s);
-    case 3: return launch_brf_rank<int16_t, 8, FUSED>(src, dst, H, W, rw, rh, mr, taps, frec, color, space, s);
-    case 5: if (FUSED) return 0; return launch_brf_rank<float, 8, false>(src, dst, H, W, rw, rh, mr, taps, frec, color, space, s);
-    case 6: if (FUSED) return 0; return launch_brf_rank<double, 8, false>(src, dst, H, W, rw, rh, mr, taps, frec, color, space, s);
+    case 0: return launch_brf_rank<uint8_t, FUSED ? 8 : kBrfTY8, FUSED>(src, dst, nf, H, W, rw, rh, mr, taps, frec, color, space, s);      // fused: taller tiles, less halo to min-max
+    case 2: return launch_brf_rank<uint16_t, 8, FUSED>(src, dst, nf, H, W, rw, rh, mr, taps, frec, color, space, s);
+    case 3: return launch_brf_rank<int16_t, 8, FUSED>(src, dst, nf, H, W, rw, rh, mr, taps, frec, color, space, s);
+    case 5: if (FUSED) return 0; return launch_brf_rank<float, 8, false>(src, dst, nf, H, W, rw, rh, mr, taps, frec, color, space, s);
+    case 6: if (FUSED) return 0; return launch_brf_rank<double, 8, false>(src, dst, nf, H, W, rw, rh, mr, taps, frec, color, space, s);
     }
     return 0;
 }
 
-int launch_brf(const void* src, void* dst, int H, int W, int depth, int kw, int kh, float frec, float color, float space, cudaStream_t s) {
-    return launch_brf_any<false>(src, dst, H, W, depth, kw, kh, 0, frec, color, space, s);
+int launch_brf(const void* src, void* dst, int nf, int H, int W, int depth, int kw, int kh, float frec, float color, float space, cudaStream_t s) {
+    return launch_brf_any<false>(src, dst, nf, H, W, depth, kw, kh, 0, frec, color, space, s);
 }
 
-int launch_minmax_brf(const void* src, void* dst, int H, int W, int depth, int minmax_r, int kw, int kh, float frec, float color, float space, cudaStream_t s) {
-    return launch_brf_any<true>(src, dst, H, W, depth, kw, kh, minmax_r, frec, color, space, s);
+int launch_minmax_brf(const void* src, void* dst, int nf, int H, int W, int depth, int minmax_r, int kw, int kh, float frec, float color, float space, cudaStream_t s) {
+    return launch_brf_any<true>(src, dst, nf, H, W, depth, kw, kh, minmax_r, frec, color, space, s);
 }
 
 }  // namespace dmc

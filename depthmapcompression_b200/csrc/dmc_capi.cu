@@ -27,8 +27,8 @@ enum { SB_IN, SB_OUT, SB_PING, SB_PONG, SB_FLOAT, SB_BITS, SB_META, SB_SCANS, SB
 // Device buffers of dmc_jpeg_decode_gray_batch.
 enum { JD_BITS, JD_META, JD_SCANS, JD_COEF, JD_OUT, JD_COUNT };
 // Device buffers of dmc_sse_gray_batch and dmc_jpeg_rd_sweep: every quality's encoder + decoder tables, the decoder's
-// FrameDescs of a group, its staged source, coded and filtered frames (the staged second batch of dmc_sse_gray_batch),
-// and the group's results (SSE, stream lengths) that one copy brings back.
+// FrameDescs of a group, its staged source, coded and filtered frames (the staged second batch of dmc_sse_gray_batch; the
+// BRF arm's frames in both sweeps), and the group's results (SSE, stream lengths) that one copy brings back.
 enum { RD_TABS, RD_DESC, RD_SRC, RD_CODED, RD_FILT, RD_RES, RD_COUNT };
 // Device buffers of dmc_jpeg_view_rd_sweep: the group's staged textures, a depth frame, the points of the coded and of the
 // filtered depth (xyz), their projections, a raw render, the coded and filtered views, and the reference views.
@@ -1214,6 +1214,21 @@ int rd_degrade(dmc_ctx* ctx, int k, const uint8_t* dsrc, int nf, int rows, int c
     return DMC_OK;
 }
 
+// The argument rules of dmc_boundary_reconstruction for a parameter block (dmc_brf_batch and the sweeps' BRF arm).
+int check_brf_params(dmc_ctx* ctx, const dmc_brf_params* b, const char* what) {
+    if (!b) return fail(ctx, DMC_ERR_ARG, std::string(what) + ": no boundary reconstruction parameters");
+    if (b->kernel_w < 1 || b->kernel_h < 1 || b->kernel_w / 2 > DMC_MAX_RADIUS || b->kernel_h / 2 > DMC_MAX_RADIUS)
+        return fail(ctx, DMC_ERR_ARG, std::string(what) + ": boundaryReconstructionFilter kernel size out of range");
+    return DMC_OK;
+}
+
+// B of nf dense 8-bit frames in one launch (the sweeps' BRF arm).
+int brf_frames(dmc_ctx* ctx, const uint8_t* src, uint8_t* dst, int nf, int rows, int cols, const dmc_brf_params& b) {
+    const int nk = launch_brf(src, dst, nf, rows, cols, DMC_8U, b.kernel_w, b.kernel_h, b.frec, b.color, b.space, ctx->stream);
+    if (nk == 0) return fail(ctx, DMC_ERR_ARG, "boundaryReconstructionFilter: window too large");
+    return after_launch(ctx, nk);
+}
+
 }  // namespace
 
 // The sweep runs group by group (a group is sized like the encoder's, counting the coded and filtered frames and the
@@ -1221,9 +1236,17 @@ int rd_degrade(dmc_ctx* ctx, int k, const uint8_t* dsrc, int nf, int rows, int c
 // Every quality's encoder tables and the decoder tables parsed from its header are built once and uploaded in one copy.
 // Per (group, quality) everything runs on ctx->stream without a host synchronisation: encode, decode into the coded
 // frames, the chain into the filtered frames, one SSE launch (source vs coded and vs filtered) and a device-side copy of
-// the stream lengths; one copy and one synchronisation per group bring the results back.
+// the stream lengths; one copy and one synchronisation per group bring the results back.  The BRF arm (b != NULL) adds, per
+// (group, quality), one batched BRF launch on the coded frames and one SSE launch; its output reuses the filtered frames'
+// buffer once their SSE is queued.
 int dmc_jpeg_rd_sweep(dmc_ctx* ctx, const void* src, int src_mem, int n_frames, int rows, int cols, const int* qualities, int n_q,
                       int flags, const dmc_chain_params* p, uint64_t* bytes, uint64_t* sse_coded, uint64_t* sse_filtered) {
+    return dmc_jpeg_rd_sweep_ex(ctx, src, src_mem, n_frames, rows, cols, qualities, n_q, flags, p, nullptr, bytes, sse_coded, sse_filtered, nullptr);
+}
+
+int dmc_jpeg_rd_sweep_ex(dmc_ctx* ctx, const void* src, int src_mem, int n_frames, int rows, int cols, const int* qualities, int n_q,
+                         int flags, const dmc_chain_params* p, const dmc_brf_params* b, uint64_t* bytes, uint64_t* sse_coded,
+                         uint64_t* sse_filtered, uint64_t* sse_brf) {
     if (!ctx) return fail(nullptr, DMC_ERR_ARG, "null context");
     if (!qualities || n_q < 1) return fail(ctx, DMC_ERR_ARG, "dmc_jpeg_rd_sweep: no qualities");
     for (int k = 0; k < n_q; k++)
@@ -1235,10 +1258,11 @@ int dmc_jpeg_rd_sweep(dmc_ctx* ctx, const void* src, int src_mem, int n_frames, 
         // (the reference's 8U range filter leaves dst unwritten for FULL_KERNEL_PAIR: there would be nothing to measure)
         if (p->brange_method != DMC_FULL_KERNEL && p->brange_method != DMC_SEPARABLE_KERNEL) return fail(ctx, DMC_ERR_ARG, "dmc_jpeg_rd_sweep: brange_method must be FULL_KERNEL or SEPARABLE_KERNEL");
     }
+    if (b) TRY(check_brf_params(ctx, b, "dmc_jpeg_rd_sweep"));
     if (src_mem != DMC_MEM_HOST && src_mem != DMC_MEM_DEVICE) return fail(ctx, DMC_ERR_ARG, "dmc_jpeg_rd_sweep: bad mem");
     uint64_t bound;
     if (dmc_jpeg_encode_bound_ex(rows, cols, flags, &bound) != DMC_OK) return fail(ctx, DMC_ERR_SIZE, "dmc_jpeg_rd_sweep: " + g_err);
-    if (n_frames < 0 || (n_frames > 0 && (!src || !bytes || !sse_coded || (p && !sse_filtered)))) return fail(ctx, DMC_ERR_SIZE, "dmc_jpeg_rd_sweep: bad arguments");
+    if (n_frames < 0 || (n_frames > 0 && (!src || !bytes || !sse_coded || (p && !sse_filtered) || (b && !sse_brf)))) return fail(ctx, DMC_ERR_SIZE, "dmc_jpeg_rd_sweep: bad arguments");
     if (n_frames == 0) return DMC_OK;
     CUDA_TRY(ctx, cudaSetDevice(ctx->device));
     cudaStream_t s = ctx->stream;
@@ -1246,16 +1270,17 @@ int dmc_jpeg_rd_sweep(dmc_ctx* ctx, const void* src, int src_mem, int n_frames, 
     const size_t fpx = (size_t)rows * cols;
     const JpegEncLayout l = jpeg_enc_layout(rows, cols, optimize);
     const size_t per = l.coef_bytes + l.info_bytes + l.word_bytes + l.slot_bytes + (optimize ? l.opt_bytes + 2 * sizeof(dmcjpeg::HuffTable) : 0) +
-                       sizeof(dmcjpeg::FrameDesc) + fpx * ((host ? 1 : 0) + 1 + (p ? 3 : 0));      // staged source, coded, filtered, ping, pong
+                       sizeof(dmcjpeg::FrameDesc) + fpx * ((host ? 1 : 0) + 1 + (p ? 3 : b ? 1 : 0));   // staged source, coded, filtered (or BRF), ping, pong
     const int group = chunk_frames(kEncGroupBytes, per, n_frames, 2048, false);
     std::vector<char> tabs;
     TRY(rd_tables(ctx, "dmc_jpeg_rd_sweep", rows, cols, qualities, n_q, tabs));
     TRY(reserve(ctx, ctx->rd[RD_DESC], (size_t)group * sizeof(dmcjpeg::FrameDesc)));
     TRY(reserve(ctx, ctx->rd[RD_CODED], fpx * group));
-    if (p) TRY(reserve(ctx, ctx->rd[RD_FILT], fpx * group));
+    if (p || b) TRY(reserve(ctx, ctx->rd[RD_FILT], fpx * group));
     if (host) TRY(reserve(ctx, ctx->rd[RD_SRC], fpx * group));
-    // results of a group of nf frames: [sse_coded][sse_filtered] (uint64, [quality][frame]), then the lengths (uint32)
-    const size_t res_bytes = (size_t)n_q * group * (2 * sizeof(uint64_t) + sizeof(uint32_t));
+    // results of a group of nf frames: [sse_coded][sse_filtered][sse_brf if b] (uint64, [quality][frame]), then the lengths (uint32)
+    const int nsse = b ? 3 : 2;
+    const size_t res_bytes = (size_t)n_q * group * (nsse * sizeof(uint64_t) + sizeof(uint32_t));
     TRY(reserve(ctx, ctx->rd[RD_RES], res_bytes));
     Slot& sl = ctx->slot[0]; sl.stream = s;
     uint8_t* coded = (uint8_t*)ctx->rd[RD_CODED].p;
@@ -1270,25 +1295,32 @@ int dmc_jpeg_rd_sweep(dmc_ctx* ctx, const void* src, int src_mem, int n_frames, 
         }
         uint64_t* d_sc = (uint64_t*)ctx->rd[RD_RES].p;
         uint64_t* d_sf = d_sc + (size_t)n_q * nf;
-        uint32_t* d_len = (uint32_t*)(d_sf + (size_t)n_q * nf);
+        uint64_t* d_sb = d_sf + (size_t)n_q * nf;
+        uint32_t* d_len = (uint32_t*)(d_sc + (size_t)nsse * n_q * nf);
         for (int k = 0; k < n_q; k++) {
             TRY(rd_degrade(ctx, k, dsrc, nf, rows, cols, optimize, coded));
             if (p) TRY(run_chain(ctx, sl, coded, filt, nf, rows, cols, *p));
             LAUNCH(ctx, launch_sse_u8(dsrc, coded, p ? filt : nullptr, d_sc + (size_t)k * nf, p ? d_sf + (size_t)k * nf : nullptr, nf, fpx, s));
+            if (b) {                                                // (stream order: the SSE above has read `filt`)
+                TRY(brf_frames(ctx, coded, filt, nf, rows, cols, *b));
+                LAUNCH(ctx, launch_sse_u8(dsrc, filt, nullptr, d_sb + (size_t)k * nf, nullptr, nf, fpx, s));
+            }
             CUDA_TRY(ctx, cudaMemcpyAsync(d_len + (size_t)k * nf, ctx->jpeg_enc[JE_LENS].p, nf * sizeof(uint32_t), cudaMemcpyDeviceToDevice, s));
         }
-        const size_t used = (size_t)n_q * nf * (2 * sizeof(uint64_t) + sizeof(uint32_t));
+        const size_t used = (size_t)n_q * nf * (nsse * sizeof(uint64_t) + sizeof(uint32_t));
         res.resize(used);
         CUDA_TRY(ctx, cudaMemcpyAsync(res.data(), ctx->rd[RD_RES].p, used, cudaMemcpyDeviceToHost, s));
         CUDA_TRY(ctx, cudaStreamSynchronize(s));
         const uint64_t* sc = (const uint64_t*)res.data();
         const uint64_t* sf = sc + (size_t)n_q * nf;
-        const uint32_t* len = (const uint32_t*)(sf + (size_t)n_q * nf);
+        const uint64_t* sb = sf + (size_t)n_q * nf;
+        const uint32_t* len = (const uint32_t*)(sc + (size_t)nsse * n_q * nf);
         for (int k = 0; k < n_q; k++)
             for (int i = 0; i < nf; i++) {
                 const size_t o = (size_t)k * n_frames + f0 + i, j = (size_t)k * nf + i;
                 bytes[o] = len[j]; sse_coded[o] = sc[j];
                 if (p) sse_filtered[o] = sf[j];
+                if (b) sse_brf[o] = sb[j];
             }
     }
     return DMC_OK;
@@ -1404,10 +1436,58 @@ int dmc_boundary_reconstruction(dmc_ctx* ctx, const dmc_image* src, dmc_image* d
     const void* in; void* out;
     TRY(stage_op(ctx, src, dst, &in, &out));
     const cudaStream_t s = ctx->stream;
-    int nk = launch_brf(in, out, src->rows, src->cols, t, kw, kh, frec, color, space, s);
+    int nk = launch_brf(in, out, 1, src->rows, src->cols, t, kw, kh, frec, color, space, s);
     if (nk == 0) return fail(ctx, DMC_ERR_ARG, "boundaryReconstructionFilter: window too large");
     TRY(after_launch(ctx, nk));
     return stage_out_end(ctx, dst, out, s);
+}
+
+// Frame batches of the boundary reconstruction filter.  Device memory: one launch per group of up to 65535 frames (the grid's
+// z); when dst overlaps src, each group goes through a group-sized scratch, in memmove order.  Host memory: the slot pipeline
+// of dmc_chain_batch.
+int dmc_brf_batch(dmc_ctx* ctx, const void* src, void* dst, int n_frames, int rows, int cols, int depth, const dmc_brf_params* b, int mem) {
+    if (!ctx) return fail(nullptr, DMC_ERR_ARG, "null context");
+    TRY(check_brf_params(ctx, b, "dmc_brf_batch"));
+    if (depth != DMC_8U && depth != DMC_16U && depth != DMC_16S && depth != DMC_32F && depth != DMC_64F) return fail(ctx, DMC_ERR_TYPE, "dmc_brf_batch: depth must be 8U, 16U, 16S, 32F or 64F");
+    if (mem != DMC_MEM_HOST && mem != DMC_MEM_DEVICE) return fail(ctx, DMC_ERR_ARG, "dmc_brf_batch: bad mem");
+    if (n_frames < 0 || rows <= 0 || cols <= 0 || (n_frames > 0 && (!src || !dst))) return fail(ctx, DMC_ERR_SIZE, "dmc_brf_batch: bad arguments");
+    if (n_frames == 0) return DMC_OK;
+    CUDA_TRY(ctx, cudaSetDevice(ctx->device));
+    const size_t fb = (size_t)rows * cols * depth_size(depth), total = fb * n_frames;
+    const dmc_brf_params& bp = *b;
+    auto brf = [&](const void* in, void* out, int nf, cudaStream_t s) {
+        const int nk = launch_brf(in, out, nf, rows, cols, depth, bp.kernel_w, bp.kernel_h, bp.frec, bp.color, bp.space, s);
+        if (nk == 0) return fail(ctx, DMC_ERR_ARG, "dmc_brf_batch: window too large");
+        return after_launch(ctx, nk);
+    };
+    if (mem == DMC_MEM_DEVICE) {
+        // Groups of ~256 MB, as dmc_chain_batch; the first group's launch fails before anything is written.  A group's CTAs read
+        // halos of its source frames while other CTAs write, so where dst overlaps src a group is filtered into scratch and
+        // copied out in stream order.  The groups then run in memmove order: a group never reads frames that an earlier group
+        // has written (with dst above src, the last group first).
+        const int group = chunk_frames(env_mib("DMC_GROUP_MB", (size_t)256 << 20), fb, n_frames, 65535, false);
+        const int ng = (n_frames + group - 1) / group;
+        const bool staged = overlaps(dst, total, src, total), backward = staged && (uintptr_t)dst > (uintptr_t)src;
+        if (staged) TRY(reserve(ctx, ctx->slot[0].buf[SB_OUT], fb * group));
+        for (int g = 0; g < ng; g++) {
+            const int f0 = (backward ? ng - 1 - g : g) * group, nf = n_frames - f0 < group ? n_frames - f0 : group;
+            uint8_t* out = (uint8_t*)dst + fb * f0;
+            TRY(brf((const uint8_t*)src + fb * f0, staged ? ctx->slot[0].buf[SB_OUT].p : out, nf, ctx->stream));
+            if (staged) CUDA_TRY(ctx, cudaMemcpyAsync(out, ctx->slot[0].buf[SB_OUT].p, fb * nf, cudaMemcpyDeviceToDevice, ctx->stream));
+        }
+        return DMC_OK;
+    }
+    // host: chunked streaming.  A chunk reads and writes only its own frames, so src == dst is safe; a dst that partly
+    // overlaps src would be read by a later chunk after an earlier one wrote it, so such a source is copied first.
+    std::vector<char> copy;
+    if (src != dst && overlaps(dst, total, src, total)) { copy.assign((const char*)src, (const char*)src + total); src = copy.data(); }
+    const int chunk = chunk_frames(env_mib("DMC_CHUNK_MB", (size_t)48 << 20), fb, n_frames, 65535, true);
+    void *din = nullptr, *dout = nullptr;
+    return stream_chunks(ctx, n_frames, chunk, ctx->gw.device >= 0, false,
+        [&](const Chunk& c) { return reserve_io(ctx, c, fb * c.nf, fb * c.nf, c.sl->buf[SB_IN], c.sl->buf[SB_OUT], &din, &dout); },
+        [&](const Chunk& c) { return cudaMemcpyAsync(din, (const uint8_t*)src + fb * c.f0, fb * c.nf, cudaMemcpyHostToDevice, c.copy); },
+        [&](const Chunk& c) { return brf(din, dout, c.nf, c.sl->stream); },
+        [&](const Chunk& c) { return cudaMemcpyAsync((uint8_t*)dst + fb * c.f0, dout, fb * c.nf, cudaMemcpyDeviceToHost, c.copy); });
 }
 
 int dmc_minmax_boundary_reconstruction(dmc_ctx* ctx, const dmc_image* src, dmc_image* dst, int minmax_r, int kw, int kh, float frec, float color, float space) {
@@ -1421,7 +1501,7 @@ int dmc_minmax_boundary_reconstruction(dmc_ctx* ctx, const dmc_image* src, dmc_i
     const void* in; void* out;
     TRY(stage_op(ctx, src, dst, &in, &out));
     const cudaStream_t s = ctx->stream;
-    int nk = launch_minmax_brf(in, out, src->rows, src->cols, t, minmax_r, kw, kh, frec, color, space, s);
+    int nk = launch_minmax_brf(in, out, 1, src->rows, src->cols, t, minmax_r, kw, kh, frec, color, space, s);
     if (nk == 0) return fail(ctx, DMC_ERR_ARG, "minmaxBoundaryReconstructionFilter: window too large");
     TRY(after_launch(ctx, nk));
     return stage_out_end(ctx, dst, out, s);
@@ -1659,10 +1739,21 @@ extern "C" {
 // filtered, both depths reprojected, and per camera both rendered and compared with the reference view in one SSE launch.
 // Every render of nf frames is one batched render; its fixed point costs one host read per iteration.  One copy per group
 // brings the results back.
+//
+// The BRF arm (b != NULL) adds per (group, quality) one batched BRF launch on the coded frames, D of its output and its points,
+// and per camera one more render and SSE launch.  Its render reuses the coded view's buffer once that view's SSE is queued.
 int dmc_jpeg_view_rd_sweep(dmc_ctx* ctx, const void* disp, const void* texture, int src_mem, int n_frames, int rows, int cols,
                            const int* qualities, int n_q, int flags, const dmc_chain_params* p, double f,
                            const double* R, const double* t, int n_views, const double* K, int is_sub, int render_flags,
                            uint64_t* bytes, uint64_t* sse_view_coded, uint64_t* sse_view_filtered) {
+    return dmc_jpeg_view_rd_sweep_ex(ctx, disp, texture, src_mem, n_frames, rows, cols, qualities, n_q, flags, p, nullptr, f, R, t, n_views, K,
+                                     is_sub, render_flags, bytes, sse_view_coded, sse_view_filtered, nullptr);
+}
+
+int dmc_jpeg_view_rd_sweep_ex(dmc_ctx* ctx, const void* disp, const void* texture, int src_mem, int n_frames, int rows, int cols,
+                              const int* qualities, int n_q, int flags, const dmc_chain_params* p, const dmc_brf_params* b, double f,
+                              const double* R, const double* t, int n_views, const double* K, int is_sub, int render_flags,
+                              uint64_t* bytes, uint64_t* sse_view_coded, uint64_t* sse_view_filtered, uint64_t* sse_view_brf) {
     if (!ctx) return fail(nullptr, DMC_ERR_ARG, "null context");
     if (!qualities || n_q < 1) return fail(ctx, DMC_ERR_ARG, "dmc_jpeg_view_rd_sweep: no qualities");
     for (int k = 0; k < n_q; k++)
@@ -1676,12 +1767,13 @@ int dmc_jpeg_view_rd_sweep(dmc_ctx* ctx, const void* disp, const void* texture, 
     if (p->brange_method != DMC_FULL_KERNEL && p->brange_method != DMC_FULL_KERNEL_PAIR && p->brange_method != DMC_SEPARABLE_KERNEL)
         return fail(ctx, DMC_ERR_ARG, "dmc_jpeg_view_rd_sweep: brange_method must be FULL_KERNEL, FULL_KERNEL_PAIR or SEPARABLE_KERNEL");
     if (n_views < 1 || !R || !t || !K) return fail(ctx, DMC_ERR_ARG, "dmc_jpeg_view_rd_sweep: at least one camera (R, t, K) is required");
+    if (b) TRY(check_brf_params(ctx, b, "dmc_jpeg_view_rd_sweep"));
     if (src_mem != DMC_MEM_HOST && src_mem != DMC_MEM_DEVICE) return fail(ctx, DMC_ERR_ARG, "dmc_jpeg_view_rd_sweep: bad mem");
     uint64_t bound;
     if (dmc_jpeg_encode_bound_ex(rows, cols, flags, &bound) != DMC_OK) return fail(ctx, DMC_ERR_SIZE, "dmc_jpeg_view_rd_sweep: " + g_err);
     const size_t fpx = (size_t)rows * cols;
     if (fpx >= ((size_t)1 << 29)) return fail(ctx, DMC_ERR_SIZE, "dmc_jpeg_view_rd_sweep: frame too large for the renderer");
-    if (n_frames < 0 || (n_frames > 0 && (!disp || !texture || !bytes || !sse_view_coded || !sse_view_filtered))) return fail(ctx, DMC_ERR_SIZE, "dmc_jpeg_view_rd_sweep: bad arguments");
+    if (n_frames < 0 || (n_frames > 0 && (!disp || !texture || !bytes || !sse_view_coded || !sse_view_filtered || (b && !sse_view_brf)))) return fail(ctx, DMC_ERR_SIZE, "dmc_jpeg_view_rd_sweep: bad arguments");
     if (n_frames == 0) return DMC_OK;
     CUDA_TRY(ctx, cudaSetDevice(ctx->device));
     cudaStream_t s = ctx->stream;
@@ -1689,9 +1781,10 @@ int dmc_jpeg_view_rd_sweep(dmc_ctx* ctx, const void* disp, const void* texture, 
     const int exact = render_flags & DMC_RENDER_EXACT_DIVIDE;
     const JpegEncLayout l = jpeg_enc_layout(rows, cols, optimize);
     // per frame: the encoder's scratch and FrameDesc; staged source and texture; coded, ping, pong, float scratch of the chain;
-    // depth, two sets of points, their projection; raw render, coded and filtered views, reference views; the render's scratch
+    // depth, two sets of points, their projection; raw render, coded and filtered views, reference views; the render's scratch;
+    // with b, the BRF frames and their points
     const size_t per = l.coef_bytes + l.info_bytes + l.word_bytes + l.slot_bytes + (optimize ? l.opt_bytes + 2 * sizeof(dmcjpeg::HuffTable) : 0) +
-                       sizeof(dmcjpeg::FrameDesc) + fpx * ((host ? 4 : 0) + 3 + 4 + 4 + 24 + 8 + 9 + 3 * (size_t)n_views) + render_scratch_bytes(1, rows, cols);
+                       sizeof(dmcjpeg::FrameDesc) + fpx * ((host ? 4 : 0) + 3 + 4 + 4 + 24 + 8 + 9 + 3 * (size_t)n_views + (b ? 1 + 12 : 0)) + render_scratch_bytes(1, rows, cols);
     // the render's attempt offsets are uint32 (at most 7 attempts a point) and the frame is a grid dimension
     const size_t cap = ((size_t)UINT32_MAX / (7 * fpx)) < 2048 ? (size_t)UINT32_MAX / (7 * fpx) : 2048;
     const int group = chunk_frames(kEncGroupBytes, per, n_frames, (int)cap, false);
@@ -1702,14 +1795,17 @@ int dmc_jpeg_view_rd_sweep(dmc_ctx* ctx, const void* disp, const void* texture, 
     TRY(reserve(ctx, ctx->rd[RD_CODED], fpx * group));
     if (host) { TRY(reserve(ctx, ctx->rd[RD_SRC], fpx * group)); TRY(reserve(ctx, ctx->vs[VS_TEX], 3 * fpx * group)); }
     TRY(reserve(ctx, ctx->vs[VS_DEPTH], 4 * fpx * group));
-    TRY(reserve(ctx, ctx->vs[VS_XYZ], 2 * 12 * fpx * group));
+    TRY(reserve(ctx, ctx->vs[VS_XYZ], (b ? 3 : 2) * 12 * fpx * group));
+    if (b) TRY(reserve(ctx, ctx->rd[RD_FILT], fpx * group));
     TRY(reserve(ctx, ctx->vs[VS_PT], 8 * fpx * group));
     TRY(reserve(ctx, ctx->vs[VS_RAW], 3 * fpx * group));
     TRY(reserve(ctx, ctx->vs[VS_VIEW], 2 * 3 * fpx * group));
     TRY(reserve(ctx, ctx->vs[VS_REF], 3 * fpx * group * (size_t)n_views));
     TRY(reserve(ctx, ctx->render[0], render_scratch_bytes(group, rows, cols)));
-    // results of a group of nf frames: [sse_view_coded][sse_view_filtered] (uint64, [quality][view][frame]), the lengths (uint32)
-    const size_t per_res = (size_t)n_q * (2 * sizeof(uint64_t) * n_views + sizeof(uint32_t));
+    // results of a group of nf frames: [sse_view_coded][sse_view_filtered][sse_view_brf if b] (uint64, [quality][view][frame]),
+    // the lengths (uint32)
+    const int nsse = b ? 3 : 2;
+    const size_t per_res = (size_t)n_q * (nsse * sizeof(uint64_t) * n_views + sizeof(uint32_t));
     TRY(reserve(ctx, ctx->rd[RD_RES], per_res * group));
     std::vector<float> kr(9 * (size_t)n_views), tt(3 * (size_t)n_views);
     for (int v = 0; v < n_views; v++) camera_floats(R + 9 * v, t + 3 * v, K, &kr[9 * v], &tt[3 * v]);
@@ -1718,12 +1814,14 @@ int dmc_jpeg_view_rd_sweep(dmc_ctx* ctx, const void* disp, const void* texture, 
     float* depth = (float*)ctx->vs[VS_DEPTH].p;
     float* pt = (float*)ctx->vs[VS_PT].p;
     uint8_t* raw = (uint8_t*)ctx->vs[VS_RAW].p;
+    uint8_t* brf8 = (uint8_t*)ctx->rd[RD_FILT].p;
     std::vector<char> res;
     for (int f0 = 0; f0 < n_frames; f0 += group) {
         const int nf = n_frames - f0 < group ? n_frames - f0 : group;
         const size_t vb = 3 * fpx * nf;           // bytes of the group's views of one camera
         float* xyz_c = (float*)ctx->vs[VS_XYZ].p;
         float* xyz_f = xyz_c + 3 * fpx * nf;
+        float* xyz_b = xyz_f + 3 * fpx * nf;
         uint8_t* view_c = (uint8_t*)ctx->vs[VS_VIEW].p;
         uint8_t* view_f = view_c + vb;
         uint8_t* ref = (uint8_t*)ctx->vs[VS_REF].p;
@@ -1739,18 +1837,27 @@ int dmc_jpeg_view_rd_sweep(dmc_ctx* ctx, const void* disp, const void* texture, 
         for (int v = 0; v < n_views; v++) TRY(render_view(ctx, dtex, xyz_c, pt, raw, ref + vb * v, nf, rows, cols, &kr[9 * v], &tt[3 * v], is_sub, exact));
         uint64_t* d_sc = (uint64_t*)ctx->rd[RD_RES].p;
         uint64_t* d_sf = d_sc + (size_t)n_q * n_views * nf;
-        uint32_t* d_len = (uint32_t*)(d_sf + (size_t)n_q * n_views * nf);
+        uint64_t* d_sb = d_sf + (size_t)n_q * n_views * nf;
+        uint32_t* d_len = (uint32_t*)(d_sc + (size_t)nsse * n_q * n_views * nf);
         for (int k = 0; k < n_q; k++) {
             TRY(rd_degrade(ctx, k, dsrc, nf, rows, cols, optimize, coded));
             CUDA_TRY(ctx, cudaMemcpyAsync(d_len + (size_t)k * nf, ctx->jpeg_enc[JE_LENS].p, nf * sizeof(uint32_t), cudaMemcpyDeviceToDevice, s));
             TRY(depth_points(ctx, coded, depth, xyz_c, nf, rows, cols, *p, f));
             TRY(run_chain(ctx, sl, coded, depth, nf, rows, cols, *p));
             LAUNCH(ctx, launch_reproject(depth, xyz_f, ctx->xtab, nf, rows, cols, DMC_32F, (float)(1.0 / f), (rows - 1) * 0.5f, s));
+            if (b) {
+                TRY(brf_frames(ctx, coded, brf8, nf, rows, cols, *b));
+                TRY(depth_points(ctx, brf8, depth, xyz_b, nf, rows, cols, *p, f));
+            }
             for (int v = 0; v < n_views; v++) {
                 TRY(render_view(ctx, dtex, xyz_c, pt, raw, view_c, nf, rows, cols, &kr[9 * v], &tt[3 * v], is_sub, exact));
                 TRY(render_view(ctx, dtex, xyz_f, pt, raw, view_f, nf, rows, cols, &kr[9 * v], &tt[3 * v], is_sub, exact));
                 const size_t o = ((size_t)k * n_views + v) * nf;
                 LAUNCH(ctx, launch_sse_u8(ref + vb * v, view_c, view_f, d_sc + o, d_sf + o, nf, 3 * fpx, s));
+                if (b) {                                            // (stream order: the SSE above has read view_c)
+                    TRY(render_view(ctx, dtex, xyz_b, pt, raw, view_c, nf, rows, cols, &kr[9 * v], &tt[3 * v], is_sub, exact));
+                    LAUNCH(ctx, launch_sse_u8(ref + vb * v, view_c, nullptr, d_sb + o, nullptr, nf, 3 * fpx, s));
+                }
             }
         }
         const size_t used = per_res * nf;
@@ -1759,13 +1866,15 @@ int dmc_jpeg_view_rd_sweep(dmc_ctx* ctx, const void* disp, const void* texture, 
         CUDA_TRY(ctx, cudaStreamSynchronize(s));
         const uint64_t* sc = (const uint64_t*)res.data();
         const uint64_t* sf = sc + (size_t)n_q * n_views * nf;
-        const uint32_t* len = (const uint32_t*)(sf + (size_t)n_q * n_views * nf);
+        const uint64_t* sb = sf + (size_t)n_q * n_views * nf;
+        const uint32_t* len = (const uint32_t*)(sc + (size_t)nsse * n_q * n_views * nf);
         for (int k = 0; k < n_q; k++)
             for (int i = 0; i < nf; i++) {
                 bytes[(size_t)k * n_frames + f0 + i] = len[(size_t)k * nf + i];
                 for (int v = 0; v < n_views; v++) {
                     const size_t o = ((size_t)k * n_views + v) * n_frames + f0 + i, j = ((size_t)k * n_views + v) * nf + i;
                     sse_view_coded[o] = sc[j]; sse_view_filtered[o] = sf[j];
+                    if (b) sse_view_brf[o] = sb[j];
                 }
             }
     }

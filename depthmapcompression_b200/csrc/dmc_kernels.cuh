@@ -36,10 +36,11 @@ enum StoreOp { STORE_F32 = 0, STORE_U16 = 1, STORE_S16 = 2 };
 int launch_bwrf32f(const void* src, void* dst, int n, int H, int W, int cn, const RowSpan& rs, float th,
                    int load_op, float maf, int store_op, cudaStream_t s);
 
-// boundaryReconstructionFilter_<T> (boundaryReconstructionFilter.cpp:12-131)
-int launch_brf(const void* src, void* dst, int H, int W, int depth, int kw, int kh, float frec, float color, float space, cudaStream_t s);
+// boundaryReconstructionFilter_<T> (boundaryReconstructionFilter.cpp:12-131) on nf dense H x W frames (1..65535, one launch);
+// returns 0 (nothing launched) for a window or frame count the kernel cannot take
+int launch_brf(const void* src, void* dst, int nf, int H, int W, int depth, int kw, int kh, float frec, float color, float space, cudaStream_t s);
 // extension (filter_ext.h): blurRemoveMinMax(minmax_r) fused into the tile staging of the boundary reconstruction filter; 8U / 16U / 16S
-int launch_minmax_brf(const void* src, void* dst, int H, int W, int depth, int minmax_r, int kw, int kh, float frec, float color, float space, cudaStream_t s);
+int launch_minmax_brf(const void* src, void* dst, int nf, int H, int W, int depth, int minmax_r, int kw, int kh, float frec, float color, float space, cudaStream_t s);
 
 // converters (depthmapUtil.cpp:685-1014); kind: 0 disp8U2depth32F, 1 depth32F2disp8U, 2 depth16U2disp8U, 3 disp16S2depth16U
 int launch_convert(int kind, const void* src, void* dst, long n, float fb, float a, float b, cudaStream_t s);

@@ -13,7 +13,7 @@ import ctypes as C
 import numpy as np
 
 from . import capi
-from .capi import lib, DmcImage, DmcChainParams, DmcError, MEM_HOST, MEM_DEVICE, FULL_KERNEL, BORDER_REPLICATE
+from .capi import lib, DmcImage, DmcChainParams, DmcBrfParams, DmcError, MEM_HOST, MEM_DEVICE, FULL_KERNEL, BORDER_REPLICATE
 
 _DEPTH = {np.dtype(np.uint8): capi.CV_8U, np.dtype(np.uint16): capi.CV_16U, np.dtype(np.int16): capi.CV_16S,
           np.dtype(np.float32): capi.CV_32F, np.dtype(np.float64): capi.CV_64F}
@@ -312,11 +312,12 @@ def psnrFromSSE(sse, pixels):
     return float(r) if r.ndim == 0 else r
 
 
-def jpegRateDistortion(frames, qualities, params=None, optimize=False, ctx=None):
-    """The JPEG rate-distortion sweep on the GPU (dmc_jpeg_rd_sweep): every frame is coded at every quality as cv2.imencode
+def jpegRateDistortion(frames, qualities, params=None, optimize=False, ctx=None, brf=None):
+    """The JPEG rate-distortion sweep on the GPU (dmc_jpeg_rd_sweep_ex): every frame is coded at every quality as cv2.imencode
     codes it (optimize: with optimised Huffman tables), decoded, and with `params` (a chain_params(CHAIN_DISP8U, ...))
-    post-filtered; no frame or stream leaves the device.  frames as for degradeJPEG.  Returns a dict of (n_q, n) arrays:
-    bytes, sse_coded, psnr_coded, and with params also sse_filtered, psnr_filtered."""
+    post-filtered; with `brf` (a brf_params(...)) the decoded frames also go through boundaryReconstructionFilter.  No frame
+    or stream leaves the device.  frames as for degradeJPEG.  Returns a dict of (n_q, n) arrays: bytes, sse_coded,
+    psnr_coded, with params also sse_filtered, psnr_filtered, and with brf also sse_brf, psnr_brf."""
     ctx = ctx or default_context()
     sp, n, rows, cols, mem, keep = _frames(frames)
     q = np.ascontiguousarray(np.asarray(qualities).ravel(), dtype=np.int32)
@@ -324,25 +325,32 @@ def jpegRateDistortion(frames, qualities, params=None, optimize=False, ctx=None)
     U64 = C.POINTER(C.c_uint64)
     nbytes, sc = np.zeros(shape, np.uint64), np.zeros(shape, np.uint64)
     sf = np.zeros(shape, np.uint64) if params is not None else None
-    ctx.check(lib.dmc_jpeg_rd_sweep(ctx.h, C.c_void_p(sp), mem, n, rows, cols, q.ctypes.data_as(C.POINTER(C.c_int)), len(q), _jpeg_flags(optimize),
-                                    C.byref(params) if params is not None else None, nbytes.ctypes.data_as(U64), sc.ctypes.data_as(U64),
-                                    sf.ctypes.data_as(U64) if sf is not None else None))
+    sb = np.zeros(shape, np.uint64) if brf is not None else None
+    ctx.check(lib.dmc_jpeg_rd_sweep_ex(ctx.h, C.c_void_p(sp), mem, n, rows, cols, q.ctypes.data_as(C.POINTER(C.c_int)), len(q), _jpeg_flags(optimize),
+                                       C.byref(params) if params is not None else None, C.byref(brf) if brf is not None else None,
+                                       nbytes.ctypes.data_as(U64), sc.ctypes.data_as(U64), sf.ctypes.data_as(U64) if sf is not None else None,
+                                       sb.ctypes.data_as(U64) if sb is not None else None))
     out = {"bytes": nbytes, "sse_coded": sc, "psnr_coded": psnrFromSSE(sc, rows * cols)}
     if sf is not None:
         out["sse_filtered"] = sf
         out["psnr_filtered"] = psnrFromSSE(sf, rows * cols)
+    if sb is not None:
+        out["sse_brf"] = sb
+        out["psnr_brf"] = psnrFromSSE(sb, rows * cols)
     return out
 
 
-def jpegViewRateDistortion(disp, texture, qualities, params, f, R, t, K, isSub=True, optimize=False, exact_divide=False, ctx=None):
-    """The view-synthesis rate-distortion sweep on the GPU (dmc_jpeg_view_rd_sweep): coded depth scored by the views it
+def jpegViewRateDistortion(disp, texture, qualities, params, f, R, t, K, isSub=True, optimize=False, exact_divide=False, ctx=None, brf=None):
+    """The view-synthesis rate-distortion sweep on the GPU (dmc_jpeg_view_rd_sweep_ex): coded depth scored by the views it
     renders, as pointcloudTest renders a decoded depth map.  For every frame, quality and camera (R[v], t[v], shared K) the
     reference view fillSmallHole(projectImagefromXYZ(texture, reprojectXYZ(D(disp), f), ...)), with D the unfiltered
     disp8U2depth32F, is compared with the view of D(decoded) and with the view of filterDisp8U2Depth32F(decoded, params).
     disp: frames as for degradeJPEG; texture: uint8 numpy [n, rows, cols, 3] (or one [rows, cols, 3] image), or (device
     pointer, n, rows, cols) when disp is a device tuple.  params: chain_params(CHAIN_DEPTH32F, ..., focus, baseline, amp).
     R: [n_views, 3, 3] (or one 3x3), t: [n_views, 3].  Returns a dict: bytes (n_q, n), and sse_view_coded, psnr_view_coded,
-    sse_view_filtered, psnr_view_filtered (n_q, n_views, n); the PSNR is cv2.PSNR of the two 8UC3 views."""
+    sse_view_filtered, psnr_view_filtered (n_q, n_views, n); the PSNR is cv2.PSNR of the two 8UC3 views.  brf (a
+    brf_params(...)): also sse_view_brf, psnr_view_brf, the view of D(boundaryReconstructionFilter(decoded)) against the
+    same reference view."""
     ctx = ctx or default_context()
     sp, n, rows, cols, mem, keep = _frames(disp)
     if isinstance(texture, tuple):
@@ -366,13 +374,19 @@ def jpegViewRateDistortion(disp, texture, qualities, params, f, R, t, K, isSub=T
     U64, DP = C.POINTER(C.c_uint64), C.POINTER(C.c_double)
     nbytes = np.zeros((len(q), n), np.uint64)
     sc, sf = np.zeros((len(q), nv, n), np.uint64), np.zeros((len(q), nv, n), np.uint64)
-    ctx.check(lib.dmc_jpeg_view_rd_sweep(ctx.h, C.c_void_p(sp), C.c_void_p(tp), mem, n, rows, cols, q.ctypes.data_as(C.POINTER(C.c_int)), len(q),
-                                         _jpeg_flags(optimize), C.byref(params), float(f), Rs.ctypes.data_as(DP), ts.ctypes.data_as(DP), nv,
-                                         Ks.ctypes.data_as(DP), int(bool(isSub)), capi.RENDER_EXACT_DIVIDE if exact_divide else 0,
-                                         nbytes.ctypes.data_as(U64), sc.ctypes.data_as(U64), sf.ctypes.data_as(U64)))
+    sb = np.zeros((len(q), nv, n), np.uint64) if brf is not None else None
+    ctx.check(lib.dmc_jpeg_view_rd_sweep_ex(ctx.h, C.c_void_p(sp), C.c_void_p(tp), mem, n, rows, cols, q.ctypes.data_as(C.POINTER(C.c_int)), len(q),
+                                            _jpeg_flags(optimize), C.byref(params), C.byref(brf) if brf is not None else None, float(f),
+                                            Rs.ctypes.data_as(DP), ts.ctypes.data_as(DP), nv, Ks.ctypes.data_as(DP), int(bool(isSub)),
+                                            capi.RENDER_EXACT_DIVIDE if exact_divide else 0, nbytes.ctypes.data_as(U64), sc.ctypes.data_as(U64),
+                                            sf.ctypes.data_as(U64), sb.ctypes.data_as(U64) if sb is not None else None))
     px = 3 * rows * cols
-    return {"bytes": nbytes, "sse_view_coded": sc, "psnr_view_coded": psnrFromSSE(sc, px),
-            "sse_view_filtered": sf, "psnr_view_filtered": psnrFromSSE(sf, px)}
+    out = {"bytes": nbytes, "sse_view_coded": sc, "psnr_view_coded": psnrFromSSE(sc, px),
+           "sse_view_filtered": sf, "psnr_view_filtered": psnrFromSSE(sf, px)}
+    if sb is not None:
+        out["sse_view_brf"] = sb
+        out["psnr_view_brf"] = psnrFromSSE(sb, px)
+    return out
 
 
 _default = {}
@@ -382,6 +396,13 @@ def default_context(device=0):
     if device not in _default:
         _default[device] = Context(device)
     return _default[device]
+
+
+def brf_params(ksize=(13, 13), frec=1.0, color=1.0, space=1.0):
+    """Parameters of boundaryReconstructionFilter(src, dest, ksize, frec, color, space) for boundaryReconstructionFilterBatch
+    and the brf= arm of the sweeps.  The defaults are pointcloudTest's call (main.cpp:306-311)."""
+    kw, kh = _ksize(ksize)
+    return DmcBrfParams(kw, kh, float(frec), float(color), float(space))
 
 
 def chain_params(chain, median_r, gaussian_r, minmax_r, brange_r, brange_th, brange_method=FULL_KERNEL, focus=0.0, baseline=0.0, amp=0.0):
@@ -538,6 +559,34 @@ def boundaryReconstructionFilter(src, dest, ksize, frec, color, space, ctx=None)
     s, d = _img(src), _img(dest)
     ctx.check(lib.dmc_boundary_reconstruction(ctx.h, C.byref(s), C.byref(d), kw, kh, frec, color, space))
     return dest
+
+
+def boundaryReconstructionFilterBatch(frames, dst=None, ksize=(13, 13), frec=1.0, color=1.0, space=1.0, ctx=None):
+    """boundaryReconstructionFilter (filter.h:45) on a batch of frames (dmc_brf_batch): every frame of the result equals
+    boundaryReconstructionFilter of that frame.  frames: numpy [n, rows, cols] (or one [rows, cols] frame) of uint8, uint16,
+    int16, float32 or float64, streamed through the device; or (device pointer, n, rows, cols[, dtype]) (dtype defaults to
+    uint8) with dst a device pointer, processed in stream order.  dst=None: a new host array; dst is frames: in place."""
+    ctx = ctx or default_context()
+    b = brf_params(ksize, frec, color, space)
+    if isinstance(frames, tuple):
+        ptr, n, rows, cols = (int(x) for x in frames[:4])
+        dt = np.dtype(frames[4] if len(frames) > 4 else np.uint8)
+        if dt not in _DEPTH:
+            raise DmcError(capi.DMC_ERR_TYPE, "unsupported dtype %s" % dt)
+        if not isinstance(dst, int):
+            raise DmcError(capi.DMC_ERR_ARG, "boundaryReconstructionFilterBatch: device frames need a device pointer dst")
+        ctx.check(lib.dmc_brf_batch(ctx.h, C.c_void_p(ptr), C.c_void_p(dst), n, rows, cols, _DEPTH[dt], C.byref(b), MEM_DEVICE))
+        return dst
+    a = frames if isinstance(frames, np.ndarray) and frames.flags.c_contiguous else np.ascontiguousarray(frames)
+    if a.ndim not in (2, 3):
+        raise DmcError(capi.DMC_ERR_SIZE, "frames must be [n, rows, cols] or [rows, cols]")
+    if a.dtype not in _DEPTH:
+        raise DmcError(capi.DMC_ERR_TYPE, "unsupported dtype %s" % a.dtype)
+    n, rows, cols = (1,) + a.shape if a.ndim == 2 else a.shape
+    if dst is None or dst.shape != a.shape or dst.dtype != a.dtype or not dst.flags.c_contiguous:
+        dst = np.empty(a.shape, a.dtype)
+    ctx.check(lib.dmc_brf_batch(ctx.h, C.c_void_p(a.ctypes.data), C.c_void_p(dst.ctypes.data), n, rows, cols, _DEPTH[a.dtype], C.byref(b), MEM_HOST))
+    return dst
 
 
 def minmaxBoundaryReconstructionFilter(src, dest, r, ksize, frec, color, space, ctx=None):

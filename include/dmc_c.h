@@ -253,6 +253,30 @@ double dmc_psnr_from_sse(uint64_t sse, uint64_t pixels);
 int dmc_jpeg_rd_sweep(dmc_ctx* ctx, const void* src, int src_mem, int n_frames, int rows, int cols, const int* qualities, int n_q,
                       int flags, const dmc_chain_params* p, uint64_t* bytes, uint64_t* sse_coded, uint64_t* sse_filtered);
 
+/* ---- the boundary reconstruction filter on frame batches, and as a third arm of both sweeps ---------------------------- */
+/* Parameters of boundaryReconstructionFilter(src, dest, Size(kernel_w, kernel_h), frec, color, space) (filter.h:45). */
+typedef struct dmc_brf_params { int kernel_w, kernel_h; float frec, color, space; } dmc_brf_params;
+/* boundaryReconstructionFilter (filter.h:45) on n dense single-channel frames of one depth (DMC_8U/16U/16S/32F/64F), host or device memory.
+ * src and dst hold n_frames dense rows x cols frames back to back in `mem`; each frame of dst equals dmc_boundary_reconstruction
+ * of that frame.  Device memory: one launch per group of frames, in stream order (dmc_synchronize before reading dst).  Host
+ * memory: chunks stream through the device as in dmc_chain_batch (pinned memory for overlap); returns when dst is valid.
+ * src == dst is legal, and so is any overlap.  Device memory: where dst overlaps src, each group of frames (~256 MB) is filtered
+ * into scratch of the group's size and copied to dst, so an in-place batch costs one group of device memory and one extra
+ * device-to-device copy of the batch.  Host memory: in place needs nothing extra; a partly overlapping source is copied on the
+ * host first.  DMC_ERR_ARG: b == NULL, a kernel side < 1 or a radius
+ * (side / 2) above DMC_MAX_RADIUS, a window the kernel cannot take; DMC_ERR_TYPE: another depth; nothing is written on error. */
+int dmc_brf_batch(dmc_ctx* ctx, const void* src, void* dst, int n_frames, int rows, int cols, int depth, const dmc_brf_params* b, int mem);
+/* dmc_jpeg_rd_sweep with a third arm.  b == NULL: exactly dmc_jpeg_rd_sweep (sse_brf may be NULL and is not written).  With b,
+ * B(x) = boundaryReconstructionFilter(x, Size(b->kernel_w, b->kernel_h), b->frec, b->color, b->space) on the 8-bit decoded
+ * disparity and
+ *          sse_brf[k*n+i]      = SSE(frame_i, B(imdecode(that stream))).
+ * The reference never runs this comparison: pointcloudTest keeps the call boundaryReconstructionFilter(disp, disp, Size(13,13),
+ * 1, 1, 1) on the decoded disparity commented out (main.cpp:306-311).  Placing B there, in place of the post filter set, is this
+ * library's definition.  b's argument rules are those of dmc_brf_batch (DMC_ERR_ARG, nothing written); p may be NULL with b set. */
+int dmc_jpeg_rd_sweep_ex(dmc_ctx* ctx, const void* src, int src_mem, int n_frames, int rows, int cols, const int* qualities, int n_q,
+                         int flags, const dmc_chain_params* p, const dmc_brf_params* b, uint64_t* bytes, uint64_t* sse_coded,
+                         uint64_t* sse_filtered, uint64_t* sse_brf);
+
 /* ---- stand-alone operators of filter.h ------------------------------------------------------------------- */
 /* binalyWeightedRangeFilter filter.h:29 (binalyWeightedRangeFilter.cpp:1106): 8U/16S/16U/32F x C1/C3 */
 int dmc_bwrf(dmc_ctx* ctx, const dmc_image* src, dmc_image* dst, int kernel_w, int kernel_h, float threshold,
@@ -339,6 +363,15 @@ int dmc_jpeg_view_rd_sweep(dmc_ctx* ctx, const void* disp, const void* texture, 
                            const int* qualities, int n_q, int flags, const dmc_chain_params* p, double f,
                            const double* R, const double* t, int n_views, const double* K, int is_sub, int render_flags,
                            uint64_t* bytes, uint64_t* sse_view_coded, uint64_t* sse_view_filtered);
+/* dmc_jpeg_view_rd_sweep with a third arm.  b == NULL: exactly dmc_jpeg_view_rd_sweep (sse_view_brf may be NULL and is not
+ * written).  With b, B as for dmc_jpeg_rd_sweep_ex on the 8-bit decoded disparity, and D and view the sweep's own:
+ *   sse_view_brf[(k*n_views + v)*n + i] = SSE(view(D(disp_i)), view(D(B(dec)))).
+ * p stays required: it supplies focus, baseline and amp for D.  As for the gray sweep, the reference never runs this: the BRF
+ * call on the decoded disparity is commented out at main.cpp:306-311, and putting B before D is this library's definition. */
+int dmc_jpeg_view_rd_sweep_ex(dmc_ctx* ctx, const void* disp, const void* texture, int src_mem, int n_frames, int rows, int cols,
+                              const int* qualities, int n_q, int flags, const dmc_chain_params* p, const dmc_brf_params* b, double f,
+                              const double* R, const double* t, int n_views, const double* K, int is_sub, int render_flags,
+                              uint64_t* bytes, uint64_t* sse_view_coded, uint64_t* sse_view_filtered, uint64_t* sse_view_brf);
 
 #ifdef __cplusplus
 }

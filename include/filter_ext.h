@@ -134,3 +134,67 @@ inline void jpegViewRateDistortionGray(const Mat& disp, const Mat& texture, cons
 		}
 	}
 }
+
+// The two sweeps above with a third arm, the boundary reconstruction filter: psnr_brf[k] = cv::PSNR(src,
+// boundaryReconstructionFilter(decoded, brf_ksize, frec, color, space)), the filter the reference keeps on the decoded
+// disparity but comments out (main.cpp:306-311).  Scoring it there, next to the post filter set, is this library's definition.
+inline void jpegRateDistortionGray(const Mat& src, const vector<int>& qualities, vector<int>& bytes, vector<double>& psnr_coded,
+                                   vector<double>& psnr_filtered, int median_r, int gaussian_r, int minmax_r, int brange_r, int brange_th,
+                                   Size brf_ksize, float frec, float color, float space, vector<double>& psnr_brf, bool optimize = false)
+{
+	dmc_dropin::require_gray8(src, "jpegRateDistortionGray");
+	const Mat s = src.isContinuous() ? src : src.clone();
+	const size_t nq = qualities.size();
+	vector<uint64_t> b(nq), sc(nq), sf(nq), sb(nq);
+	dmc_chain_params p = {DMC_CHAIN_DISP8U, median_r, gaussian_r, minmax_r, brange_r, (float)brange_th, DMC_FULL_KERNEL, 0, 0, 0};
+	dmc_brf_params bp = {brf_ksize.width, brf_ksize.height, frec, color, space};
+	dmc_dropin::check(dmc_jpeg_rd_sweep_ex(dmc_dropin::context(), s.data, DMC_MEM_HOST, 1, s.rows, s.cols, qualities.data(), (int)nq,
+	                                       optimize ? DMC_JPEG_OPTIMIZE_HUFFMAN : 0, &p, &bp, b.data(), sc.data(), sf.data(), sb.data()), "jpegRateDistortionGray");
+	const uint64_t pixels = (uint64_t)s.rows * s.cols;
+	bytes.resize(nq); psnr_coded.resize(nq); psnr_filtered.resize(nq); psnr_brf.resize(nq);
+	for (size_t k = 0; k < nq; k++) {
+		bytes[k] = (int)b[k];
+		psnr_coded[k] = dmc_psnr_from_sse(sc[k], pixels);
+		psnr_filtered[k] = dmc_psnr_from_sse(sf[k], pixels);
+		psnr_brf[k] = dmc_psnr_from_sse(sb[k], pixels);
+	}
+}
+
+// psnr_brf[k][v] = cv::PSNR of the reference view against the view rendered from
+// disp8U2depth32F(boundaryReconstructionFilter(decoded, brf_ksize, frec, color, space), focus*baseline, amp).
+inline void jpegViewRateDistortionGray(const Mat& disp, const Mat& texture, const vector<int>& qualities, double focus, double baseline, double amp,
+                                       int median_r, int gaussian_r, int minmax_r, int brange_r, float brange_th, double f,
+                                       const vector<Mat>& R, const vector<Mat>& t, const Mat& K, bool isSub, vector<int>& bytes,
+                                       vector<vector<double> >& psnr_coded, vector<vector<double> >& psnr_filtered,
+                                       Size brf_ksize, float frec, float color, float space, vector<vector<double> >& psnr_brf, bool optimize = false)
+{
+	dmc_dropin::require_gray8(disp, "jpegViewRateDistortionGray");
+	if (texture.type() != CV_8UC3 || texture.rows != disp.rows || texture.cols != disp.cols) {
+#ifdef DMC_MINICV_HPP
+		throw cv::Exception("jpegViewRateDistortionGray: texture must be CV_8UC3 of the size of disp", __FILE__, __LINE__);
+#else
+		CV_Error(cv::Error::StsAssert, "jpegViewRateDistortionGray: texture must be CV_8UC3 of the size of disp");
+#endif
+	}
+	const Mat s = disp.isContinuous() ? disp : disp.clone();
+	const Mat tex = texture.isContinuous() ? texture : texture.clone();
+	const size_t nq = qualities.size(), nv = R.size() < t.size() ? R.size() : t.size();
+	vector<double> r(9 * nv), tt(3 * nv), k(9);
+	for (size_t v = 0; v < nv; v++) dmc_dropin::camera(R[v], t[v], K, &r[9 * v], &tt[3 * v], &k[0], "jpegViewRateDistortionGray");
+	vector<uint64_t> b(nq), sc(nq * nv), sf(nq * nv), sb(nq * nv);
+	dmc_chain_params p = {DMC_CHAIN_DEPTH32F, median_r, gaussian_r, minmax_r, brange_r, brange_th, DMC_FULL_KERNEL, focus, baseline, amp};
+	dmc_brf_params bp = {brf_ksize.width, brf_ksize.height, frec, color, space};
+	dmc_dropin::check(dmc_jpeg_view_rd_sweep_ex(dmc_dropin::context(), s.data, tex.data, DMC_MEM_HOST, 1, s.rows, s.cols, qualities.data(), (int)nq,
+	                                            optimize ? DMC_JPEG_OPTIMIZE_HUFFMAN : 0, &p, &bp, f, nv ? &r[0] : 0, nv ? &tt[0] : 0, (int)nv, &k[0], isSub ? 1 : 0, 0,
+	                                            b.data(), sc.data(), sf.data(), sb.data()), "jpegViewRateDistortionGray");
+	const uint64_t pixels = 3 * (uint64_t)s.rows * s.cols;
+	bytes.resize(nq); psnr_coded.assign(nq, vector<double>(nv)); psnr_filtered.assign(nq, vector<double>(nv)); psnr_brf.assign(nq, vector<double>(nv));
+	for (size_t q = 0; q < nq; q++) {
+		bytes[q] = (int)b[q];
+		for (size_t v = 0; v < nv; v++) {
+			psnr_coded[q][v] = dmc_psnr_from_sse(sc[q * nv + v], pixels);
+			psnr_filtered[q][v] = dmc_psnr_from_sse(sf[q * nv + v], pixels);
+			psnr_brf[q][v] = dmc_psnr_from_sse(sb[q * nv + v], pixels);
+		}
+	}
+}
