@@ -9,6 +9,8 @@ import ctypes as C
 import numpy as np
 import pytest
 
+from _util import ntaps
+
 pytestmark = pytest.mark.gpu
 
 C0 = 128
@@ -19,16 +21,6 @@ def dmc():
     import depthmapcompression_b200 as m
     m.default_context(0)          # raises loudly without a GPU / without the built library
     return m
-
-
-def ntaps(r):
-    n = 0
-    for dy in range(-r, r + 1):
-        lim, j = r * r - dy * dy, 0
-        while (j + 1) * (j + 1) <= lim:
-            j += 1
-        n += 2 * j + 1
-    return n
 
 
 def rows_per_thread(r, H, W):
