@@ -33,6 +33,7 @@ EXPORTS = [
     "dmc_chain_batch_jpeg", "dmc_jpeg_probe", "dmc_jpeg_encode_bound", "dmc_jpeg_encode_gray_batch", "dmc_jpeg_degrade_gray_batch", "dmc_jpeg_encode_bound_ex", "dmc_jpeg_encode_gray_batch_ex", "dmc_jpeg_degrade_gray_batch_ex", "dmc_split_bgr_line_interleave", "dmc_project_points", "dmc_project_image_from_xyz", "dmc_fill_small_hole", "dmc_hostlink_probe", "dmc_release_device", "dmc_set_gateway", "dmc_get_gateway", "dmc_sched_get_routing",
     "dmc_sse_gray_batch", "dmc_psnr_from_sse", "dmc_jpeg_rd_sweep", "dmc_jpeg_view_rd_sweep",
     "dmc_brf_batch", "dmc_jpeg_rd_sweep_ex", "dmc_jpeg_view_rd_sweep_ex",
+    "dmc_prepare_disp_batch", "dmc_render_view_batch",
 ]
 MAX_DEVICES = 16
 RENDER_EXACT_DIVIDE = 1
@@ -122,6 +123,8 @@ def _load():
         "dmc_fill_small_hole": (I, [P, IMG, IMG]), "dmc_split_bgr_line_interleave": (I, [P, IMG, IMG]),
         "dmc_hostlink_probe": (I, [C.POINTER(I), I, C.POINTER(DmcHostlinkInfo)]), "dmc_release_device": (I, [I]), "dmc_set_gateway": (I, [P, I]), "dmc_get_gateway": (I, [P]),
         "dmc_sched_get_routing": (I, [P, C.POINTER(I), C.POINTER(D), C.POINTER(D)]),
+        "dmc_prepare_disp_batch": (I, [P, P, P, I, I, I, F, F, F, I, I]),
+        "dmc_render_view_batch": (I, [P, P, I, P, I, I, I, I, D, C.POINTER(D), C.POINTER(D), I, C.POINTER(D), I, I, P]),
         "dmc_fill_occlusion": (I, [P, IMG, I, I]), "dmc_reproject_xyz": (I, [P, IMG, IMG, D]), "dmc_transpose": (I, [P, IMG, IMG]),
     }
     for name, (res, args) in sig.items():

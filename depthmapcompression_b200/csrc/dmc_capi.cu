@@ -1585,6 +1585,45 @@ int dmc_transpose(dmc_ctx* ctx, const dmc_image* src, dmc_image* dst) {
     return stage_out_end(ctx, dst, out, s);
 }
 
+// pointcloudTest's preparation on frame batches.  Device memory: groups of ~256 MB of source and output, each through a
+// group-sized scratch for the first pass when passes = 2.  Host memory: the slot pipeline of dmc_chain_batch.
+int dmc_prepare_disp_batch(dmc_ctx* ctx, const void* depth16, void* disp8, int n_frames, int rows, int cols, float focal_baseline,
+                           float a, float b, int passes, int mem) {
+    if (!ctx) return fail(nullptr, DMC_ERR_ARG, "null context");
+    if (passes != 1 && passes != 2) return fail(ctx, DMC_ERR_ARG, "dmc_prepare_disp_batch: passes must be 1 or 2");
+    if (mem != DMC_MEM_HOST && mem != DMC_MEM_DEVICE) return fail(ctx, DMC_ERR_ARG, "dmc_prepare_disp_batch: bad mem");
+    if (n_frames < 0 || rows <= 0 || cols <= 0 || (n_frames > 0 && (!depth16 || !disp8))) return fail(ctx, DMC_ERR_SIZE, "dmc_prepare_disp_batch: bad arguments");
+    if (cols < 2) return fail(ctx, DMC_ERR_SIZE, "dmc_prepare_disp_batch: fillOcclusion needs at least 2 columns");
+    if (passes == 2 && rows < 2) return fail(ctx, DMC_ERR_SIZE, "dmc_prepare_disp_batch: the column pass needs at least 2 rows");
+    const size_t fpx = (size_t)rows * cols;
+    if (overlaps(disp8, fpx * n_frames, depth16, 2 * fpx * n_frames)) return fail(ctx, DMC_ERR_ARG, "dmc_prepare_disp_batch: depth16 and disp8 overlap");
+    if (n_frames == 0) return DMC_OK;
+    CUDA_TRY(ctx, cudaSetDevice(ctx->device));
+    auto prepare = [&](const void* in, void* out, uint8_t* scratch, int nf, cudaStream_t s) {
+        return after_launch(ctx, launch_prepare_disp((const uint16_t*)in, (uint8_t*)out, scratch, nf, rows, cols, focal_baseline, a, b, passes, s));
+    };
+    if (mem == DMC_MEM_DEVICE) {
+        const int group = chunk_frames(env_mib("DMC_GROUP_MB", (size_t)256 << 20), 3 * fpx, n_frames, 65535, false);
+        uint8_t* scratch = nullptr;
+        if (passes == 2) { TRY(reserve(ctx, ctx->slot[0].buf[SB_PING], fpx * group)); scratch = (uint8_t*)ctx->slot[0].buf[SB_PING].p; }
+        for (int f0 = 0; f0 < n_frames; f0 += group) {
+            const int nf = n_frames - f0 < group ? n_frames - f0 : group;
+            TRY(prepare((const uint16_t*)depth16 + fpx * f0, (uint8_t*)disp8 + fpx * f0, scratch, nf, ctx->stream));
+        }
+        return DMC_OK;
+    }
+    const int chunk = chunk_frames(env_mib("DMC_CHUNK_MB", (size_t)48 << 20), 2 * fpx, n_frames, 65535, true);
+    void *din = nullptr, *dout = nullptr;
+    return stream_chunks(ctx, n_frames, chunk, ctx->gw.device >= 0, false,
+        [&](const Chunk& c) {
+            if (passes == 2) TRY(reserve(ctx, c.sl->buf[SB_PING], fpx * c.nf));
+            return reserve_io(ctx, c, 2 * fpx * c.nf, fpx * c.nf, c.sl->buf[SB_IN], c.sl->buf[SB_OUT], &din, &dout);
+        },
+        [&](const Chunk& c) { return cudaMemcpyAsync(din, (const uint16_t*)depth16 + fpx * c.f0, 2 * fpx * c.nf, cudaMemcpyHostToDevice, c.copy); },
+        [&](const Chunk& c) { return prepare(din, dout, (uint8_t*)c.sl->buf[SB_PING].p, c.nf, c.sl->stream); },
+        [&](const Chunk& c) { return cudaMemcpyAsync((uint8_t*)disp8 + fpx * c.f0, dout, fpx * c.nf, cudaMemcpyDeviceToHost, c.copy); });
+}
+
 }  // extern "C"
 
 namespace {
@@ -1722,12 +1761,27 @@ int render_view(dmc_ctx* ctx, const uint8_t* tex, const float* xyz, float* pt, u
 }
 
 // D(x) of nf 8-bit frames: disp8U2depth32F(x, focus * baseline, amp, 0), one launch per frame because the converter's
-// SIMD body / scalar tail split is per call; then reprojectXYZ into xyz.
-int depth_points(dmc_ctx* ctx, const uint8_t* disp, float* depth, float* xyz, int nf, int rows, int cols, const dmc_chain_params& p, double f) {
+// SIMD body / scalar tail split is per call.
+int disp_depth(dmc_ctx* ctx, const uint8_t* disp, float* depth, int nf, int rows, int cols, const dmc_chain_params& p) {
     const size_t fpx = (size_t)rows * cols;
     for (int i = 0; i < nf; i++)
         LAUNCH(ctx, launch_convert(0, disp + fpx * i, depth + fpx * i, (long)fpx, (float)(p.focus * p.baseline), (float)p.amp, 0.f, ctx->stream));
+    return DMC_OK;
+}
+
+// D(x) of nf 8-bit frames, then reprojectXYZ into xyz.
+int depth_points(dmc_ctx* ctx, const uint8_t* disp, float* depth, float* xyz, int nf, int rows, int cols, const dmc_chain_params& p, double f) {
+    TRY(disp_depth(ctx, disp, depth, nf, rows, cols, p));
     LAUNCH(ctx, launch_reproject(depth, xyz, ctx->xtab, nf, rows, cols, DMC_32F, (float)(1.0 / f), (rows - 1) * 0.5f, ctx->stream));
+    return DMC_OK;
+}
+
+// The views of a group of nf frames: reprojectXYZ of their depths (dtype) into xyz, then for every camera v render_view
+// into out + v * view_stride.  kr, tt: the n_views cameras of camera_floats; ctx->xtab holds reproject_table(cols, f).
+int render_views(dmc_ctx* ctx, const void* depth, int dtype, const uint8_t* tex, float* xyz, float* pt, uint8_t* raw, uint8_t* out, size_t view_stride,
+                 int nf, int rows, int cols, double f, const float* kr, const float* tt, int n_views, int is_sub, int exact) {
+    LAUNCH(ctx, launch_reproject(depth, xyz, ctx->xtab, nf, rows, cols, dtype, (float)(1.0 / f), (rows - 1) * 0.5f, ctx->stream));
+    for (int v = 0; v < n_views; v++) TRY(render_view(ctx, tex, xyz, pt, raw, out + view_stride * v, nf, rows, cols, kr + 9 * v, tt + 3 * v, is_sub, exact));
     return DMC_OK;
 }
 }  // namespace
@@ -1833,8 +1887,8 @@ int dmc_jpeg_view_rd_sweep_ex(dmc_ctx* ctx, const void* disp, const void* textur
             dsrc = (const uint8_t*)ctx->rd[RD_SRC].p;
             dtex = (const uint8_t*)ctx->vs[VS_TEX].p;
         }
-        TRY(depth_points(ctx, dsrc, depth, xyz_c, nf, rows, cols, *p, f));
-        for (int v = 0; v < n_views; v++) TRY(render_view(ctx, dtex, xyz_c, pt, raw, ref + vb * v, nf, rows, cols, &kr[9 * v], &tt[3 * v], is_sub, exact));
+        TRY(disp_depth(ctx, dsrc, depth, nf, rows, cols, *p));
+        TRY(render_views(ctx, depth, DMC_32F, dtex, xyz_c, pt, raw, ref, vb, nf, rows, cols, f, kr.data(), tt.data(), n_views, is_sub, exact));
         uint64_t* d_sc = (uint64_t*)ctx->rd[RD_RES].p;
         uint64_t* d_sf = d_sc + (size_t)n_q * n_views * nf;
         uint64_t* d_sb = d_sf + (size_t)n_q * n_views * nf;
@@ -1878,6 +1932,66 @@ int dmc_jpeg_view_rd_sweep_ex(dmc_ctx* ctx, const void* disp, const void* textur
                 }
             }
     }
+    return DMC_OK;
+}
+
+// Views of frame batches: group by group (sized like dmc_jpeg_view_rd_sweep's groups: the render's scratch, the points, their
+// projection, a raw render, and for host memory the staged depths, textures and views), render_views.  Device memory writes
+// the views in place; host memory stages each group and copies its views back per camera.
+int dmc_render_view_batch(dmc_ctx* ctx, const void* depth, int depth_type, const void* texture, int mem, int n_frames, int rows, int cols,
+                          double f, const double* R, const double* t, int n_views, const double* K, int is_sub, int render_flags, void* views) {
+    if (!ctx) return fail(nullptr, DMC_ERR_ARG, "null context");
+    if (n_views < 1 || !R || !t || !K) return fail(ctx, DMC_ERR_ARG, "dmc_render_view_batch: at least one camera (R, t, K) is required");
+    if (render_flags & ~DMC_RENDER_EXACT_DIVIDE) return fail(ctx, DMC_ERR_ARG, "dmc_render_view_batch: unknown render_flags " + std::to_string(render_flags));
+    if (depth_type != DMC_8U && depth_type != DMC_16S && depth_type != DMC_16U && depth_type != DMC_32F)
+        return fail(ctx, DMC_ERR_ARG, "dmc_render_view_batch: depth_type must be DMC_8U, DMC_16S, DMC_16U or DMC_32F");
+    if (mem != DMC_MEM_HOST && mem != DMC_MEM_DEVICE) return fail(ctx, DMC_ERR_ARG, "dmc_render_view_batch: bad mem");
+    if (n_frames < 0 || rows <= 0 || cols <= 0 || (n_frames > 0 && (!depth || !texture || !views))) return fail(ctx, DMC_ERR_SIZE, "dmc_render_view_batch: bad arguments");
+    const size_t fpx = (size_t)rows * cols, db = depth_size(depth_type) * fpx, vb1 = 3 * fpx;
+    if (fpx >= ((size_t)1 << 29)) return fail(ctx, DMC_ERR_SIZE, "dmc_render_view_batch: frame too large for the renderer");
+    const size_t vbytes = vb1 * n_frames * (size_t)n_views;
+    if (overlaps(views, vbytes, depth, db * n_frames) || overlaps(views, vbytes, texture, vb1 * n_frames))
+        return fail(ctx, DMC_ERR_ARG, "dmc_render_view_batch: views overlap depth or texture");
+    if (n_frames == 0) return DMC_OK;
+    CUDA_TRY(ctx, cudaSetDevice(ctx->device));
+    const cudaStream_t s = ctx->stream;
+    const bool host = mem == DMC_MEM_HOST;
+    const int exact = render_flags & DMC_RENDER_EXACT_DIVIDE;
+    const size_t per = fpx * (12 + 8 + 3 + (host ? depth_size(depth_type) + 3 + 3 * (size_t)n_views : 0)) + render_scratch_bytes(1, rows, cols);
+    // the render's attempt offsets are uint32 (at most 7 attempts a point) and the frame is a grid dimension
+    const size_t cap = ((size_t)UINT32_MAX / (7 * fpx)) < 2048 ? (size_t)UINT32_MAX / (7 * fpx) : 2048;
+    const int group = chunk_frames(env_mib("DMC_GROUP_MB", kEncGroupBytes), per, n_frames, (int)cap, false);
+    TRY(reproject_table(ctx, cols, f));
+    if (host) {
+        TRY(reserve(ctx, ctx->vs[VS_DEPTH], db * group));
+        TRY(reserve(ctx, ctx->vs[VS_TEX], vb1 * group));
+        TRY(reserve(ctx, ctx->vs[VS_VIEW], vb1 * group * (size_t)n_views));
+    }
+    TRY(reserve(ctx, ctx->vs[VS_XYZ], 12 * fpx * group));
+    TRY(reserve(ctx, ctx->vs[VS_PT], 8 * fpx * group));
+    TRY(reserve(ctx, ctx->vs[VS_RAW], vb1 * group));
+    TRY(reserve(ctx, ctx->render[0], render_scratch_bytes(group, rows, cols)));
+    std::vector<float> kr(9 * (size_t)n_views), tt(3 * (size_t)n_views);
+    for (int v = 0; v < n_views; v++) camera_floats(R + 9 * v, t + 3 * v, K, &kr[9 * v], &tt[3 * v]);
+    ctx->slot[0].stream = s;
+    for (int f0 = 0; f0 < n_frames; f0 += group) {
+        const int nf = n_frames - f0 < group ? n_frames - f0 : group;
+        const void* d = (const uint8_t*)depth + db * f0;
+        const uint8_t* tex = (const uint8_t*)texture + vb1 * f0;
+        uint8_t* out = (uint8_t*)views + vb1 * f0;
+        size_t stride = vb1 * n_frames;
+        if (host) {
+            CUDA_TRY(ctx, cudaMemcpyAsync(ctx->vs[VS_DEPTH].p, d, db * nf, cudaMemcpyHostToDevice, s));
+            CUDA_TRY(ctx, cudaMemcpyAsync(ctx->vs[VS_TEX].p, tex, vb1 * nf, cudaMemcpyHostToDevice, s));
+            d = ctx->vs[VS_DEPTH].p; tex = (const uint8_t*)ctx->vs[VS_TEX].p; out = (uint8_t*)ctx->vs[VS_VIEW].p; stride = vb1 * nf;
+        }
+        TRY(render_views(ctx, d, depth_type, tex, (float*)ctx->vs[VS_XYZ].p, (float*)ctx->vs[VS_PT].p, (uint8_t*)ctx->vs[VS_RAW].p, out, stride,
+                         nf, rows, cols, f, kr.data(), tt.data(), n_views, is_sub, exact));
+        if (host)
+            for (int v = 0; v < n_views; v++)
+                CUDA_TRY(ctx, cudaMemcpyAsync((uint8_t*)views + vb1 * ((size_t)v * n_frames + f0), out + stride * v, vb1 * nf, cudaMemcpyDeviceToHost, s));
+    }
+    if (host) CUDA_TRY(ctx, cudaStreamSynchronize(s));
     return DMC_OK;
 }
 

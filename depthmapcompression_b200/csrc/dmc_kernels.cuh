@@ -48,6 +48,9 @@ int launch_f32_to_u16(const float* src, uint16_t* dst, long n, cudaStream_t s); 
 // fillOcclusion_<T> / Inv_ (depthmapUtil.cpp:548-636): `pristine` is an untouched copy of `img`
 int launch_fill_occlusion(void* img, const void* pristine, int H, int W, int depth, double invalid, int inv, cudaStream_t s);
 int launch_transpose(const void* src, void* dst, int H, int W, int elem_size, cudaStream_t s);   // cv::transpose, single channel
+// pointcloudTest's preparation of nf frames (dmc_prepare.cu): depth16U2disp8U -> fillOcclusion(0, FILL_DISPARITY), and with
+// passes = 2 the column fill (transpose -> fillOcclusion -> transpose) from `scratch` (nf frames of 8 bits) into dst
+int launch_prepare_disp(const uint16_t* src, uint8_t* dst, uint8_t* scratch, int nf, int rows, int cols, float fb, float a, float b, int passes, cudaStream_t s);
 // reprojectXYZ_<T> (depthmapUtil.cpp:450-481) of `frames` frames: xtab[i] = running FP32 sum along the row, computed by the
 // host and shared by the frames
 int launch_reproject(const void* depth, float* xyz, const float* xtab, int frames, int H, int W, int dtype, float fyinv, float ch, cudaStream_t s);

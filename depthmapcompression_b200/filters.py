@@ -589,6 +589,71 @@ def boundaryReconstructionFilterBatch(frames, dst=None, ksize=(13, 13), frec=1.0
     return dst
 
 
+def prepareDisparityBatch(depth16, focal_baseline, a=1.0, b=0.0, passes=2, dst=None, ctx=None):
+    """pointcloudTest's preparation of sensor depth on a batch (dmc_prepare_disp_batch): every frame of the result equals
+    fillOcclusion(depth16U2disp8U(frame, focal_baseline, a, b), 0, FILL_DISPARITY), and with passes=2 (pointcloudTest,
+    main.cpp:254-260) that filled again around a transpose; passes=1 is simpleTest's call.  depth16: uint16 numpy
+    [n, rows, cols] (or one [rows, cols] frame), streamed through the device; or (device pointer, n, rows, cols) with dst a
+    device pointer, processed in stream order.  dst=None: a new uint8 host array."""
+    ctx = ctx or default_context()
+    if isinstance(depth16, tuple):
+        ptr, n, rows, cols = (int(x) for x in depth16)
+        if not isinstance(dst, int):
+            raise DmcError(capi.DMC_ERR_ARG, "prepareDisparityBatch: device frames need a device pointer dst")
+        ctx.check(lib.dmc_prepare_disp_batch(ctx.h, C.c_void_p(ptr), C.c_void_p(dst), n, rows, cols, focal_baseline, a, b, int(passes), MEM_DEVICE))
+        return dst
+    s = np.ascontiguousarray(depth16)
+    if s.dtype != np.uint16 or s.ndim not in (2, 3):
+        raise DmcError(capi.DMC_ERR_TYPE, "prepareDisparityBatch: depth16 must be uint16 [n, rows, cols] or [rows, cols]")
+    n, rows, cols = (1,) + s.shape if s.ndim == 2 else s.shape
+    if dst is None or dst.shape != s.shape or dst.dtype != np.uint8 or not dst.flags.c_contiguous:
+        dst = np.empty(s.shape, np.uint8)
+    ctx.check(lib.dmc_prepare_disp_batch(ctx.h, C.c_void_p(s.ctypes.data), C.c_void_p(dst.ctypes.data), n, rows, cols, focal_baseline, a, b, int(passes), MEM_HOST))
+    return dst
+
+
+def renderViewBatch(depth, texture, f, R, t, K, isSub=True, exact_divide=False, dst=None, ctx=None):
+    """pointcloudTest's views of a batch (dmc_render_view_batch): views[v, i] = fillSmallHole(projectImagefromXYZ(texture[i],
+    reprojectXYZ(depth[i], f), R[v], t[v], K, isSub)), the fill in place (main.cpp:321-355).  depth: numpy [n, rows, cols]
+    (or one [rows, cols] frame) of uint8, int16, uint16 or float32 (filterDisp8U2Depth32F's output as it is); texture: uint8
+    [n, rows, cols, 3] (or one [rows, cols, 3] image).  Or device tuples (pointer, n, rows, cols[, dtype]) for depth (dtype
+    defaults to float32) and (pointer, n, rows, cols) for texture, with dst a device pointer, processed in stream order.
+    R: [n_views, 3, 3] (or one 3x3), t: [n_views, 3].  Returns uint8 [n_views, n, rows, cols, 3] (dst=None: a new host array)."""
+    ctx = ctx or default_context()
+    Rs = np.ascontiguousarray(R, np.float64).reshape(-1, 9)
+    ts = np.ascontiguousarray(t, np.float64).reshape(-1, 3)
+    Ks = np.ascontiguousarray(K, np.float64).reshape(9)
+    if Rs.shape[0] != ts.shape[0]:
+        raise DmcError(capi.DMC_ERR_ARG, "renderViewBatch: R and t must hold one camera each")
+    nv = Rs.shape[0]
+    if isinstance(depth, tuple):
+        dp, n, rows, cols = (int(x) for x in depth[:4])
+        dt = np.dtype(depth[4] if len(depth) > 4 else np.float32)
+        if not isinstance(texture, tuple) or tuple(int(x) for x in texture[1:4]) != (n, rows, cols):
+            raise DmcError(capi.DMC_ERR_SIZE, "renderViewBatch: device depth needs a device texture tuple of the same batch")
+        if not isinstance(dst, int):
+            raise DmcError(capi.DMC_ERR_ARG, "renderViewBatch: device frames need a device pointer dst")
+        tp, mem, out = int(texture[0]), MEM_DEVICE, dst
+    else:
+        d, tex = np.ascontiguousarray(depth), np.ascontiguousarray(texture)
+        if d.ndim not in (2, 3) or tex.dtype != np.uint8 or tex.ndim != d.ndim + 1 or tex.shape[:-1] != d.shape or tex.shape[-1] != 3:
+            raise DmcError(capi.DMC_ERR_SIZE, "renderViewBatch: depth [n, rows, cols] and texture uint8 [n, rows, cols, 3] of one batch")
+        dt = d.dtype
+        n, rows, cols = (1,) + d.shape if d.ndim == 2 else d.shape
+        dp, tp, mem = d.ctypes.data, tex.ctypes.data, MEM_HOST
+        shape = (nv, n, rows, cols, 3)
+        if dst is None or dst.shape != shape or dst.dtype != np.uint8 or not dst.flags.c_contiguous:
+            dst = np.empty(shape, np.uint8)
+        out = dst.ctypes.data
+    if dt not in _DEPTH or _DEPTH[dt] == capi.CV_64F:
+        raise DmcError(capi.DMC_ERR_TYPE, "renderViewBatch: depth must be uint8, int16, uint16 or float32")
+    DP = C.POINTER(C.c_double)
+    ctx.check(lib.dmc_render_view_batch(ctx.h, C.c_void_p(dp), _DEPTH[dt], C.c_void_p(tp), mem, n, rows, cols, float(f), Rs.ctypes.data_as(DP),
+                                        ts.ctypes.data_as(DP), nv, Ks.ctypes.data_as(DP), int(bool(isSub)),
+                                        capi.RENDER_EXACT_DIVIDE if exact_divide else 0, C.c_void_p(out)))
+    return dst
+
+
 def minmaxBoundaryReconstructionFilter(src, dest, r, ksize, frec, color, space, ctx=None):
     """Extension (filter_ext.h): blurRemoveMinMax(r) fused into boundaryReconstructionFilter, one kernel, src read once;
     bit-identical to the two reference calls.  8U / 16U / 16S, single channel."""

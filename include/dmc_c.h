@@ -373,6 +373,31 @@ int dmc_jpeg_view_rd_sweep_ex(dmc_ctx* ctx, const void* disp, const void* textur
                               const double* R, const double* t, int n_views, const double* K, int is_sub, int render_flags,
                               uint64_t* bytes, uint64_t* sse_view_coded, uint64_t* sse_view_filtered, uint64_t* sse_view_brf);
 
+/* ---- pointcloudTest's frame loop on batches: preparation and views ------------------------------------------------ */
+/* Preparation of sensor depth (main.cpp:254-260, :511-512) on n_frames dense 16UC1 frames (depth16) into n_frames dense 8UC1
+ * frames (disp8), both in `mem`:
+ *   passes = 1: disp8_i = fillOcclusion(depth16U2disp8U(depth16_i, focal_baseline, a, b), 0, FILL_DISPARITY)  (simpleTest);
+ *   passes = 2: that, then transpose, fillOcclusion(0, FILL_DISPARITY) and transpose back                       (pointcloudTest).
+ * Every frame equals, bit for bit, that sequence of single-image calls on the frame alone: the converter's SIMD body and
+ * scalar tail split per frame, and no frame reads its neighbour.  Device memory: groups of frames (~256 MB, DMC_GROUP_MB)
+ * in stream order (dmc_synchronize before reading disp8).  Host memory: chunks stream through the device as in
+ * dmc_chain_batch; returns when disp8 is valid.  DMC_ERR_ARG: passes not 1 or 2, depth16 and disp8 overlapping, a bad mem;
+ * DMC_ERR_SIZE: cols < 2, rows < 2 with passes = 2, a negative count or size, a NULL buffer; nothing is written on error. */
+int dmc_prepare_disp_batch(dmc_ctx* ctx, const void* depth16, void* disp8, int n_frames, int rows, int cols, float focal_baseline,
+                           float a, float b, int passes, int mem);
+/* Views of frame batches (main.cpp:321-355): for every frame i of depth (n_frames dense rows x cols frames of depth_type
+ * DMC_8U, DMC_16S, DMC_16U or DMC_32F, the depths reprojectXYZ takes; dmc_chain_batch's DMC_CHAIN_DEPTH32F output as it is)
+ * with its texture i (dense 8UC3) and every camera v (R + 9v, t + 3v: row-major doubles; K shared),
+ *   views[v*n_frames + i] = fillSmallHole(projectImagefromXYZ(texture_i, reprojectXYZ(depth_i, f), R_v, t_v, K, is_sub)),
+ * the fill in place as at main.cpp:355; each view is a dense rows x cols 8UC3 image.  This is the view of
+ * dmc_jpeg_view_rd_sweep, through the same render.  depth, texture and views are all in `mem`.  render_flags:
+ * DMC_RENDER_EXACT_DIVIDE or 0.  Frames run in groups sized like the sweep's.  Device memory: in stream order; host
+ * memory: returns when views is valid.  DMC_ERR_ARG (nothing written): n_views < 1, a NULL camera, unknown render_flags,
+ * views overlapping depth or texture, another depth_type, a bad mem; DMC_ERR_SIZE: rows * cols >= 2^29, a negative count
+ * or size, a NULL buffer. */
+int dmc_render_view_batch(dmc_ctx* ctx, const void* depth, int depth_type, const void* texture, int mem, int n_frames, int rows, int cols,
+                          double f, const double* R, const double* t, int n_views, const double* K, int is_sub, int render_flags, void* views);
+
 #ifdef __cplusplus
 }
 #endif

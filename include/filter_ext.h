@@ -3,6 +3,7 @@
 #pragma once
 #include "filter.h"
 #include "util.h"
+#include <cstring>
 
 // Joint ("colour-guided") binary-weighted range filter: `src` (CV_8UC1 depth / disparity) is averaged over the window
 // of binalyWeightedRangeFilter with the binary weights computed on `guide` (CV_8UC3: the saturated L1 colour distance of
@@ -195,6 +196,78 @@ inline void jpegViewRateDistortionGray(const Mat& disp, const Mat& texture, cons
 			psnr_coded[q][v] = dmc_psnr_from_sse(sc[q * nv + v], pixels);
 			psnr_filtered[q][v] = dmc_psnr_from_sse(sf[q * nv + v], pixels);
 			psnr_brf[q][v] = dmc_psnr_from_sse(sb[q * nv + v], pixels);
+		}
+	}
+}
+
+namespace dmc_dropin {
+inline void require(bool ok, const char* what) {
+	if (ok) return;
+#ifdef DMC_MINICV_HPP
+	throw cv::Exception(what, __FILE__, __LINE__);
+#else
+	CV_Error(cv::Error::StsAssert, what);
+#endif
+}
+// frames of one size and type, packed back to back (row by row: any row step)
+inline vector<uchar> pack(const vector<Mat>& frames, int type, const char* what) {
+	const Mat& f0 = frames[0];
+	const size_t row = (size_t)f0.cols * f0.elemSize();
+	vector<uchar> out(row * f0.rows * frames.size());
+	for (size_t i = 0; i < frames.size(); i++) {
+		require(frames[i].type() == type && frames[i].rows == f0.rows && frames[i].cols == f0.cols, what);
+		for (int y = 0; y < f0.rows; y++) memcpy(&out[(i * f0.rows + y) * row], frames[i].ptr(y), row);
+	}
+	return out;
+}
+}  // namespace dmc_dropin
+
+// pointcloudTest's preparation of sensor depth (main.cpp:254-260) on a batch: disp8[i] = fillOcclusion(depth16U2disp8U(
+// depth16[i], focal_baseline, a, b), 0, FILL_DISPARITY), and with passes = 2 that filled again around a transpose (passes = 1
+// is simpleTest's call, main.cpp:511-512).  depth16: CV_16UC1 frames of one size.  Bit-identical to those calls frame by frame.
+inline void prepareDisparityBatch(const vector<Mat>& depth16, vector<Mat>& disp8, float focal_baseline, float a = 1.f, float b = 0.f, int passes = 2)
+{
+	disp8.clear();
+	if (depth16.empty()) return;
+	const int n = (int)depth16.size(), rows = depth16[0].rows, cols = depth16[0].cols;
+	const vector<uchar> src = dmc_dropin::pack(depth16, CV_16UC1, "prepareDisparityBatch: depth16 must be CV_16UC1 frames of one size");
+	vector<uchar> dst((size_t)n * rows * cols);
+	dmc_dropin::check(dmc_prepare_disp_batch(dmc_dropin::context(), src.data(), dst.data(), n, rows, cols, focal_baseline, a, b, passes, DMC_MEM_HOST),
+	                  "prepareDisparityBatch");
+	disp8.resize(n);
+	for (int i = 0; i < n; i++) {
+		disp8[i].create(rows, cols, CV_8UC1);
+		memcpy(disp8[i].data, &dst[(size_t)i * rows * cols], (size_t)rows * cols);
+	}
+}
+
+// pointcloudTest's views (main.cpp:321-355) of a batch: views[v][i] = fillSmallHole(projectImagefromXYZ(texture[i],
+// reprojectXYZ(depth[i], f), R[v], t[v], K, isSub)), the fill in place.  depth: frames of one size and one of the types
+// reprojectXYZ takes (CV_8U, CV_16S, CV_16U, CV_32F: filterDisp8U2Depth32F's output as it is); texture: CV_8UC3 of that size.
+inline void renderViewBatch(const vector<Mat>& depth, const vector<Mat>& texture, double f, const vector<Mat>& R, const vector<Mat>& t, const Mat& K,
+                            bool isSub, vector<vector<Mat> >& views)
+{
+	views.clear();
+	dmc_dropin::require(!R.empty() && R.size() == t.size(), "renderViewBatch: R and t must hold one camera each");
+	dmc_dropin::require(depth.size() == texture.size(), "renderViewBatch: one texture per depth frame");
+	const size_t nv = R.size();
+	vector<double> r(9 * nv), tt(3 * nv), k(9);
+	for (size_t v = 0; v < nv; v++) dmc_dropin::camera(R[v], t[v], K, &r[9 * v], &tt[3 * v], &k[0], "renderViewBatch");
+	views.assign(nv, vector<Mat>());
+	if (depth.empty()) return;
+	const int n = (int)depth.size(), rows = depth[0].rows, cols = depth[0].cols, type = depth[0].type();
+	const vector<uchar> d = dmc_dropin::pack(depth, type, "renderViewBatch: depth frames must share one size and type");
+	const vector<uchar> tex = dmc_dropin::pack(texture, CV_8UC3, "renderViewBatch: texture must be CV_8UC3 frames of the depth's size");
+	dmc_dropin::require(texture[0].rows == rows && texture[0].cols == cols, "renderViewBatch: texture must be CV_8UC3 frames of the depth's size");
+	const size_t vb = (size_t)rows * cols * 3;
+	vector<uchar> out(vb * n * nv);
+	dmc_dropin::check(dmc_render_view_batch(dmc_dropin::context(), d.data(), type, tex.data(), DMC_MEM_HOST, n, rows, cols, f, &r[0], &tt[0], (int)nv, &k[0],
+	                                        isSub ? 1 : 0, 0, out.data()), "renderViewBatch");
+	for (size_t v = 0; v < nv; v++) {
+		views[v].resize(n);
+		for (int i = 0; i < n; i++) {
+			views[v][i].create(rows, cols, CV_8UC3);
+			memcpy(views[v][i].data, &out[(v * n + i) * vb], vb);
 		}
 	}
 }
