@@ -1669,10 +1669,10 @@ void camera_floats(const double* R, const double* t, const double* K, float kr[9
 // projectImagefromXYZ's splat of `frames` frames (pt already projected) into dest (and depth, if not NULL).
 int render(dmc_ctx* ctx, const uint8_t* image, const float* xyz, const float* pt, int frames, int rows, int cols, int is_sub, uint8_t* dest, float* depth) {
     TRY(reserve(ctx, ctx->render[0], render_scratch_bytes(frames, rows, cols)));
-    TRY(reserve(ctx, ctx->render[1], 64));
+    TRY(reserve(ctx, ctx->render[1], sizeof(int) * (1 + (size_t)frames)));        // the sweeps' change flags: any, then per frame
     if (!ctx->render_flag) CUDA_TRY(ctx, cudaHostAlloc((void**)&ctx->render_flag, 64, cudaHostAllocDefault));
     const int nk = launch_render(image, xyz, pt, frames, rows, cols, is_sub, dest, depth, ctx->render[0].p, (int*)ctx->render[1].p, ctx->render_flag, ctx->stream);
-    if (nk < 0) return fail(ctx, DMC_ERR_CUDA, std::string("projectImagefromXYZ: the splat did not settle: ") + cudaGetErrorString(cudaGetLastError()));
+    if (nk < 0) return fail(ctx, DMC_ERR_CUDA, std::string("projectImagefromXYZ: the splat failed: ") + cudaGetErrorString(cudaGetLastError()));
     return after_launch(ctx, nk);
 }
 }  // namespace

@@ -13,13 +13,19 @@
 //   * attempts are binned per z-tested pixel (count / exclusive scan / fill / per-pixel sort by time), then the fired bits
 //     of the primaries are iterated to their fixed point: one thread per pixel walks its time-sorted list with a running
 //     minimum.  Whether a primary fires depends only on attempts of EARLIER points, so the fixed point is unique and an
-//     iteration that changes nothing has reached it (typically 3-5 iterations).
+//     iteration that changes nothing has reached it.  Natural scenes settle in 3-5 iterations, but the count has no such
+//     bound: point k's primary can depend on point k-1's through a neighbour attempt that z-tests k's pixel, and each such
+//     link of a chain can cost an iteration (a 3 x W image can chain W/2 points).  So after max(32, n / 1024) iterations
+//     (n pixels a frame) the frames that still changed are finished by splat_serial_kernel, one thread per frame replaying
+//     the serial loop to get `fired`.  The cap is a choice: n / 1024 sweeps cost less than one serial replay of the frame
+//     (DESIGN.md section 6 has the times), and 32 alone would send some coded 1080p views, which need more, to the replay.
 //   * the colour of a pixel is that of the LATEST fired attempt that colours it (atomicMax on time), its depth the final
 //     running minimum.
 //   * a batch of F frames (one camera) is rendered at once: the kernels take the frame from the grid, a pixel's global
 //     index is frame * n + local, while times, coloured pixels and the `fired` bits stay frame-local.  Only interior points
 //     make attempts, so no attempt reaches into another frame.  One scan covers all F * n counters, and the fixed point
-//     is iterated until no frame changed (one host read per iteration for the whole batch).
+//     is iterated until no frame changed (one host read per iteration for the whole batch); the last iteration before the
+//     serial finish also reports each frame's own change, so the finish replays only the frames that have not settled.
 //
 // The projection uses the reference's reciprocal: _mm_rcp_ps (:78) is a 2048-entry look-up on Intel CPUs, carried here as
 // a table (dmc_rcp_intel.inc, verified against the instruction on all 2^32 operands by tools/gen_rcp_table.c); the last
@@ -86,17 +92,19 @@ __device__ __forceinline__ void for_each_attempt(const float2* __restrict__ pt, 
 // time = frame-local point * 8 + ordinal; c = frame-local coloured pixel.  Pixel lists hold one frame's attempts only.
 struct Attempt { uint32_t time; float z; uint32_t c; };
 
-// frame = blockIdx.z; counters, cursors and offsets are indexed by the global pixel frame * n + q
-__global__ void attempts_count_kernel(const float2* __restrict__ pt, uint32_t* __restrict__ cnt, int rows, int cols, int is_sub) {
-    const int i = blockIdx.x * blockDim.x + threadIdx.x + 1, j = blockIdx.y + 1;
+// The kernels over interior points take row j = j0 + blockIdx.y + 1 (gridDim.y is at most 65535: launch_interior splits
+// taller images into several launches) and frame = blockIdx.z.  Counters, cursors and offsets are indexed by the global
+// pixel frame * n + q.
+__global__ void attempts_count_kernel(const float2* __restrict__ pt, uint32_t* __restrict__ cnt, int rows, int cols, int is_sub, int j0) {
+    const int i = blockIdx.x * blockDim.x + threadIdx.x + 1, j = j0 + blockIdx.y + 1;
     if (i >= cols - 1 || j >= rows - 1) return;
     const long base = (long)blockIdx.z * rows * cols;
     for_each_attempt(pt + base, (long)j * cols + i, rows, cols, is_sub, [&](int, long q, long) { atomicAdd(&cnt[base + q], 1u); });
 }
 
 __global__ void attempts_fill_kernel(const float2* __restrict__ pt, const float* __restrict__ xyz, const uint32_t* __restrict__ offs, uint32_t* __restrict__ cursor,
-                                     Attempt* __restrict__ att, int rows, int cols, int is_sub) {
-    const int i = blockIdx.x * blockDim.x + threadIdx.x + 1, j = blockIdx.y + 1;
+                                     Attempt* __restrict__ att, int rows, int cols, int is_sub, int j0) {
+    const int i = blockIdx.x * blockDim.x + threadIdx.x + 1, j = j0 + blockIdx.y + 1;
     if (i >= cols - 1 || j >= rows - 1) return;
     const long base = (long)blockIdx.z * rows * cols, p = (long)j * cols + i;
     const float z = xyz[3 * (base + p) + 2];
@@ -105,6 +113,15 @@ __global__ void attempts_fill_kernel(const float2* __restrict__ pt, const float*
         Attempt a; a.time = (uint32_t)p * 8u + (uint32_t)ord; a.z = z; a.c = (uint32_t)c;
         att[slot] = a;
     });
+}
+
+// kernel<<<...>>>(args..., j0) over the interior rows of `frames` frames, at most 65535 rows a launch -> launches
+template <class Kernel, class... Args>
+int launch_interior(Kernel kernel, int frames, int rows, int cols, cudaStream_t s, Args... args) {
+    int nk = 0;
+    for (int j0 = 0; j0 < rows - 2; j0 += 65535, nk++)
+        kernel<<<dim3((cols + 255) / 256, rows - 2 - j0 < 65535 ? rows - 2 - j0 : 65535, frames), 256, 0, s>>>(args..., j0);
+    return nk;
 }
 
 // exclusive scan of n counters: per-block sums, scan of the sums by one block, add
@@ -184,10 +201,11 @@ __global__ void attempts_sort_kernel(const uint32_t* __restrict__ offs, const ui
 }
 
 // One sweep of the fixed-point iteration over every frame; FINAL: also emits colours and depth.  `changed` is shared by
-// the frames: the batch iterates until no frame changed.
+// the frames: the batch iterates until no frame changed.  frame_changed (the last sweep before the serial finish only,
+// NULL in the others) receives each frame's own flag.
 template <bool FINAL>
 __global__ void attempts_sweep_kernel(const uint32_t* __restrict__ offs, const uint32_t* __restrict__ cnt, const Attempt* __restrict__ att, uint8_t* fired,
-                                      int* __restrict__ changed, uint32_t* __restrict__ ckey, float* __restrict__ depth, long n) {
+                                      int* __restrict__ changed, int* __restrict__ frame_changed, uint32_t* __restrict__ ckey, float* __restrict__ depth, long n) {
     const long q = (long)blockIdx.x * blockDim.x + threadIdx.x;
     if (q >= n) return;
     const long base = (long)blockIdx.y * n, g = base + q;
@@ -201,9 +219,33 @@ __global__ void attempts_sweep_kernel(const uint32_t* __restrict__ offs, const u
         const bool considered = ord == 0u || fr[p] != 0;
         const bool fires = considered && cur > e.z;     // `*zbuff > z` :325 (false for NaN)
         if (fires) { cur = e.z; if (FINAL) atomicMax(&ckey[base + e.c], e.time + 1u); }
-        if (!FINAL && ord == 0u && (fr[p] != 0) != fires) { fr[p] = fires ? 1 : 0; *changed = 1; }
+        if (!FINAL && ord == 0u && (fr[p] != 0) != fires) { fr[p] = fires ? 1 : 0; *changed = 1; if (frame_changed) frame_changed[blockIdx.y] = 1; }
     }
     if (FINAL && depth) depth[g] = cur;
+}
+
+// The serial splat (ref:depthmapUtil.cpp:320-445) of the frames whose last sweep still changed, one thread per frame: a
+// point's primary fires iff it is below the z-buffer at that moment, and only then do its neighbour attempts write.  Only
+// `fired` is kept: the FINAL sweep then emits colours and depth from it as after a settled iteration.  zbuf: n floats a
+// frame.
+__global__ void splat_serial_kernel(const float2* __restrict__ pt, const float* __restrict__ xyz, const int* __restrict__ frame_changed,
+                                    uint8_t* __restrict__ fired, float* __restrict__ zbuf, int frames, int rows, int cols, int is_sub) {
+    const int f = blockIdx.x * blockDim.x + threadIdx.x;
+    if (f >= frames || !frame_changed[f]) return;
+    const long n = (long)rows * cols, base = (long)f * n;
+    float* zb = zbuf + base;
+    uint8_t* fr = fired + base;
+    for (long q = 0; q < n; q++) zb[q] = 10000.f;
+    for (int j = 1; j < rows - 1; j++)
+        for (int i = 1; i < cols - 1; i++) {
+            const long p = (long)j * cols + i;
+            const float z = xyz[3 * (base + p) + 2];
+            bool won = false;
+            for_each_attempt(pt + base, p, rows, cols, is_sub, [&](int ord, long q, long) {
+                if (ord == 0) { won = zb[q] > z; fr[p] = won ? 1 : 0; if (won) zb[q] = z; }
+                else if (won && zb[q] > z) zb[q] = z;
+            });
+        }
 }
 
 __global__ void render_resolve_kernel(const uint8_t* __restrict__ image, const uint32_t* __restrict__ ckey, uint8_t* __restrict__ dest, long n) {
@@ -217,9 +259,10 @@ __global__ void render_resolve_kernel(const uint8_t* __restrict__ image, const u
 }
 
 // fillSmallHole :187-283: a pixel whose GREEN is 0 becomes the mean of the neighbours whose BLUE is not 0 (s[lstep+1-1]);
-// cvRound of a double quotient; border pixels and non-holes keep dst's previous content.  Frame = blockIdx.z.
-__global__ void fill_small_hole_kernel(const uint8_t* __restrict__ src, uint8_t* __restrict__ dst, int rows, int cols) {
-    const int i = blockIdx.x * blockDim.x + threadIdx.x + 1, j = blockIdx.y + 1;
+// cvRound of a double quotient; border pixels and non-holes keep dst's previous content.  Row j0 + blockIdx.y + 1, frame =
+// blockIdx.z.
+__global__ void fill_small_hole_kernel(const uint8_t* __restrict__ src, uint8_t* __restrict__ dst, int rows, int cols, int j0) {
+    const int i = blockIdx.x * blockDim.x + threadIdx.x + 1, j = j0 + blockIdx.y + 1;
     if (i >= cols - 1 || j >= rows - 1) return;
     const long step = (long)cols * 3, frame = (long)blockIdx.z * rows * step;
     const uint8_t* s = src + frame + j * step + 3 * i;
@@ -271,8 +314,11 @@ size_t render_scratch_bytes(int frames, int rows, int cols) {
 
 // Everything after the projection, up to the fixed point, for `frames` frames of rows x cols at once (one scan over all
 // their counters: the caller keeps frames * rows * cols * 7 below 2^32).  `changed_host` is pinned memory the sweeps report
-// through: one read per iteration for the whole batch.  Returns the number of kernels launched, or -1 if the iteration did
-// not settle (cannot happen: see the header).
+// through: one read per iteration for the whole batch; changed_dev holds 1 + frames ints (the shared flag, then the
+// frames' own).  After render_sweep_cap(rows * cols) iterations the frames that still changed are finished by the serial
+// splat (see the header), so the work is bounded whatever the input.  Returns the number of kernels launched, or -1 on a
+// CUDA error.
+int render_sweep_cap(long n) { return n / 1024 > 32 ? (int)(n / 1024) : 32; }
 int launch_render(const uint8_t* image, const float* xyz, const float* pt, int frames, int rows, int cols, int is_sub, uint8_t* dest, float* depth,
                   void* scratch, int* changed_dev, int* changed_host, cudaStream_t s) {
     const long n = (long)rows * cols, nt = n * frames;
@@ -283,37 +329,39 @@ int launch_render(const uint8_t* image, const float* xyz, const float* pt, int f
     uint8_t* fired = (uint8_t*)(att + (size_t)nt * 7);
     int nk = 0;
     cudaMemsetAsync(cnt, 0, (size_t)nt * 4, s); cudaMemsetAsync(cursor, 0, (size_t)nt * 4, s); cudaMemsetAsync(fired, 1, (size_t)nt, s);
-    dim3 grid((cols + 255) / 256, rows > 2 ? rows - 2 : 1, frames);
-    if (rows > 2 && cols > 2) { attempts_count_kernel<<<grid, 256, 0, s>>>((const float2*)pt, cnt, rows, cols, is_sub); nk++; }
+    if (cols > 2) nk += launch_interior(attempts_count_kernel, frames, rows, cols, s, (const float2*)pt, cnt, rows, cols, is_sub);
     scan_blocks_kernel<<<nb, kScanT, 0, s>>>(cnt, offs, sums, nt);
     scan_sums_kernel<<<1, 1024, 0, s>>>(sums, nb);
     scan_add_kernel<<<nb, kScanT, 0, s>>>(offs, sums, nt);
     nk += 3;
-    if (rows > 2 && cols > 2) { attempts_fill_kernel<<<grid, 256, 0, s>>>((const float2*)pt, xyz, offs, cursor, att, rows, cols, is_sub); nk++; }
+    if (cols > 2) nk += launch_interior(attempts_fill_kernel, frames, rows, cols, s, (const float2*)pt, xyz, offs, cursor, att, rows, cols, is_sub);
     const dim3 gq((unsigned)((n + 255) / 256), frames);
     attempts_sort_kernel<<<gq, 256, 0, s>>>(offs, cnt, att, n); nk++;
     if (is_sub) {
+        const int cap = render_sweep_cap(n);
         for (int it = 0;; it++) {
-            if (it > 100000) return -1;
-            cudaMemsetAsync(changed_dev, 0, sizeof(int), s);
-            attempts_sweep_kernel<false><<<gq, 256, 0, s>>>(offs, cnt, att, fired, changed_dev, nullptr, nullptr, n); nk++;
+            if (it == cap) {                        // not settled: the serial splat finishes the frames that still changed
+                splat_serial_kernel<<<(frames + 31) / 32, 32, 0, s>>>((const float2*)pt, xyz, changed_dev + 1, fired, (float*)cursor, frames, rows, cols, is_sub); nk++;
+                break;
+            }
+            int* frame_changed = it == cap - 1 ? changed_dev + 1 : nullptr;
+            cudaMemsetAsync(changed_dev, 0, sizeof(int) * (frame_changed ? 1 + (size_t)frames : 1), s);
+            attempts_sweep_kernel<false><<<gq, 256, 0, s>>>(offs, cnt, att, fired, changed_dev, frame_changed, nullptr, nullptr, n); nk++;
             cudaMemcpyAsync(changed_host, changed_dev, sizeof(int), cudaMemcpyDeviceToHost, s);
             if (cudaStreamSynchronize(s) != cudaSuccess) return -1;
             if (!*changed_host) break;
         }
     }
-    uint32_t* ckey = cursor;                            // the fill cursors are no longer needed
+    uint32_t* ckey = cursor;                            // the fill cursors (and the serial splat's z-buffer) are no longer needed
     cudaMemsetAsync(ckey, 0, (size_t)nt * 4, s);
-    attempts_sweep_kernel<true><<<gq, 256, 0, s>>>(offs, cnt, att, fired, nullptr, ckey, depth, n);
+    attempts_sweep_kernel<true><<<gq, 256, 0, s>>>(offs, cnt, att, fired, nullptr, nullptr, ckey, depth, n);
     render_resolve_kernel<<<gq, 256, 0, s>>>(image, ckey, dest, n);
     return nk + 2;
 }
 
 int launch_fill_small_hole(const uint8_t* src, uint8_t* dst, int frames, int rows, int cols, cudaStream_t s) {
     if (rows <= 2 || cols <= 2 || frames <= 0) return 0;
-    dim3 grid((cols + 255) / 256, rows - 2, frames);
-    fill_small_hole_kernel<<<grid, 256, 0, s>>>(src, dst, rows, cols);
-    return 1;
+    return launch_interior(fill_small_hole_kernel, frames, rows, cols, s, src, dst, rows, cols);
 }
 
 }  // namespace dmc
