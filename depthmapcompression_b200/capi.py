@@ -34,6 +34,7 @@ EXPORTS = [
     "dmc_sse_gray_batch", "dmc_psnr_from_sse", "dmc_jpeg_rd_sweep", "dmc_jpeg_view_rd_sweep",
     "dmc_brf_batch", "dmc_jpeg_rd_sweep_ex", "dmc_jpeg_view_rd_sweep_ex",
     "dmc_prepare_disp_batch", "dmc_render_view_batch",
+    "dmc_ssim_batch", "dmc_jpeg_rd_sweep_ssim", "dmc_jpeg_view_rd_sweep_ssim",
 ]
 MAX_DEVICES = 16
 RENDER_EXACT_DIVIDE = 1
@@ -106,6 +107,13 @@ def _load():
         "dmc_jpeg_view_rd_sweep_ex": (I, [P, P, P, I, I, I, I, C.POINTER(I), I, I, C.POINTER(DmcChainParams), C.POINTER(DmcBrfParams), D, C.POINTER(D),
                                           C.POINTER(D), I, C.POINTER(D), I, I, C.POINTER(C.c_uint64), C.POINTER(C.c_uint64), C.POINTER(C.c_uint64),
                                           C.POINTER(C.c_uint64)]),
+        "dmc_ssim_batch": (I, [P, P, P, I, I, I, I, I, C.POINTER(D)]),
+        "dmc_jpeg_rd_sweep_ssim": (I, [P, P, I, I, I, I, C.POINTER(I), I, I, C.POINTER(DmcChainParams), C.POINTER(DmcBrfParams),
+                                       C.POINTER(C.c_uint64), C.POINTER(C.c_uint64), C.POINTER(C.c_uint64), C.POINTER(C.c_uint64),
+                                       C.POINTER(D), C.POINTER(D), C.POINTER(D)]),
+        "dmc_jpeg_view_rd_sweep_ssim": (I, [P, P, P, I, I, I, I, C.POINTER(I), I, I, C.POINTER(DmcChainParams), C.POINTER(DmcBrfParams), D, C.POINTER(D),
+                                            C.POINTER(D), I, C.POINTER(D), I, I, C.POINTER(C.c_uint64), C.POINTER(C.c_uint64), C.POINTER(C.c_uint64),
+                                            C.POINTER(C.c_uint64), C.POINTER(D), C.POINTER(D), C.POINTER(D)]),
         "dmc_sched_create": (I, [C.POINTER(I), I, C.POINTER(P)]), "dmc_sched_destroy": (None, [P]), "dmc_sched_device_count": (I, [P]),
         "dmc_sched_last_error": (C.c_char_p, [P]), "dmc_sched_chain_batch": (I, [P, P, P, I, I, I, C.POINTER(DmcChainParams)]),
         "dmc_multi_chain_batch": (I, [C.POINTER(I), I, P, P, I, I, I, C.POINTER(DmcChainParams), C.c_char_p, C.c_size_t]),

@@ -29,7 +29,8 @@ enum { JD_BITS, JD_META, JD_SCANS, JD_COEF, JD_OUT, JD_COUNT };
 // Device buffers of dmc_sse_gray_batch and dmc_jpeg_rd_sweep: every quality's encoder + decoder tables, the decoder's
 // FrameDescs of a group, its staged source, coded and filtered frames (the staged second batch of dmc_sse_gray_batch; the
 // BRF arm's frames in both sweeps), and the group's results (SSE, stream lengths) that one copy brings back.
-enum { RD_TABS, RD_DESC, RD_SRC, RD_CODED, RD_FILT, RD_RES, RD_COUNT };
+// RD_SSIM: the per-tile sums of the SSIM launches (dmc_ssim_batch and the sweeps' SSIM outputs).
+enum { RD_TABS, RD_DESC, RD_SRC, RD_CODED, RD_FILT, RD_RES, RD_SSIM, RD_COUNT };
 // Device buffers of dmc_jpeg_view_rd_sweep: the group's staged textures, a depth frame, the points of the coded and of the
 // filtered depth (xyz), their projections, a raw render, the coded and filtered views, and the reference views.
 enum { VS_TEX, VS_DEPTH, VS_XYZ, VS_PT, VS_RAW, VS_VIEW, VS_REF, VS_COUNT };
@@ -1177,6 +1178,44 @@ int dmc_sse_gray_batch(dmc_ctx* ctx, const void* a, const void* b, int n_frames,
     return DMC_OK;
 }
 
+// Groups of ~256 MB of frames (host frames are copied in first, once when a and b are the same pointer); the per-tile sums
+// of a group go to RD_SSIM, every frame's MSSIM to RD_RES, and one copy at the end brings them back.
+int dmc_ssim_batch(dmc_ctx* ctx, const void* a, const void* b, int n_frames, int rows, int cols, int channels, int mem, double* mssim) {
+    if (!ctx) return fail(nullptr, DMC_ERR_ARG, "null context");
+    if (mem != DMC_MEM_HOST && mem != DMC_MEM_DEVICE) return fail(ctx, DMC_ERR_ARG, "dmc_ssim_batch: bad mem");
+    if (channels != 1 && channels != 3) return fail(ctx, DMC_ERR_ARG, "dmc_ssim_batch: channels must be 1 or 3");
+    if (rows < 11 || cols < 11) return fail(ctx, DMC_ERR_SIZE, "dmc_ssim_batch: frames must be at least 11 x 11 (the SSIM window)");
+    if (n_frames < 0 || (n_frames > 0 && (!a || !b || !mssim))) return fail(ctx, DMC_ERR_SIZE, "dmc_ssim_batch: bad arguments");
+    if (n_frames == 0) return DMC_OK;
+    CUDA_TRY(ctx, cudaSetDevice(ctx->device));
+    cudaStream_t s = ctx->stream;
+    const bool host = mem == DMC_MEM_HOST;
+    const size_t fb = (size_t)rows * cols * channels;
+    const int group = chunk_frames((size_t)256 << 20, fb, n_frames, INT_MAX, false);
+    TRY(reserve(ctx, ctx->rd[RD_SSIM], ssim_partial_bytes(rows, cols, channels) * group));
+    TRY(reserve(ctx, ctx->rd[RD_RES], (size_t)n_frames * sizeof(double)));
+    if (host) {
+        TRY(reserve(ctx, ctx->rd[RD_SRC], fb * group));
+        if (b != a) TRY(reserve(ctx, ctx->rd[RD_CODED], fb * group));
+    }
+    double* dres = (double*)ctx->rd[RD_RES].p;
+    for (int f0 = 0; f0 < n_frames; f0 += group) {
+        const int nf = n_frames - f0 < group ? n_frames - f0 : group;
+        const uint8_t* da = (const uint8_t*)a + fb * f0;
+        const uint8_t* db = (const uint8_t*)b + fb * f0;
+        if (host) {
+            CUDA_TRY(ctx, cudaMemcpyAsync(ctx->rd[RD_SRC].p, da, fb * nf, cudaMemcpyHostToDevice, s));
+            if (b != a) CUDA_TRY(ctx, cudaMemcpyAsync(ctx->rd[RD_CODED].p, db, fb * nf, cudaMemcpyHostToDevice, s));
+            da = (const uint8_t*)ctx->rd[RD_SRC].p;
+            db = b != a ? (const uint8_t*)ctx->rd[RD_CODED].p : da;
+        }
+        LAUNCH(ctx, launch_ssim_u8(da, db, (double*)ctx->rd[RD_SSIM].p, dres + f0, nf, rows, cols, channels, s));
+    }
+    CUDA_TRY(ctx, cudaMemcpyAsync(mssim, dres, (size_t)n_frames * sizeof(double), cudaMemcpyDeviceToHost, s));
+    CUDA_TRY(ctx, cudaStreamSynchronize(s));
+    return DMC_OK;
+}
+
 namespace {
 
 // The sweeps' per-quality tables in RD_TABS, kRdRec bytes a quality: [EncTables][DC, AC HuffTable][QuantTable].
@@ -1229,6 +1268,12 @@ int brf_frames(dmc_ctx* ctx, const uint8_t* src, uint8_t* dst, int nf, int rows,
     return after_launch(ctx, nk);
 }
 
+// MSSIM of nf pairs of dense 8-bit frames (the sweeps' SSIM outputs) into out (device), per-tile sums in RD_SSIM.
+int ssim_frames(dmc_ctx* ctx, const uint8_t* a, const uint8_t* b, int nf, int rows, int cols, int channels, double* out) {
+    LAUNCH(ctx, launch_ssim_u8(a, b, (double*)ctx->rd[RD_SSIM].p, out, nf, rows, cols, channels, ctx->stream));
+    return DMC_OK;
+}
+
 }  // namespace
 
 // The sweep runs group by group (a group is sized like the encoder's, counting the coded and filtered frames and the
@@ -1238,7 +1283,8 @@ int brf_frames(dmc_ctx* ctx, const uint8_t* src, uint8_t* dst, int nf, int rows,
 // frames, the chain into the filtered frames, one SSE launch (source vs coded and vs filtered) and a device-side copy of
 // the stream lengths; one copy and one synchronisation per group bring the results back.  The BRF arm (b != NULL) adds, per
 // (group, quality), one batched BRF launch on the coded frames and one SSE launch; its output reuses the filtered frames'
-// buffer once their SSE is queued.
+// buffer once their SSE is queued.  The SSIM outputs (ssim_coded != NULL) add per (group, quality) one SSIM launch pair per
+// arm, queued next to the arm's SSE launch on the same frames; their results ride in the group's one copy.
 int dmc_jpeg_rd_sweep(dmc_ctx* ctx, const void* src, int src_mem, int n_frames, int rows, int cols, const int* qualities, int n_q,
                       int flags, const dmc_chain_params* p, uint64_t* bytes, uint64_t* sse_coded, uint64_t* sse_filtered) {
     return dmc_jpeg_rd_sweep_ex(ctx, src, src_mem, n_frames, rows, cols, qualities, n_q, flags, p, nullptr, bytes, sse_coded, sse_filtered, nullptr);
@@ -1247,6 +1293,13 @@ int dmc_jpeg_rd_sweep(dmc_ctx* ctx, const void* src, int src_mem, int n_frames, 
 int dmc_jpeg_rd_sweep_ex(dmc_ctx* ctx, const void* src, int src_mem, int n_frames, int rows, int cols, const int* qualities, int n_q,
                          int flags, const dmc_chain_params* p, const dmc_brf_params* b, uint64_t* bytes, uint64_t* sse_coded,
                          uint64_t* sse_filtered, uint64_t* sse_brf) {
+    return dmc_jpeg_rd_sweep_ssim(ctx, src, src_mem, n_frames, rows, cols, qualities, n_q, flags, p, b, bytes, sse_coded, sse_filtered, sse_brf,
+                                  nullptr, nullptr, nullptr);
+}
+
+int dmc_jpeg_rd_sweep_ssim(dmc_ctx* ctx, const void* src, int src_mem, int n_frames, int rows, int cols, const int* qualities, int n_q,
+                           int flags, const dmc_chain_params* p, const dmc_brf_params* b, uint64_t* bytes, uint64_t* sse_coded,
+                           uint64_t* sse_filtered, uint64_t* sse_brf, double* ssim_coded, double* ssim_filtered, double* ssim_brf) {
     if (!ctx) return fail(nullptr, DMC_ERR_ARG, "null context");
     if (!qualities || n_q < 1) return fail(ctx, DMC_ERR_ARG, "dmc_jpeg_rd_sweep: no qualities");
     for (int k = 0; k < n_q; k++)
@@ -1262,7 +1315,10 @@ int dmc_jpeg_rd_sweep_ex(dmc_ctx* ctx, const void* src, int src_mem, int n_frame
     if (src_mem != DMC_MEM_HOST && src_mem != DMC_MEM_DEVICE) return fail(ctx, DMC_ERR_ARG, "dmc_jpeg_rd_sweep: bad mem");
     uint64_t bound;
     if (dmc_jpeg_encode_bound_ex(rows, cols, flags, &bound) != DMC_OK) return fail(ctx, DMC_ERR_SIZE, "dmc_jpeg_rd_sweep: " + g_err);
-    if (n_frames < 0 || (n_frames > 0 && (!src || !bytes || !sse_coded || (p && !sse_filtered) || (b && !sse_brf)))) return fail(ctx, DMC_ERR_SIZE, "dmc_jpeg_rd_sweep: bad arguments");
+    const bool ssim = ssim_coded != nullptr;
+    if (ssim && (rows < 11 || cols < 11)) return fail(ctx, DMC_ERR_SIZE, "dmc_jpeg_rd_sweep: SSIM needs frames of at least 11 x 11 (the window)");
+    if (n_frames < 0 || (n_frames > 0 && (!src || !bytes || !sse_coded || (p && !sse_filtered) || (b && !sse_brf) || (ssim && ((p && !ssim_filtered) || (b && !ssim_brf))))))
+        return fail(ctx, DMC_ERR_SIZE, "dmc_jpeg_rd_sweep: bad arguments");
     if (n_frames == 0) return DMC_OK;
     CUDA_TRY(ctx, cudaSetDevice(ctx->device));
     cudaStream_t s = ctx->stream;
@@ -1270,7 +1326,8 @@ int dmc_jpeg_rd_sweep_ex(dmc_ctx* ctx, const void* src, int src_mem, int n_frame
     const size_t fpx = (size_t)rows * cols;
     const JpegEncLayout l = jpeg_enc_layout(rows, cols, optimize);
     const size_t per = l.coef_bytes + l.info_bytes + l.word_bytes + l.slot_bytes + (optimize ? l.opt_bytes + 2 * sizeof(dmcjpeg::HuffTable) : 0) +
-                       sizeof(dmcjpeg::FrameDesc) + fpx * ((host ? 1 : 0) + 1 + (p ? 3 : b ? 1 : 0));   // staged source, coded, filtered (or BRF), ping, pong
+                       sizeof(dmcjpeg::FrameDesc) + fpx * ((host ? 1 : 0) + 1 + (p ? 3 : b ? 1 : 0)) +   // staged source, coded, filtered (or BRF), ping, pong
+                       (ssim ? ssim_partial_bytes(rows, cols, 1) : 0);
     const int group = chunk_frames(kEncGroupBytes, per, n_frames, 2048, false);
     std::vector<char> tabs;
     TRY(rd_tables(ctx, "dmc_jpeg_rd_sweep", rows, cols, qualities, n_q, tabs));
@@ -1278,9 +1335,12 @@ int dmc_jpeg_rd_sweep_ex(dmc_ctx* ctx, const void* src, int src_mem, int n_frame
     TRY(reserve(ctx, ctx->rd[RD_CODED], fpx * group));
     if (p || b) TRY(reserve(ctx, ctx->rd[RD_FILT], fpx * group));
     if (host) TRY(reserve(ctx, ctx->rd[RD_SRC], fpx * group));
-    // results of a group of nf frames: [sse_coded][sse_filtered][sse_brf if b] (uint64, [quality][frame]), then the lengths (uint32)
-    const int nsse = b ? 3 : 2;
-    const size_t res_bytes = (size_t)n_q * group * (nsse * sizeof(uint64_t) + sizeof(uint32_t));
+    if (ssim) TRY(reserve(ctx, ctx->rd[RD_SSIM], ssim_partial_bytes(rows, cols, 1) * group));
+    // results of a group of nf frames: [sse_coded][sse_filtered][sse_brf if b] (uint64, [quality][frame]), with SSIM
+    // [ssim_coded][ssim_filtered][ssim_brf if b] (double, [quality][frame]), then the lengths (uint32)
+    const int nsse = b ? 3 : 2, nssim = ssim ? nsse : 0;
+    const size_t per_q = (nsse + nssim) * sizeof(uint64_t) + sizeof(uint32_t);
+    const size_t res_bytes = (size_t)n_q * group * per_q;
     TRY(reserve(ctx, ctx->rd[RD_RES], res_bytes));
     Slot& sl = ctx->slot[0]; sl.stream = s;
     uint8_t* coded = (uint8_t*)ctx->rd[RD_CODED].p;
@@ -1296,31 +1356,47 @@ int dmc_jpeg_rd_sweep_ex(dmc_ctx* ctx, const void* src, int src_mem, int n_frame
         uint64_t* d_sc = (uint64_t*)ctx->rd[RD_RES].p;
         uint64_t* d_sf = d_sc + (size_t)n_q * nf;
         uint64_t* d_sb = d_sf + (size_t)n_q * nf;
-        uint32_t* d_len = (uint32_t*)(d_sc + (size_t)nsse * n_q * nf);
+        double* d_qc = (double*)(d_sc + (size_t)nsse * n_q * nf);
+        double* d_qf = d_qc + (size_t)n_q * nf;
+        double* d_qb = d_qf + (size_t)n_q * nf;
+        uint32_t* d_len = (uint32_t*)(d_sc + (size_t)(nsse + nssim) * n_q * nf);
         for (int k = 0; k < n_q; k++) {
             TRY(rd_degrade(ctx, k, dsrc, nf, rows, cols, optimize, coded));
             if (p) TRY(run_chain(ctx, sl, coded, filt, nf, rows, cols, *p));
             LAUNCH(ctx, launch_sse_u8(dsrc, coded, p ? filt : nullptr, d_sc + (size_t)k * nf, p ? d_sf + (size_t)k * nf : nullptr, nf, fpx, s));
-            if (b) {                                                // (stream order: the SSE above has read `filt`)
+            if (ssim) {
+                TRY(ssim_frames(ctx, dsrc, coded, nf, rows, cols, 1, d_qc + (size_t)k * nf));
+                if (p) TRY(ssim_frames(ctx, dsrc, filt, nf, rows, cols, 1, d_qf + (size_t)k * nf));
+            }
+            if (b) {                                                // (stream order: the SSE and SSIM above have read `filt`)
                 TRY(brf_frames(ctx, coded, filt, nf, rows, cols, *b));
                 LAUNCH(ctx, launch_sse_u8(dsrc, filt, nullptr, d_sb + (size_t)k * nf, nullptr, nf, fpx, s));
+                if (ssim) TRY(ssim_frames(ctx, dsrc, filt, nf, rows, cols, 1, d_qb + (size_t)k * nf));
             }
             CUDA_TRY(ctx, cudaMemcpyAsync(d_len + (size_t)k * nf, ctx->jpeg_enc[JE_LENS].p, nf * sizeof(uint32_t), cudaMemcpyDeviceToDevice, s));
         }
-        const size_t used = (size_t)n_q * nf * (nsse * sizeof(uint64_t) + sizeof(uint32_t));
+        const size_t used = (size_t)n_q * nf * per_q;
         res.resize(used);
         CUDA_TRY(ctx, cudaMemcpyAsync(res.data(), ctx->rd[RD_RES].p, used, cudaMemcpyDeviceToHost, s));
         CUDA_TRY(ctx, cudaStreamSynchronize(s));
         const uint64_t* sc = (const uint64_t*)res.data();
         const uint64_t* sf = sc + (size_t)n_q * nf;
         const uint64_t* sb = sf + (size_t)n_q * nf;
-        const uint32_t* len = (const uint32_t*)(sc + (size_t)nsse * n_q * nf);
+        const double* qc = (const double*)(sc + (size_t)nsse * n_q * nf);
+        const double* qf = qc + (size_t)n_q * nf;
+        const double* qb = qf + (size_t)n_q * nf;
+        const uint32_t* len = (const uint32_t*)(sc + (size_t)(nsse + nssim) * n_q * nf);
         for (int k = 0; k < n_q; k++)
             for (int i = 0; i < nf; i++) {
                 const size_t o = (size_t)k * n_frames + f0 + i, j = (size_t)k * nf + i;
                 bytes[o] = len[j]; sse_coded[o] = sc[j];
                 if (p) sse_filtered[o] = sf[j];
                 if (b) sse_brf[o] = sb[j];
+                if (ssim) {
+                    ssim_coded[o] = qc[j];
+                    if (p) ssim_filtered[o] = qf[j];
+                    if (b) ssim_brf[o] = qb[j];
+                }
             }
     }
     return DMC_OK;
@@ -1796,6 +1872,8 @@ extern "C" {
 //
 // The BRF arm (b != NULL) adds per (group, quality) one batched BRF launch on the coded frames, D of its output and its points,
 // and per camera one more render and SSE launch.  Its render reuses the coded view's buffer once that view's SSE is queued.
+// The SSIM outputs (ssim_view_coded != NULL) add per camera one SSIM launch pair per arm next to the arm's SSE launch, before the
+// coded view's buffer is reused; their results ride in the group's one copy.
 int dmc_jpeg_view_rd_sweep(dmc_ctx* ctx, const void* disp, const void* texture, int src_mem, int n_frames, int rows, int cols,
                            const int* qualities, int n_q, int flags, const dmc_chain_params* p, double f,
                            const double* R, const double* t, int n_views, const double* K, int is_sub, int render_flags,
@@ -1808,6 +1886,15 @@ int dmc_jpeg_view_rd_sweep_ex(dmc_ctx* ctx, const void* disp, const void* textur
                               const int* qualities, int n_q, int flags, const dmc_chain_params* p, const dmc_brf_params* b, double f,
                               const double* R, const double* t, int n_views, const double* K, int is_sub, int render_flags,
                               uint64_t* bytes, uint64_t* sse_view_coded, uint64_t* sse_view_filtered, uint64_t* sse_view_brf) {
+    return dmc_jpeg_view_rd_sweep_ssim(ctx, disp, texture, src_mem, n_frames, rows, cols, qualities, n_q, flags, p, b, f, R, t, n_views, K, is_sub,
+                                       render_flags, bytes, sse_view_coded, sse_view_filtered, sse_view_brf, nullptr, nullptr, nullptr);
+}
+
+int dmc_jpeg_view_rd_sweep_ssim(dmc_ctx* ctx, const void* disp, const void* texture, int src_mem, int n_frames, int rows, int cols,
+                                const int* qualities, int n_q, int flags, const dmc_chain_params* p, const dmc_brf_params* b, double f,
+                                const double* R, const double* t, int n_views, const double* K, int is_sub, int render_flags,
+                                uint64_t* bytes, uint64_t* sse_view_coded, uint64_t* sse_view_filtered, uint64_t* sse_view_brf,
+                                double* ssim_view_coded, double* ssim_view_filtered, double* ssim_view_brf) {
     if (!ctx) return fail(nullptr, DMC_ERR_ARG, "null context");
     if (!qualities || n_q < 1) return fail(ctx, DMC_ERR_ARG, "dmc_jpeg_view_rd_sweep: no qualities");
     for (int k = 0; k < n_q; k++)
@@ -1827,7 +1914,11 @@ int dmc_jpeg_view_rd_sweep_ex(dmc_ctx* ctx, const void* disp, const void* textur
     if (dmc_jpeg_encode_bound_ex(rows, cols, flags, &bound) != DMC_OK) return fail(ctx, DMC_ERR_SIZE, "dmc_jpeg_view_rd_sweep: " + g_err);
     const size_t fpx = (size_t)rows * cols;
     if (fpx >= ((size_t)1 << 29)) return fail(ctx, DMC_ERR_SIZE, "dmc_jpeg_view_rd_sweep: frame too large for the renderer");
-    if (n_frames < 0 || (n_frames > 0 && (!disp || !texture || !bytes || !sse_view_coded || !sse_view_filtered || (b && !sse_view_brf)))) return fail(ctx, DMC_ERR_SIZE, "dmc_jpeg_view_rd_sweep: bad arguments");
+    const bool ssim = ssim_view_coded != nullptr;
+    if (ssim && (rows < 11 || cols < 11)) return fail(ctx, DMC_ERR_SIZE, "dmc_jpeg_view_rd_sweep: SSIM needs frames of at least 11 x 11 (the window)");
+    if (n_frames < 0 || (n_frames > 0 && (!disp || !texture || !bytes || !sse_view_coded || !sse_view_filtered || (b && !sse_view_brf) ||
+                                          (ssim && (!ssim_view_filtered || (b && !ssim_view_brf))))))
+        return fail(ctx, DMC_ERR_SIZE, "dmc_jpeg_view_rd_sweep: bad arguments");
     if (n_frames == 0) return DMC_OK;
     CUDA_TRY(ctx, cudaSetDevice(ctx->device));
     cudaStream_t s = ctx->stream;
@@ -1838,7 +1929,8 @@ int dmc_jpeg_view_rd_sweep_ex(dmc_ctx* ctx, const void* disp, const void* textur
     // depth, two sets of points, their projection; raw render, coded and filtered views, reference views; the render's scratch;
     // with b, the BRF frames and their points
     const size_t per = l.coef_bytes + l.info_bytes + l.word_bytes + l.slot_bytes + (optimize ? l.opt_bytes + 2 * sizeof(dmcjpeg::HuffTable) : 0) +
-                       sizeof(dmcjpeg::FrameDesc) + fpx * ((host ? 4 : 0) + 3 + 4 + 4 + 24 + 8 + 9 + 3 * (size_t)n_views + (b ? 1 + 12 : 0)) + render_scratch_bytes(1, rows, cols);
+                       sizeof(dmcjpeg::FrameDesc) + fpx * ((host ? 4 : 0) + 3 + 4 + 4 + 24 + 8 + 9 + 3 * (size_t)n_views + (b ? 1 + 12 : 0)) + render_scratch_bytes(1, rows, cols) +
+                       (ssim ? ssim_partial_bytes(rows, cols, 3) : 0);
     // the render's attempt offsets are uint32 (at most 7 attempts a point) and the frame is a grid dimension
     const size_t cap = ((size_t)UINT32_MAX / (7 * fpx)) < 2048 ? (size_t)UINT32_MAX / (7 * fpx) : 2048;
     const int group = chunk_frames(kEncGroupBytes, per, n_frames, (int)cap, false);
@@ -1856,10 +1948,11 @@ int dmc_jpeg_view_rd_sweep_ex(dmc_ctx* ctx, const void* disp, const void* textur
     TRY(reserve(ctx, ctx->vs[VS_VIEW], 2 * 3 * fpx * group));
     TRY(reserve(ctx, ctx->vs[VS_REF], 3 * fpx * group * (size_t)n_views));
     TRY(reserve(ctx, ctx->render[0], render_scratch_bytes(group, rows, cols)));
+    if (ssim) TRY(reserve(ctx, ctx->rd[RD_SSIM], ssim_partial_bytes(rows, cols, 3) * group));
     // results of a group of nf frames: [sse_view_coded][sse_view_filtered][sse_view_brf if b] (uint64, [quality][view][frame]),
-    // the lengths (uint32)
-    const int nsse = b ? 3 : 2;
-    const size_t per_res = (size_t)n_q * (nsse * sizeof(uint64_t) * n_views + sizeof(uint32_t));
+    // with SSIM [ssim_view_coded][ssim_view_filtered][ssim_view_brf if b] (double, [quality][view][frame]), the lengths (uint32)
+    const int nsse = b ? 3 : 2, nssim = ssim ? nsse : 0;
+    const size_t per_res = (size_t)n_q * ((nsse + nssim) * sizeof(uint64_t) * n_views + sizeof(uint32_t));
     TRY(reserve(ctx, ctx->rd[RD_RES], per_res * group));
     std::vector<float> kr(9 * (size_t)n_views), tt(3 * (size_t)n_views);
     for (int v = 0; v < n_views; v++) camera_floats(R + 9 * v, t + 3 * v, K, &kr[9 * v], &tt[3 * v]);
@@ -1892,7 +1985,10 @@ int dmc_jpeg_view_rd_sweep_ex(dmc_ctx* ctx, const void* disp, const void* textur
         uint64_t* d_sc = (uint64_t*)ctx->rd[RD_RES].p;
         uint64_t* d_sf = d_sc + (size_t)n_q * n_views * nf;
         uint64_t* d_sb = d_sf + (size_t)n_q * n_views * nf;
-        uint32_t* d_len = (uint32_t*)(d_sc + (size_t)nsse * n_q * n_views * nf);
+        double* d_qc = (double*)(d_sc + (size_t)nsse * n_q * n_views * nf);
+        double* d_qf = d_qc + (size_t)n_q * n_views * nf;
+        double* d_qb = d_qf + (size_t)n_q * n_views * nf;
+        uint32_t* d_len = (uint32_t*)(d_sc + (size_t)(nsse + nssim) * n_q * n_views * nf);
         for (int k = 0; k < n_q; k++) {
             TRY(rd_degrade(ctx, k, dsrc, nf, rows, cols, optimize, coded));
             CUDA_TRY(ctx, cudaMemcpyAsync(d_len + (size_t)k * nf, ctx->jpeg_enc[JE_LENS].p, nf * sizeof(uint32_t), cudaMemcpyDeviceToDevice, s));
@@ -1908,9 +2004,14 @@ int dmc_jpeg_view_rd_sweep_ex(dmc_ctx* ctx, const void* disp, const void* textur
                 TRY(render_view(ctx, dtex, xyz_f, pt, raw, view_f, nf, rows, cols, &kr[9 * v], &tt[3 * v], is_sub, exact));
                 const size_t o = ((size_t)k * n_views + v) * nf;
                 LAUNCH(ctx, launch_sse_u8(ref + vb * v, view_c, view_f, d_sc + o, d_sf + o, nf, 3 * fpx, s));
-                if (b) {                                            // (stream order: the SSE above has read view_c)
+                if (ssim) {
+                    TRY(ssim_frames(ctx, ref + vb * v, view_c, nf, rows, cols, 3, d_qc + o));
+                    TRY(ssim_frames(ctx, ref + vb * v, view_f, nf, rows, cols, 3, d_qf + o));
+                }
+                if (b) {                                            // (stream order: the SSE and SSIM above have read view_c)
                     TRY(render_view(ctx, dtex, xyz_b, pt, raw, view_c, nf, rows, cols, &kr[9 * v], &tt[3 * v], is_sub, exact));
                     LAUNCH(ctx, launch_sse_u8(ref + vb * v, view_c, nullptr, d_sb + o, nullptr, nf, 3 * fpx, s));
+                    if (ssim) TRY(ssim_frames(ctx, ref + vb * v, view_c, nf, rows, cols, 3, d_qb + o));
                 }
             }
         }
@@ -1921,7 +2022,10 @@ int dmc_jpeg_view_rd_sweep_ex(dmc_ctx* ctx, const void* disp, const void* textur
         const uint64_t* sc = (const uint64_t*)res.data();
         const uint64_t* sf = sc + (size_t)n_q * n_views * nf;
         const uint64_t* sb = sf + (size_t)n_q * n_views * nf;
-        const uint32_t* len = (const uint32_t*)(sc + (size_t)nsse * n_q * n_views * nf);
+        const double* qc = (const double*)(sc + (size_t)nsse * n_q * n_views * nf);
+        const double* qf = qc + (size_t)n_q * n_views * nf;
+        const double* qb = qf + (size_t)n_q * n_views * nf;
+        const uint32_t* len = (const uint32_t*)(sc + (size_t)(nsse + nssim) * n_q * n_views * nf);
         for (int k = 0; k < n_q; k++)
             for (int i = 0; i < nf; i++) {
                 bytes[(size_t)k * n_frames + f0 + i] = len[(size_t)k * nf + i];
@@ -1929,6 +2033,10 @@ int dmc_jpeg_view_rd_sweep_ex(dmc_ctx* ctx, const void* disp, const void* textur
                     const size_t o = ((size_t)k * n_views + v) * n_frames + f0 + i, j = ((size_t)k * n_views + v) * nf + i;
                     sse_view_coded[o] = sc[j]; sse_view_filtered[o] = sf[j];
                     if (b) sse_view_brf[o] = sb[j];
+                    if (ssim) {
+                        ssim_view_coded[o] = qc[j]; ssim_view_filtered[o] = qf[j];
+                        if (b) ssim_view_brf[o] = qb[j];
+                    }
                 }
             }
     }

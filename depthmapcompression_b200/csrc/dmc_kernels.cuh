@@ -104,6 +104,11 @@ namespace dmc {
 // Exact per-frame sum of squared differences of n dense 8-bit frames of frame_bytes each (dmc_metrics.cu): sse0[f] = SSE(a, b0)
 // and, when b1 != nullptr, sse1[f] = SSE(a, b1) in the same launch (a is read once).  Zeroes the outputs first.
 int launch_sse_u8(const uint8_t* a, const uint8_t* b0, const uint8_t* b1, uint64_t* sse0, uint64_t* sse1, int n, size_t frame_bytes, cudaStream_t s);
+// SSIM of n dense rows x cols 8-bit frames of `channels` (1 or 3, interleaved) channels, rows and cols >= 11 (dmc_metrics.cu):
+// mssim[f] = MSSIM(a_f, b_f), the definition of dmc_ssim_batch.  `partial` holds n x ssim_partial_bytes(rows, cols, channels)
+// bytes of per-tile sums; mssim (device, n doubles) is written in stream order.  Deterministic: no floating-point atomics.
+size_t ssim_partial_bytes(int rows, int cols, int channels);
+int launch_ssim_u8(const uint8_t* a, const uint8_t* b, double* partial, double* mssim, int n, int rows, int cols, int channels, cudaStream_t s);
 }
 
 namespace dmc {

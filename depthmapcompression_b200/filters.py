@@ -302,6 +302,37 @@ def frameSSE(a, b, ctx=None):
     return sse
 
 
+def _ssim_frames(frames, channels):
+    """numpy uint8 [n, rows, cols], [rows, cols], [n, rows, cols, 3] or [rows, cols, 3] (a trailing 3 is a colour frame: a gray
+    frame needs cols >= 11), or (device pointer, n, rows, cols) with `channels` -> (pointer, n, rows, cols, channels, mem, array)"""
+    if isinstance(frames, tuple):
+        ptr, n, rows, cols = (int(x) for x in frames)
+        return ptr, n, rows, cols, int(channels), MEM_DEVICE, None
+    a = np.ascontiguousarray(frames)
+    if a.dtype != np.uint8 or a.ndim not in (2, 3, 4) or (a.ndim == 4 and a.shape[-1] != 3):
+        raise DmcError(capi.DMC_ERR_TYPE, "frames must be uint8 [n, rows, cols], [rows, cols], [n, rows, cols, 3] or [rows, cols, 3]")
+    cn = 3 if a.ndim == 4 or (a.ndim == 3 and a.shape[-1] == 3) else 1
+    shape = a.shape[:-1] if cn == 3 else a.shape
+    n, rows, cols = (1,) + shape if len(shape) == 2 else shape
+    return a.ctypes.data, n, rows, cols, cn, MEM_HOST, a
+
+
+def frameSSIM(a, b, ctx=None, channels=1):
+    """Per-frame mean structural similarity of two batches of 8-bit frames on the GPU (dmc_ssim_batch; the definition of
+    Wang et al. 2004 and of skimage's structural_similarity(data_range=255, gaussian_weights=True, sigma=1.5,
+    use_sample_covariance=False), channels averaged).  a, b: uint8 numpy [n, rows, cols] or [rows, cols] (gray), [n, rows, cols, 3]
+    or [rows, cols, 3] (interleaved colour), or both (device pointer, n, rows, cols) with channels= 1 or 3.  Frames of at least
+    11 x 11.  -> np.float64[n]"""
+    ctx = ctx or default_context()
+    ap, n, rows, cols, cn, mem, ka = _ssim_frames(a, channels)
+    bp, bn, brows, bcols, bcn, bmem, kb = _ssim_frames(b, channels)
+    if (n, rows, cols, cn, mem) != (bn, brows, bcols, bcn, bmem):
+        raise DmcError(capi.DMC_ERR_SIZE, "frameSSIM: a and b must be batches of one shape in the same memory")
+    out = np.zeros(n, np.float64)
+    ctx.check(lib.dmc_ssim_batch(ctx.h, C.c_void_p(ap), C.c_void_p(bp), n, rows, cols, cn, mem, out.ctypes.data_as(C.POINTER(C.c_double))))
+    return out
+
+
 _psnr = np.vectorize(lambda sse, pixels: lib.dmc_psnr_from_sse(int(sse), int(pixels)), otypes=[np.float64])
 
 
@@ -312,12 +343,13 @@ def psnrFromSSE(sse, pixels):
     return float(r) if r.ndim == 0 else r
 
 
-def jpegRateDistortion(frames, qualities, params=None, optimize=False, ctx=None, brf=None):
-    """The JPEG rate-distortion sweep on the GPU (dmc_jpeg_rd_sweep_ex): every frame is coded at every quality as cv2.imencode
+def jpegRateDistortion(frames, qualities, params=None, optimize=False, ctx=None, brf=None, ssim=False):
+    """The JPEG rate-distortion sweep on the GPU (dmc_jpeg_rd_sweep_ssim): every frame is coded at every quality as cv2.imencode
     codes it (optimize: with optimised Huffman tables), decoded, and with `params` (a chain_params(CHAIN_DISP8U, ...))
     post-filtered; with `brf` (a brf_params(...)) the decoded frames also go through boundaryReconstructionFilter.  No frame
     or stream leaves the device.  frames as for degradeJPEG.  Returns a dict of (n_q, n) arrays: bytes, sse_coded,
-    psnr_coded, with params also sse_filtered, psnr_filtered, and with brf also sse_brf, psnr_brf."""
+    psnr_coded, with params also sse_filtered, psnr_filtered, and with brf also sse_brf, psnr_brf.  ssim=True adds the
+    frameSSIM of every arm against the source: ssim_coded (and ssim_filtered, ssim_brf with params, brf), float64."""
     ctx = ctx or default_context()
     sp, n, rows, cols, mem, keep = _frames(frames)
     q = np.ascontiguousarray(np.asarray(qualities).ravel(), dtype=np.int32)
@@ -326,10 +358,14 @@ def jpegRateDistortion(frames, qualities, params=None, optimize=False, ctx=None,
     nbytes, sc = np.zeros(shape, np.uint64), np.zeros(shape, np.uint64)
     sf = np.zeros(shape, np.uint64) if params is not None else None
     sb = np.zeros(shape, np.uint64) if brf is not None else None
-    ctx.check(lib.dmc_jpeg_rd_sweep_ex(ctx.h, C.c_void_p(sp), mem, n, rows, cols, q.ctypes.data_as(C.POINTER(C.c_int)), len(q), _jpeg_flags(optimize),
-                                       C.byref(params) if params is not None else None, C.byref(brf) if brf is not None else None,
-                                       nbytes.ctypes.data_as(U64), sc.ctypes.data_as(U64), sf.ctypes.data_as(U64) if sf is not None else None,
-                                       sb.ctypes.data_as(U64) if sb is not None else None))
+    qs = {k: np.zeros(shape, np.float64) for k, on in (("ssim_coded", True), ("ssim_filtered", params is not None), ("ssim_brf", brf is not None))
+          if ssim and on}
+    DP = C.POINTER(C.c_double)
+    ctx.check(lib.dmc_jpeg_rd_sweep_ssim(ctx.h, C.c_void_p(sp), mem, n, rows, cols, q.ctypes.data_as(C.POINTER(C.c_int)), len(q), _jpeg_flags(optimize),
+                                         C.byref(params) if params is not None else None, C.byref(brf) if brf is not None else None,
+                                         nbytes.ctypes.data_as(U64), sc.ctypes.data_as(U64), sf.ctypes.data_as(U64) if sf is not None else None,
+                                         sb.ctypes.data_as(U64) if sb is not None else None,
+                                         *[qs[k].ctypes.data_as(DP) if k in qs else None for k in ("ssim_coded", "ssim_filtered", "ssim_brf")]))
     out = {"bytes": nbytes, "sse_coded": sc, "psnr_coded": psnrFromSSE(sc, rows * cols)}
     if sf is not None:
         out["sse_filtered"] = sf
@@ -337,11 +373,13 @@ def jpegRateDistortion(frames, qualities, params=None, optimize=False, ctx=None,
     if sb is not None:
         out["sse_brf"] = sb
         out["psnr_brf"] = psnrFromSSE(sb, rows * cols)
+    out.update(qs)
     return out
 
 
-def jpegViewRateDistortion(disp, texture, qualities, params, f, R, t, K, isSub=True, optimize=False, exact_divide=False, ctx=None, brf=None):
-    """The view-synthesis rate-distortion sweep on the GPU (dmc_jpeg_view_rd_sweep_ex): coded depth scored by the views it
+def jpegViewRateDistortion(disp, texture, qualities, params, f, R, t, K, isSub=True, optimize=False, exact_divide=False, ctx=None, brf=None,
+                           ssim=False):
+    """The view-synthesis rate-distortion sweep on the GPU (dmc_jpeg_view_rd_sweep_ssim): coded depth scored by the views it
     renders, as pointcloudTest renders a decoded depth map.  For every frame, quality and camera (R[v], t[v], shared K) the
     reference view fillSmallHole(projectImagefromXYZ(texture, reprojectXYZ(D(disp), f), ...)), with D the unfiltered
     disp8U2depth32F, is compared with the view of D(decoded) and with the view of filterDisp8U2Depth32F(decoded, params).
@@ -350,7 +388,8 @@ def jpegViewRateDistortion(disp, texture, qualities, params, f, R, t, K, isSub=T
     R: [n_views, 3, 3] (or one 3x3), t: [n_views, 3].  Returns a dict: bytes (n_q, n), and sse_view_coded, psnr_view_coded,
     sse_view_filtered, psnr_view_filtered (n_q, n_views, n); the PSNR is cv2.PSNR of the two 8UC3 views.  brf (a
     brf_params(...)): also sse_view_brf, psnr_view_brf, the view of D(boundaryReconstructionFilter(decoded)) against the
-    same reference view."""
+    same reference view.  ssim=True adds the frameSSIM of the 8UC3 views against the reference view: ssim_view_coded,
+    ssim_view_filtered (and ssim_view_brf with brf), float64 (n_q, n_views, n)."""
     ctx = ctx or default_context()
     sp, n, rows, cols, mem, keep = _frames(disp)
     if isinstance(texture, tuple):
@@ -375,17 +414,21 @@ def jpegViewRateDistortion(disp, texture, qualities, params, f, R, t, K, isSub=T
     nbytes = np.zeros((len(q), n), np.uint64)
     sc, sf = np.zeros((len(q), nv, n), np.uint64), np.zeros((len(q), nv, n), np.uint64)
     sb = np.zeros((len(q), nv, n), np.uint64) if brf is not None else None
-    ctx.check(lib.dmc_jpeg_view_rd_sweep_ex(ctx.h, C.c_void_p(sp), C.c_void_p(tp), mem, n, rows, cols, q.ctypes.data_as(C.POINTER(C.c_int)), len(q),
-                                            _jpeg_flags(optimize), C.byref(params), C.byref(brf) if brf is not None else None, float(f),
-                                            Rs.ctypes.data_as(DP), ts.ctypes.data_as(DP), nv, Ks.ctypes.data_as(DP), int(bool(isSub)),
-                                            capi.RENDER_EXACT_DIVIDE if exact_divide else 0, nbytes.ctypes.data_as(U64), sc.ctypes.data_as(U64),
-                                            sf.ctypes.data_as(U64), sb.ctypes.data_as(U64) if sb is not None else None))
+    qs = {k: np.zeros((len(q), nv, n), np.float64) for k, on in (("ssim_view_coded", True), ("ssim_view_filtered", True), ("ssim_view_brf", brf is not None))
+          if ssim and on}
+    ctx.check(lib.dmc_jpeg_view_rd_sweep_ssim(ctx.h, C.c_void_p(sp), C.c_void_p(tp), mem, n, rows, cols, q.ctypes.data_as(C.POINTER(C.c_int)), len(q),
+                                              _jpeg_flags(optimize), C.byref(params), C.byref(brf) if brf is not None else None, float(f),
+                                              Rs.ctypes.data_as(DP), ts.ctypes.data_as(DP), nv, Ks.ctypes.data_as(DP), int(bool(isSub)),
+                                              capi.RENDER_EXACT_DIVIDE if exact_divide else 0, nbytes.ctypes.data_as(U64), sc.ctypes.data_as(U64),
+                                              sf.ctypes.data_as(U64), sb.ctypes.data_as(U64) if sb is not None else None,
+                                              *[qs[k].ctypes.data_as(DP) if k in qs else None for k in ("ssim_view_coded", "ssim_view_filtered", "ssim_view_brf")]))
     px = 3 * rows * cols
     out = {"bytes": nbytes, "sse_view_coded": sc, "psnr_view_coded": psnrFromSSE(sc, px),
            "sse_view_filtered": sf, "psnr_view_filtered": psnrFromSSE(sf, px)}
     if sb is not None:
         out["sse_view_brf"] = sb
         out["psnr_view_brf"] = psnrFromSSE(sb, px)
+    out.update(qs)
     return out
 
 

@@ -277,6 +277,39 @@ int dmc_jpeg_rd_sweep_ex(dmc_ctx* ctx, const void* src, int src_mem, int n_frame
                          int flags, const dmc_chain_params* p, const dmc_brf_params* b, uint64_t* bytes, uint64_t* sse_coded,
                          uint64_t* sse_filtered, uint64_t* sse_brf);
 
+/* ---- structural similarity (SSIM) ---------------------------------------------------------------------------------------- */
+/* Per-frame mean structural similarity of two batches of n dense rows x cols 8-bit frames of `channels` interleaved channels
+ * (1: 8UC1, 3: 8UC3 such as the sweeps' BGR views), both in `mem`; mssim (host, n_frames entries).  The definition is that of
+ * Wang, Bovik, Sheikh and Simoncelli (2004), ssim_index.m, and of skimage.metrics.structural_similarity(a, b, data_range=255,
+ * gaussian_weights=True, sigma=1.5, use_sample_covariance=False[, channel_axis=-1]):
+ *   window   w = g g^T, g_i = exp(-i^2 / 4.5) for i = -5..5, normalised to sum 1 in double;
+ *   at every window position that lies wholly inside the frame ((rows - 10) x (cols - 10) of them), per channel:
+ *            mu_x = sum w x, mu_y = sum w y, s_x = sum w x^2 - mu_x^2, s_y = sum w y^2 - mu_y^2, s_xy = sum w x y - mu_x mu_y,
+ *            S = ((2 mu_x mu_y + C1)(2 s_xy + C2)) / ((mu_x^2 + mu_y^2 + C1)(s_x + s_y + C2)),  C1 = (0.01 * 255)^2, C2 = (0.03 * 255)^2;
+ *   MSSIM    the mean of S over the positions; with 3 channels the mean of the three channels' MSSIMs.
+ * Computed in FP64 (in FP32, E[x^2] - mu^2 cancels to about 4e-3 on sigma^2 near 255).  Deterministic: a frame's result is
+ * the same bits alone, in any batch, inside a sweep, from host or device memory.  a == b and any alignment are legal.
+ * DMC_ERR_ARG: channels not 1 or 3, a bad mem; DMC_ERR_SIZE: rows or cols below 11, a negative count, a NULL pointer;
+ * nothing is written on error.  Returns when mssim is valid. */
+int dmc_ssim_batch(dmc_ctx* ctx, const void* a, const void* b, int n_frames, int rows, int cols, int channels, int mem, double* mssim);
+/* dmc_jpeg_rd_sweep_ex with SSIM outputs, in the layout of the SSE arrays ([k*n+i]): ssim_coded = MSSIM(frame, decoded),
+ * ssim_filtered = MSSIM(frame, chain(decoded)), ssim_brf = MSSIM(frame, B(decoded)).  SSIM is computed iff ssim_coded != NULL;
+ * then ssim_filtered is required iff p != NULL and ssim_brf iff b != NULL (DMC_ERR_SIZE), and frames below 11 x 11 are
+ * DMC_ERR_SIZE.  With ssim_coded == NULL this is dmc_jpeg_rd_sweep_ex: the same launches, the same results.  bytes and the SSE
+ * outputs are the same with and without SSIM. */
+int dmc_jpeg_rd_sweep_ssim(dmc_ctx* ctx, const void* src, int src_mem, int n_frames, int rows, int cols, const int* qualities, int n_q,
+                           int flags, const dmc_chain_params* p, const dmc_brf_params* b, uint64_t* bytes, uint64_t* sse_coded,
+                           uint64_t* sse_filtered, uint64_t* sse_brf, double* ssim_coded, double* ssim_filtered, double* ssim_brf);
+/* dmc_jpeg_view_rd_sweep_ex with SSIM outputs of the 8UC3 views, in the layout of the SSE arrays ([(k*n_views + v)*n + i]):
+ * MSSIM(view(D(disp_i)), the arm's view).  SSIM is computed iff ssim_view_coded != NULL; then ssim_view_filtered is required and
+ * ssim_view_brf iff b != NULL (DMC_ERR_SIZE), and frames below 11 x 11 are DMC_ERR_SIZE.  With ssim_view_coded == NULL this is
+ * dmc_jpeg_view_rd_sweep_ex. */
+int dmc_jpeg_view_rd_sweep_ssim(dmc_ctx* ctx, const void* disp, const void* texture, int src_mem, int n_frames, int rows, int cols,
+                                const int* qualities, int n_q, int flags, const dmc_chain_params* p, const dmc_brf_params* b, double f,
+                                const double* R, const double* t, int n_views, const double* K, int is_sub, int render_flags,
+                                uint64_t* bytes, uint64_t* sse_view_coded, uint64_t* sse_view_filtered, uint64_t* sse_view_brf,
+                                double* ssim_view_coded, double* ssim_view_filtered, double* ssim_view_brf);
+
 /* ---- stand-alone operators of filter.h ------------------------------------------------------------------- */
 /* binalyWeightedRangeFilter filter.h:29 (binalyWeightedRangeFilter.cpp:1106): 8U/16S/16U/32F x C1/C3 */
 int dmc_bwrf(dmc_ctx* ctx, const dmc_image* src, dmc_image* dst, int kernel_w, int kernel_h, float threshold,

@@ -271,3 +271,19 @@ inline void renderViewBatch(const vector<Mat>& depth, const vector<Mat>& texture
 		}
 	}
 }
+
+// Mean structural similarity (SSIM, Wang et al. 2004) of two CV_8UC1 or CV_8UC3 images of one size and type in host memory,
+// on the GPU (dmc_ssim_batch): 11x11 Gaussian window with sigma 1.5, only window positions inside the image, C1 = (0.01*255)^2,
+// C2 = (0.03*255)^2, FP64; for CV_8UC3 the mean of the three channels' values.  Both sides at least 11 x 11.
+inline double structuralSimilarity(const Mat& a, const Mat& b)
+{
+	const int type = a.type();
+	dmc_dropin::require((type == CV_8UC1 || type == CV_8UC3) && b.type() == type && a.rows == b.rows && a.cols == b.cols,
+	                    "structuralSimilarity: a and b must be CV_8UC1 or CV_8UC3 images of one size and type");
+	const Mat x = a.isContinuous() ? a : a.clone();
+	const Mat y = b.isContinuous() ? b : b.clone();
+	double mssim = 0;
+	dmc_dropin::check(dmc_ssim_batch(dmc_dropin::context(), x.data, y.data, 1, x.rows, x.cols, type == CV_8UC3 ? 3 : 1, DMC_MEM_HOST, &mssim),
+	                  "structuralSimilarity");
+	return mssim;
+}
