@@ -253,7 +253,9 @@ int range_filter_32f(dmc_ctx* ctx, const void* src, void* dst, Buf& tmp, int n, 
     if (method == DMC_FULL_KERNEL || method == DMC_FULL_KERNEL_PAIR) {
         // FULL_KERNEL_PAIR has no deterministic reference output (racy scatter, unwritten tail columns); it computes
         // the FULL_KERNEL result that it approximates.  No bit-parity claim for that method (DESIGN.md).
-        if (kw == 0 || kh == 0) { kw = 1; kh = 1; if (load_op == LOAD_F32 && store_op == STORE_F32) return copy_unless_same(ctx, dst, src, count * sizeof(float), s); }
+        // an empty window copies the image (:980), so a 16-bit source comes back unchanged through its float round trip: one
+        // tap that passes at any threshold (v / 1 = v), not the 1x1 filter, whose tap a negative or NaN threshold rejects
+        if (kw == 0 || kh == 0) { kw = 1; kh = 1; threshold = FLT_MAX; if (load_op == LOAD_F32 && store_op == STORE_F32) return copy_unless_same(ctx, dst, src, count * sizeof(float), s); }
         RowSpan rs = make_rowspan(kw, kh);
         LAUNCH(ctx, launch_bwrf32f(src, dst, n, H, W, cn, rs, threshold, load_op, maf, store_op, s));
         return DMC_OK;

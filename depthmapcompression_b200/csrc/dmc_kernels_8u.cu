@@ -133,6 +133,11 @@ template <> __device__ __forceinline__ double absdiff_cv<double>(double a, doubl
 
 // MODE 0: blur-remove select; 1: max only; 2: min only.  The channel is blockIdx.z % cn (planes are filtered
 // independently, minmaxFilter.cpp:189-213).
+// Visiting order (cv::dilate / cv::erode as the reference build's cv:: stand-in states them, DESIGN.md §2): each pass
+// starts at the window's centre and then folds every tap in order (left to right, top to bottom) with m = v > m ? v : m.
+// For ordered values the order is free, but a NaN sticks only where the fold starts and of +0 / -0 the first one seen
+// wins, so float results follow the reference only in this order.  Clamped border taps repeat a neighbour and change
+// nothing.
 template <typename T, int MODE>
 __global__ void __launch_bounds__(256) minmax_kernel(const T* __restrict__ src, T* __restrict__ dst, int H, int W, int cn, int rx, int ry) {
     extern __shared__ unsigned char smraw[];
@@ -153,16 +158,16 @@ __global__ void __launch_bounds__(256) minmax_kernel(const T* __restrict__ src, 
     for (int idx = tid; idx < TH * kTX; idx += 256) {
         int ty = idx / kTX, tx = idx - ty * kTX;
         const T* p = sin + ty * TW + tx;
-        T mx = p[0], mn = p[0];
-        for (int i = 1; i <= 2 * rx; i++) { T v = p[i]; mx = v > mx ? v : mx; mn = v < mn ? v : mn; }
+        T mx = p[rx], mn = p[rx];                 // centre first: see the visiting order above
+        for (int i = 0; i <= 2 * rx; i++) { T v = p[i]; mx = v > mx ? v : mx; mn = v < mn ? v : mn; }
         smx[idx] = mx; smn[idx] = mn;
     }
     __syncthreads();
     for (int ly = threadIdx.y; ly < kTY; ly += blockDim.y) {
         int x = x0 + threadIdx.x, y = y0 + ly;
         if (x >= W || y >= H) continue;
-        T mx = smx[ly * kTX + threadIdx.x], mn = smn[ly * kTX + threadIdx.x];
-        for (int i = 1; i <= 2 * ry; i++) {
+        T mx = smx[(ly + ry) * kTX + threadIdx.x], mn = smn[(ly + ry) * kTX + threadIdx.x];
+        for (int i = 0; i <= 2 * ry; i++) {
             T a = smx[(ly + i) * kTX + threadIdx.x], b = smn[(ly + i) * kTX + threadIdx.x];
             mx = a > mx ? a : mx; mn = b < mn ? b : mn;
         }

@@ -98,3 +98,31 @@ def make_image(rs, H, W, dtype=np.uint8, cn=1, kind="pw"):
     elif dtype in (np.float32, np.float64):
         a = a * 3.7 + 0.25 * rs.randint(0, 4, size=shape)
     return np.ascontiguousarray(a.astype(dtype))
+
+
+def special_floats(dtype, nan=True, negzero=True):
+    """IEEE values a float min / max can get wrong: infinities, the largest finite values, the smallest normal value
+    and its neighbours (FLT_MIN seeds maxFilter), subnormals, zeros and NaN."""
+    f = np.finfo(dtype); t = dtype(f.tiny); z = dtype(0)
+    v = [z, np.inf, -np.inf, f.max, -f.max, t, -t, np.nextafter(t, z), np.nextafter(t, dtype(1)), -np.nextafter(t, z),
+         t / dtype(4), -t / dtype(4), f.smallest_subnormal, -f.smallest_subnormal]
+    if negzero:
+        v.append(-z)
+    if nan:
+        v.append(np.nan)
+    return np.array(v, dtype)
+
+
+def special_image(rs, H, W, dtype, cn=1, nan=True, negzero=True, p=0.2):
+    """Half-integers in -1.5..1.5 (many ties and zeros) with a fraction `p` of the pixels, and every corner, replaced by
+    special_floats.  With `negzero` the zeros take random signs."""
+    shape = (H, W) if cn == 1 else (H, W, cn)
+    a = (rs.randint(-3, 4, size=shape) * 0.5).astype(dtype)
+    if negzero:
+        a[(a == 0) & (rs.rand(*shape) < 0.5)] = -0.0
+    sp = special_floats(dtype, nan, negzero)
+    pick = rs.rand(*shape) < p
+    a[pick] = sp[rs.randint(0, len(sp), size=int(pick.sum()))]
+    for y, x in ((0, 0), (0, W - 1), (H - 1, 0), (H - 1, W - 1)):
+        a[y, x] = sp[rs.randint(0, len(sp), size=a[y, x].shape)]
+    return np.ascontiguousarray(a)

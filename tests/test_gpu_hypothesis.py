@@ -57,7 +57,7 @@ def test_chain_entry_points(dmc, port, H, W, seed, smooth, mr, gr, mmr, br, th, 
 @settings(**COMMON)
 @given(H=st.integers(1, 60), W=st.integers(1, 140), seed=st.integers(0, 10**6), smooth=st.booleans(),
        kw=st.integers(0, 15), kh=st.integers(0, 15), th=st.floats(0, 255.9), method=st.sampled_from([0, 1, 2]),
-       tc=st.sampled_from([(np.uint8, 1), (np.uint8, 3), (np.uint16, 1), (np.int16, 1), (np.float32, 1), (np.float32, 3)]))
+       tc=st.sampled_from([(np.uint8, 1), (np.uint8, 3), (np.uint16, 1), (np.int16, 1), (np.uint16, 3), (np.int16, 3), (np.float32, 1), (np.float32, 3)]))
 def test_range_filter(dmc, port, H, W, seed, smooth, kw, kh, th, method, tc):
     dt, cn = tc
     b = _image(seed, H, W, dt, cn, smooth)

@@ -45,7 +45,7 @@ while time.time() - t0 < budget:
     H = int(rs.choice([rs.randint(1, 20), rs.randint(20, 140), 64 * rs.randint(1, 4) + rs.randint(-2, 3)]))
     W = max(W, 1); H = max(H, 1)
     a = image(H, W)
-    op = rs.randint(12)
+    op = rs.randint(13)
     if op == 0:
         k = int(rs.choice([3, 5, 7, 9, 13, 17, 21])); same(dmc.medianBlur(a, None, k) if hasattr(dmc, "medianBlur") else pfs(a, None, k // 2, 0, 0, 0, 0), port.post_filter_set(a, k // 2, 0, 0, 0, 0), "median k%d %dx%d" % (k, H, W))
     elif op == 1:
@@ -84,12 +84,21 @@ while time.time() - t0 < budget:
         same(dmc.minmaxBoundaryReconstructionFilter(b, None, r, (k, k), 1.0, 1.0, 1.0), port.brf(port.blur_remove_minmax(b, r), k, k, 1.0, 1.0, 1.0), "fused r%d k%d %s %dx%d" % (r, k, np.dtype(dt).name, H, W))
     elif op == 10:      # 32-bit range filter on 16-bit sources (integer mode up to radius 9, float mode at 10) and on floats
         dt = [np.uint16, np.int16, np.float32][rs.randint(3)]
-        scale = int(rs.choice([1, 16, 257]))
+        scale = int(rs.choice([1, 16, 257])); a = image(H, W, int(rs.choice([1, 3])))
         b = (a.astype(np.int32) * scale - (30000 if dt == np.int16 else 0)).clip(-32768, 65535).astype(dt) if dt != np.float32 else (a * 3.7).astype(np.float32)
         r = int(rs.randint(1, 11)); th = float(rs.choice([0, 0.5, 3, 10.9, 40, 160, 5000, 70000])); k = 2 * r + 1
         got = dmc.binalyWeightedRangeFilter(b, None, (k, k), th, dmc.FULL_KERNEL); want = port.bwrf(b, k, k, th)
         if r % 8 == 5 and W % 4 == 0: got[:, -1] = want[:, -1]      # the reference's own undefined read (masked in tests/ too)
-        same(got, want, "bwrf32 %s r%d th%s %dx%d" % (np.dtype(dt).name, r, th, H, W))
+        same(got, want, "bwrf32 %sC%d r%d th%s %dx%d" % (np.dtype(dt).name, a.size // (H * W), r, th, H, W))
+    elif op == 11:      # blurRemoveMinMax on the wider types, NaN and zeros of both signs in the float images
+        dt = [np.uint16, np.int16, np.float32, np.float64][rs.randint(4)]; cn = int(rs.choice([1, 3])); c = image(H, W, cn)
+        if dt in (np.float32, np.float64):
+            b = (c.astype(dt) - 128) * dt(0.5)
+            sel = rs.rand(*b.shape); b[sel < 0.03] = np.nan; b[(sel >= 0.03) & (sel < 0.1)] = -0.0
+        else:
+            b = (c.astype(np.int32) * 257 - (32768 if dt == np.int16 else 0)).astype(dt)
+        r = int(rs.randint(0, 11))
+        same(dmc.blurRemoveMinMax(b, None, r), port.blur_remove_minmax(b, r), "minmaxT %sC%d r%d %dx%d" % (np.dtype(dt).name, cn, r, H, W))
     else:               # pinned host images (filtered in place over the host link)
         b = np.maximum(a, 1)
         if b.nbytes:
