@@ -30,7 +30,7 @@ EXPORTS = [
     "dmc_small_gaussian", "dmc_median_blur",
     "dmc_disp8u2depth32f", "dmc_depth32f2disp8u", "dmc_depth16u2disp8u", "dmc_disp16s2depth16u",
     "dmc_fill_occlusion", "dmc_reproject_xyz", "dmc_transpose",
-    "dmc_chain_batch_jpeg", "dmc_jpeg_probe", "dmc_jpeg_encode_bound", "dmc_jpeg_encode_gray_batch", "dmc_jpeg_degrade_gray_batch", "dmc_jpeg_encode_bound_ex", "dmc_jpeg_encode_gray_batch_ex", "dmc_jpeg_degrade_gray_batch_ex", "dmc_split_bgr_line_interleave", "dmc_project_points", "dmc_project_image_from_xyz", "dmc_fill_small_hole", "dmc_hostlink_probe", "dmc_release_device", "dmc_set_gateway", "dmc_get_gateway", "dmc_sched_get_routing",
+    "dmc_chain_batch_jpeg", "dmc_jpeg_probe", "dmc_jpeg_decode_color_batch", "dmc_jpeg_probe_color", "dmc_jpeg_encode_bound", "dmc_jpeg_encode_gray_batch", "dmc_jpeg_degrade_gray_batch", "dmc_jpeg_encode_bound_ex", "dmc_jpeg_encode_gray_batch_ex", "dmc_jpeg_degrade_gray_batch_ex", "dmc_split_bgr_line_interleave", "dmc_project_points", "dmc_project_image_from_xyz", "dmc_fill_small_hole", "dmc_hostlink_probe", "dmc_release_device", "dmc_set_gateway", "dmc_get_gateway", "dmc_sched_get_routing",
     "dmc_sse_gray_batch", "dmc_psnr_from_sse", "dmc_jpeg_rd_sweep", "dmc_jpeg_view_rd_sweep",
     "dmc_brf_batch", "dmc_jpeg_rd_sweep_ex", "dmc_jpeg_view_rd_sweep_ex",
     "dmc_prepare_disp_batch", "dmc_render_view_batch",
@@ -90,6 +90,8 @@ def _load():
         "dmc_jpeg_decode_gray_batch": (I, [P, P, P, I, I, I, P, I]),
         "dmc_chain_batch_jpeg": (I, [P, P, P, I, I, I, P, I, C.POINTER(DmcChainParams)]),
         "dmc_jpeg_probe": (I, [P, C.c_size_t, C.POINTER(I), C.POINTER(I), C.c_char_p, C.c_size_t]),
+        "dmc_jpeg_decode_color_batch": (I, [P, P, P, I, I, I, P, I]),
+        "dmc_jpeg_probe_color": (I, [P, C.c_size_t, C.POINTER(I), C.POINTER(I), C.POINTER(I), C.c_char_p, C.c_size_t]),
         "dmc_jpeg_encode_bound": (I, [I, I, C.POINTER(C.c_uint64)]),
         "dmc_jpeg_encode_gray_batch": (I, [P, P, I, I, I, I, I, P, I, C.c_uint64, C.POINTER(C.c_uint64)]),
         "dmc_jpeg_degrade_gray_batch": (I, [P, P, P, I, I, I, I, I, C.POINTER(C.c_uint64)]),

@@ -26,6 +26,8 @@ constexpr int kSlots = 4;        // streaming pipeline depth (H2D / kernels / D2
 enum { SB_IN, SB_OUT, SB_PING, SB_PONG, SB_FLOAT, SB_BITS, SB_META, SB_SCANS, SB_COEF, SB_COUNT };
 // Device buffers of dmc_jpeg_decode_gray_batch.
 enum { JD_BITS, JD_META, JD_SCANS, JD_COEF, JD_OUT, JD_COUNT };
+// Device buffers of dmc_jpeg_decode_color_batch: those of the gray decoder plus the component planes.
+enum { JC_BITS, JC_META, JC_SCANS, JC_PLANES, JC_COEF, JC_OUT, JC_COUNT };
 // Device buffers of dmc_sse_gray_batch and dmc_jpeg_rd_sweep: every quality's encoder + decoder tables, the decoder's
 // FrameDescs of a group, its staged source, coded and filtered frames (the staged second batch of dmc_sse_gray_batch; the
 // BRF arm's frames in both sweeps), and the group's results (SSE, stream lengths) that one copy brings back.
@@ -59,6 +61,7 @@ struct dmc_ctx {
     struct Gateway { int device = -1; cudaStream_t stream[kSlots] = {}; Buf in[kSlots], out[kSlots]; cudaEvent_t ev_in[kSlots] = {}, ev_out[kSlots] = {}, ev_done[kSlots] = {}; } gw;
     Buf render[2]; int* render_flag = nullptr;      // point-cloud render: attempt lists etc., device flag; pinned host flag
     Buf jpeg[JD_COUNT];
+    Buf jpeg_color[JC_COUNT];
     Buf rd[RD_COUNT];
     Buf vs[VS_COUNT];
     Buf jpeg_enc[11];            // JPEG encode: tables, staged frames, coefficients, block records, scan words, slots, lengths + offsets, staged output, decoder tables + descriptors,
@@ -561,6 +564,7 @@ void dmc_destroy(dmc_ctx* ctx) {
     drop_gateway(ctx);
     drop_graph(ctx);
     for (auto& b : ctx->jpeg) if (b.p) cudaFree(b.p);
+    for (auto& b : ctx->jpeg_color) if (b.p) cudaFree(b.p);
     for (auto& b : ctx->jpeg_enc) if (b.p) cudaFree(b.p);
     for (auto& b : ctx->rd) if (b.p) cudaFree(b.p);
     for (auto& b : ctx->render) if (b.p) cudaFree(b.p);
@@ -973,6 +977,112 @@ int dmc_jpeg_decode_gray_batch(dmc_ctx* ctx, const void* blob, const uint64_t* o
         LAUNCH(ctx, launch_jpeg_decode((const uint8_t*)ctx->jpeg[JD_BITS].p, dm, dm + g.o_huff, dm + g.o_quant, (uint8_t*)ctx->jpeg[JD_SCANS].p, (int16_t*)ctx->jpeg[JD_COEF].p,
                                        out, nf, g.n_restart, rows, cols, s));
         if (dst_mem == DMC_MEM_HOST) CUDA_TRY(ctx, cudaMemcpyAsync((uint8_t*)dst + fpx * f0, out, fpx * nf, cudaMemcpyDeviceToHost, s));
+        CUDA_TRY(ctx, cudaStreamSynchronize(s));     // the pageable metadata block is reused by the next group
+    }
+    return DMC_OK;
+}
+
+// ---- colour JPEG decode ------------------------------------------------------------------------------------------
+namespace {
+
+// Device scratch of the colour decoder's frames in one call: the group is as large as this allows (at least one frame,
+// at most 2048).  A 1080p frame needs about 3.6 MB at 4:2:0 and 7 MB at 4:4:4 (planes and de-stuffed scan).
+constexpr size_t kColorGroupBytes = (size_t)4 << 30;
+
+// One group of colour streams: descriptors and de-duplicated tables, packed into one metadata block
+// [ColorFrameDesc...][HuffTable...][QuantTable...][YccTables] with 16-byte aligned parts.
+struct JpegColorGroup {
+    std::vector<dmcjpeg::ColorFrameDesc> desc; JpegTablePools pools;
+    size_t scratch_bytes = 0, plane_bytes = 0, coef_blocks = 0; int n_restart = 0; uint32_t max_blocks = 0;
+    size_t o_huff = 0, o_quant = 0, o_ycc = 0, meta_bytes = 0;
+};
+
+// Parses streams f0, f0 + 1, ... into g until the group holds 2048 frames, the budget is spent or the streams end; at
+// least one frame.  Returns the number of frames taken in *nf.
+int jpeg_color_parse_group(dmc_ctx* ctx, const uint8_t* blob, const uint64_t* offsets, int f0, int n_frames, int rows, int cols, size_t out_frame_bytes,
+                           JpegColorGroup* g, int* nf) {
+    g->desc.clear(); g->pools.q.clear(); g->pools.h.clear();
+    g->scratch_bytes = g->plane_bytes = g->coef_blocks = 0; g->n_restart = 0; g->max_blocks = 0;
+    const uint64_t b0 = offsets[f0];
+    size_t used = 0;
+    int i = f0;
+    for (; i < n_frames && i - f0 < 2048; i++) {
+        const uint64_t o = offsets[i], e = offsets[i + 1];
+        if (e < o || o < b0) return fail(ctx, DMC_ERR_ARG, "dmc_jpeg_decode_color_batch: offsets must be non-decreasing");
+        dmcjpeg::ColorFrameDesc d;
+        std::string why = jpeg_parse_color_frame(blob + o, e - o, o - b0, rows, cols, g->pools, &d);
+        if (!why.empty()) return fail(ctx, DMC_ERR_TYPE, "JPEG frame " + std::to_string(i) + ": " + why);
+        if (d.scan_end - d.scan_offset >= (1ull << 28)) return fail(ctx, DMC_ERR_SIZE, "JPEG frame " + std::to_string(i) + ": scan larger than 256 MB");
+        const size_t sb = jpeg_scratch_bytes(d.scan_end - d.scan_offset), pb = (dmcjpeg::color_plane_bytes(d) + 63) & ~(size_t)63;
+        const size_t cb = d.restart_interval ? (size_t)dmcjpeg::color_blocks(d) * 128 : 0;
+        const size_t cost = sb + pb + cb + out_frame_bytes;
+        if (i > f0 && used + cost > kColorGroupBytes) break;     // (its tables stay in the pools unused; harmless)
+        used += cost;
+        d.ds_offset = g->scratch_bytes; d.plane_offset = g->plane_bytes; d.coef_offset = g->coef_blocks;
+        g->scratch_bytes += sb; g->plane_bytes += pb;
+        if (d.restart_interval) {
+            g->n_restart++; g->coef_blocks += dmcjpeg::color_blocks(d);
+            if (dmcjpeg::color_blocks(d) > g->max_blocks) g->max_blocks = dmcjpeg::color_blocks(d);
+        }
+        g->desc.push_back(d);
+    }
+    *nf = i - f0;
+    g->o_huff = (g->desc.size() * sizeof(dmcjpeg::ColorFrameDesc) + 15) & ~(size_t)15;
+    g->o_quant = (g->o_huff + g->pools.h.items.size() * sizeof(dmcjpeg::HuffTable) + 15) & ~(size_t)15;
+    g->o_ycc = (g->o_quant + g->pools.q.items.size() * sizeof(dmcjpeg::QuantTable) + 15) & ~(size_t)15;
+    g->meta_bytes = g->o_ycc + sizeof(dmcjpeg::YccTables);
+    return DMC_OK;
+}
+
+}  // namespace
+
+int dmc_jpeg_probe_color(const void* stream, size_t len, int* rows, int* cols, int* components, char* err, size_t err_len) {
+    JpegTablePools pools; dmcjpeg::ColorFrameDesc d;
+    int r = 0, c = 0, n = 0;
+    std::string why = stream ? jpeg_parse_color_frame((const uint8_t*)stream, len, 0, -1, -1, pools, &d, &r, &c, &n) : std::string("null stream");
+    if (rows) *rows = r;
+    if (cols) *cols = c;
+    if (components) *components = n;
+    if (err && err_len) { strncpy(err, why.c_str(), err_len - 1); err[err_len - 1] = 0; }
+    return why.empty() ? DMC_OK : DMC_ERR_TYPE;
+}
+
+int dmc_jpeg_decode_color_batch(dmc_ctx* ctx, const void* blob, const uint64_t* offsets, int n_frames, int rows, int cols, void* dst, int dst_mem) {
+    if (!ctx) return fail(nullptr, DMC_ERR_ARG, "null context");
+    if (!blob || !offsets || !dst || n_frames < 0 || rows <= 0 || cols <= 0 || rows > 65535 || cols > 65535) return fail(ctx, DMC_ERR_SIZE, "dmc_jpeg_decode_color_batch: bad arguments");
+    if (dst_mem != DMC_MEM_HOST && dst_mem != DMC_MEM_DEVICE) return fail(ctx, DMC_ERR_ARG, "dmc_jpeg_decode_color_batch: bad mem");
+    if (n_frames == 0) return DMC_OK;
+    CUDA_TRY(ctx, cudaSetDevice(ctx->device));
+    cudaStream_t s = ctx->stream;
+    const size_t fbytes = (size_t)rows * cols * 3;
+    const bool host_out = dst_mem == DMC_MEM_HOST;
+    JpegColorGroup g;
+    std::vector<char> meta;
+    dmcjpeg::YccTables ycc;
+    dmcjpeg::make_ycc_tables(&ycc);
+    for (int f0 = 0, nf = 0; f0 < n_frames; f0 += nf) {
+        TRY(jpeg_color_parse_group(ctx, (const uint8_t*)blob, offsets, f0, n_frames, rows, cols, host_out ? fbytes : 0, &g, &nf));
+        const uint64_t b0 = offsets[f0], b1 = offsets[f0 + nf];
+        TRY(reserve(ctx, ctx->jpeg_color[JC_BITS], (size_t)(b1 - b0) + 16));
+        TRY(reserve(ctx, ctx->jpeg_color[JC_META], g.meta_bytes));
+        TRY(reserve(ctx, ctx->jpeg_color[JC_SCANS], g.scratch_bytes + 16));
+        TRY(reserve(ctx, ctx->jpeg_color[JC_PLANES], g.plane_bytes));
+        if (g.n_restart) TRY(reserve(ctx, ctx->jpeg_color[JC_COEF], g.coef_blocks * 64 * sizeof(int16_t)));
+        uint8_t* out = (uint8_t*)dst + fbytes * f0;
+        if (host_out) { TRY(reserve(ctx, ctx->jpeg_color[JC_OUT], fbytes * nf)); out = (uint8_t*)ctx->jpeg_color[JC_OUT].p; }
+        meta.resize(g.meta_bytes);
+        memcpy(meta.data(), g.desc.data(), g.desc.size() * sizeof(dmcjpeg::ColorFrameDesc));
+        memcpy(meta.data() + g.o_huff, g.pools.h.items.data(), g.pools.h.items.size() * sizeof(dmcjpeg::HuffTable));
+        memcpy(meta.data() + g.o_quant, g.pools.q.items.data(), g.pools.q.items.size() * sizeof(dmcjpeg::QuantTable));
+        memcpy(meta.data() + g.o_ycc, &ycc, sizeof ycc);
+        CUDA_TRY(ctx, cudaMemcpyAsync(ctx->jpeg_color[JC_BITS].p, (const uint8_t*)blob + b0, (size_t)(b1 - b0), cudaMemcpyHostToDevice, s));
+        CUDA_TRY(ctx, cudaMemcpyAsync(ctx->jpeg_color[JC_META].p, meta.data(), g.meta_bytes, cudaMemcpyHostToDevice, s));
+        if (g.n_restart) CUDA_TRY(ctx, cudaMemsetAsync(ctx->jpeg_color[JC_COEF].p, 0, g.coef_blocks * 64 * sizeof(int16_t), s));
+        const char* dm = (const char*)ctx->jpeg_color[JC_META].p;
+        LAUNCH(ctx, launch_jpeg_color_decode((const uint8_t*)ctx->jpeg_color[JC_BITS].p, dm, dm + g.o_huff, dm + g.o_quant, dm + g.o_ycc,
+                                             (uint8_t*)ctx->jpeg_color[JC_SCANS].p, (uint8_t*)ctx->jpeg_color[JC_PLANES].p, (int16_t*)ctx->jpeg_color[JC_COEF].p,
+                                             out, nf, g.n_restart, g.max_blocks, rows, cols, s));
+        if (host_out) CUDA_TRY(ctx, cudaMemcpyAsync((uint8_t*)dst + fbytes * f0, out, fbytes * nf, cudaMemcpyDeviceToHost, s));
         CUDA_TRY(ctx, cudaStreamSynchronize(s));     // the pageable metadata block is reused by the next group
     }
     return DMC_OK;

@@ -85,6 +85,12 @@ namespace dmc {
 size_t jpeg_scratch_bytes(uint64_t scan_bytes);
 int launch_jpeg_decode(const uint8_t* blob, const void* desc, const void* hts, const void* qts, uint8_t* scratch, int16_t* coefs, uint8_t* dst,
                        int n, int n_restart, int H, int W, cudaStream_t s);
+// Baseline colour JPEG decoding (dmc_jpeg_color.cu) to dense BGR in dst.  desc: n ColorFrameDescs whose ds_offset points
+// into `scratch` (jpeg_scratch_bytes per frame), plane_offset into `planes` (color_plane_bytes) and, for the n_restart
+// frames with restart intervals, coef_offset into `coefs` (color_blocks * 64 int16, zero on entry); max_blocks: the
+// largest color_blocks of those frames.  ycc: the YccTables.
+int launch_jpeg_color_decode(const uint8_t* blob, const void* desc, const void* hts, const void* qts, const void* ycc, uint8_t* scratch, uint8_t* planes,
+                             int16_t* coefs, uint8_t* dst, int n, int n_restart, uint32_t max_blocks, int H, int W, cudaStream_t s);
 // Baseline grayscale JPEG encoding (dmc_jpeg_enc.cu).  Per-frame scratch of a rows x cols frame: int16 coefficients, block
 // records, packed scan words (reused by the decoder as de-stuffing scratch) and the slot the frame's stream is written to.
 // optimize: optimised Huffman tables, which take opt_bytes more per frame (symbol counts, the frame's code tables and header).

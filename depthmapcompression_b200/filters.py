@@ -216,6 +216,36 @@ def jpegDecodeGrayBatch(streams, rows, cols, dst=None, ctx=None):
     return dst
 
 
+def jpegProbeColor(stream):
+    """dmc_jpeg_probe_color (host only): -> (rows, cols, components) of a stream jpegDecodeColorBatch can decode
+    (components 1 or 3); raises DmcError with the reason otherwise (malformed / progressive / CMYK / RGB ...)."""
+    a = np.frombuffer(stream, np.uint8) if not isinstance(stream, np.ndarray) else np.ascontiguousarray(stream).ravel()
+    r, c, n = C.c_int(), C.c_int(), C.c_int(); err = C.create_string_buffer(256)
+    rc = lib.dmc_jpeg_probe_color(C.c_void_p(a.ctypes.data if a.size else None), a.size, C.byref(r), C.byref(c), C.byref(n), err, 256)
+    if rc != capi.DMC_OK:
+        raise DmcError(rc, err.value.decode())
+    return r.value, c.value, n.value
+
+
+def jpegDecodeColorBatch(streams, rows, cols, dst=None, ctx=None):
+    """Baseline colour (or one-component) JPEG bitstreams (list of bytes, or a (blob, offsets) pair) -> [n, rows, cols, 3]
+    uint8 BGR, bit-identical to cv2.imdecode(buf, cv2.IMREAD_COLOR | cv2.IMREAD_IGNORE_ORIENTATION).  dst: None (new host
+    array), a host array of that shape, or a device pointer (int) -- a device batch that renderViewBatch takes as its
+    texture tuple (pointer, n, rows, cols)."""
+    ctx = ctx or default_context()
+    blob, offsets = streams if isinstance(streams, tuple) else pack_streams(streams)
+    n = len(offsets) - 1
+    device = isinstance(dst, int)
+    if dst is None:
+        dst = np.empty((n, max(rows, 0), max(cols, 0), 3), np.uint8)
+    elif not device and (dst.dtype != np.uint8 or dst.size != n * rows * cols * 3 or not dst.flags.c_contiguous):
+        raise DmcError(capi.DMC_ERR_SIZE, "jpegDecodeColorBatch: dst must be a contiguous uint8 array of n x rows x cols x 3")
+    dp = C.c_void_p(dst if device else dst.ctypes.data)
+    ctx.check(lib.dmc_jpeg_decode_color_batch(ctx.h, C.c_void_p(blob.ctypes.data), C.c_void_p(offsets.ctypes.data), n, rows, cols, dp,
+                                              MEM_DEVICE if device else MEM_HOST))
+    return dst
+
+
 def _jpeg_flags(optimize):
     return capi.JPEG_OPTIMIZE_HUFFMAN if optimize else 0
 

@@ -192,6 +192,23 @@ int dmc_chain_batch_jpeg(dmc_ctx* ctx, const void* blob, const uint64_t* offsets
  * not (DMC_ERR_TYPE + message in err, may be NULL).  Needs no context and no GPU.  Malformed, truncated or hostile
  * streams (bad segment lengths, Huffman tables that are not prefix codes, ...) are refused here, never crashed on. */
 int dmc_jpeg_probe(const void* stream, size_t len, int* rows, int* cols, char* err, size_t err_len);
+/* Frame-parallel baseline colour JPEG decode.  The output of frame i is a dense rows x cols 8UC3 BGR image equal to
+ * cv::imdecode(buf, IMREAD_COLOR | IMREAD_IGNORE_ORIENTATION) with libjpeg-turbo 3.1.2 (cv2 4.13): islow IDCT, fancy
+ * upsampling, libjpeg's YCbCr -> RGB tables; pixels as stored, so for streams without an EXIF orientation tag (cv2's own
+ * streams never carry one) it is plain IMREAD_COLOR.  Accepted: SOF0 / SOF1 at 8-bit precision with three components in
+ * one interleaved scan, chroma sampled 1x1 and luma 1x1, 2x1, 2x2, 1x2 or 4x1 (4:4:4, 4:2:2, 4:2:0, 4:4:0, 4:1:1: every
+ * sampling cv::imencode writes), standard or optimised Huffman tables, with or without restart intervals; and
+ * one-component streams, which decode to B = G = R = Y.  Refused with a reason (DMC_ERR_TYPE): progressive, arithmetic,
+ * lossless, 12-bit, non-interleaved multi-scan colour, CMYK / YCCK, and streams libjpeg treats as RGB (Adobe transform 0
+ * without JFIF, or component IDs 'R' 'G' 'B' without JFIF or Adobe markers).  blob / offsets as for
+ * dmc_jpeg_decode_gray_batch; one batch may mix samplings, table kinds and component counts at one rows x cols.
+ * dst receives n_frames x rows x cols x 3 bytes (dst_mem: host or device; a device dst is a texture batch that
+ * dmc_render_view_batch takes as it is).  Returns when dst is valid. */
+int dmc_jpeg_decode_color_batch(dmc_ctx* ctx, const void* blob, const uint64_t* offsets, int n_frames, int rows, int cols,
+                                void* dst, int dst_mem);
+/* Host-only: whether dmc_jpeg_decode_color_batch can decode this stream (DMC_OK, with its size and component count, 1 or
+ * 3) or why not (DMC_ERR_TYPE + message in err, may be NULL).  Needs no context and no GPU. */
+int dmc_jpeg_probe_color(const void* stream, size_t len, int* rows, int* cols, int* components, char* err, size_t err_len);
 
 /* ---- encode (SURVEY.md 8f-5) ----------------------------------------------------------------------------------- */
 /* Baseline JPEG encoding of 8UC1 frames, byte-identical to cv::imencode(".jpg", img, {IMWRITE_JPEG_QUALITY, quality}) with

@@ -287,3 +287,19 @@ inline double structuralSimilarity(const Mat& a, const Mat& b)
 	                  "structuralSimilarity");
 	return mssim;
 }
+
+// Baseline colour JPEG decoding on the GPU: dst = cv::imdecode(buf, IMREAD_COLOR), a CV_8UC3 BGR image, bit for bit
+// (libjpeg-turbo's islow IDCT, fancy upsampling and colour conversion; one-component streams give B = G = R = Y).  Streams
+// the decoder does not take (progressive, arithmetic, 12-bit, CMYK, RGB-coded, ...) throw with the reason.
+inline void jpegDecodeColor(const vector<uchar>& buf, Mat& dst)
+{
+	int rows = 0, cols = 0, nc = 0;
+	char why[256] = {0};
+	if (dmc_jpeg_probe_color(buf.empty() ? 0 : buf.data(), buf.size(), &rows, &cols, &nc, why, sizeof why) != DMC_OK)
+		dmc_dropin::require(false, (std::string("jpegDecodeColor: ") + why).c_str());
+	dst.create(rows, cols, CV_8UC3);
+	Mat out = dst.isContinuous() ? dst : Mat(rows, cols, CV_8UC3);
+	const uint64_t off[2] = {0, (uint64_t)buf.size()};
+	dmc_dropin::check(dmc_jpeg_decode_color_batch(dmc_dropin::context(), buf.data(), off, 1, rows, cols, out.data, DMC_MEM_HOST), "jpegDecodeColor");
+	if (out.data != dst.data) out.copyTo(dst);
+}
