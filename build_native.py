@@ -16,7 +16,7 @@ ROOT = os.path.dirname(os.path.abspath(__file__))
 HERE = os.path.join(ROOT, "depthmapcompression_b200")
 CSRC = os.path.join(HERE, "csrc")
 LIB = os.path.join(HERE, "libdmc_b200.so")
-SOURCES = ["dmc_kernels_8u.cu", "dmc_bwrf8u_h2.cu", "dmc_bwrf8u_c3_h2.cu", "dmc_joint_bwrf.cu", "dmc_front8u.cu", "dmc_kernels_32f.cu", "dmc_prepare.cu", "dmc_brf.cu", "dmc_bwrf32f_tiled.cu", "dmc_jpeg.cu", "dmc_jpeg_color.cu", "dmc_jpeg_enc.cu", "dmc_metrics.cu", "dmc_hostlink.cu", "dmc_render.cu", "dmc_capi.cu"]
+SOURCES = ["dmc_kernels_8u.cu", "dmc_bwrf8u_h2.cu", "dmc_bwrf8u_c3_h2.cu", "dmc_joint_bwrf.cu", "dmc_front8u.cu", "dmc_kernels_32f.cu", "dmc_prepare.cu", "dmc_brf.cu", "dmc_bwrf32f_tiled.cu", "dmc_jpeg.cu", "dmc_jpeg_color.cu", "dmc_jpeg_enc.cu", "dmc_jpeg_color_enc.cu", "dmc_metrics.cu", "dmc_hostlink.cu", "dmc_render.cu", "dmc_capi.cu"]
 NVCC_FLAGS = ["-gencode", "arch=compute_100a,code=sm_100a", "-O3", "-lineinfo", "-fmad=false", "-std=c++17",
               "-Xcompiler", "-fPIC", "-Xcompiler", "-O2", "--shared", "-Xptxas", "-v", "--threads", "0"]
 

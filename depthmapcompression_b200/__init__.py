@@ -11,5 +11,5 @@ from .capi import (FULL_KERNEL, FULL_KERNEL_PAIR, SEPARABLE_KERNEL, FILL_DISPARI
 from .filters import (Context, PostFilterSet, binalyWeightedRangeFilter, jointBinalyWeightedRangeFilter, blurRemoveMinMax, blurRemoveMinMaxBase,  # noqa: F401
                       maxFilter, minFilter, boundaryReconstructionFilter, minmaxBoundaryReconstructionFilter, smallGaussianBlur, medianBlur,
                       disp8U2depth32F, depth32F2disp8U, depth16U2disp8U, disp16S2depth16U, fillOcclusion,
-                      reprojectXYZ, transpose, default_context, jpegDecodeGrayBatch, jpegProbe, jpegDecodeColorBatch, jpegProbeColor, jpegEncodeGrayBatch, jpegEncodeBound, degradeJPEG, frameSSE, frameSSIM, psnrFromSSE, jpegRateDistortion, jpegViewRateDistortion, boundaryReconstructionFilterBatch, brf_params, prepareDisparityBatch, renderViewBatch, pack_streams, multi_chain_batch, FrameBatchScheduler, hostlink_probe,
+                      reprojectXYZ, transpose, default_context, jpegDecodeGrayBatch, jpegProbe, jpegDecodeColorBatch, jpegProbeColor, jpegEncodeGrayBatch, jpegEncodeBound, degradeJPEG, jpegEncodeColorBatch, jpegEncodeColorBound, degradeJPEGColor, frameSSE, frameSSIM, psnrFromSSE, jpegRateDistortion, jpegViewRateDistortion, boundaryReconstructionFilterBatch, brf_params, prepareDisparityBatch, renderViewBatch, pack_streams, multi_chain_batch, FrameBatchScheduler, hostlink_probe,
                       projectPointsSimple, projectImagefromXYZ, fillSmallHole, pinned_empty, pinned_free, host_register, host_unregister)

@@ -13,6 +13,7 @@ DMC_OK, DMC_UNSUPPORTED = 0, 1
 DMC_ERR_TYPE, DMC_ERR_SIZE, DMC_ERR_CUDA, DMC_ERR_ARG = -1, -2, -3, -4
 MEM_HOST, MEM_DEVICE = 0, 1
 JPEG_OPTIMIZE_HUFFMAN = 1
+DMC_JPEG_SAMPLING_444, DMC_JPEG_SAMPLING_422, DMC_JPEG_SAMPLING_420, DMC_JPEG_SAMPLING_440, DMC_JPEG_SAMPLING_411 = 0x111111, 0x211111, 0x221111, 0x121111, 0x411111
 CV_8U, CV_16U, CV_16S, CV_32F, CV_64F = 0, 2, 3, 5, 6
 FULL_KERNEL, FULL_KERNEL_PAIR, SEPARABLE_KERNEL = 0, 1, 2       # filter.h:23-28
 FILL_DISPARITY, FILL_DEPTH = 0, 1                               # util.h:19-23
@@ -30,7 +31,7 @@ EXPORTS = [
     "dmc_small_gaussian", "dmc_median_blur",
     "dmc_disp8u2depth32f", "dmc_depth32f2disp8u", "dmc_depth16u2disp8u", "dmc_disp16s2depth16u",
     "dmc_fill_occlusion", "dmc_reproject_xyz", "dmc_transpose",
-    "dmc_chain_batch_jpeg", "dmc_jpeg_probe", "dmc_jpeg_decode_color_batch", "dmc_jpeg_probe_color", "dmc_jpeg_encode_bound", "dmc_jpeg_encode_gray_batch", "dmc_jpeg_degrade_gray_batch", "dmc_jpeg_encode_bound_ex", "dmc_jpeg_encode_gray_batch_ex", "dmc_jpeg_degrade_gray_batch_ex", "dmc_split_bgr_line_interleave", "dmc_project_points", "dmc_project_image_from_xyz", "dmc_fill_small_hole", "dmc_hostlink_probe", "dmc_release_device", "dmc_set_gateway", "dmc_get_gateway", "dmc_sched_get_routing",
+    "dmc_chain_batch_jpeg", "dmc_jpeg_probe", "dmc_jpeg_decode_color_batch", "dmc_jpeg_probe_color", "dmc_jpeg_encode_bound", "dmc_jpeg_encode_gray_batch", "dmc_jpeg_degrade_gray_batch", "dmc_jpeg_encode_bound_ex", "dmc_jpeg_encode_gray_batch_ex", "dmc_jpeg_degrade_gray_batch_ex", "dmc_jpeg_encode_color_bound", "dmc_jpeg_encode_color_batch", "dmc_jpeg_degrade_color_batch", "dmc_split_bgr_line_interleave", "dmc_project_points", "dmc_project_image_from_xyz", "dmc_fill_small_hole", "dmc_hostlink_probe", "dmc_release_device", "dmc_set_gateway", "dmc_get_gateway", "dmc_sched_get_routing",
     "dmc_sse_gray_batch", "dmc_psnr_from_sse", "dmc_jpeg_rd_sweep", "dmc_jpeg_view_rd_sweep",
     "dmc_brf_batch", "dmc_jpeg_rd_sweep_ex", "dmc_jpeg_view_rd_sweep_ex",
     "dmc_prepare_disp_batch", "dmc_render_view_batch",
@@ -98,6 +99,9 @@ def _load():
         "dmc_jpeg_encode_bound_ex": (I, [I, I, I, C.POINTER(C.c_uint64)]),
         "dmc_jpeg_encode_gray_batch_ex": (I, [P, P, I, I, I, I, I, I, P, I, C.c_uint64, C.POINTER(C.c_uint64)]),
         "dmc_jpeg_degrade_gray_batch_ex": (I, [P, P, P, I, I, I, I, I, I, C.POINTER(C.c_uint64)]),
+        "dmc_jpeg_encode_color_bound": (I, [I, I, I, C.POINTER(C.c_uint64)]),
+        "dmc_jpeg_encode_color_batch": (I, [P, P, I, I, I, I, I, I, P, I, C.c_uint64, C.POINTER(C.c_uint64)]),
+        "dmc_jpeg_degrade_color_batch": (I, [P, P, P, I, I, I, I, I, I, C.POINTER(C.c_uint64)]),
         "dmc_sse_gray_batch": (I, [P, P, P, I, I, I, I, C.POINTER(C.c_uint64)]),
         "dmc_psnr_from_sse": (D, [C.c_uint64, C.c_uint64]),
         "dmc_jpeg_rd_sweep": (I, [P, P, I, I, I, I, C.POINTER(I), I, I, C.POINTER(DmcChainParams), C.POINTER(C.c_uint64), C.POINTER(C.c_uint64), C.POINTER(C.c_uint64)]),

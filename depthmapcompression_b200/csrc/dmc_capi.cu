@@ -4,6 +4,7 @@
 #include "../../include/dmc_c.h"
 #include "dmc_common.cuh"
 #include "dmc_jpeg_enc_core.h"
+#include "dmc_jpeg_color_enc_core.h"
 #include "dmc_kernels.cuh"
 
 #include <limits.h>
@@ -64,8 +65,8 @@ struct dmc_ctx {
     Buf jpeg_color[JC_COUNT];
     Buf rd[RD_COUNT];
     Buf vs[VS_COUNT];
-    Buf jpeg_enc[11];            // JPEG encode: tables, staged frames, coefficients, block records, scan words, slots, lengths + offsets, staged output, decoder tables + descriptors,
-                                 // optimised-table scratch, per-frame decoder Huffman tables
+    Buf jpeg_enc[12];            // JPEG encode: tables, staged frames, coefficients, block records, scan words, slots, lengths + offsets, staged output, decoder tables + descriptors,
+                                 // optimised-table scratch, per-frame decoder Huffman tables, colour decoder planes
     // optional per-stage CUDA-event timing of the chain (bench.py's live roofline measurement)
     int lanes = 1;               // concurrent frame groups in the device-resident batch path
     int profile_mask = 0;
@@ -1106,7 +1107,7 @@ namespace {
 // frame needs about 26 MB (slot 13.4 MB, scan words 6.7 MB, coefficients 4.1 MB, staged frame).
 constexpr size_t kEncGroupBytes = (size_t)4 << 30;
 
-enum { JE_TABS, JE_SRC, JE_COEF, JE_INFO, JE_WORDS, JE_SLOTS, JE_LENS, JE_OUT, JE_DEC, JE_OPT, JE_HUFF };
+enum { JE_TABS, JE_SRC, JE_COEF, JE_INFO, JE_WORDS, JE_SLOTS, JE_LENS, JE_OUT, JE_DEC, JE_OPT, JE_HUFF, JE_PLANES };
 
 // Checks the arguments shared by the encode entry points, uploads the encoder tables and returns the group size.
 int jpeg_enc_prepare(dmc_ctx* ctx, const char* what, int rows, int cols, int quality, int flags, int mem_a, int mem_b, int* group) {
@@ -1248,6 +1249,156 @@ int dmc_jpeg_degrade_gray_batch_ex(dmc_ctx* ctx, const void* src, void* dst, int
 
 int dmc_jpeg_degrade_gray_batch(dmc_ctx* ctx, const void* src, void* dst, int n_frames, int rows, int cols, int quality, int mem, uint64_t* bytes) {
     return dmc_jpeg_degrade_gray_batch_ex(ctx, src, dst, n_frames, rows, cols, quality, 0, mem, bytes);
+}
+
+// ---- colour JPEG encode --------------------------------------------------------------------------------------------------
+int dmc_jpeg_encode_color_bound(int rows, int cols, int sampling, uint64_t* bytes) {
+    if (!bytes) return fail(nullptr, DMC_ERR_ARG, "dmc_jpeg_encode_color_bound: null bytes");
+    int hy, vy;
+    if (!dmcjpeg::color_sampling_factors(sampling, &hy, &vy)) return fail(nullptr, DMC_ERR_ARG, "colour JPEG encode: unknown sampling " + std::to_string(sampling));
+    if (rows <= 0 || cols <= 0 || rows > 65535 || cols > 65535) return fail(nullptr, DMC_ERR_SIZE, "colour JPEG encode: frame size must be 1..65535 x 1..65535");
+    *bytes = dmcjpeg::jpeg_encode_color_bound(rows, cols, hy, vy);
+    if (*bytes > dmcjpeg::kEncMaxStreamBytes) return fail(nullptr, DMC_ERR_SIZE, "colour JPEG encode: the worst-case stream of a " + std::to_string(rows) + " x " + std::to_string(cols) + " frame exceeds 256 MB");
+    return DMC_OK;
+}
+
+namespace {
+
+// The decoder's view of the encoder's header: the ColorFrameDesc template (geometry, table indices), the tables it
+// refers to (four Huffman tables; one quantisation table when quality makes K.1 and K.2 equal, as at 100, else two),
+// and the component-plane bytes of one frame.
+struct ColorDecodeTemplate { dmcjpeg::ColorFrameDesc d; JpegTablePools pools; uint64_t plane_bytes = 0; };
+
+// The colour counterpart of jpeg_enc_prepare: checks the shared arguments, uploads the encoder tables and returns the luma
+// factors and the group size.  dec != nullptr: also parses the header into *dec, and the group holds the planes too.
+int jpeg_color_enc_prepare(dmc_ctx* ctx, const char* what, int rows, int cols, int quality, int sampling, int mem_a, int mem_b,
+                           int* hy, int* vy, int* group, ColorDecodeTemplate* dec) {
+    if (quality < 0 || quality > 100) return fail(ctx, DMC_ERR_ARG, std::string(what) + ": quality must be in 0..100");
+    if ((mem_a != DMC_MEM_HOST && mem_a != DMC_MEM_DEVICE) || (mem_b != DMC_MEM_HOST && mem_b != DMC_MEM_DEVICE)) return fail(ctx, DMC_ERR_ARG, std::string(what) + ": bad mem");
+    uint64_t bound;
+    const int rc = dmc_jpeg_encode_color_bound(rows, cols, sampling, &bound);
+    if (rc != DMC_OK) return fail(ctx, rc, std::string(what) + ": " + g_err);
+    dmcjpeg::color_sampling_factors(sampling, hy, vy);
+    dmcjpeg::EncColorTables t;
+    dmcjpeg::make_enc_color_tables(quality, rows, cols, *hy, *vy, &t);
+    if (dec) {
+        const std::string why = jpeg_parse_color_frame(t.header, dmcjpeg::kColorEncHeaderBytes, 0, rows, cols, dec->pools, &dec->d);
+        if (!why.empty() || dec->pools.h.items.size() != 4 || dec->pools.q.items.size() > 2 || dec->d.nc != 3 || dec->d.hy != *hy || dec->d.vy != *vy)
+            return fail(ctx, DMC_ERR_TYPE, std::string(what) + ": encoder header does not parse: " + why);
+        dec->plane_bytes = (dmcjpeg::color_plane_bytes(dec->d) + 63) & ~(uint64_t)63;
+    }
+    CUDA_TRY(ctx, cudaSetDevice(ctx->device));
+    const JpegEncLayout l = jpeg_color_enc_layout(rows, cols, *hy, *vy);
+    const size_t per = l.coef_bytes + l.info_bytes + l.word_bytes + l.slot_bytes + 2 * (size_t)rows * cols * 3 + (dec ? dec->plane_bytes : 0);
+    *group = chunk_frames(kEncGroupBytes, per, INT_MAX, 2048, false);
+    TRY(reserve(ctx, ctx->jpeg_enc[JE_TABS], sizeof t));
+    CUDA_TRY(ctx, cudaMemcpyAsync(ctx->jpeg_enc[JE_TABS].p, &t, sizeof t, cudaMemcpyHostToDevice, ctx->stream));
+    CUDA_TRY(ctx, cudaStreamSynchronize(ctx->stream));          // (t lives on this stack frame)
+    return DMC_OK;
+}
+
+// Encodes frames [f0, f0 + nf) of src into the slots (lengths in JE_LENS); desc: also write the decoder's ColorFrameDescs
+// there, from the template tmpl, with planes plane_bytes apart.
+int jpeg_color_enc_group(dmc_ctx* ctx, const uint8_t* src, int src_mem, int f0, int nf, int rows, int cols, int hy, int vy, void* desc,
+                         const dmcjpeg::ColorFrameDesc* tmpl, uint64_t plane_bytes) {
+    cudaStream_t s = ctx->stream;
+    const size_t fbytes = (size_t)rows * cols * 3;
+    const JpegEncLayout l = jpeg_color_enc_layout(rows, cols, hy, vy);
+    const uint8_t* dsrc = src + fbytes * f0;
+    if (src_mem == DMC_MEM_HOST) {
+        TRY(reserve(ctx, ctx->jpeg_enc[JE_SRC], fbytes * nf));
+        CUDA_TRY(ctx, cudaMemcpyAsync(ctx->jpeg_enc[JE_SRC].p, dsrc, fbytes * nf, cudaMemcpyHostToDevice, s));
+        dsrc = (const uint8_t*)ctx->jpeg_enc[JE_SRC].p;
+    }
+    TRY(reserve(ctx, ctx->jpeg_enc[JE_COEF], l.coef_bytes * nf));
+    TRY(reserve(ctx, ctx->jpeg_enc[JE_INFO], l.info_bytes * nf));
+    TRY(reserve(ctx, ctx->jpeg_enc[JE_WORDS], l.word_bytes * nf));
+    TRY(reserve(ctx, ctx->jpeg_enc[JE_SLOTS], l.slot_bytes * nf));
+    TRY(reserve(ctx, ctx->jpeg_enc[JE_LENS], (size_t)nf * (sizeof(uint32_t) + sizeof(uint64_t)) + 16));
+    LAUNCH(ctx, launch_jpeg_color_encode(dsrc, ctx->jpeg_enc[JE_TABS].p, ctx->jpeg_enc[JE_COEF].p, ctx->jpeg_enc[JE_INFO].p, ctx->jpeg_enc[JE_WORDS].p,
+                                         (uint8_t*)ctx->jpeg_enc[JE_SLOTS].p, (uint32_t*)ctx->jpeg_enc[JE_LENS].p, desc, tmpl, plane_bytes, nf, rows, cols, hy, vy, s));
+    return DMC_OK;
+}
+
+}  // namespace
+
+// As dmc_jpeg_encode_gray_batch: group by group into the slots, then the gather kernel places the streams.
+int dmc_jpeg_encode_color_batch(dmc_ctx* ctx, const void* src, int src_mem, int n_frames, int rows, int cols, int quality, int sampling,
+                                void* blob, int blob_mem, uint64_t capacity, uint64_t* offsets) {
+    if (!ctx) return fail(nullptr, DMC_ERR_ARG, "null context");
+    if (!offsets || n_frames < 0 || (n_frames > 0 && (!src || !blob))) return fail(ctx, DMC_ERR_SIZE, "dmc_jpeg_encode_color_batch: bad arguments");
+    int hy, vy, group;
+    TRY(jpeg_color_enc_prepare(ctx, "dmc_jpeg_encode_color_batch", rows, cols, quality, sampling, src_mem, blob_mem, &hy, &vy, &group, nullptr));
+    offsets[0] = 0;
+    cudaStream_t s = ctx->stream;
+    const JpegEncLayout l = jpeg_color_enc_layout(rows, cols, hy, vy);
+    std::vector<uint32_t> lens; std::vector<uint64_t> offs;
+    for (int f0 = 0; f0 < n_frames; f0 += group) {
+        const int nf = n_frames - f0 < group ? n_frames - f0 : group;
+        TRY(jpeg_color_enc_group(ctx, (const uint8_t*)src, src_mem, f0, nf, rows, cols, hy, vy, nullptr, nullptr, 0));
+        lens.resize(nf); offs.resize(nf);
+        CUDA_TRY(ctx, cudaMemcpyAsync(lens.data(), ctx->jpeg_enc[JE_LENS].p, nf * sizeof(uint32_t), cudaMemcpyDeviceToHost, s));
+        CUDA_TRY(ctx, cudaStreamSynchronize(s));
+        const uint64_t base = offsets[f0];
+        uint64_t end = base, longest = 0;
+        for (int i = 0; i < nf; i++) { offs[i] = end - base; end += lens[i]; if (lens[i] > longest) longest = lens[i]; }
+        if (end > capacity)
+            return fail(ctx, DMC_ERR_SIZE, "dmc_jpeg_encode_color_batch: the streams of frames 0.." + std::to_string(f0 + nf - 1) + " need " + std::to_string(end) +
+                                               " bytes, capacity is " + std::to_string(capacity));
+        for (int i = 0; i < nf; i++) offsets[f0 + i + 1] = base + offs[i] + lens[i];
+        uint64_t* d_offs = enc_offs(ctx, nf);
+        CUDA_TRY(ctx, cudaMemcpyAsync(d_offs, offs.data(), nf * sizeof(uint64_t), cudaMemcpyHostToDevice, s));
+        uint8_t* dst = (uint8_t*)blob + base;
+        if (blob_mem == DMC_MEM_HOST) { TRY(reserve(ctx, ctx->jpeg_enc[JE_OUT], end - base)); dst = (uint8_t*)ctx->jpeg_enc[JE_OUT].p; }
+        LAUNCH(ctx, launch_jpeg_enc_gather((const uint8_t*)ctx->jpeg_enc[JE_SLOTS].p, l.slot_bytes, (const uint32_t*)ctx->jpeg_enc[JE_LENS].p, d_offs, dst, nf, longest, s));
+        if (blob_mem == DMC_MEM_HOST) CUDA_TRY(ctx, cudaMemcpyAsync((uint8_t*)blob + base, dst, end - base, cudaMemcpyDeviceToHost, s));
+        CUDA_TRY(ctx, cudaStreamSynchronize(s));     // offs is reused by the next group
+    }
+    return DMC_OK;
+}
+
+// Encode into the slots, then decode every slot in place with the decoder of dmc_jpeg_decode_color_batch.  Its tables
+// come from parsing the encoder's 623-byte header once; the encoder writes each frame's ColorFrameDesc from that parse.
+// The decoder de-stuffs each scan into the frame's scan words: it writes the de-stuffed scan (at most the unstuffed
+// scan, blocks * 1660 bits) and at most 12 bytes of padding words behind it, which jpeg_color_enc_layout's word_bytes
+// holds.  The component planes take one more scratch region per group.
+int dmc_jpeg_degrade_color_batch(dmc_ctx* ctx, const void* src, void* dst, int n_frames, int rows, int cols, int quality, int sampling, int mem, uint64_t* bytes) {
+    if (!ctx) return fail(nullptr, DMC_ERR_ARG, "null context");
+    if (n_frames < 0 || (n_frames > 0 && (!src || !dst))) return fail(ctx, DMC_ERR_SIZE, "dmc_jpeg_degrade_color_batch: bad arguments");
+    int hy, vy, group;
+    ColorDecodeTemplate dec;
+    TRY(jpeg_color_enc_prepare(ctx, "dmc_jpeg_degrade_color_batch", rows, cols, quality, sampling, mem, mem, &hy, &vy, &group, &dec));
+    if (n_frames == 0) return DMC_OK;
+    cudaStream_t s = ctx->stream;
+    const size_t fbytes = (size_t)rows * cols * 3;
+    // decoder metadata: [4 HuffTables][1 or 2 QuantTables][YccTables][ColorFrameDesc per frame], 16-byte aligned parts
+    const size_t o_q = 4 * sizeof(dmcjpeg::HuffTable), o_ycc = (o_q + 2 * sizeof(dmcjpeg::QuantTable) + 15) & ~(size_t)15;
+    const size_t o_desc = (o_ycc + sizeof(dmcjpeg::YccTables) + 15) & ~(size_t)15;
+    dmcjpeg::YccTables ycc;
+    dmcjpeg::make_ycc_tables(&ycc);
+    TRY(reserve(ctx, ctx->jpeg_enc[JE_DEC], o_desc + (size_t)group * sizeof(dmcjpeg::ColorFrameDesc)));
+    TRY(reserve(ctx, ctx->jpeg_enc[JE_PLANES], (size_t)group * dec.plane_bytes));
+    char* dm = (char*)ctx->jpeg_enc[JE_DEC].p;
+    CUDA_TRY(ctx, cudaMemcpyAsync(dm, dec.pools.h.items.data(), o_q, cudaMemcpyHostToDevice, s));
+    CUDA_TRY(ctx, cudaMemcpyAsync(dm + o_q, dec.pools.q.items.data(), dec.pools.q.items.size() * sizeof(dmcjpeg::QuantTable), cudaMemcpyHostToDevice, s));
+    CUDA_TRY(ctx, cudaMemcpyAsync(dm + o_ycc, &ycc, sizeof ycc, cudaMemcpyHostToDevice, s));
+    std::vector<uint32_t> lens;
+    for (int f0 = 0; f0 < n_frames; f0 += group) {
+        const int nf = n_frames - f0 < group ? n_frames - f0 : group;
+        TRY(jpeg_color_enc_group(ctx, (const uint8_t*)src, mem, f0, nf, rows, cols, hy, vy, dm + o_desc, &dec.d, dec.plane_bytes));
+        uint8_t* out = (uint8_t*)dst + fbytes * f0;
+        if (mem == DMC_MEM_HOST) { TRY(reserve(ctx, ctx->jpeg_enc[JE_OUT], fbytes * nf)); out = (uint8_t*)ctx->jpeg_enc[JE_OUT].p; }
+        LAUNCH(ctx, launch_jpeg_color_decode((const uint8_t*)ctx->jpeg_enc[JE_SLOTS].p, dm + o_desc, dm, dm + o_q, dm + o_ycc, (uint8_t*)ctx->jpeg_enc[JE_WORDS].p,
+                                             (uint8_t*)ctx->jpeg_enc[JE_PLANES].p, nullptr, out, nf, 0, 0, rows, cols, s));
+        if (mem == DMC_MEM_HOST) CUDA_TRY(ctx, cudaMemcpyAsync((uint8_t*)dst + fbytes * f0, out, fbytes * nf, cudaMemcpyDeviceToHost, s));
+        if (bytes) {
+            lens.resize(nf);
+            CUDA_TRY(ctx, cudaMemcpyAsync(lens.data(), ctx->jpeg_enc[JE_LENS].p, nf * sizeof(uint32_t), cudaMemcpyDeviceToHost, s));
+        }
+        CUDA_TRY(ctx, cudaStreamSynchronize(s));
+        if (bytes) for (int i = 0; i < nf; i++) bytes[f0 + i] = lens[i];
+    }
+    return DMC_OK;
 }
 
 // ---- distortion and the rate-distortion sweep ----------------------------------------------------------------------------

@@ -82,15 +82,17 @@ static const uint8_t kStdAcVals[162] = {
     0xb2, 0xb3, 0xb4, 0xb5, 0xb6, 0xb7, 0xb8, 0xb9, 0xba, 0xc2, 0xc3, 0xc4, 0xc5, 0xc6, 0xc7, 0xc8, 0xc9, 0xca, 0xd2, 0xd3, 0xd4, 0xd5, 0xd6,
     0xd7, 0xd8, 0xd9, 0xda, 0xe1, 0xe2, 0xe3, 0xe4, 0xe5, 0xe6, 0xe7, 0xe8, 0xe9, 0xea, 0xf1, 0xf2, 0xf3, 0xf4, 0xf5, 0xf6, 0xf7, 0xf8, 0xf9, 0xfa};
 
-// cv2 clamps the quality to [0, 100]; libjpeg treats 0 as 1.  quant[] in natural order.
-inline void quality_table(int quality, uint8_t quant[64]) {
+// cv2 clamps the quality to [0, 100]; libjpeg treats 0 as 1.  std[] and quant[] in natural order.
+inline void scale_quant_table(const uint8_t* std, int quality, uint8_t quant[64]) {
     int q = quality < 1 ? 1 : (quality > 100 ? 100 : quality);
     const int scale = q < 50 ? 5000 / q : 200 - 2 * q;
     for (int i = 0; i < 64; i++) {
-        const int v = ((int)std_luminance_quant()[i] * scale + 50) / 100;
+        const int v = ((int)std[i] * scale + 50) / 100;
         quant[i] = (uint8_t)(v < 1 ? 1 : (v > 255 ? 255 : v));
     }
 }
+
+inline void quality_table(int quality, uint8_t quant[64]) { scale_quant_table(std_luminance_quant(), quality, quant); }
 
 // jcdctmgr's canonical code assignment (jpeg_make_c_derived_tbl): (length << 16) | code per symbol.
 inline void make_code_table(const uint8_t bits[16], const uint8_t* vals, uint32_t* out, int nout) {
@@ -102,11 +104,13 @@ inline void make_code_table(const uint8_t bits[16], const uint8_t* vals, uint32_
     }
 }
 
+// SOI and the JFIF 1.1 APP0 segment cv2 writes (no thumbnail, 1:1 aspect)
+static const uint8_t kSoiApp0[20] = {0xFF, 0xD8, 0xFF, 0xE0, 0x00, 0x10, 'J', 'F', 'I', 'F', 0x00, 0x01, 0x01, 0x00, 0x00, 0x01, 0x00, 0x01, 0x00, 0x00};
+
 // The 328 header bytes cv2.imencode writes for an 8UC1 image.
 inline void build_header(const uint8_t quant[64], int rows, int cols, uint8_t* h) {
-    static const uint8_t app0[20] = {0xFF, 0xD8, 0xFF, 0xE0, 0x00, 0x10, 'J', 'F', 'I', 'F', 0x00, 0x01, 0x01, 0x00, 0x00, 0x01, 0x00, 0x01, 0x00, 0x00};
     uint8_t* p = h;
-    memcpy(p, app0, 20); p += 20;
+    memcpy(p, kSoiApp0, 20); p += 20;
     *p++ = 0xFF; *p++ = 0xDB; *p++ = 0x00; *p++ = 0x43; *p++ = 0x00;
     for (int k = 0; k < 64; k++) *p++ = quant[zigzag_to_natural(k)];
     const uint8_t sof[13] = {0xFF, 0xC0, 0x00, 0x0B, 0x08, (uint8_t)(rows >> 8), (uint8_t)rows, (uint8_t)(cols >> 8), (uint8_t)cols, 0x01, 0x01, 0x11, 0x00};

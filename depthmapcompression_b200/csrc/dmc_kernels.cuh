@@ -102,6 +102,14 @@ JpegEncLayout jpeg_enc_layout(int rows, int cols, bool optimize = false);
 // then refer to the HuffTable pair huff[2 f], huff[2 f + 1], which the encoder writes when huff != nullptr.
 int launch_jpeg_encode(const uint8_t* src, const void* tabs, void* coefs, void* info, void* words, uint8_t* slots, uint32_t* lens, void* desc,
                        int n, int H, int W, cudaStream_t s, void* opt = nullptr, void* huff = nullptr);
+// Baseline colour JPEG encoding (dmc_jpeg_color_enc.cu) of n dense 8UC3 BGR frames with luma factors hy x vy: the per-frame
+// scratch has the gray encoder's parts (opt_bytes = 0), sized by jpeg_color_enc_layout.  tabs: a device EncColorTables.
+// With desc != nullptr the encoder also writes the ColorFrameDesc that decodes slot f in place: *tmpl (the header's
+// parse: geometry and table indices) with scan_offset / scan_end relative to `slots`, ds_offset relative to `words` and
+// plane_offset = f * plane_bytes.
+JpegEncLayout jpeg_color_enc_layout(int rows, int cols, int hy, int vy);
+int launch_jpeg_color_encode(const uint8_t* src, const void* tabs, void* coefs, void* info, void* words, uint8_t* slots, uint32_t* lens,
+                             void* desc, const dmcjpeg::ColorFrameDesc* tmpl, uint64_t plane_bytes, int n, int H, int W, int hy, int vy, cudaStream_t s);
 // copies stream f (lens[f] bytes of slot f) to dst + offs[f]; max_len >= every lens[f]
 int launch_jpeg_enc_gather(const uint8_t* slots, size_t slot_bytes, const uint32_t* lens, const uint64_t* offs, uint8_t* dst, int n, uint64_t max_len, cudaStream_t s);
 }

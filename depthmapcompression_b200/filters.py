@@ -319,6 +319,90 @@ def degradeJPEG(frames, quality, dst=None, ctx=None, optimize=False):
     return dst, nbytes
 
 
+JPEG_SAMPLINGS = {"444": capi.DMC_JPEG_SAMPLING_444, "422": capi.DMC_JPEG_SAMPLING_422, "420": capi.DMC_JPEG_SAMPLING_420,
+                  "440": capi.DMC_JPEG_SAMPLING_440, "411": capi.DMC_JPEG_SAMPLING_411}
+
+
+def _sampling(sampling):
+    """"444" / "422" / "420" / "440" / "411", or the value of a cv2.IMWRITE_JPEG_SAMPLING_FACTOR_* constant -> that value"""
+    if isinstance(sampling, str):
+        if sampling not in JPEG_SAMPLINGS:
+            raise DmcError(capi.DMC_ERR_ARG, "unknown JPEG sampling %r (one of %s)" % (sampling, ", ".join(JPEG_SAMPLINGS)))
+        return JPEG_SAMPLINGS[sampling]
+    return int(sampling)
+
+
+def _color_frames(frames):
+    """numpy [n, rows, cols, 3] / [rows, cols, 3] uint8, or (device pointer, n, rows, cols) -> (pointer, n, rows, cols, mem, array)"""
+    if isinstance(frames, tuple):
+        ptr, n, rows, cols = frames
+        return int(ptr), int(n), int(rows), int(cols), MEM_DEVICE, None
+    a = np.ascontiguousarray(frames)
+    if a.dtype != np.uint8 or a.ndim not in (3, 4) or a.shape[-1] != 3:
+        raise DmcError(capi.DMC_ERR_TYPE, "frames must be uint8 [n, rows, cols, 3] or [rows, cols, 3]")
+    n, rows, cols = (1,) + a.shape[:2] if a.ndim == 3 else a.shape[:3]
+    return a.ctypes.data, n, rows, cols, MEM_HOST, a
+
+
+def jpegEncodeColorBound(rows, cols, sampling="420"):
+    """dmc_jpeg_encode_color_bound (host only): worst-case bytes of one rows x cols colour stream at `sampling`; raises
+    DmcError for sizes or samplings the encoder refuses."""
+    b = C.c_uint64()
+    rc = lib.dmc_jpeg_encode_color_bound(int(rows), int(cols), _sampling(sampling), C.byref(b))
+    if rc != capi.DMC_OK:
+        raise DmcError(rc, (lib.dmc_last_error(None) or b"").decode())
+    return int(b.value)
+
+
+def jpegEncodeColorBatch(frames, quality, sampling="420", ctx=None, blob=None):
+    """Baseline colour JPEG encode of 8UC3 BGR frames on the GPU, byte-identical to cv2.imencode(".jpg", f,
+    [IMWRITE_JPEG_QUALITY, quality, IMWRITE_JPEG_SAMPLING_FACTOR, s]) of each frame.  sampling: "444", "422", "420"
+    (cv2's default), "440", "411", or a cv2.IMWRITE_JPEG_SAMPLING_FACTOR_* value.  frames: uint8 numpy [n, rows, cols, 3]
+    (or one [rows, cols, 3] frame), or (device pointer, n, rows, cols).  Returns (blob, offsets) in the layout of
+    pack_streams, ready for jpegDecodeColorBatch.  blob=None: a new host array; blob=(device pointer, capacity): the
+    streams go to device memory and (pointer, offsets) is returned."""
+    ctx = ctx or default_context()
+    sp, n, rows, cols, smem, keep = _color_frames(frames)
+    s = _sampling(sampling)
+    offsets = np.zeros(n + 1, np.uint64)
+    if blob is None:
+        cap = n * jpegEncodeColorBound(rows, cols, s)
+        host = np.empty(cap, np.uint8)          # pages the streams never reach are never touched
+        bp, bmem = host.ctypes.data, MEM_HOST
+    else:
+        bp, cap = int(blob[0]), int(blob[1])
+        bmem = MEM_DEVICE
+    ctx.check(lib.dmc_jpeg_encode_color_batch(ctx.h, C.c_void_p(sp), smem, n, rows, cols, int(quality), s, C.c_void_p(bp), bmem,
+                                              cap, offsets.ctypes.data_as(C.POINTER(C.c_uint64))))
+    if blob is None:
+        return host[:int(offsets[-1])].copy(), offsets
+    return bp, offsets
+
+
+def degradeJPEGColor(frames, quality, sampling="420", dst=None, ctx=None):
+    """A colour JPEG round trip on the device: decoded = cv2.imdecode(cv2.imencode(f, [IMWRITE_JPEG_QUALITY, quality,
+    IMWRITE_JPEG_SAMPLING_FACTOR, s]), IMREAD_COLOR) for every frame, and the stream sizes in bytes; the streams never
+    leave the device.  frames as for jpegEncodeColorBatch (one [rows, cols, 3] frame: nbytes is an int); device frames
+    need a device pointer dst, which may equal the frames' pointer, and the result is then a texture batch that
+    renderViewBatch takes as (pointer, n, rows, cols).  Returns (decoded, nbytes)."""
+    ctx = ctx or default_context()
+    sp, n, rows, cols, mem, a = _color_frames(frames)
+    if mem == MEM_DEVICE:
+        if not isinstance(dst, int):
+            raise DmcError(capi.DMC_ERR_ARG, "degradeJPEGColor: device frames need a device pointer dst")
+        dp = dst
+    else:
+        if dst is None or dst.shape != a.shape or dst.dtype != np.uint8 or not dst.flags.c_contiguous:
+            dst = np.empty(a.shape, np.uint8)
+        dp = dst.ctypes.data
+    nbytes = np.zeros(n, np.uint64)
+    ctx.check(lib.dmc_jpeg_degrade_color_batch(ctx.h, C.c_void_p(sp), C.c_void_p(dp), n, rows, cols, int(quality), _sampling(sampling), mem,
+                                               nbytes.ctypes.data_as(C.POINTER(C.c_uint64))))
+    if a is not None and a.ndim == 3:
+        return dst, int(nbytes[0])
+    return dst, nbytes
+
+
 def frameSSE(a, b, ctx=None):
     """Exact per-frame sum of squared differences of two batches of 8-bit frames on the GPU (dmc_sse_gray_batch).  a, b:
     uint8 numpy [n, rows, cols] (or one [rows, cols] frame), or both (device pointer, n, rows, cols).  -> np.uint64[n]"""

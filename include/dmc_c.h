@@ -250,6 +250,33 @@ int dmc_jpeg_degrade_gray_batch(dmc_ctx* ctx, const void* src, void* dst, int n_
 int dmc_jpeg_degrade_gray_batch_ex(dmc_ctx* ctx, const void* src, void* dst, int n_frames, int rows, int cols, int quality, int flags,
                                    int mem, uint64_t* bytes);
 
+/* Baseline colour JPEG encoding of dense 8UC3 BGR frames, byte-identical to cv::imencode(".jpg", img,
+ * {IMWRITE_JPEG_QUALITY, quality, IMWRITE_JPEG_SAMPLING_FACTOR, sampling}) with libjpeg-turbo 3.1.2 (cv2 4.13): libjpeg's
+ * RGB -> YCbCr conversion and chroma downsampling (no smoothing), the standard luminance and chrominance tables of ITU
+ * T.81 K.1-K.6 scaled by quality, one interleaved scan, no restart intervals.  `sampling` is one of cv::IMWRITE_JPEG_SAMPLING_
+ * FACTOR_*'s values below (anything else is DMC_ERR_ARG); cv::imencode's default is 4:2:0.  Other rules as for the gray
+ * encoder: quality 0..100, sizes 1..65535, DMC_ERR_SIZE for frames whose bound exceeds 256 MB. */
+enum {
+    DMC_JPEG_SAMPLING_444 = 0x111111,
+    DMC_JPEG_SAMPLING_422 = 0x211111,
+    DMC_JPEG_SAMPLING_420 = 0x221111,
+    DMC_JPEG_SAMPLING_440 = 0x121111,
+    DMC_JPEG_SAMPLING_411 = 0x411111
+};
+/* Host only, needs no GPU: the worst-case stream size of one rows x cols colour frame (1660 bits per 8x8 block, the dummy
+ * blocks of partial MCUs included). */
+int dmc_jpeg_encode_color_bound(int rows, int cols, int sampling, uint64_t* bytes);
+/* src: n_frames dense rows x cols x 3 frames (src_mem: host or device).  blob, capacity and offsets as for
+ * dmc_jpeg_encode_gray_batch (n_frames x dmc_jpeg_encode_color_bound always suffices); dmc_jpeg_decode_color_batch takes
+ * blob and offsets as they are.  Returns when offsets and blob are valid. */
+int dmc_jpeg_encode_color_batch(dmc_ctx* ctx, const void* src, int src_mem, int n_frames, int rows, int cols, int quality, int sampling,
+                                void* blob, int blob_mem, uint64_t capacity, uint64_t* offsets);
+/* A colour JPEG round trip for a batch, entirely on the device: dst = cv::imdecode(cv::imencode(src, {QUALITY, quality,
+ * SAMPLING_FACTOR, sampling}), IMREAD_COLOR) for every frame (src, dst: n_frames dense 8UC3 frames in `mem`; they may
+ * alias).  bytes (host, n_frames entries, may be NULL) receives the stream sizes.  Returns when dst and bytes are valid. */
+int dmc_jpeg_degrade_color_batch(dmc_ctx* ctx, const void* src, void* dst, int n_frames, int rows, int cols, int quality, int sampling,
+                                 int mem, uint64_t* bytes);
+
 /* ---- distortion and the JPEG rate-distortion sweep ---------------------------------------------------------- */
 /* Per-frame sum of squared differences of two batches of n dense rows x cols 8UC1 frames (both in `mem`), exact:
  * sse[i] = sum over the pixels of (a_i - b_i)^2 (host, n_frames entries).  a and b may be the same pointer.

@@ -71,6 +71,48 @@ inline int degradeJPEGGray(const Mat& src, Mat& dest, int quality, bool optimize
 	return (int)bytes;
 }
 
+namespace dmc_dropin {
+inline void require_color8(const Mat& m, const char* what) {
+	if (m.type() == CV_8UC3 && !m.empty()) return;
+#ifdef DMC_MINICV_HPP
+	throw cv::Exception((std::string(what) + ": src must be a non-empty CV_8UC3 image").c_str(), __FILE__, __LINE__);
+#else
+	CV_Error(cv::Error::StsAssert, std::string(what) + ": src must be a non-empty CV_8UC3 image");
+#endif
+}
+}  // namespace dmc_dropin
+
+// Baseline colour JPEG encoding of a CV_8UC3 (BGR) image on the GPU: `buf` receives the same bytes as
+// cv::imencode(".jpg", src, buf, {IMWRITE_JPEG_QUALITY, quality, IMWRITE_JPEG_SAMPLING_FACTOR, sampling}) with
+// libjpeg-turbo.  quality in 0..100; sampling one of DMC_JPEG_SAMPLING_* (the values of cv::IMWRITE_JPEG_SAMPLING_FACTOR_*).
+inline void jpegEncodeColor(const Mat& src, vector<uchar>& buf, int quality, int sampling = DMC_JPEG_SAMPLING_420)
+{
+	dmc_dropin::require_color8(src, "jpegEncodeColor");
+	const Mat s = src.isContinuous() ? src : src.clone();
+	uint64_t cap = 0, off[2] = {0, 0};
+	dmc_dropin::check(dmc_jpeg_encode_color_bound(s.rows, s.cols, sampling, &cap), "jpegEncodeColor");
+	buf.resize((size_t)cap);
+	dmc_dropin::check(dmc_jpeg_encode_color_batch(dmc_dropin::context(), s.data, DMC_MEM_HOST, 1, s.rows, s.cols, quality, sampling, buf.data(), DMC_MEM_HOST, cap, off), "jpegEncodeColor");
+	buf.resize((size_t)off[1]);
+}
+
+// Colour JPEG round trip of a CV_8UC3 image on the GPU, the stream never leaving the device:
+// dest = cv::imdecode(cv::imencode(".jpg", src, {IMWRITE_JPEG_QUALITY, quality, IMWRITE_JPEG_SAMPLING_FACTOR, sampling}),
+// IMREAD_COLOR).  Returns the stream's size in bytes.
+inline int degradeJPEGColor(const Mat& src, Mat& dest, int quality, int sampling = DMC_JPEG_SAMPLING_420)
+{
+	dmc_dropin::require_color8(src, "degradeJPEGColor");
+	const Mat s = src.isContinuous() ? src : src.clone();
+	Mat d;
+	if (dest.data != src.data && dest.size() == src.size() && dest.type() == CV_8UC3 && dest.isContinuous()) d = dest;
+	else d.create(src.size(), CV_8UC3);
+	uint64_t bytes = 0;
+	dmc_dropin::check(dmc_jpeg_degrade_color_batch(dmc_dropin::context(), s.data, d.data, 1, s.rows, s.cols, quality, sampling, DMC_MEM_HOST, &bytes),
+	                  "degradeJPEGColor");
+	if (d.data != dest.data) dest = d;
+	return (int)bytes;
+}
+
 // The JPEG rate-distortion sweep of one CV_8UC1 image on the GPU (the reference's simpleTest, main.cpp:516-526, for several
 // qualities at once): for every qualities[k], bytes[k] = the size of cv::imencode(".jpg", src, {IMWRITE_JPEG_QUALITY, q}
 // [, IMWRITE_JPEG_OPTIMIZE, 1]), psnr_coded[k] = cv::PSNR(src, the decoded image) and psnr_filtered[k] = cv::PSNR(src,
