@@ -30,12 +30,17 @@ def assert_bits_equal(a, b, msg=""):
     if not bits_equal(a, b):
         a = np.asarray(a); b = np.asarray(b)
         if a.shape == b.shape and a.dtype == b.dtype:
-            with np.errstate(invalid="ignore"):
-                bad = ~((a == b) | (np.isnan(a) & np.isnan(b))) if a.dtype.kind == "f" else (a != b)
+            if a.dtype.kind == "f":     # the rule of bits_equal: bits differ (-0.0 vs +0.0 too), unless both are NaN
+                na, nb = np.isnan(a), np.isnan(b)
+                iv = np.dtype("u%d" % a.dtype.itemsize)
+                bad = (na != nb) | (~na & ~nb & (a.view(iv) != b.view(iv)))
+            else:
+                bad = a != b
             idx = np.argwhere(bad)
-            first = tuple(idx[0]) if len(idx) else None
+            first = tuple(int(i) for i in idx[0]) if len(idx) else None
             raise AssertionError("%s: %d of %d elements differ; first at %s: got %r expected %r"
-                                 % (msg, int(bad.sum()), a.size, first, a[first] if first else None, b[first] if first else None))
+                                 % (msg, int(bad.sum()), a.size, first, a[first] if first is not None else None,
+                                    b[first] if first is not None else None))
         raise AssertionError("%s: shape/dtype mismatch %s %s vs %s %s" % (msg, a.shape, a.dtype, b.shape, b.dtype))
 
 

@@ -106,6 +106,7 @@ def test_unaligned_device_pointers(dmc, port, offs, shape):
     d_in = torch.zeros(H * W + 64, dtype=torch.uint8, device="cuda")
     d_out = torch.zeros(H * W + 64, dtype=torch.uint8, device="cuda")
     d_in[so:so + H * W] = torch.from_numpy(img.reshape(-1)).cuda()
+    torch.cuda.synchronize()                # the copy runs on torch's stream, the filter on the context's own
     ctx = dmc.default_context(0)
     for r in (2, 5):
         s8 = DmcImage(d_in.data_ptr() + so, H, W, 0, W, 1)

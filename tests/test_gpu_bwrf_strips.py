@@ -153,6 +153,7 @@ def test_unaligned_device_pointers(dmc, port, offs, shape):
     for r in (2, 5):
         img = strip_image(taps_per_tile(rs, H, W, rows_per_thread(r, H, W), [31, 33, 1]), H, W, rows_per_thread(r, H, W), 6)
         d_in[so:so + H * W] = torch.from_numpy(img.reshape(-1)).cuda()
+        torch.cuda.synchronize()            # the copy runs on torch's stream, the filter on the context's own
         s8 = DmcImage(d_in.data_ptr() + so, H, W, 0, W, 1)
         o8 = DmcImage(d_out.data_ptr() + do, H, W, 0, W, 1)
         ctx.check(lib.dmc_bwrf(ctx.h, C.byref(s8), C.byref(o8), 2 * r + 1, 2 * r + 1, 10.0, 0, 1))

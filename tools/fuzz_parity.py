@@ -5,8 +5,10 @@ and operators, and compares every result with the CPU oracle bit for bit."""
 import os, sys, time
 import numpy as np
 sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
+sys.path.insert(0, os.path.join(os.path.dirname(os.path.dirname(os.path.abspath(__file__))), "tests"))
 import depthmapcompression_b200 as dmc
 from oracle import oracle_py as O
+import _float_edge_cases as E
 
 budget = float(sys.argv[1]) if len(sys.argv) > 1 else 120.0
 port = O.Port(); pfs = dmc.PostFilterSet(); rs = np.random.RandomState(int(os.environ.get("FUZZ_SEED", "12345")))
@@ -87,6 +89,10 @@ while time.time() - t0 < budget:
         scale = int(rs.choice([1, 16, 257])); a = image(H, W, int(rs.choice([1, 3])))
         b = (a.astype(np.int32) * scale - (30000 if dt == np.int16 else 0)).clip(-32768, 65535).astype(dt) if dt != np.float32 else (a * 3.7).astype(np.float32)
         r = int(rs.randint(1, 11)); th = float(rs.choice([0, 0.5, 3, 10.9, 40, 160, 5000, 70000])); k = 2 * r + 1
+        if dt == np.float32 and rs.randint(3) == 0:     # IEEE edge values, with thresholds that their distances meet exactly
+            cases = E.CASES_C1 if a.ndim == 2 else E.CASES_C3
+            case = cases[rs.randint(len(cases))]; b = case.image(H, W); ths = E.all_thresholds(case)
+            th = float(ths[rs.randint(len(ths))])
         got = dmc.binalyWeightedRangeFilter(b, None, (k, k), th, dmc.FULL_KERNEL); want = port.bwrf(b, k, k, th)
         if r % 8 == 5 and W % 4 == 0: got[:, -1] = want[:, -1]      # the reference's own undefined read (masked in tests/ too)
         same(got, want, "bwrf32 %sC%d r%d th%s %dx%d" % (np.dtype(dt).name, a.size // (H * W), r, th, H, W))
